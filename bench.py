@@ -42,9 +42,11 @@ def parse_args():
     ap.add_argument("--frames", type=int, default=16, help="T: frames per stream per step")
     ap.add_argument("--ring", type=int, default=32, help="frames per stream resident in HBM")
     ap.add_argument("--e2e-steps", type=int, default=32)
-    ap.add_argument("--min-seconds", type=float, default=2.0,
-                    help="the timed region repeats the K-step block until it lasts at least this long (sustained clocks); "
-                         "0 = exactly K steps")
+    ap.add_argument("--min-seconds", type=float, default=0.0,
+                    help="repeat the K-step block until the timed region lasts at least this long (sustained clocks); "
+                         "0 = exactly K timed steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
     ap.add_argument("--size", default="1920x1080", help="frame size WxH (the headline metric is 1080p)")
     ap.add_argument("--distinct", type=int, default=0, help="distinct synthetic clips (0 = one per stream); "
                     "streams reuse them round-robin (large-batch sweeps)")
@@ -207,20 +209,22 @@ def workload_config(args, kw, info):
 
 
 def time_engine(eng, ring_dev, args, torch, dist, world):
-    """warm-up, then EXACTLY K timed steps bracketed by barrier + synchronize; returns ms (max over ranks)."""
+    """warm-up, then EXACTLY K timed steps (a multiple of K with --min-seconds) between two CUDA events; returns ms (max
+    over ranks), the step count, the launch count and the device stats of the last step."""
     R, T = args.ring, args.frames
     nslots = R // T
 
     def step(i):
         a = (i % nslots) * T
-        eng.process(ring_dev[:, a:a + T], sync=False)
+        return eng.process(ring_dev[:, a:a + T], sync=False)
 
+    eng.timing(enable=False)                 # warm-up calls stay out of the kernel-group times
     for i in range(args.warmup):
         step(i)
-    torch.cuda.synchronize()
     # how often the K-step block must repeat for the timed region to last --min-seconds (same count on every rank)
     reps = 1
     if getattr(args, "min_seconds", 0) > 0:
+        torch.cuda.synchronize()
         c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         c0.record()
         for i in range(args.steps):
@@ -231,17 +235,18 @@ def time_engine(eng, ring_dev, args, torch, dist, world):
         if world > 1:
             dist.all_reduce(est, op=dist.ReduceOp.MIN)
         reps = max(1, int(-(-args.min_seconds // max(float(est.item()), 1e-6))))
-    if hasattr(eng, "timing"):
-        eng.timing(reset=True)
+    eng.timing(enable=True, reset=True)      # no call is pending, so neither waits for the device
     if world > 1:
         dist.barrier()
-    torch.cuda.synchronize()
+        torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     from find_motion_b200.engine import launch_count
     l0 = launch_count()
+    # queued behind the warm-up steps still in flight: the K timed steps start on a busy device, as inside a long run,
+    # rather than after an idle gap and the launch latency of their first step
     e0.record()
     for i in range(args.steps * reps):
-        step(args.warmup + i)
+        stats = step(args.warmup + i)
     e1.record()
     launches = launch_count() - l0
     torch.cuda.synchronize()
@@ -253,7 +258,7 @@ def time_engine(eng, ring_dev, args, torch, dist, world):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     eng.check()
-    return ms, args.steps * reps, launches
+    return ms, args.steps * reps, launches, stats
 
 
 def main():
@@ -286,14 +291,14 @@ def measure(eng, ring_dev, args, torch, dist, world, S, T, launch_count, local):
     eng.reset()
     sampler = ClockSampler(local)
     sampler.start()
-    ms, timed_steps, launches = time_engine(eng, ring_dev, args, torch, dist, world)
+    ms, timed_steps, launches, stats = time_engine(eng, ring_dev, args, torch, dist, world)
     clocks = sampler.stop()
     groups = eng.timing()                    # reset at the start of the timed region: timed steps only
     fps = S * T * timed_steps * world / (ms / 1e3)
     per_call = {k: v[0] / max(1, v[1]) for k, v in groups.items()}
     eng.timing(enable=False)
     return {"fps": fps, "ms": ms, "timed_steps": timed_steps, "step_ms": ms / timed_steps, "per_call": per_call,
-            "launches": int(launches), "clocks": clocks}
+            "launches": int(launches), "clocks": clocks, "last_stats": stats}
 
 
 def roofline_of(m, info, S, T, traffic=None):
@@ -328,6 +333,38 @@ def ncu_traffic_for(args, info, name):
         return None
 
 
+DUMP_BG_VALUES = 1 << 20       # background values kept over all streams (8 MB)
+DUMP_COMPONENT_ROWS = 1 << 19  # contour records kept (28 MB); the whole dump stays under 64 MB
+
+
+def dump_outputs(path, eng, stats_dev, S, T, prefix=""):
+    """What the last timed step computed, as float64 DIR/<prefix><name>.npy, so that two builds run with the same
+    arguments (hence the same seeded inputs) can be compared file by file:
+      <stats field>      [S, T]  the per-frame stats fm_process returns, one file per field (n_contours, movement, ...)
+      components         [n, 7]  every contour record of the step: stream, frame, area_x2, x, y, w, h (the library's
+                                 sorted order; a fixed seeded sample of rows past DUMP_COMPONENT_ROWS)
+      background_sample  [S, k]  the float64 background after the step at k fixed seeded pixels (row-major index)"""
+    import numpy as np
+    from find_motion_b200.engine import STATS_DTYPE
+    out = {}
+    stats = stats_dev.cpu().numpy().view(STATS_DTYPE).reshape(S, T)
+    for name in STATS_DTYPE.names:
+        out[name] = stats[name].astype(np.float64)
+    rows = [(s, t, a2, *box) for s in range(S) for t in range(T) for a2, box in eng.components(s, t)[1]]
+    comps = np.array(rows, np.float64).reshape(-1, 7)
+    if len(comps) > DUMP_COMPONENT_ROWS:
+        comps = comps[np.sort(np.random.default_rng(1).choice(len(comps), DUMP_COMPONENT_ROWS, replace=False))]
+    out["components"] = comps
+    n = eng.w * eng.h
+    idx = np.sort(np.random.default_rng(0).choice(n, min(n, max(1, DUMP_BG_VALUES // S)), replace=False))
+    out["background_sample"] = np.stack(
+        [eng.planes(s, T - 1, gray=False, blur=False, thresh=False)["bg"].ravel()[idx] for s in range(S)])
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20, "dump larger than 64 MB"
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, prefix + name + ".npy"), a)
+
+
 def run_b200(args):
 
     import numpy as np
@@ -346,6 +383,7 @@ def run_b200(args):
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     assert args.ring % args.frames == 0 and args.ring >= args.frames
+    assert args.steps >= 1, "--steps: at least one timed step"
 
     kw = tuning(args.mode, args.blur_scale)
     S, T, R = args.streams, args.frames, args.ring
@@ -383,6 +421,8 @@ def run_b200(args):
     eng = MotionEngine(W, H, n_streams=S, max_frames=T, device=local, **fe, **kw)
     info = dict(eng.info, w=eng.w, h=eng.h)
     m = measure(eng, ring_dev, args, torch, dist, world, S, T, launch_count, local)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, m["last_stats"], S, T, "" if world == 1 else f"rank{rank}_")
     name = "fused" if info["front_end"] == 0 else ("wide" if args.mode == "full" else "default")
     roofline = roofline_of(m, info, S, T, ncu_traffic_for(args, info, name))
 
@@ -486,10 +526,8 @@ def secondary_regimes(args, ring_dev, torch, dist, launch_count, local):
         kw = tuning(mode, bs)
         try:
             with MotionEngine(W, H, n_streams=S, max_frames=T, **kw) as eng:
-                a = argparse.Namespace(**vars(args))
-                a.steps, a.warmup, a.min_seconds = max(3, min(40, args.steps // 4)), 3, min(args.min_seconds, 1.0)
                 info = dict(eng.info, w=eng.w, h=eng.h)
-                m = measure(eng, ring_dev, a, torch, dist, 1, S, T, launch_count, local)
+                m = measure(eng, ring_dev, args, torch, dist, 1, S, T, launch_count, local)
                 out[name] = {"value": round(m["fps"], 1), "unit": "frames/s", "proc": f"{eng.w}x{eng.h}",
                              "gaussian": eng.info["gaussian"], "timed_steps": m["timed_steps"],
                              "ms_per_step": round(m["step_ms"], 4),
