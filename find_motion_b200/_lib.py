@@ -54,6 +54,7 @@ FLAG_NO_UMMA = 8
 FLAG_UMMA_APRON = 16
 FLAG_UMMA = 32
 FLAG_NO_ROWS = 64
+FLAG_UPSCALE = 128
 
 # every symbol include/fm_gpu.h declares: name -> (restype, argtypes)
 _P = C.c_void_p

@@ -47,7 +47,7 @@ struct fm_ctx {
     int S, Tmax, W, H, w, h, k, wpr;
     int N;                     // w*h
     int ntiles;                // ceil(N / FM_TILE_PX)
-    int resize_mode;           // 0 identity, 1 general tables, 2 integer ratio
+    int resize_mode;           // 0 identity, 1 general tables, 2 integer ratio, 3 upscale (FM_FLAG_UPSCALE, k_upscale.cu)
     bool fused;                // K1 fused stencil+background kernel drives the front end
     bool wide_fused;           // wide Gaussian: the vertical pass runs the temporal stage too (k_wide_vt)
     bool umma;                 // blur + temporal stage on tcgen05 tensor cores (k_umma.cu), k <= 97
@@ -65,6 +65,7 @@ struct fm_ctx {
     int *g4start, *g4n, *g4off;   // x taps regrouped in 4-pixel groups with zero-weight padding (k_resize_gray_g4)
     float4 *g4w;
     int g4max;                    // most tap groups of any destination column
+    int2 *uxt, *uyt;              // upscale taps (mode 3): [w] / [h] (source index, a0 | a1 << 16)
     struct RowsPlan *rows;        // plan of the row-per-lane resize kernel (k_resize_rows.cu); null: not applicable
     // planes
     uint8_t *gray;             // [S][Tmax][h][w]
@@ -159,6 +160,10 @@ size_t fm_fused_bg_doubles(const fm_ctx *c);
 int fm_launch_bg_export_fused(fm_ctx *c, int stream, double *dst_dev, cudaStream_t st);
 int fm_launch_resize_bgr(int device, const uint8_t *src_dev, int W, int H, int w, int h, int mode, int fx, int fy,
                          const ResizeTab &xt, const ResizeTab &yt, uint8_t *dst_dev, cudaStream_t st);
+size_t fm_upscale_smem(int w);
+int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, int T, int F, int W, int H, int w,
+                      int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
+                      cudaStream_t st);
 int fm_rows_plan(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx);
 void fm_rows_free(fm_ctx *c);
 int fm_rows_plan_describe(int W, int w, int h, const int *xstart, const int *xidx, const float *xwt, const int *ystart,
@@ -175,6 +180,11 @@ int fm_ccl_alloc(CclScratch *s, int frames, int h, int cap);
 void fm_ccl_free(CclScratch *s);
 int fm_ccl_plane(int device, const uint8_t *plane_host, int w, int h, int max_n, fm_component *out,
                  int *n);
+
+// gray (SURVEY.md A.2): Y = (3735 B + 19235 G + 9798 R + 16384) >> 15
+__device__ __forceinline__ uint32_t fm_gray(uint32_t b, uint32_t g, uint32_t r) {
+    return (3735u * b + 19235u * g + 9798u * r + 16384u) >> 15;
+}
 
 __device__ __forceinline__ int fm_reflect101(int i, int n) {
     // BORDER_REFLECT_101 for any offset

@@ -117,6 +117,23 @@ static HostTab area_tab(int src, int dst) {
     return t;
 }
 
+// One axis of INTER_AREA with dst >= src: cv2 takes its linear interpolation with area-style offsets there
+// (cv::resize, `area_mode`), fixed point with INTER_RESIZE_COEF_SCALE = 2048.  Per destination index: the first source
+// index and the weights a0 | a1 << 16 of it and of the next one (clamped to the border).  float where cv2 uses float.
+static std::vector<int2> upscale_tab(int src, int dst) {
+    std::vector<int2> t(dst);
+    const double inv = (double)dst / (double)src, scale = 1.0 / inv;
+    for (int d = 0; d < dst; d++) {
+        int sx = (int)floor(d * scale);
+        float fx = (float)((d + 1) - (sx + 1) * inv);
+        fx = fx <= 0 ? 0.f : fx - (float)(int)floorf(fx);
+        if (sx >= src - 1) { fx = 0.f; sx = src - 1; }
+        const int a0 = (int)lrintf((1.f - fx) * 2048.f), a1 = (int)lrintf(fx * 2048.f);   // saturate_cast<short>
+        t[d] = make_int2(sx, a0 | (a1 << 16));
+    }
+    return t;
+}
+
 template <typename T>
 static int upload(T **dst, const std::vector<T> &v) {
     FM_CUDA(cudaMalloc(dst, std::max<size_t>(v.size(), 1) * sizeof(T)));
@@ -149,6 +166,7 @@ extern "C" int fm_ctx_destroy(fm_ctx *c) {
     cudaDeviceSynchronize();
     cudaFree(c->coef); cudaFree(c->wtab); cudaFree(c->uband); cudaFree(c->uband_f); cudaFree(c->gpad);
     cudaFree(c->g4start); cudaFree(c->g4n); cudaFree(c->g4off); cudaFree(c->g4w);
+    cudaFree(c->uxt); cudaFree(c->uyt);
     fm_rows_free(c);
     cudaFree(c->xtab.start); cudaFree(c->xtab.idx); cudaFree(c->xtab.wt);
     cudaFree(c->ytab.start); cudaFree(c->ytab.idx); cudaFree(c->ytab.wt);
@@ -183,10 +201,10 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
         fm_set_error("invalid configuration (streams/geometry/max_frames/box_size/blur_scale/min_box_scale)");
         return FM_EINVAL;
     }
-    if (cfg->box_size > cfg->frame_width) {
-        // INTER_AREA with a destination wider than the source is a bilinear-style upscale in cv2
-        // that this library does not reproduce (SURVEY.md A.1)
-        fm_set_error("box_size %d > frame width %d: upscaling resize is not supported", cfg->box_size,
+    if (cfg->box_size > cfg->frame_width && !(cfg->flags & FM_FLAG_UPSCALE)) {
+        // INTER_AREA with a destination wider than the source is cv2's fixed-point linear upscale (SURVEY.md A.1):
+        // opt-in with FM_FLAG_UPSCALE, so that binders of the earlier ABI keep their range check
+        fm_set_error("box_size %d > frame width %d: upscaling resize needs FM_FLAG_UPSCALE", cfg->box_size,
                      cfg->frame_width);
         return FM_ERANGE;
     }
@@ -240,8 +258,17 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     // resize mode (cv2::resize INTER_AREA dispatch)
     if (c->w == c->W && c->h == c->H) {
         c->resize_mode = 0;
+    } else if (c->w > c->W || c->h > c->H) {
+        // imutils.resize keeps the aspect ratio, so h >= H whenever w > W: both axes go up (or stay)
+        if (!(cfg->flags & FM_FLAG_UPSCALE) || c->w < c->W || c->h < c->H) {
+            fm_set_error("upscaling resize needs FM_FLAG_UPSCALE");
+            return fail(FM_ERANGE);
+        }
+        c->resize_mode = 3;
+        if (fm_upscale_smem(c->w) > 200 * 1024) { fm_set_error("processing width %d too large to upscale", c->w); return fail(FM_ERANGE); }
+        if ((rc = upload(&c->uxt, upscale_tab(c->W, c->w)))) return fail(rc);
+        if ((rc = upload(&c->uyt, upscale_tab(c->H, c->h)))) return fail(rc);
     } else {
-        if (c->h > c->H) { fm_set_error("upscaling resize is not supported"); return fail(FM_ERANGE); }
         double sx = 1.0 / ((double)c->w / W), sy = 1.0 / ((double)c->h / H);
         int isx = (int)nearbyint(sx), isy = (int)nearbyint(sy);
         bool fast = fabs(sx - isx) < 2.220446049250313e-16 && fabs(sy - isy) < 2.220446049250313e-16;
@@ -729,7 +756,6 @@ extern "C" int fm_debug_rows_plan(int W, int H, int box_size, fm_rows_plan_info 
 
 extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H, int width, uint8_t *out_host, int *out_height) {
     if (!bgr_host || !out_host || W < 1 || H < 1 || width < 1) { fm_set_error("bad argument"); return FM_EINVAL; }
-    if (width > W) { fm_set_error("width %d > frame width %d: upscaling resize is not supported", width, W); return FM_ERANGE; }
     int ndev = 0;
     FM_CUDA(cudaGetDeviceCount(&ndev));
     if (device < 0 || device >= ndev) { fm_set_error("CUDA device %d not present", device); return FM_ECUDA; }
@@ -738,6 +764,24 @@ extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H,
     if (h < 1) { fm_set_error("resized height is zero"); return FM_ERANGE; }
     if (out_height) *out_height = h;
     if (width == W && h == H) { memcpy(out_host, bgr_host, (size_t)W * H * 3); return FM_OK; }
+    if (width > W) {                                                          // h >= H: cv2's fixed-point linear upscale
+        struct UpTabs {
+            int2 *x = nullptr, *y = nullptr;
+            ~UpTabs() { cudaFree(x); cudaFree(y); }
+        } ut;
+        int rc;
+        if ((rc = upload(&ut.x, upscale_tab(W, width)))) return rc;
+        if ((rc = upload(&ut.y, upscale_tab(H, h)))) return rc;
+        DevBuf src, dst;
+        FM_CUDA(cudaMalloc(&src.p, (size_t)W * H * 3));
+        FM_CUDA(cudaMalloc(&dst.p, (size_t)width * h * 3));
+        FM_CUDA(cudaMemcpy(src.p, bgr_host, (size_t)W * H * 3, cudaMemcpyHostToDevice));
+        if ((rc = fm_launch_upscale(device, (const uint8_t *)src.p, 0, 0, 1, 1, W, H, width, h, ut.x, ut.y, nullptr, nullptr,
+                                    (uint8_t *)dst.p, 0)))
+            return rc;
+        FM_CUDA(cudaMemcpy(out_host, dst.p, (size_t)width * h * 3, cudaMemcpyDeviceToHost));
+        return FM_OK;
+    }
     const double sx = 1.0 / ((double)width / W), sy = 1.0 / ((double)h / H);
     const int isx = (int)nearbyint(sx), isy = (int)nearbyint(sy);
     const bool fast = fabs(sx - isx) < 2.220446049250313e-16 && fabs(sy - isy) < 2.220446049250313e-16;

@@ -3,13 +3,6 @@
 // Replaces VideoMotion.blur_frame + mask_off_areas (find_motion/find_motion.py:487-494, 619-635).
 #include "fm_common.cuh"
 
-// ---------------------------------------------------------------------------------------------
-// gray (SURVEY.md A.2): Y = (3735 B + 19235 G + 9798 R + 16384) >> 15
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t fm_gray(uint32_t b, uint32_t g, uint32_t r) {
-    return (3735u * b + 19235u * g + 9798u * r + 16384u) >> 15;
-}
-
 // identity-resize mode: one thread per 4 pixels of a frame (12 bytes in, 4 bytes out)
 __global__ void __launch_bounds__(256) k_gray(const uint8_t *__restrict__ frames, size_t sstride,
                                               size_t fstride, int T, int N, uint8_t *__restrict__ gray,
@@ -460,7 +453,12 @@ int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t 
     // every Gaussian the fused stencil does not take goes to the tensor-core blur (k_wide.cu)
     if (c->resize_mode == 0)          // gray fused into the first kernel of the blur
         return c->umma ? fm_launch_umma_blur(c, frames, sstride, fstride, T, st) : fm_launch_wide_blur(c, frames, sstride, fstride, T, st);
-    {
+    if (c->resize_mode == 3) {        // upscale + gray into the gray plane (k_upscale.cu)
+        int rc;
+        if ((rc = fm_launch_upscale(c->cfg.device, frames, sstride, fstride, T, F, c->W, c->H, c->w, c->h, c->uxt, c->uyt,
+                                    c->nvalid, c->gray, nullptr, st)))
+            return rc;
+    } else {
         K0Params p;
         p.frames = frames; p.sstride = sstride; p.fstride = fstride;
         p.T = T; p.W = c->W; p.H = c->H; p.w = c->w; p.h = c->h;

@@ -19,7 +19,10 @@ STATS_DTYPE = np.dtype([(n, np.int32) for n in ("n_contours", "n_counted", "move
 class MotionEngine:
     def __init__(self, frame_width, frame_height, n_streams=1, max_frames=8, device=0, fps=30, box_size=100,
                  min_box_scale=50, cache_time=2.0, min_time=0.5, threshold=7, avg=0.1, blur_scale=20,
-                 mask_areas=None, max_components=256, keep_planes=False, no_fused=False, no_umma=False, umma_apron=False, umma=False, no_rows=False):
+                 mask_areas=None, max_components=256, keep_planes=False, no_fused=False, no_umma=False, umma_apron=False, umma=False, no_rows=False,
+                 upscale=False):
+        """upscale: accept box_size > frame_width (cv2's INTER_AREA upscale, bit-exact, as imutils.resize does it);
+        without it such a geometry raises, as in earlier releases."""
         self._lib = _lib.load()
         self._ctx = C.c_void_p()
         cfg = _lib.fm_config(
@@ -29,7 +32,7 @@ class MotionEngine:
             cache_time=float(cache_time), max_components=max_components,
             flags=(_lib.FLAG_KEEP_PLANES if keep_planes else 0) | (_lib.FLAG_NO_FUSED if no_fused else 0) |
             (_lib.FLAG_NO_UMMA if no_umma else 0) | (_lib.FLAG_UMMA_APRON if umma_apron else 0) | (_lib.FLAG_UMMA if umma else 0) |
-            (_lib.FLAG_NO_ROWS if no_rows else 0))
+            (_lib.FLAG_NO_ROWS if no_rows else 0) | (_lib.FLAG_UPSCALE if upscale else 0))
         _lib.check(self._lib.fm_ctx_create(C.byref(cfg), C.byref(self._ctx)))
         self.device = device
         self.n_streams, self.max_frames = n_streams, max_frames
@@ -248,7 +251,7 @@ class PinnedBatch:
 
 def resize_area(frame: np.ndarray, width: int = 300, device: int = 0) -> np.ndarray:
     """imutils.resize(frame, width=width) (cv2.INTER_AREA) of one BGR frame on the GPU: the input plane of the
-    reference's find_objects (find_motion.py:703-706).  Bit-exact with cv2."""
+    reference's find_objects (find_motion.py:703-706).  Bit-exact with cv2, also for width > frame width (upscale)."""
     lib = _lib.load()
     frame = np.ascontiguousarray(frame, np.uint8)
     H, W, ch = frame.shape

@@ -21,6 +21,7 @@ There is no data-path collective: streams are independent (SURVEY.md 8e).
 """
 from __future__ import annotations
 
+import functools
 import logging
 import queue
 import threading
@@ -28,6 +29,7 @@ import time
 import typing
 from concurrent.futures import ThreadPoolExecutor
 
+from . import engine as _engine
 from .engine import MotionEngine, PinnedBatch
 from .video_motion import VideoMotion
 
@@ -72,7 +74,11 @@ class _GroupDriver:
 
     def __init__(self, device, geom, kw, streams, chunk, source_q, results, stream_cls, max_latency=None,
                  engine_factory=None, buffer_factory=None):
-        self.engine_factory = engine_factory or MotionEngine
+        factory = engine_factory or MotionEngine
+        if factory is _engine.MotionEngine:
+            # the reference upscales frames narrower than box_size (imutils.resize): so does the library's engine
+            factory = functools.partial(factory, upscale=True)
+        self.engine_factory = factory
         self.buffer_factory = buffer_factory or PinnedBatch
         self.device, self.geom, self.kw = device, geom, kw
         self.S, self.T = streams, chunk

@@ -117,7 +117,7 @@ class VideoMotion(object):
             return False
         if self._own_engine:
             self.engine = MotionEngine(self.frame_width, self.frame_height, n_streams=1, max_frames=self.chunk,
-                                       device=self.device, mask_areas=self.mask_areas, **self._tuning)
+                                       device=self.device, mask_areas=self.mask_areas, upscale=True, **self._tuning)
         if self.engine is not None:
             self._adopt_info(self.engine.info)
         return True

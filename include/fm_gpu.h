@@ -62,6 +62,9 @@ typedef struct fm_config {
                                    either flag the library picks the faster path for the geometry (measured: DESIGN.md) */
 #define FM_FLAG_NO_ROWS     64  /* default (resize) mode: never take the row-per-lane INTER_AREA kernel (k_resize_rows.cu);
                                    the warp-per-destination-row kernels instead (A/B testing) */
+#define FM_FLAG_UPSCALE     128 /* accept box_size > frame_width: cv2's INTER_AREA upscale (a fixed-point linear interpolation,
+                                   SURVEY.md A.1), bit-exact, as imutils.resize does it.  Without the flag such a
+                                   configuration is refused with FM_ERANGE */
 
 /* Derived parameters, exactly as the reference computes them (SURVEY.md A.0). */
 typedef struct fm_info {
@@ -114,7 +117,9 @@ const char *fm_last_error(void);
 int fm_version(void);
 
 /* Replaces VideoMotion.__init__ + _calc_min_area + _make_gaussian + _load_video
- * (find_motion.py:299-380, 402-424, 478-484) for n_streams streams. */
+ * (find_motion.py:299-380, 402-424, 478-484) for n_streams streams.  box_size > frame_width (a processing plane larger
+ * than the frame, which imutils.resize produces with cv2's INTER_AREA upscale) needs FM_FLAG_UPSCALE; without it
+ * fm_ctx_create returns FM_ERANGE. */
 int fm_ctx_create(const fm_config *cfg, fm_ctx **out);
 int fm_ctx_destroy(fm_ctx *ctx);
 int fm_ctx_info(const fm_ctx *ctx, fm_info *info);
@@ -194,7 +199,8 @@ int fm_debug_components(int device, const uint8_t *plane, int w, int h, int max_
                         fm_component *out, int *n);
 
 /* The detector input plane of find_objects (find_motion.py:703-706): imutils.resize(frame.raw, width=300), i.e.
- * cv2.resize(INTER_AREA) of one BGR frame to (width, int(H * width / W)), bit-exact (SURVEY.md A.1).  Host buffers;
+ * cv2.resize(INTER_AREA) of one BGR frame to (width, int(H * width / W)), bit-exact (SURVEY.md A.1), also for width > W
+ * (cv2's fixed-point upscale; no flag needed here).  Host buffers;
  * out_host holds width * out_height * 3 bytes.  The detectors themselves stay on the host. */
 int fm_resize_area(int device, const uint8_t *bgr_host, int frame_width, int frame_height, int width,
                    uint8_t *out_host, int *out_height);
