@@ -30,6 +30,11 @@ struct ResizeTab {             // INTER_AREA decimation tables of one axis (SURV
     int max_taps;
 };
 
+struct FmClipCopy {            // one whole-frame copy of the device clip path (k_clips.cu)
+    const uint8_t *src;
+    uint8_t *dst;
+};
+
 struct CclScratch {            // run-based labelling scratch for `frames` frames at a time
     int frames;                // sub-batch capacity
     int cap;                   // run slots per row
@@ -102,6 +107,13 @@ struct fm_ctx {
     cudaStream_t own_stream;   // compute
     cudaStream_t copy_stream;  // host -> device frame copies
     cudaEvent_t ev_copied[2], ev_done[2];
+    // device look-back cache (FM_FLAG_DEVICE_CLIPS, k_clips.cu)
+    uint8_t *clip_ring;        // [S][cache_frames] raw BGR frames, slots of clip_slot_bytes; null when cache_frames == 0
+    size_t clip_slot_bytes;    // H * W * 3 rounded up to 256
+    long long *clip_base;      // [S] absolute frame number of the next frame of each stream
+    FmClipCopy *clip_list;     // gather list [S * (cache_frames + Tmax)], then store list [S * min(cache_frames, Tmax)]
+    int *clip_count;           // [2] entries of the two lists in the current call
+    int clip_sms;              // multiprocessors of the device (grid of the copy kernels)
     // timing
     bool timing;               // bracket the kernel groups with events (no sync inside fm_process)
     cudaEvent_t *evs;          // [FM_TIMING_RING][4]
@@ -176,6 +188,10 @@ int fm_umma_init(fm_ctx *c, const int *taps);
 size_t fm_umma_bg_doubles(const fm_ctx *c);
 int fm_launch_umma_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
 int fm_launch_bg_export_umma(fm_ctx *c, int stream, double *dst_dev, cudaStream_t st);
+int fm_clips_alloc(fm_ctx *c);
+void fm_clips_free(fm_ctx *c);
+int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
+                    size_t ostride, cudaStream_t st);
 int fm_ccl_alloc(CclScratch *s, int frames, int h, int cap);
 void fm_ccl_free(CclScratch *s);
 int fm_ccl_plane(int device, const uint8_t *plane_host, int w, int h, int max_n, fm_component *out,

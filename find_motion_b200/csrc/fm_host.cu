@@ -168,6 +168,7 @@ extern "C" int fm_ctx_destroy(fm_ctx *c) {
     cudaFree(c->g4start); cudaFree(c->g4n); cudaFree(c->g4off); cudaFree(c->g4w);
     cudaFree(c->uxt); cudaFree(c->uyt);
     fm_rows_free(c);
+    fm_clips_free(c);
     cudaFree(c->xtab.start); cudaFree(c->xtab.idx); cudaFree(c->xtab.wt);
     cudaFree(c->ytab.start); cudaFree(c->ytab.idx); cudaFree(c->ytab.wt);
     cudaFree(c->gray); cudaFree(c->hor); cudaFree(c->blur); cudaFree(c->bg);
@@ -379,6 +380,7 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     int nb = (int)std::min<size_t>(F, std::max<size_t>(1, budget / per_frame));
     if ((rc = fm_ccl_alloc(&c->ccl, nb, c->h, cap))) return fail(rc);
     if ((rc = fm_ccl_configure(c))) return fail(rc);
+    if ((cfg->flags & FM_FLAG_DEVICE_CLIPS) && (rc = fm_clips_alloc(c))) return fail(rc);
     FM_TRY(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
     FM_TRY(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     for (int i = 0; i < 2; i++) {
@@ -462,8 +464,10 @@ static int timing_drain(fm_ctx *c) {
     return FM_OK;
 }
 
-extern "C" int fm_process_ragged(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
-                                 int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev) {
+// out: the motion-clip frames of fm_process_clip (null from the other entry points, which with FM_FLAG_DEVICE_CLIPS
+// still keep the device ring up to date)
+static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride, int n_frames,
+                   const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev, uint8_t *out, size_t out_stride) {
     if (!c || !frames) { fm_set_error("null argument"); return FM_EINVAL; }
     if (n_frames < 1 || n_frames > c->Tmax) {
         fm_set_error("n_frames %d outside [1, max_frames=%d]", n_frames, c->Tmax);
@@ -504,14 +508,39 @@ extern "C" int fm_process_ragged(fm_ctx *c, const uint8_t *frames, size_t stream
     }
     if ((rc = fm_launch_morph_ccl(c, n_frames, st, stats_dev))) return rc;
     if (ev) FM_CUDA(cudaEventRecord(ev[3], st));
+    if ((c->cfg.flags & FM_FLAG_DEVICE_CLIPS) &&
+        (rc = fm_launch_clips(c, frames, stream_stride, frame_stride, n_frames, out, out_stride, st)))
+        return rc;
     c->last_T = n_frames;
     c->planes_valid = true;
     return FM_OK;
 }
 
+extern "C" int fm_process_ragged(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
+                                 int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev) {
+    return process(c, frames, stream_stride, frame_stride, n_frames, n_valid, cuda_stream, stats_dev, nullptr, 0);
+}
+
+extern "C" int fm_process_clip(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
+                               int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev,
+                               uint8_t *out_dev, size_t out_stream_stride, int out_capacity) {
+    if (!c || !frames || !out_dev) { fm_set_error("null argument"); return FM_EINVAL; }
+    if (!(c->cfg.flags & FM_FLAG_DEVICE_CLIPS)) {
+        fm_set_error("fm_process_clip needs a context created with FM_FLAG_DEVICE_CLIPS");
+        return FM_EINVAL;
+    }
+    if ((long long)out_capacity < (long long)c->info.cache_frames + n_frames) {
+        fm_set_error("out_capacity %d < cache_frames %d + n_frames %d (the most frames one call can write)", out_capacity,
+                     c->info.cache_frames, n_frames);
+        return FM_EINVAL;
+    }
+    return process(c, frames, stream_stride, frame_stride, n_frames, n_valid, cuda_stream, stats_dev, out_dev,
+                   out_stream_stride);
+}
+
 extern "C" int fm_process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
                           int n_frames, void *cuda_stream, fm_frame_stats *stats_dev) {
-    return fm_process_ragged(c, frames, stream_stride, frame_stride, n_frames, nullptr, cuda_stream, stats_dev);
+    return process(c, frames, stream_stride, frame_stride, n_frames, nullptr, cuda_stream, stats_dev, nullptr, 0);
 }
 
 // ---- host buffers: pipelined (submit / wait on two slots) and the blocking form built on it ----

@@ -20,9 +20,11 @@ class MotionEngine:
     def __init__(self, frame_width, frame_height, n_streams=1, max_frames=8, device=0, fps=30, box_size=100,
                  min_box_scale=50, cache_time=2.0, min_time=0.5, threshold=7, avg=0.1, blur_scale=20,
                  mask_areas=None, max_components=256, keep_planes=False, no_fused=False, no_umma=False, umma_apron=False, umma=False, no_rows=False,
-                 upscale=False):
+                 upscale=False, device_clips=False):
         """upscale: accept box_size > frame_width (cv2's INTER_AREA upscale, bit-exact, as imutils.resize does it);
-        without it such a geometry raises, as in earlier releases."""
+        without it such a geometry raises, as in earlier releases.
+        device_clips: keep the look-back cache of raw frames on the GPU (n_streams x cache_frames frames) so that
+        process_clip can hand out the frames the reference writes to its *_motion.avi."""
         self._lib = _lib.load()
         self._ctx = C.c_void_p()
         cfg = _lib.fm_config(
@@ -32,7 +34,8 @@ class MotionEngine:
             cache_time=float(cache_time), max_components=max_components,
             flags=(_lib.FLAG_KEEP_PLANES if keep_planes else 0) | (_lib.FLAG_NO_FUSED if no_fused else 0) |
             (_lib.FLAG_NO_UMMA if no_umma else 0) | (_lib.FLAG_UMMA_APRON if umma_apron else 0) | (_lib.FLAG_UMMA if umma else 0) |
-            (_lib.FLAG_NO_ROWS if no_rows else 0) | (_lib.FLAG_UPSCALE if upscale else 0))
+            (_lib.FLAG_NO_ROWS if no_rows else 0) | (_lib.FLAG_UPSCALE if upscale else 0) |
+            (_lib.FLAG_DEVICE_CLIPS if device_clips else 0))
         _lib.check(self._lib.fm_ctx_create(C.byref(cfg), C.byref(self._ctx)))
         self.device = device
         self.n_streams, self.max_frames = n_streams, max_frames
@@ -43,6 +46,7 @@ class MotionEngine:
         self.w, self.h = inf.proc_width, inf.proc_height
         self.max_components = inf.max_components
         self._stats_dev = None
+        self._clips_out = None
         self._inflight = {}
         if mask_areas:
             self.set_masks(mask_areas)
@@ -113,6 +117,40 @@ class MotionEngine:
         host = self._stats_dev[:need].cpu().numpy()
         self.check()
         return host.view(STATS_DTYPE).reshape(S, T)
+
+    def process_clip(self, frames, n_valid=None, out=None):
+        """process() that also returns the frames the reference writes to its *_motion.avi in this call (needs
+        device_clips=True).  frames: CUDA uint8 tensor [n_streams, T, H, W, 3].  out: optional CUDA uint8 tensor
+        [n_streams, >= cache_frames + T, H, W, 3] (dense frames) for them; by default one of
+        [n_streams, cache_frames + max_frames, H, W, 3] is allocated once and reused, so the views returned by one call
+        are overwritten by the next.  Runs on the current torch stream and synchronises.
+        Returns (stats [n_streams, T], clips): clips[s] is a view [n_out, H, W, 3] of `out` holding, in order, the
+        cached frames each frame of stream s flushes and the frame itself where it is written."""
+        import torch
+
+        assert frames.is_cuda and frames.dtype == torch.uint8 and frames.dim() == 5, "uint8 CUDA [S,T,H,W,3]"
+        S, T, H, W, ch = frames.shape
+        assert (S, H, W, ch) == (self.n_streams, self.H, self.W, 3), "frame geometry mismatch"
+        assert frames[0, 0].is_contiguous()
+        if out is None:
+            if self._clips_out is None:
+                self._clips_out = torch.empty((S, self.info["cache_frames"] + self.max_frames, H, W, 3), dtype=torch.uint8,
+                                              device=frames.device)
+            out = self._clips_out
+        assert out.is_cuda and out.dtype == torch.uint8 and out.dim() == 5 and out.shape[0] == S and \
+            tuple(out.shape[2:]) == (H, W, 3) and out[0].is_contiguous(), "uint8 CUDA [S, capacity, H, W, 3]"
+        need = S * T * STATS_DTYPE.itemsize
+        if self._stats_dev is None or self._stats_dev.numel() < need:
+            self._stats_dev = torch.empty(S * self.max_frames * STATS_DTYPE.itemsize, dtype=torch.uint8,
+                                          device=frames.device)
+        st = torch.cuda.current_stream(frames.device).cuda_stream
+        _lib.check(self._lib.fm_process_clip(self._ctx, frames.data_ptr(), frames.stride(0), frames.stride(1), T,
+                                             self._nvalid(n_valid, S, T), C.c_void_p(st), self._stats_dev.data_ptr(),
+                                             out.data_ptr(), out.stride(0), out.shape[1]))
+        stats = self._stats_dev[:need].cpu().numpy().view(STATS_DTYPE).reshape(S, T)
+        self.check()
+        n_out = (stats["wrote"].astype(np.int64) + stats["n_flush"]).sum(axis=1)
+        return stats, [out[s, :int(n_out[s])] for s in range(S)]
 
     def check(self):
         """Synchronise and raise if a call since the last check hit a device-side capacity error."""

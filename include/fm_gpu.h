@@ -65,6 +65,9 @@ typedef struct fm_config {
 #define FM_FLAG_UPSCALE     128 /* accept box_size > frame_width: cv2's INTER_AREA upscale (a fixed-point linear interpolation,
                                    SURVEY.md A.1), bit-exact, as imutils.resize does it.  Without the flag such a
                                    configuration is refused with FM_ERANGE */
+#define FM_FLAG_DEVICE_CLIPS 256 /* keep the look-back cache of raw frames on the device (a ring of cache_frames frames per
+                                   stream, n_streams * cache_frames * H * W * 3 bytes) and accept fm_process_clip.  Every
+                                   hot-path call then keeps that ring up to date, so they mix freely with fm_process_clip */
 
 /* Derived parameters, exactly as the reference computes them (SURVEY.md A.0). */
 typedef struct fm_info {
@@ -149,6 +152,19 @@ int fm_process(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, size_t 
  * left untouched (background, counters), the stats of frames t >= n_valid[s] are zero. */
 int fm_process_ragged(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
                       int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev);
+
+/* fm_process_ragged that also hands out the frames the reference writes to its *_motion.avi in this call (needs
+ * FM_FLAG_DEVICE_CLIPS).  For stream s, with n_out[s] = sum of wrote + n_flush over its valid frames, it writes
+ * n_out[s] raw BGR frames densely to the DEVICE buffer
+ *   out_dev + s * out_stream_stride + i * H*W*3          (i < n_out[s])
+ * in the reference's order: for each frame in order, the n_flush cached frames it flushes (oldest first, taken from the
+ * device ring or from this call's input), then the frame itself if `wrote` (find_motion.py:561-570, 583).  n_out
+ * follows from the stats.  out_capacity is the room per stream in frames and must be at least cache_frames + n_frames,
+ * the most one call can write (the whole cache plus every frame); otherwise, or without the flag, FM_EINVAL.
+ * Asynchronous on `cuda_stream` like fm_process. */
+int fm_process_clip(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
+                    int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev,
+                    uint8_t *out_dev, size_t out_stream_stride, int out_capacity);
 
 /* Same with HOST buffers: copies the frames host->device (pinned memory recommended), runs the
  * path, copies the stats back and synchronises.  This is the call a drop-in adapter makes. */
