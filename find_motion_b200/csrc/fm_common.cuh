@@ -7,6 +7,7 @@
 #include <stdint.h>
 
 #include <atomic>
+#include <utility>
 
 #include "../../include/fm_gpu.h"
 
@@ -79,11 +80,13 @@ struct fm_ctx {
     double *bg;                // [S][ntiles][8][32][2]  float64 background, tiled
     uint32_t *maskbits;        // [S][h][wpr]  1 = zero the blur here
     uint32_t *maskflat;        // [S][ntiles*16] same mask, flat bit order (fused kernels)
-    uint32_t *tflat;           // [S][Tmax][ntiles*16]  raw threshold, flat bit order
+    uint32_t *tflat;           // [slots][S][Tmax][ntiles*16]  raw threshold, flat bit order (fm_tflat)
     uint32_t *dil;             // [S][Tmax][h][wpr]  dilated threshold, row-padded bit plane
     uint32_t *fill;            // [S][Tmax][h][wpr]  dilated threshold with holes filled
     int *any;                  // [S][Tmax][4] range of set pixels: (max y, max h-1-y, max word column j, max wpr-1-j), -1 = none
-    int *rawrange;             // [S][Tmax][2] row range of the RAW threshold (written by the temporal kernels)
+    int *rawrange;             // [slots][S][Tmax][2] row range of the RAW threshold (written by the temporal kernels, fm_rawrange)
+    int slot;                  // per-call slot of tflat / rawrange the next call uses (alternates with the fused front end)
+    int *bg_valid;             // [2][S] the fused front end's own "background exists" flag, indexed by slot
     int *heavy;                // [S][Tmax] frame needs the global-memory labelling kernel
     int *ncomp;                // [S][Tmax]
     int *ncounted;             // [S][Tmax]
@@ -115,8 +118,10 @@ struct fm_ctx {
     int *clip_count;           // [2] entries of the two lists in the current call
     int clip_sms;              // multiprocessors of the device (grid of the copy kernels)
     // timing
-    bool timing;               // bracket the kernel groups with events (no sync inside fm_process)
+    bool timing;               // time the kernel groups: events around them, or stamps with the fused front end (no sync inside fm_process)
     cudaEvent_t *evs;          // [FM_TIMING_RING][4]
+    unsigned long long *stamps;   // [FM_TIMING_RING][4] fused front end: %globaltimer of the groups (fm_stamp_*)
+    unsigned long long *stamp;    // the stamps of the call being enqueued, null when none are taken
     int ev_pending;
     double t_ms[3];
     int64_t t_calls;
@@ -148,6 +153,47 @@ void fm_set_error(const char *fmt, ...);
             return FM_ECUDA;                                                      \
         }                                                                         \
     } while (0)
+
+// The fused front end of call i+1 runs while the contour stage of call i still reads its raw threshold bits and
+// ranges, so those two buffers have two slots used by alternate calls (one slot with the other front ends).  Layout of
+// `rawrange`: [range slot 0][any][range slot 1], each range slot S*Tmax*2 ints: a range slot and `any` are adjacent in
+// both parities, so one fill clears both.
+inline uint32_t *fm_tflat(const fm_ctx *c) {
+    return c->tflat + (size_t)c->slot * c->S * c->Tmax * c->ntiles * FM_TILE_WORDS;
+}
+inline int *fm_rawrange(const fm_ctx *c) { return c->rawrange + (size_t)c->slot * 6 * c->S * c->Tmax; }
+
+// Programmatic dependent launch (sm_90+): the kernel may start while the kernel before it in `st` still runs, once
+// every CTA of that one has executed griddepcontrol.launch_dependents (or exited).  It must execute
+// griddepcontrol.wait before it touches what its predecessor writes; that wait returns when the predecessor has
+// completed and its memory is visible.  After any other stream operation it is an ordinary launch.
+template <typename... KArgs, typename... Args>
+cudaError_t fm_launch_chained(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                              Args &&...args) {
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
+// Group times of a chained call: events recorded between two chained kernels would sit in the chain, so the kernels of a
+// group stamp %globaltimer (ns) themselves.  stamp[0] / stamp[2]: NOT of the earliest start of the front end / contour
+// stage (atomicMax of ~t is a minimum, and 0 is the cleared value of both kinds), stamp[1] / stamp[3]: latest end.
+__device__ __forceinline__ unsigned long long fm_globaltimer() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+__device__ __forceinline__ void fm_stamp_start(unsigned long long *stamp) {
+    if (stamp && threadIdx.x == 0) atomicMax(stamp, ~fm_globaltimer());
+}
+__device__ __forceinline__ void fm_stamp_end(unsigned long long *stamp) {
+    if (stamp && threadIdx.x == 0) atomicMax(stamp + 1, fm_globaltimer());
+}
+__device__ __forceinline__ void fm_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+__device__ __forceinline__ void fm_wait_predecessor() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 // stage launchers (each enqueues on `st`, returns FM_OK / error)
 int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T,

@@ -174,7 +174,7 @@ extern "C" int fm_ctx_destroy(fm_ctx *c) {
     cudaFree(c->gray); cudaFree(c->hor); cudaFree(c->blur); cudaFree(c->bg);
     cudaFree(c->maskbits); cudaFree(c->maskflat); cudaFree(c->tflat); cudaFree(c->dil); cudaFree(c->fill);
     cudaFree(c->heavy); cudaFree(c->rawrange); cudaFree(c->ncomp); cudaFree(c->comps); cudaFree(c->stats);      // any / ncounted live inside rawrange / ncomp
-    cudaFree(c->state); cudaFree(c->errflag); cudaFree(c->nvalid);
+    cudaFree(c->state); cudaFree(c->bg_valid); cudaFree(c->errflag); cudaFree(c->nvalid);
     free(c->nvalid_host);
     fm_ccl_free(&c->ccl);
     for (int i = 0; i < 2; i++) {
@@ -190,6 +190,7 @@ extern "C" int fm_ctx_destroy(fm_ctx *c) {
         for (int i = 0; i < 4 * FM_TIMING_RING; i++) cudaEventDestroy(c->evs[i]);
         delete[] c->evs;
     }
+    cudaFree(c->stamps);
     delete c;
     return FM_OK;
 }
@@ -346,12 +347,15 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     ALLOC(c->bg, bg_doubles * sizeof(double));
     ALLOC(c->maskbits, (size_t)c->S * c->h * c->wpr * 4);
     ALLOC(c->maskflat, (size_t)c->S * flatw * 4);
-    ALLOC(c->tflat, (F * flatw + FM_TILE_WORDS) * 4);
+    // two slots of the raw threshold bits and ranges with the fused front end, which overlaps the previous call's
+    // contour stage (fm_tflat, fm_rawrange)
+    const size_t slots = c->fused ? 2 : 1;
+    ALLOC(c->tflat, (slots * F * flatw + FM_TILE_WORDS) * 4);
     ALLOC(c->dil, F * c->h * c->wpr * 4);
     ALLOC(c->fill, F * c->h * c->wpr * 4);
-    // ranges of the raw ([F][2]) and of the dilated mask ([F][4]) share one allocation, and so do the two counters:
-    // one memset each per call
-    ALLOC(c->rawrange, F * 6 * sizeof(int));
+    // ranges of the raw ([slots][F][2]) and of the dilated mask ([F][4]) share one allocation, and so do the two
+    // counters: one clear each per call
+    ALLOC(c->rawrange, F * (4 + 2 * slots) * sizeof(int));
     c->any = c->rawrange + 2 * F;
     ALLOC(c->ncomp, (F * 2 + 4) * sizeof(int));        // + the frame counter of the decision tail
     c->ncounted = c->ncomp + F;
@@ -359,6 +363,7 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     ALLOC(c->comps, F * c->maxc * sizeof(fm_component));
     ALLOC(c->stats, F * sizeof(fm_frame_stats));
     ALLOC(c->state, (size_t)c->S * sizeof(StreamState));
+    ALLOC(c->bg_valid, 2 * (size_t)c->S * sizeof(int));
     ALLOC(c->errflag, sizeof(int));
     ALLOC(c->nvalid, (size_t)c->S * sizeof(int));
     c->nvalid_host = (int *)malloc((size_t)c->S * sizeof(int));
@@ -367,9 +372,12 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     FM_TRY(cudaMemcpy(c->nvalid, c->nvalid_host, (size_t)c->S * sizeof(int), cudaMemcpyHostToDevice));
     FM_TRY(cudaMemset(c->maskbits, 0, (size_t)c->S * c->h * c->wpr * 4));
     FM_TRY(cudaMemset(c->maskflat, 0, (size_t)c->S * flatw * 4));
-    FM_TRY(cudaMemset(c->tflat, 0, (F * flatw + FM_TILE_WORDS) * 4));
+    FM_TRY(cudaMemset(c->tflat, 0, (slots * F * flatw + FM_TILE_WORDS) * 4));
     FM_TRY(cudaMemset(c->bg, 0, bg_doubles * sizeof(double)));
     FM_TRY(cudaMemset(c->state, 0, (size_t)c->S * sizeof(StreamState)));
+    FM_TRY(cudaMemset(c->bg_valid, 0, 2 * (size_t)c->S * sizeof(int)));
+    FM_TRY(cudaMemset(c->rawrange, 0xFF, F * (4 + 2 * slots) * sizeof(int)));      // the fused front end clears them
+    FM_TRY(cudaMemset(c->ncomp, 0, (F * 2 + 4) * sizeof(int)));                    //   for the call after it
     FM_TRY(cudaMemset(c->errflag, 0, sizeof(int)));
     FM_TRY(cudaMemset(c->heavy, 0, F * sizeof(int)));
     // contour scratch: a dilated plane has runs >= 3 px separated by >= 1 px, so a row holds at
@@ -406,9 +414,11 @@ extern "C" int fm_ctx_reset(fm_ctx *c, int stream) {
     FM_CUDA(cudaDeviceSynchronize());
     if (stream < 0) {
         FM_CUDA(cudaMemset(c->state, 0, (size_t)c->S * sizeof(StreamState)));
+        FM_CUDA(cudaMemset(c->bg_valid, 0, 2 * (size_t)c->S * sizeof(int)));
         FM_CUDA(cudaMemset(c->errflag, 0, sizeof(int)));
     } else {
         FM_CUDA(cudaMemset(c->state + stream, 0, sizeof(StreamState)));
+        for (int i = 0; i < 2; i++) FM_CUDA(cudaMemset(c->bg_valid + (size_t)i * c->S + stream, 0, sizeof(int)));
     }
     return FM_OK;
 }
@@ -450,6 +460,21 @@ extern "C" int fm_ctx_set_masks(fm_ctx *c, int stream, int n_polys, const int32_
 // the hot path
 // --------------------------------------------------------------------------------------------
 static int timing_drain(fm_ctx *c) {
+    if (c->fused) {     // group stamps taken by the kernels (the chained launches carry no events)
+        if (!c->ev_pending) return FM_OK;
+        std::vector<unsigned long long> st((size_t)4 * c->ev_pending);
+        FM_CUDA(cudaDeviceSynchronize());
+        FM_CUDA(cudaMemcpy(st.data(), c->stamps, st.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+        FM_CUDA(cudaMemset(c->stamps, 0, st.size() * sizeof(unsigned long long)));
+        for (int i = 0; i < c->ev_pending; i++) {
+            const unsigned long long *q = &st[4 * (size_t)i];
+            c->t_ms[0] += (double)(q[1] - ~q[0]) * 1e-6;     // front end: first CTA start .. last CTA end
+            c->t_ms[2] += (double)(q[3] - ~q[2]) * 1e-6;     // contour stage (the temporal stage is inside K1)
+            c->t_calls++;
+        }
+        c->ev_pending = 0;
+        return FM_OK;
+    }
     for (int i = 0; i < c->ev_pending; i++) {
         cudaEvent_t *ev = c->evs + 4 * i;
         FM_CUDA(cudaEventSynchronize(ev[3]));
@@ -486,27 +511,32 @@ static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_
         // pageable source: the runtime stages the bytes before returning, so nvalid_host may change right after
         if (changed) FM_CUDA(cudaMemcpyAsync(c->nvalid, c->nvalid_host, (size_t)c->S * sizeof(int), cudaMemcpyHostToDevice, st));
     }
-    {   // per-frame result slots of the call: ranges = -1 (nothing set), counters = 0
+    if (!c->fused) {   // per-frame result slots of the call: ranges = -1 (nothing set), counters = 0
+        // (the fused front end clears them itself for the call after it, so that no memset ends the launch chain)
         const size_t Fmax = (size_t)c->S * c->Tmax;
         FM_CUDA(cudaMemsetAsync(c->rawrange, 0xFF, Fmax * 6 * sizeof(int), st));
         FM_CUDA(cudaMemsetAsync(c->ncomp, 0, (Fmax * 2 + 4) * sizeof(int), st));
     }
     cudaEvent_t *ev = nullptr;
+    c->stamp = nullptr;
     if (c->timing) {
         if (c->ev_pending == FM_TIMING_RING && (rc = timing_drain(c))) return rc;
-        ev = c->evs + 4 * c->ev_pending++;
-        FM_CUDA(cudaEventRecord(ev[0], st));
+        if (c->fused) c->stamp = c->stamps + 4 * c->ev_pending++;
+        else { ev = c->evs + 4 * c->ev_pending++; FM_CUDA(cudaEventRecord(ev[0], st)); }
     }
     if (c->fused) {
-        if ((rc = fm_launch_fused(c, frames, stream_stride, frame_stride, n_frames, st))) return rc;
-        if (ev) { FM_CUDA(cudaEventRecord(ev[1], st)); FM_CUDA(cudaEventRecord(ev[2], st)); }
+        rc = fm_launch_fused(c, frames, stream_stride, frame_stride, n_frames, st);
+        if (rc) { if (c->stamp) c->ev_pending--; c->stamp = nullptr; return rc; }
     } else {
         if ((rc = fm_launch_frontend(c, frames, stream_stride, frame_stride, n_frames, st))) return rc;
         if (ev) FM_CUDA(cudaEventRecord(ev[1], st));
         if (!c->wide_fused && !c->umma && (rc = fm_launch_temporal(c, n_frames, st))) return rc;
         if (ev) FM_CUDA(cudaEventRecord(ev[2], st));
     }
-    if ((rc = fm_launch_morph_ccl(c, n_frames, st, stats_dev))) return rc;
+    rc = fm_launch_morph_ccl(c, n_frames, st, stats_dev);
+    c->stamp = nullptr;
+    if (rc) return rc;
+    if (c->fused) c->slot ^= 1;
     if (ev) FM_CUDA(cudaEventRecord(ev[3], st));
     if ((c->cfg.flags & FM_FLAG_DEVICE_CLIPS) &&
         (rc = fm_launch_clips(c, frames, stream_stride, frame_stride, n_frames, out, out_stride, st)))
@@ -619,6 +649,8 @@ extern "C" int fm_submit_reset(fm_ctx *c, int stream) {
     if (stream < 0 || stream >= c->S) { fm_set_error("stream %d out of range", stream); return FM_EINVAL; }
     FM_CUDA(cudaSetDevice(c->cfg.device));
     FM_CUDA(cudaMemsetAsync(c->state + stream, 0, sizeof(StreamState), c->own_stream));
+    for (int i = 0; i < 2; i++)
+        FM_CUDA(cudaMemsetAsync(c->bg_valid + (size_t)i * c->S + stream, 0, sizeof(int), c->own_stream));
     return FM_OK;
 }
 
@@ -858,7 +890,11 @@ extern "C" int fm_debug_components(int device, const uint8_t *plane, int w, int 
 extern "C" int fm_timing_enable(fm_ctx *c, int on) {
     if (!c) return FM_EINVAL;
     FM_CUDA(cudaSetDevice(c->cfg.device));
-    if (on && !c->evs) {
+    if (on && c->fused && !c->stamps) {
+        FM_CUDA(cudaMalloc(&c->stamps, (size_t)4 * FM_TIMING_RING * sizeof(unsigned long long)));
+        FM_CUDA(cudaMemset(c->stamps, 0, (size_t)4 * FM_TIMING_RING * sizeof(unsigned long long)));
+    }
+    if (on && !c->fused && !c->evs) {
         c->evs = new cudaEvent_t[4 * FM_TIMING_RING];
         for (int i = 0; i < 4 * FM_TIMING_RING; i++) FM_CUDA(cudaEventCreate(&c->evs[i]));
     }

@@ -74,7 +74,12 @@ struct FusedParams {
     const uint32_t *maskbits;   // [S][h][wpr]
     uint32_t *tbits;            // [S][T][flatwords]  (row-padded == flat because w % 32 == 0)
     size_t flatwords;
-    const StreamState *state;
+    const int *bg_in;           // [S] bg_valid slot of this call: the stream has a background
+    int *bg_out;                // [S] bg_valid slot of the next call
+    int *clear_ff;              // filled with -1 after the wait at the end: the other range slot and `any`
+    int *clear_zero;            //   ... and zeroed: the contour counters
+    int n_ff, n_zero;
+    unsigned long long *stamp;  // front-end group stamps of the call (null: timing off)
     int b0, b1, b2, shift, rnd; // taps / g, and the rounding of the final shift (packed in both lanes)
     int threshold;
     double alpha, beta;
@@ -236,6 +241,25 @@ __device__ __forceinline__ uint32_t fused_rows(const uint32_t *shw, double (&bg)
     return __brev(bits) >> (32 - FT_PX);      // the first pixel was pushed first: bit idx = pixel idx
 }
 
+// End of every CTA of K1.  K1 of call i+1 is launched as a programmatic dependent of k_decide of call i (fm_host.cu), so
+// it starts while the contour stage of call i still runs and may do all its own work then: it reads only the frames,
+// the mask, n_valid, its background and bg_valid, and writes the other tflat / rawrange slot.  The wait here keeps the
+// chain transitive: K1(i+1) cannot complete before decide(i) has, and decide(i) waits for the labelling kernels of
+// call i, which wait for K1(i).  So the contour stage of call i+1 (an ordinary launch after K1(i+1)) never runs ahead
+// of call i, and K1(i+2) never writes the slot the contour stage of call i reads.  Past the wait, the contour stage of
+// call i is complete, so this is where the per-call result slots are cleared: the range slot call i used (call i+1
+// uses it next), `any` and the counters, which the contour stage of call i+1 fills.
+__device__ __forceinline__ void fused_exit(const FusedParams &p) {
+    fm_stamp_end(p.stamp);                       // this CTA's own work is done; the wait below is not the front end's
+    fm_wait_predecessor();
+    const int nthreads = gridDim.x * gridDim.y * gridDim.z * FUSED_THREADS;
+    for (int i = ((blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * FUSED_THREADS + threadIdx.x;
+         i < p.n_ff + p.n_zero; i += nthreads) {
+        if (i < p.n_ff) p.clear_ff[i] = -1;
+        else p.clear_zero[i - p.n_ff] = 0;
+    }
+}
+
 template <bool KEEP, bool SAFE>
 __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const __grid_constant__ CUtensorMap tmap, FusedParams p) {
     extern __shared__ __align__(128) unsigned char fsm[];
@@ -249,9 +273,15 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
     const int x0 = tx * FT_W, y0 = ty * FT_H;
     const int w = p.w, h = p.h;
     const bool border = (x0 == 0) || (x0 + FT_W >= w) || (y0 == 0) || (y0 + FT_H >= h);
-    const bool has_bg = p.state[s].has_bg != 0;
+    fm_stamp_start(p.stamp);
+    // not StreamState::has_bg: k_decide of the previous call may still be running and writes it
+    const bool has_bg = p.bg_in[s] != 0;
     const int Ts = min(p.T, __ldg(p.nvalid + s));            // frames of this stream that are real
-    if (Ts <= 0) return;
+    if (tid == 0 && tx == 0 && ty == 0) p.bg_out[s] = has_bg || Ts > 0;
+    if (Ts <= 0) {
+        fused_exit(p);
+        return;
+    }
 
     // this thread's pixels: row y0 + tid / 8, columns x0 + 8 (tid % 8) .. + 7 and the same 64 pixels further right
     const int trow = tid >> 3, xg = tid & 7;
@@ -407,6 +437,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
     }
 #pragma unroll
     for (int i = 0; i < FT_PX / 2; i++) bgt[i * 32] = make_double2(bg[2 * i], bg[2 * i + 1]);
+    fused_exit(p);
 }
 
 // tiled background -> row-major float64 plane
@@ -472,9 +503,17 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     p.T = T; p.nvalid = c->nvalid;
     p.w = c->w; p.h = c->h; p.wpr = c->wpr;
     p.tilesX = (c->w + FT_W - 1) / FT_W; p.tilesY = (c->h + FT_H - 1) / FT_H;
-    p.bg = c->bg; p.maskbits = c->maskbits; p.tbits = c->tflat;
+    p.bg = c->bg; p.maskbits = c->maskbits; p.tbits = fm_tflat(c);
     p.flatwords = (size_t)c->ntiles * FM_TILE_WORDS;
-    p.state = c->state;
+    p.bg_in = c->bg_valid + (size_t)c->slot * c->S;
+    p.bg_out = c->bg_valid + (size_t)(c->slot ^ 1) * c->S;
+    {
+        const int Fmax = c->S * c->Tmax;
+        p.clear_ff = c->rawrange + (c->slot ? 0 : 2 * Fmax);      // [range slot 0][any] or [any][range slot 1]
+        p.n_ff = 6 * Fmax;
+        p.clear_zero = c->ncomp;                                   // ncomp, ncounted and the frame counter
+        p.n_zero = 2 * Fmax + 4;
+    }
     // taps / g for k in {1,3,5}: [0,0,1,0,0] g=256, [0,1,2,1,0] g=64, [1,4,6,4,1] g=16
     int lg;
     if (c->k == 1) { p.b0 = 0; p.b1 = 0; p.b2 = 1; lg = 8; }
@@ -486,7 +525,8 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     p.threshold = c->cfg.threshold;
     p.alpha = c->cfg.avg; p.beta = 1.0 - p.alpha;
     p.gray_out = c->gray; p.blur_out = c->blur;
-    p.rawrange = c->rawrange;
+    p.rawrange = fm_rawrange(c);
+    p.stamp = c->stamp;
     const bool keep = (c->cfg.flags & FM_FLAG_KEEP_PLANES) != 0;
     const bool safe = p.alpha >= 0.0 && p.alpha <= 1.0 && p.threshold >= 0;
     fused_bfr(p);
@@ -496,13 +536,10 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     if ((rc = fm_ensure_smem((const void *)k_fused<true, false>, FUSED_SMEM, c->cfg.device))) return rc;
     if ((rc = fm_ensure_smem((const void *)k_fused<false, true>, FUSED_SMEM, c->cfg.device))) return rc;
     if ((rc = fm_ensure_smem((const void *)k_fused<false, false>, FUSED_SMEM, c->cfg.device))) return rc;
-    if (keep) {
-        if (safe) k_fused<true, true><<<grid, FUSED_THREADS, FUSED_SMEM, st>>>(tmap, p);
-        else k_fused<true, false><<<grid, FUSED_THREADS, FUSED_SMEM, st>>>(tmap, p);
-    } else {
-        if (safe) k_fused<false, true><<<grid, FUSED_THREADS, FUSED_SMEM, st>>>(tmap, p);
-        else k_fused<false, false><<<grid, FUSED_THREADS, FUSED_SMEM, st>>>(tmap, p);
-    }
+    // a programmatic dependent of the contour stage of the previous call: see fused_exit
+    void (*kern)(const CUtensorMap, FusedParams) = keep ? (safe ? k_fused<true, true> : k_fused<true, false>)
+                                                        : (safe ? k_fused<false, true> : k_fused<false, false>);
+    (void)fm_launch_chained(kern, grid, dim3(FUSED_THREADS), FUSED_SMEM, st, tmap, p);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }

@@ -145,7 +145,9 @@ template <bool ALIGNED>
 __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) k_dilate(const uint32_t *__restrict__ tflat,
                                                                  uint32_t *__restrict__ dil, int *__restrict__ rowrange,
                                                                  const int *__restrict__ rawrange, int F, int w, int h,
-                                                                 int wpr, int flatwords, int T, int t0, int Th) {
+                                                                 int wpr, int flatwords, int T, int t0, int Th,
+                                                                 unsigned long long *stamp) {
+    fm_stamp_start(stamp);
     // F = S*Th local frames: local frame lf is frame t0 + lf % Th of stream lf / Th, stored at s*T + t
     int warp = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
     int lane = threadIdx.x & 31;
@@ -195,6 +197,7 @@ struct CclArgs {
     int *ncomp, *ncounted;     // [F]
     fm_component *comps;       // [F][maxc]
     int maxc, min_area, max_area;
+    unsigned long long *stamp; // contour-stage stamps of the call (null: timing off): &stamps[2]
 };
 
 // INVERT: runs of zeros (background pass).  Planes written earlier in the same kernel are read
@@ -440,6 +443,7 @@ struct DecideArgs {
     fm_frame_stats *stats, *stats_out;
     const int *nvalid;
     int *done;                 // frames labelled so far in this call (cleared with the counters)
+    unsigned long long *stamp; // contour-stage stamps of the call (null: timing off): &stamps[2]
     int S, T, total, cache_frames, min_movement_frames;
 };
 
@@ -498,23 +502,39 @@ __device__ __forceinline__ void decide_stream(const DecideArgs &d, const int *nc
 
 // decisions of the call, one thread per stream (measured: a "last CTA done" tail inside the labelling kernel and an in-kernel
 // call of the global-memory fallback made the labelling kernel 15 us slower than these two tiny extra launches cost)
+// The contour stage is a chain of programmatic dependent launches (fm_launch_chained): each kernel lets the next one
+// start at its entry and waits for its predecessor before its first read of it, so the next call's fused front end can
+// take the SMs this stage leaves idle (see fused_exit in k_fused.cu).
 __global__ void k_decide(DecideArgs d, const int *__restrict__ ncomp, const int *__restrict__ ncounted) {
+    fm_launch_dependents();
+    fm_wait_predecessor();
     int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s < d.S) decide_stream(d, ncomp, ncounted, s);
+    fm_stamp_end(d.stamp);                            // the last kernel of the stage: its end is the stage's
 }
 
+// One CTA per frame, or, as the fallback of k_ccl_frame_smem (heavy != null), CCL_FALLBACK_CTAS CTAs that take the frames
+// in turn: the fallback is a programmatic dependent of k_ccl_frame_smem, and a CTA waiting for it holds a whole SM
+// (1024 threads x 56 registers), so one CTA per frame would take every SM the labelling kernel leaves free, and the next
+// call's front end, further down the chain, could not start before the labelling kernel ends.
+#define CCL_FALLBACK_CTAS 16
 __global__ void __launch_bounds__(CCL_THREADS, 1) k_ccl_frame(CclArgs a, const int *__restrict__ heavy) {
-    const int lf = blockIdx.x, lg = a.f0 + lf, f = (lg / a.Th) * a.T + a.t0 + lg % a.Th;
-    if (heavy && !heavy[f]) return;                 // already labelled by k_ccl_frame_smem
-    int ylo = 0, yhi = a.h - 1;
-    bool work = true;
-    if (a.rowrange) {
-        int ymax = a.rowrange[4 * f], ymin = a.h - 1 - a.rowrange[4 * f + 1];
-        if (ymax < 0) work = false;                 // no set pixel in this frame
-        ylo = max(ymin - 1, 0);
-        yhi = min(ymax + 1, a.h - 1);
+    fm_launch_dependents();
+    fm_stamp_start(a.stamp);
+    fm_wait_predecessor();
+    for (int lf = blockIdx.x; lf < a.nf; lf += gridDim.x) {
+        const int lg = a.f0 + lf, f = (lg / a.Th) * a.T + a.t0 + lg % a.Th;
+        if (heavy && !heavy[f]) continue;           // already labelled by k_ccl_frame_smem
+        int ylo = 0, yhi = a.h - 1;
+        bool work = true;
+        if (a.rowrange) {
+            int ymax = a.rowrange[4 * f], ymin = a.h - 1 - a.rowrange[4 * f + 1];
+            if (ymax < 0) work = false;             // no set pixel in this frame
+            ylo = max(ymin - 1, 0);
+            yhi = min(ymax + 1, a.h - 1);
+        }
+        if (work) ccl_frame_global(a, lf, f, ylo, yhi);     // scratch slot lf: frames share nothing
     }
-    if (work) ccl_frame_global(a, lf, f, ylo, yhi);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -890,6 +910,8 @@ __device__ __forceinline__ bool ccl_window(const CclArgs &a, int f, int &ylo, in
 
 __global__ void __launch_bounds__(CCL2_THREADS, 1) k_ccl_frame_smem(CclArgs a, int *__restrict__ heavy) {
     extern __shared__ __align__(16) unsigned char csm[];
+    fm_launch_dependents();                           // an ordinary launch: what it reads is complete
+    fm_stamp_start(a.stamp);
     const int lf = blockIdx.x, lg = a.f0 + lf, f = (lg / a.Th) * a.T + a.t0 + lg % a.Th;
     int ylo, yhi, jlo, jhi;
     bool is_heavy = false;
@@ -986,7 +1008,8 @@ int fm_ccl_configure(fm_ctx *c) {          // fm_ctx_create: fail here, not at t
 static int ccl_run(const CclScratch &sc, const uint32_t *plane, uint32_t *fill, int *rowrange, int F, int w,
                    int h, int wpr, int *ncomp, int *ncounted, fm_component *comps, int maxc, int min_area,
                    int max_area, int *errflag, int *heavy, int T, int t0, int Th, cudaStream_t st,
-                   const uint32_t *raw = nullptr, const int *rawrange = nullptr, int flatwords = 0) {
+                   const uint32_t *raw = nullptr, const int *rawrange = nullptr, int flatwords = 0,
+                   unsigned long long *stamp = nullptr) {
     for (int f0 = 0; f0 < F; f0 += sc.frames) {
         int nf = F - f0 < sc.frames ? F - f0 : sc.frames;
         CclArgs a;
@@ -1000,6 +1023,7 @@ static int ccl_run(const CclScratch &sc, const uint32_t *plane, uint32_t *fill, 
         a.ncomp = ncomp; a.ncounted = ncounted; a.comps = comps; a.maxc = maxc;
         a.min_area = min_area; a.max_area = max_area;
         a.cache_words = 0;
+        a.stamp = stamp;
         size_t smem = 0;
         if (heavy && ccl_smem_plan(h, wpr, &smem, &a.cache_words)) {
             int dev = 0;
@@ -1010,10 +1034,11 @@ static int ccl_run(const CclScratch &sc, const uint32_t *plane, uint32_t *fill, 
             FM_LAUNCH_CHECK();
             // the global-memory kernel takes the frames that overflowed the shared tables; on small planes (default mode:
             // 100 x 56) no frame can hold more than CCL2_CAP runs of either polarity, and the idle launch is left out
-            if ((size_t)h * (w / 2 + 2) > CCL2_CAP) k_ccl_frame<<<nf, CCL_THREADS, 0, st>>>(a, heavy);
+            if ((size_t)h * (w / 2 + 2) > CCL2_CAP)
+                (void)fm_launch_chained(k_ccl_frame, nf < CCL_FALLBACK_CTAS ? nf : CCL_FALLBACK_CTAS, CCL_THREADS, 0, st, a, (const int *)heavy);
         } else {
             a.raw = nullptr;
-            k_ccl_frame<<<nf, CCL_THREADS, 0, st>>>(a, nullptr);
+            (void)fm_launch_chained(k_ccl_frame, nf, CCL_THREADS, 0, st, a, (const int *)nullptr);
         }
         FM_LAUNCH_CHECK();
     }
@@ -1021,36 +1046,39 @@ static int ccl_run(const CclScratch &sc, const uint32_t *plane, uint32_t *fill, 
 }
 
 // Dilation + contours + decisions of a T-frame call.  The per-frame result slots (ranges, counts, the frame counter of
-// the decision tail) are cleared by fm_process before the front end runs; frames beyond a stream's n_valid keep an
-// empty range and leave at once.
+// the decision tail) are cleared before this stage runs (by fm_process, or by the fused front end: fused_exit); frames
+// beyond a stream's n_valid keep an empty range and leave at once.
 int fm_launch_morph_ccl(fm_ctx *c, int T, cudaStream_t st, fm_frame_stats *stats_out) {
     const int F = c->S * T;
     size_t smem_plan = 0;
     int cw_plan = 0, rc;
     const bool smem_ok = ccl_smem_plan(c->h, c->wpr, &smem_plan, &cw_plan);
+    unsigned long long *stamp = c->stamp ? c->stamp + 2 : nullptr;
     // With enough frames to fill the GPU (one CTA per frame) the shared-memory labelling kernel dilates the raw
     // threshold bits of its frame itself; with few frames the grid-wide k_dilate (one warp per row) is faster.
     if (smem_ok && F >= 32) {
         rc = ccl_run(c->ccl, c->dil, c->fill, c->any, F, c->w, c->h, c->wpr, c->ncomp, c->ncounted, c->comps, c->maxc,
-                     c->info.min_area, c->info.max_area, c->errflag, c->heavy, T, 0, T, st, c->tflat, c->rawrange,
-                     c->ntiles * FM_TILE_WORDS);
+                     c->info.min_area, c->info.max_area, c->errflag, c->heavy, T, 0, T, st, fm_tflat(c), fm_rawrange(c),
+                     c->ntiles * FM_TILE_WORDS, stamp);
     } else {
         int blocks = (F * c->h + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
         if (c->w % 32 == 0)
-            k_dilate<true><<<blocks, 32 * WARPS_PER_BLOCK, 0, st>>>(c->tflat, c->dil, c->any, c->rawrange, F, c->w, c->h,
-                                                                   c->wpr, c->ntiles * FM_TILE_WORDS, T, 0, T);
+            k_dilate<true><<<blocks, 32 * WARPS_PER_BLOCK, 0, st>>>(fm_tflat(c), c->dil, c->any, fm_rawrange(c), F, c->w, c->h,
+                                                                   c->wpr, c->ntiles * FM_TILE_WORDS, T, 0, T, stamp);
         else
-            k_dilate<false><<<blocks, 32 * WARPS_PER_BLOCK, 0, st>>>(c->tflat, c->dil, c->any, c->rawrange, F, c->w, c->h,
-                                                                    c->wpr, c->ntiles * FM_TILE_WORDS, T, 0, T);
+            k_dilate<false><<<blocks, 32 * WARPS_PER_BLOCK, 0, st>>>(fm_tflat(c), c->dil, c->any, fm_rawrange(c), F, c->w, c->h,
+                                                                    c->wpr, c->ntiles * FM_TILE_WORDS, T, 0, T, stamp);
         FM_LAUNCH_CHECK();
         rc = ccl_run(c->ccl, c->dil, c->fill, c->any, F, c->w, c->h, c->wpr, c->ncomp, c->ncounted, c->comps, c->maxc,
-                     c->info.min_area, c->info.max_area, c->errflag, smem_ok ? c->heavy : nullptr, T, 0, T, st);
+                     c->info.min_area, c->info.max_area, c->errflag, smem_ok ? c->heavy : nullptr, T, 0, T, st, nullptr,
+                     nullptr, 0, stamp);
     }
     if (rc) return rc;
     DecideArgs d;
     d.state = c->state; d.stats = c->stats; d.stats_out = stats_out; d.nvalid = c->nvalid; d.done = nullptr;
+    d.stamp = stamp;
     d.S = c->S; d.T = T; d.total = F; d.cache_frames = c->info.cache_frames; d.min_movement_frames = c->info.min_movement_frames;
-    k_decide<<<(c->S + 127) / 128, 128, 0, st>>>(d, c->ncomp, c->ncounted);
+    (void)fm_launch_chained(k_decide, (c->S + 127) / 128, 128, 0, st, d, (const int *)c->ncomp, (const int *)c->ncounted);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }
