@@ -3,6 +3,7 @@
 // reference's cv2 call chain, find_motion/find_motion.py:487-494, 619-700, 549-589).
 #pragma once
 
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -10,6 +11,7 @@
 #include <utility>
 
 #include "../../include/fm_gpu.h"
+#include "fm_device.cuh"
 
 #define FM_MAX_K 1024          // widest supported Gaussian (taps)
 #define FM_TILE_PX 512         // pixels per background tile: 32 lanes x 16 px
@@ -195,6 +197,16 @@ __device__ __forceinline__ void fm_stamp_end(unsigned long long *stamp) {
 __device__ __forceinline__ void fm_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void fm_wait_predecessor() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
+// cuTensorMapEncodeTiled of the driver (null when it is not available)
+typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
+                                    const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
+                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+PFN_encodeTiled fm_tma_encoder();
+// The call's frames as a 4-D u32 tensor map (W*3/4 words, H rows, T frames, S streams) with boxes of box_words x box_rows
+// (out-of-range elements are zero-filled).  FM_EINVAL unless the frames, their strides and rows are 16-byte aligned.
+int fm_frames_tmap(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, int box_words, int box_rows,
+                   CUtensorMap *out);
+
 // stage launchers (each enqueues on `st`, returns FM_OK / error)
 int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T,
                        cudaStream_t st);
@@ -238,22 +250,8 @@ int fm_clips_alloc(fm_ctx *c);
 void fm_clips_free(fm_ctx *c);
 int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
                     size_t ostride, cudaStream_t st);
+int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
 int fm_ccl_alloc(CclScratch *s, int frames, int h, int cap);
 void fm_ccl_free(CclScratch *s);
 int fm_ccl_plane(int device, const uint8_t *plane_host, int w, int h, int max_n, fm_component *out,
                  int *n);
-
-// gray (SURVEY.md A.2): Y = (3735 B + 19235 G + 9798 R + 16384) >> 15
-__device__ __forceinline__ uint32_t fm_gray(uint32_t b, uint32_t g, uint32_t r) {
-    return (3735u * b + 19235u * g + 9798u * r + 16384u) >> 15;
-}
-
-__device__ __forceinline__ int fm_reflect101(int i, int n) {
-    // BORDER_REFLECT_101 for any offset
-    if ((unsigned)i < (unsigned)n) return i;
-    if (n == 1) return 0;
-    int p = 2 * (n - 1);
-    i %= p;
-    if (i < 0) i += p;
-    return i >= n ? p - i : i;
-}

@@ -41,6 +41,39 @@ void fm_set_error(const char *fmt, ...) {
     va_end(ap);
 }
 
+PFN_encodeTiled fm_tma_encoder() {
+    static PFN_encodeTiled fn = nullptr;
+    if (!fn) {
+        void *sym = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &q) == cudaSuccess &&
+            q == cudaDriverEntryPointSuccess)
+            fn = (PFN_encodeTiled)sym;
+    }
+    return fn;
+}
+
+int fm_frames_tmap(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, int box_words, int box_rows,
+                   CUtensorMap *out) {
+    const size_t row = (size_t)c->W * 3, dense = row * c->H;
+    if ((((uintptr_t)frames) | sstride | fstride | row) & 15) {
+        fm_set_error("the TMA front ends need 16-byte aligned frames, strides and rows");
+        return FM_EINVAL;
+    }
+    PFN_encodeTiled enc = fm_tma_encoder();
+    if (!enc) { fm_set_error("cuTensorMapEncodeTiled not available"); return FM_ECUDA; }
+    // the stride of a dimension of extent 1 is never applied: the dense size stands in for it (the caller's may be 0)
+    cuuint64_t dims[4] = {(cuuint64_t)row / 4, (cuuint64_t)c->H, (cuuint64_t)T, (cuuint64_t)c->S};
+    cuuint64_t strides[3] = {(cuuint64_t)row, (cuuint64_t)(T > 1 ? fstride : dense),
+                             (cuuint64_t)(c->S > 1 ? sstride : (T > 1 ? fstride * T : dense))};
+    cuuint32_t box[4] = {(cuuint32_t)box_words, (cuuint32_t)box_rows, 1, 1};
+    cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, (void *)frames, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { fm_set_error("cuTensorMapEncodeTiled (frames) failed (%d)", (int)r); return FM_ECUDA; }
+    return FM_OK;
+}
+
 extern "C" const char *fm_last_error(void) { return g_err; }
 extern "C" int fm_version(void) { return 100; }
 extern "C" uint64_t fm_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }

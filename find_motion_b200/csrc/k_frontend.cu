@@ -16,16 +16,7 @@ __global__ void __launch_bounds__(256) k_gray(const uint8_t *__restrict__ frames
     if (i4 >= N) return;
     if (i4 + 4 <= N && ((((uintptr_t)src) & 3) == 0) && ((((uintptr_t)dst) & 3) == 0)) {
         const uint32_t *p = reinterpret_cast<const uint32_t *>(src + (size_t)i4 * 3);
-        uint32_t w0 = __ldg(p), w1 = __ldg(p + 1), w2 = __ldg(p + 2);
-        // two 16-bit x 8-bit dot products per pixel on doubled coefficients: Y is byte 2 of the sum
-        const uint32_t C_BG = 7470u | (38470u << 16), C_R = 19596u;
-        const uint32_t C_xB = 7470u << 16, C_GR = 38470u | (19596u << 16);
-        uint32_t p1 = __funnelshift_r(w0, w1, 24), p2 = __funnelshift_r(w1, w2, 16);
-        uint32_t t0 = __dp2a_hi(C_R, w0, __dp2a_lo(C_BG, w0, 32768u));
-        uint32_t t1 = __dp2a_hi(C_R, p1, __dp2a_lo(C_BG, p1, 32768u));
-        uint32_t t2 = __dp2a_hi(C_R, p2, __dp2a_lo(C_BG, p2, 32768u));
-        uint32_t t3 = __dp2a_hi(C_GR, w2, __dp2a_lo(C_xB, w2, 32768u));
-        *reinterpret_cast<uint32_t *>(dst + i4) = __byte_perm(__byte_perm(t0, t1, 0x0062), __byte_perm(t2, t3, 0x0062), 0x5410);
+        *reinterpret_cast<uint32_t *>(dst + i4) = fm_gray4(__ldg(p), __ldg(p + 1), __ldg(p + 2));
     } else {
         for (int i = i4; i < min(i4 + 4, N); i++) {
             const uint8_t *p = src + (size_t)i * 3;
@@ -288,14 +279,7 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_warp(K0Params p,
 // Same decomposition for 4-byte aligned rows: every lane walks its taps in groups of 4 source pixels
 // (12 bytes = three aligned 32-bit shared loads), the tap list padded to group boundaries with zero
 // weights (x + 0*y == x exactly, so the strictly ordered float32 chains are unchanged).  Bytes become
-// floats with PRMT into the mantissa of 2^23 -- no byte loads, no XU conversions -- and the bias leaves
-// inside the tap product.
-// rn(byte * a) in one FFMA: (2^23 + byte) * a - 2^23 * a is exactly byte * a before the single rounding (2^23 * a is
-// exact), i.e. the same float32 as the reference's unfused product; na = -(2^23 * a)
-__device__ __forceinline__ float byte_mul(uint32_t w, int i, float a, float na) {
-    return __fmaf_rn(__uint_as_float(__byte_perm(w, 0x4B000000u, 0x7540u | (uint32_t)i)), a, na);
-}
-
+// floats with PRMT into the mantissa of 2^23 (fm_byte_mul) and the bias leaves inside the tap product.
 struct K0GParams {
     const int *g4start;      // [w] first source pixel of the column's first group (multiple of 4)
     const int *g4n;          // [w] groups
@@ -399,12 +383,12 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
         const uint32_t *wp = reinterpret_cast<const uint32_t *>(rowbuf + mis - b_lo + 3 * gs);
         float b0 = 0.f, b1 = 0.f, b2 = 0.f;
 #define FM_G4(W0, W1, W2, a, n)                                                                               \
-        b0 = __fadd_rn(b0, byte_mul(W0, 0, a.x, n.x)); b1 = __fadd_rn(b1, byte_mul(W0, 1, a.x, n.x));       \
-        b2 = __fadd_rn(b2, byte_mul(W0, 2, a.x, n.x)); b0 = __fadd_rn(b0, byte_mul(W0, 3, a.y, n.y));       \
-        b1 = __fadd_rn(b1, byte_mul(W1, 0, a.y, n.y)); b2 = __fadd_rn(b2, byte_mul(W1, 1, a.y, n.y));       \
-        b0 = __fadd_rn(b0, byte_mul(W1, 2, a.z, n.z)); b1 = __fadd_rn(b1, byte_mul(W1, 3, a.z, n.z));       \
-        b2 = __fadd_rn(b2, byte_mul(W2, 0, a.z, n.z)); b0 = __fadd_rn(b0, byte_mul(W2, 1, a.w, n.w));       \
-        b1 = __fadd_rn(b1, byte_mul(W2, 2, a.w, n.w)); b2 = __fadd_rn(b2, byte_mul(W2, 3, a.w, n.w));
+        b0 = __fadd_rn(b0, fm_byte_mul(W0, 0, a.x, n.x)); b1 = __fadd_rn(b1, fm_byte_mul(W0, 1, a.x, n.x));       \
+        b2 = __fadd_rn(b2, fm_byte_mul(W0, 2, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(W0, 3, a.y, n.y));       \
+        b1 = __fadd_rn(b1, fm_byte_mul(W1, 0, a.y, n.y)); b2 = __fadd_rn(b2, fm_byte_mul(W1, 1, a.y, n.y));       \
+        b0 = __fadd_rn(b0, fm_byte_mul(W1, 2, a.z, n.z)); b1 = __fadd_rn(b1, fm_byte_mul(W1, 3, a.z, n.z));       \
+        b2 = __fadd_rn(b2, fm_byte_mul(W2, 0, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(W2, 1, a.w, n.w));       \
+        b1 = __fadd_rn(b1, fm_byte_mul(W2, 2, a.w, n.w)); b2 = __fadd_rn(b2, fm_byte_mul(W2, 3, a.w, n.w));
         if (inreg) {            // the column's weights live in registers for all source rows
 #pragma unroll
             for (int g = 0; g < K0_RG; g++) {

@@ -39,33 +39,6 @@
 #define RAW_BYTES (RAW_PITCH * FG_ROWS)                 // bytes one TMA box delivers
 #define RAW_STAGE ((RAW_BYTES + 127) / 128 * 128)        // stage stride (TMA destinations are 128 B aligned)
 
-// ---- TMA / mbarrier primitives (sm_100a PTX) ----
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_LOOP:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra WAIT_DONE;\n"
-        "bra WAIT_LOOP;\n"
-        "WAIT_DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_load_4d(void *dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, int c2,
-                                            int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-        ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-
 struct FusedParams {
     int T, w, h, wpr;           // T = frames per stream of the call
     const int *nvalid;          // [S] real frames of each stream in this call (ragged batches), <= T
@@ -108,50 +81,6 @@ static void fused_bfr(FusedParams &p) {
             }
         p.bfr[lane] = make_uint4(v[0], v[1], v[2], v[3]);
     }
-}
-
-__device__ __forceinline__ uint32_t gray4(uint32_t w0, uint32_t w1, uint32_t w2) {
-    // 4 BGR pixels in 3 words -> 4 gray bytes.  Y = (3735 B + 19235 G + 9798 R + 16384) >> 15 computed as
-    // (7470 B + 38470 G + 19596 R + 32768) >> 16 with two 16-bit x 8-bit dot products per pixel (IDP.2A);
-    // the lo/hi byte-pair selection of IDP.2A picks each pixel's bytes straight out of the three words.
-    // The result is byte 2 of the accumulator.
-    const uint32_t C_BG = 7470u | (38470u << 16), C_R = 19596u;              // byte pairs [B,G], [R,x]
-    const uint32_t C_xB = 7470u << 16, C_GR = 38470u | (19596u << 16);       // byte pairs [x,B], [G,R]
-    uint32_t t0 = __dp2a_hi(C_R, w0, __dp2a_lo(C_BG, w0, 32768u));           // w0 = [B0,G0,R0,B1]
-    uint32_t t1 = __dp2a_hi(C_xB, w0, __dp2a_lo(C_GR, w1, 32768u));          // w1 = [G1,R1,B2,G2]
-    uint32_t t2 = __dp2a_hi(C_BG, w1, __dp2a_lo(C_R, w2, 32768u));           // w2 = [R2,B3,G3,R3]
-    uint32_t t3 = __dp2a_hi(C_GR, w2, __dp2a_lo(C_xB, w2, 32768u));
-    return __byte_perm(__byte_perm(t0, t1, 0x0062), __byte_perm(t2, t3, 0x0062), 0x5410);
-}
-
-// ---- tensor-core primitives for the horizontal pass ----
-__device__ __forceinline__ void ldsm_x4(uint32_t addr, uint32_t &r0, uint32_t &r1, uint32_t &r2, uint32_t &r3) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-__device__ __forceinline__ void imma_u8(int (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0,
-                                        uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%10,%10,%10,%10};"
-                 : "=r"(d[0]), "=r"(d[1]), "=r"(d[2]), "=r"(d[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1), "r"(0));
-}
-
-__device__ __forceinline__ double u8_to_f64(uint32_t v) {
-    return __int2double_rn((int)v);          // exact for 0..255; one XU op instead of MOV + DADD
-}
-
-template <bool SAFE>
-__device__ __forceinline__ int bg8_magic(double b) {
-    // 0x4B400000 + rne(|float32(b)|) saturated to 255
-    float f = __double2float_rn(b);
-    if (!SAFE) f = fminf(fabsf(f), 255.0f);
-    return __float_as_int(__fadd_rn(f, 12582912.0f));
-}
-
-// bits = 2 * bits + (d > thr2) in two instructions: d + ~thr2 carries out exactly when d > thr2 (unsigned), and the
-// carry is shifted into the accumulator by an add-with-carry.
-__device__ __forceinline__ void push_gt(uint32_t &bits, uint32_t d, uint32_t nthr2) {
-    asm("{\n .reg .u32 t;\n add.cc.u32 t, %1, %2;\n addc.u32 %0, %0, %0;\n}" : "+r"(bits) : "r"(d), "r"(nthr2));
 }
 
 // 8x8 transpose of 4-bit elements across the 8 lanes of a lane octet: in: lane i holds e[r] (nibble r)
@@ -210,8 +139,8 @@ __device__ __forceinline__ uint32_t fused_rows(const uint32_t *shw, double (&bg)
             if (SH8) { o.x = __byte_perm(v[0], v[1], 0x7531); o.y = __byte_perm(v[2], v[3], 0x7531); }
             else { o.x = __byte_perm(v[0], v[1], 0x6420); o.y = __byte_perm(v[2], v[3], 0x6420); }
             const uint32_t mk = (M >> (8 * seg)) & 0xFFu;
-            o.x &= ~((((mk & 0xFu) * 0x00204081u) & 0x01010101u) * 0xFFu);
-            o.y &= ~(((((mk >> 4) & 0xFu) * 0x00204081u) & 0x01010101u) * 0xFFu);
+            o.x = fm_clear_masked4(o.x, mk & 0xFu);
+            o.y = fm_clear_masked4(o.y, (mk >> 4) & 0xFu);
             *reinterpret_cast<uint2 *>(blur_out + 64 * seg) = o;
         }
 #pragma unroll
@@ -220,22 +149,7 @@ __device__ __forceinline__ uint32_t fused_rows(const uint32_t *shw, double (&bg)
             uint32_t sv = SH8 ? __byte_perm(v[c >> 1], 0, (c & 1) ? 0x4443 : 0x4441)
                               : ((c & 1) ? (v[c >> 1] >> 16) : (v[c >> 1] & 0xFFFFu));
             if (MASKED && (M & (1u << idx))) sv = 0;          // mask_off_areas paints BLACK into blur
-            if (SAFE) {
-                // rn(blur * alpha) without an int -> double conversion (the XU pipe converts 16 lanes/clk/SM):
-                // X = 2^52 + blur is assembled from its bit pattern, and X * alpha - 2^52 * alpha is exactly
-                // blur * alpha before the single rounding of the FMA (2^52 * alpha is exact).
-                const double X = __hiloint2double(0x43300000, (int)sv);
-                if (INIT) bg[idx] = X - 4503599627370496.0;   // ref_frame = blur.astype(float)
-                int q = bg8_magic<SAFE>(bg[idx]);
-                push_gt(bits, (unsigned)(q - qoff - (int)sv), nthr2);           // |bg8 - blur| > threshold
-                bg[idx] = __fma_rn(bg[idx], p.beta, __fma_rn(X, p.alpha, nC));
-            } else {
-                const double sd = u8_to_f64(sv);
-                if (INIT) bg[idx] = sd;
-                int q = bg8_magic<SAFE>(bg[idx]);
-                push_gt(bits, (unsigned)(q - qoff - (int)sv), nthr2);
-                bg[idx] = __fma_rn(bg[idx], p.beta, __dmul_rn(sd, p.alpha));
-            }
+            fm_temporal_px<SAFE, INIT>(sv, bg[idx], bits, p.threshold, qoff, nthr2, p.alpha, p.beta, nC);
         }
     }
     return __brev(bits) >> (32 - FT_PX);      // the first pixel was pushed first: bit idx = pixel idx
@@ -307,15 +221,15 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
     // TMA pipeline: frame t+1 lands in the other stage while frame t is being processed
     const int cx = (x0 * 3) / 4 - 4, cy = y0 - 2;        // box origin in (u32 column, row); OOB is zero-filled
     if (tid == 0) {
-        mbar_init(&bars[0], 1);
-        mbar_init(&bars[1], 1);
+        fm_mbar_init(&bars[0], 1);
+        fm_mbar_init(&bars[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     }
     __syncthreads();
     if (tid == 0) {
-        mbar_expect_tx(&bars[0], RAW_BYTES);
-        tma_load_4d(raw, &tmap, &bars[0], cx, cy, 0, s);
+        fm_mbar_expect_tx(&bars[0], RAW_BYTES);
+        fm_tma_load_4d(raw, &tmap, &bars[0], cx, cy, 0, s);
     }
     // the thread's two bytes of the bit plane (row py, pixels px .. px+7 and px+64 .. px+71)
     uint8_t *tb = reinterpret_cast<uint8_t *>(p.tbits + ((size_t)s * p.T) * p.flatwords + (size_t)py * p.wpr) + (px >> 3);
@@ -330,17 +244,17 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
     // A-fragment row addresses of LDSM.x4 (lane L supplies row L&7 of matrix L>>3; matrices: rows 0-7 / 8-15 of
     // bytes 0-15, then of bytes 16-31) and D-fragment store positions
     const int hwin = warp & 7;                                  // the warp's 16-column window of the horizontal pass
-    const uint32_t sg_lane = smem_u32(sg) + ((lane & 7) + 8 * ((lane >> 3) & 1)) * (FG_WORDS * 4) + 16 * hwin + 16 * (lane >> 4);
+    const uint32_t sg_lane = fm_smem_u32(sg) + ((lane & 7) + 8 * ((lane >> 3) & 1)) * (FG_WORDS * 4) + 16 * hwin + 16 * (lane >> 4);
     uint32_t *sh_lane = sh + (lane >> 2) * FH_WORDS + 8 * hwin + (lane & 3);
 
     for (int t = 0; t < Ts; t++) {
         // No barrier here: every thread that gets this far has passed the second barrier of frame t-1, i.e. all
         // conversions out of raw stage (t+1)&1 (frame t-1) and all reads of the gray plane are complete.
         if (tid == 0 && t + 1 < Ts) {
-            mbar_expect_tx(&bars[(t + 1) & 1], RAW_BYTES);
-            tma_load_4d(raw + ((t + 1) & 1) * RAW_STAGE, &tmap, &bars[(t + 1) & 1], cx, cy, t + 1, s);
+            fm_mbar_expect_tx(&bars[(t + 1) & 1], RAW_BYTES);
+            fm_tma_load_4d(raw + ((t + 1) & 1) * RAW_STAGE, &tmap, &bars[(t + 1) & 1], cx, cy, t + 1, s);
         }
-        mbar_wait(&bars[t & 1], (t >> 1) & 1);
+        fm_mbar_wait(&bars[t & 1], (t >> 1) & 1);
         // ---- staged BGR -> gray bytes in shared memory (tile + halo) ----
         {
             // the staged rows are dense (pitch 432 B = 36 groups of 4 pixels = 12 B, the first at byte 4 because the
@@ -356,7 +270,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
                     const unsigned char *q = rs + u * 24;
                     const uint32_t a0 = *reinterpret_cast<const uint32_t *>(q), a5 = *reinterpret_cast<const uint32_t *>(q + 20);
                     const uint2 a12 = *reinterpret_cast<const uint2 *>(q + 4), a34 = *reinterpret_cast<const uint2 *>(q + 12);
-                    const uint32_t g0 = gray4(a0, a12.x, a12.y), g1 = gray4(a34.x, a34.y, a5);
+                    const uint32_t g0 = fm_gray4(a0, a12.x, a12.y), g1 = fm_gray4(a34.x, a34.y, a5);
                     *reinterpret_cast<uint2 *>(sg + 2 * u) = make_uint2(g0, g1);
                 }
             }
@@ -397,13 +311,13 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
             uint32_t a[NMB][4];
 #pragma unroll
             for (int i = 0; i < NMB; i++)
-                if (MBS == 1 || mb0 + i * MBS < FH_MB) ldsm_x4(sg_lane + (mb0 + i * MBS) * (16 * FG_WORDS * 4), a[i][0], a[i][1], a[i][2], a[i][3]);
+                if (MBS == 1 || mb0 + i * MBS < FH_MB) fm_ldsm_x4(sg_lane + (mb0 + i * MBS) * (16 * FG_WORDS * 4), a[i]);
 #pragma unroll
             for (int i = 0; i < NMB; i++) {
                 if (MBS == 1 || mb0 + i * MBS < FH_MB) {
                     int d0[4], d1[4];
-                    imma_u8(d0, a[i][0], a[i][1], a[i][2], a[i][3], bfr[0][0], bfr[0][1]);
-                    imma_u8(d1, a[i][0], a[i][1], a[i][2], a[i][3], bfr[1][0], bfr[1][1]);
+                    fm_imma0(d0, a[i][0], a[i][1], a[i][2], a[i][3], bfr[0][0], bfr[0][1], 0);
+                    fm_imma0(d1, a[i][0], a[i][1], a[i][2], a[i][3], bfr[1][0], bfr[1][1], 0);
                     uint32_t *o = sh_lane + (mb0 + i * MBS) * (16 * FH_WORDS);
                     o[0] = __byte_perm(d0[0], d0[1], 0x5410);
                     o[4] = __byte_perm(d1[0], d1[1], 0x5410);
@@ -464,41 +378,12 @@ size_t fm_fused_bg_doubles(const fm_ctx *c) {
     return (size_t)c->S * tilesX * tilesY * FT_W * FT_H;
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                    const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-PFN_encodeTiled fm_tma_encoder() {
-    static PFN_encodeTiled fn = nullptr;
-    if (!fn) {
-        void *sym = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            fn = (PFN_encodeTiled)sym;
-    }
-    return fn;
-}
-
 #define FUSED_SMEM (2 * RAW_STAGE + FH_ROWS * FG_WORDS * 4 + FH_ROWS * FH_WORDS * 4 + 16)
 
 int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
-    if ((((uintptr_t)frames) & 15) || (sstride & 15) || (fstride & 15)) {
-        fm_set_error("fused front end needs 16-byte aligned frames and strides (TMA)");
-        return FM_EINVAL;
-    }
-    PFN_encodeTiled enc = fm_tma_encoder();
-    if (!enc) { fm_set_error("cuTensorMapEncodeTiled not available"); return FM_ECUDA; }
-    // the call's frames as a 4-D u32 tensor: (W*3/4 words, H rows, T frames, S streams)
     CUtensorMap tmap;
-    cuuint64_t dims[4] = {(cuuint64_t)c->W * 3 / 4, (cuuint64_t)c->H, (cuuint64_t)T, (cuuint64_t)c->S};
-    cuuint64_t strides[3] = {(cuuint64_t)c->W * 3, (cuuint64_t)fstride, (cuuint64_t)(c->S > 1 ? sstride : fstride * T)};
-    cuuint32_t box[4] = {RAW_PITCH / 4, FG_ROWS, 1, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, (void *)frames, dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { fm_set_error("cuTensorMapEncodeTiled failed (%d)", (int)r); return FM_ECUDA; }
+    int rc = fm_frames_tmap(c, frames, sstride, fstride, T, RAW_PITCH / 4, FG_ROWS, &tmap);
+    if (rc) return rc;
     FusedParams p;
     p.T = T; p.nvalid = c->nvalid;
     p.w = c->w; p.h = c->h; p.wpr = c->wpr;
@@ -531,7 +416,6 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     const bool safe = p.alpha >= 0.0 && p.alpha <= 1.0 && p.threshold >= 0;
     fused_bfr(p);
     dim3 grid(p.tilesX, p.tilesY, c->S);
-    int rc;
     if ((rc = fm_ensure_smem((const void *)k_fused<true, true>, FUSED_SMEM, c->cfg.device))) return rc;
     if ((rc = fm_ensure_smem((const void *)k_fused<true, false>, FUSED_SMEM, c->cfg.device))) return rc;
     if ((rc = fm_ensure_smem((const void *)k_fused<false, true>, FUSED_SMEM, c->cfg.device))) return rc;

@@ -52,40 +52,6 @@ struct RowsParams {
     const int *nvalid;
 };
 
-// ---- TMA / mbarrier primitives (sm_100a PTX) ----
-__device__ __forceinline__ uint32_t rr_smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void rr_mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(rr_smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void rr_mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(rr_smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void rr_mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "RR_WAIT_LOOP:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra RR_WAIT_DONE;\n"
-        "bra RR_WAIT_LOOP;\n"
-        "RR_WAIT_DONE:\n"
-        "}\n" ::"r"(rr_smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void rr_tma_load_4d(void *dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, int c2,
-                                               int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-        ::"r"(rr_smem_u32(dst)), "l"(map), "r"(rr_smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-
-// rn(byte * a) in one FFMA: (2^23 + byte) * a - 2^23 * a is exactly byte * a before the single rounding (2^23 * a is
-// exact), i.e. the same float32 as the reference's unfused product; na = -(2^23 * a).  The byte is placed into the
-// mantissa of 2^23 by PRMT.
-__device__ __forceinline__ float rr_byte_mul(uint32_t w, int i, float a, float na) {
-    return __fmaf_rn(__uint_as_float(__byte_perm(w, 0x4B000000u, 0x7540u | (uint32_t)i)), a, na);
-}
-
 __device__ __forceinline__ uint4 rr_lds128(uint32_t addr) {
     uint4 v;
     asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
@@ -113,12 +79,12 @@ __device__ __forceinline__ void rr_col_pass(uint32_t blk, uint32_t sel, const fl
         const uint32_t X1 = __byte_perm(W[WO + 3 * g + 1], W[WO + 3 * g + 2], sel);
         const uint32_t X2 = __byte_perm(W[WO + 3 * g + 2], W[WO + 3 * g + 3], sel);
         // pixels in source order, channels B G R of each: the strictly ordered chains of resizeArea_
-        b0 = __fadd_rn(b0, rr_byte_mul(X0, 0, a.x, n.x)); b1 = __fadd_rn(b1, rr_byte_mul(X0, 1, a.x, n.x));
-        b2 = __fadd_rn(b2, rr_byte_mul(X0, 2, a.x, n.x)); b0 = __fadd_rn(b0, rr_byte_mul(X0, 3, a.y, n.y));
-        b1 = __fadd_rn(b1, rr_byte_mul(X1, 0, a.y, n.y)); b2 = __fadd_rn(b2, rr_byte_mul(X1, 1, a.y, n.y));
-        b0 = __fadd_rn(b0, rr_byte_mul(X1, 2, a.z, n.z)); b1 = __fadd_rn(b1, rr_byte_mul(X1, 3, a.z, n.z));
-        b2 = __fadd_rn(b2, rr_byte_mul(X2, 0, a.z, n.z)); b0 = __fadd_rn(b0, rr_byte_mul(X2, 1, a.w, n.w));
-        b1 = __fadd_rn(b1, rr_byte_mul(X2, 2, a.w, n.w)); b2 = __fadd_rn(b2, rr_byte_mul(X2, 3, a.w, n.w));
+        b0 = __fadd_rn(b0, fm_byte_mul(X0, 0, a.x, n.x)); b1 = __fadd_rn(b1, fm_byte_mul(X0, 1, a.x, n.x));
+        b2 = __fadd_rn(b2, fm_byte_mul(X0, 2, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(X0, 3, a.y, n.y));
+        b1 = __fadd_rn(b1, fm_byte_mul(X1, 0, a.y, n.y)); b2 = __fadd_rn(b2, fm_byte_mul(X1, 1, a.y, n.y));
+        b0 = __fadd_rn(b0, fm_byte_mul(X1, 2, a.z, n.z)); b1 = __fadd_rn(b1, fm_byte_mul(X1, 3, a.z, n.z));
+        b2 = __fadd_rn(b2, fm_byte_mul(X2, 0, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(X2, 1, a.w, n.w));
+        b1 = __fadd_rn(b1, fm_byte_mul(X2, 2, a.w, n.w)); b2 = __fadd_rn(b2, fm_byte_mul(X2, 3, a.w, n.w));
     }
 }
 
@@ -174,8 +140,8 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
     constexpr int NT = RR_THREADS + 32;
 
     if (tid == 0) {
-        rr_mbar_init(&bars[0], 1);
-        rr_mbar_init(&bars[1], 1);
+        fm_mbar_init(&bars[0], 1);
+        fm_mbar_init(&bars[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     }
@@ -184,11 +150,11 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
         // =========================== phase 1: one source row per thread ===========================
         const bool rowlive = (tid & ~31) < nrows;           // warp-uniform: this warp holds rows of the band
         for (int i = 0; i < nch; i++) {
-            rr_mbar_wait(&bars[i & 1], (i >> 1) & 1);
+            fm_mbar_wait(&bars[i & 1], (i >> 1) & 1);
             if (i >= 2) rr_bar_sync(3 + (i & 1), NT);       // phase 2 of chunk i - 2 has consumed this hs buffer
             const int dx0 = dxa + i * CX, cxn = min(CX, dxb - dx0);
             if (rowlive) {
-                const uint32_t myrow = rr_smem_u32(stage) + (uint32_t)(i & 1) * p.stage_stride + (uint32_t)min(tid, p.NR - 1) * BW;
+                const uint32_t myrow = fm_smem_u32(stage) + (uint32_t)(i & 1) * p.stage_stride + (uint32_t)min(tid, p.NR - 1) * BW;
                 float *hw = hs + (i & 1) * hsbuf + tid;
                 int4 cnext = __ldg(p.coltab + dx0);
 #pragma unroll 1
@@ -227,8 +193,8 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
     for (int i = lane; i < ytn; i += 32) yw[i] = __ldg(p.ywt + yb + i);
     const uint32_t box_bytes = (uint32_t)p.NR * (uint32_t)BW;
     auto issue = [&](int i) {                 // chunk i of the segment -> stage i & 1 (rows past the image are zero-filled)
-        rr_mbar_expect_tx(&bars[i & 1], box_bytes);
-        rr_tma_load_4d(stage + (size_t)(i & 1) * p.stage_stride, &tmap, &bars[i & 1], __ldg(p.cstartw + ch0 + i), R0, t, s);
+        fm_mbar_expect_tx(&bars[i & 1], box_bytes);
+        fm_tma_load_4d(stage + (size_t)(i & 1) * p.stage_stride, &tmap, &bars[i & 1], __ldg(p.cstartw + ch0 + i), R0, t, s);
     };
     if (lane == 0) {
         issue(0);
@@ -263,7 +229,7 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
         const int dyl = i / dxun, dxo = i - dyl * dxun;
         const unsigned char *q = bgr + (dyl * DXU + dxo) * 3;
         p.gray[((size_t)f * p.h + dy0 + dyl) * p.w + dxa + dxo] =
-            (uint8_t)((3735u * q[0] + 19235u * q[1] + 9798u * q[2] + 16384u) >> 15);
+            (uint8_t)fm_gray(q[0], q[1], q[2]);
     }
 }
 
@@ -426,30 +392,15 @@ int fm_rows_plan_describe(int W, int w, int h, const int *xstart, const int *xid
     return FM_OK;
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                    const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-PFN_encodeTiled fm_tma_encoder();
-
 bool fm_rows_usable(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride) {
     return c->rows && ((((uintptr_t)frames) | sstride | fstride) & 15) == 0;
 }
 
 int fm_launch_resize_rows(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
     const RowsPlan *r = c->rows;
-    PFN_encodeTiled enc = fm_tma_encoder();
-    if (!enc) { fm_set_error("cuTensorMapEncodeTiled not available"); return FM_ECUDA; }
-    // the call's frames as a 4-D u32 tensor: (W*3/4 words, H rows, T frames, S streams)
     CUtensorMap tmap;
-    cuuint64_t dims[4] = {(cuuint64_t)c->W * 3 / 4, (cuuint64_t)c->H, (cuuint64_t)T, (cuuint64_t)c->S};
-    cuuint64_t strides[3] = {(cuuint64_t)c->W * 3, (cuuint64_t)(T > 1 ? fstride : (size_t)c->W * 3 * c->H),
-                             (cuuint64_t)(c->S > 1 ? sstride : (T > 1 ? fstride * T : (size_t)c->W * 3 * c->H))};
-    cuuint32_t box[4] = {(cuuint32_t)(r->BW / 4), (cuuint32_t)r->NR, 1, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult cr = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, (void *)frames, dims, strides, box, estr,
-                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) { fm_set_error("cuTensorMapEncodeTiled failed (%d)", (int)cr); return FM_ECUDA; }
+    int rc = fm_frames_tmap(c, frames, sstride, fstride, T, r->BW / 4, r->NR, &tmap);
+    if (rc) return rc;
     RowsParams p;
     p.T = T; p.w = c->w; p.h = c->h;
     p.D = r->D; p.NR = r->NR; p.NRp = r->NRp; p.CX = r->CX; p.NCHU = r->NCHU; p.BW = r->BW;

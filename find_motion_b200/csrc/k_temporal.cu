@@ -10,23 +10,9 @@
 // One lane owns 16 consecutive pixels; a warp owns a 512-pixel tile.  The background tile is
 // stored [8][32] double2 so that every 128-bit access of the warp is one contiguous 512 B run.
 
-__device__ __forceinline__ double fm_u8_to_f64(uint32_t v) {
-    // exact: 2^52 + v, minus 2^52 (avoids the slow I2F.F64 conversion)
-    return __hiloint2double(0x43300000, (int)v) - 4503599627370496.0;
-}
-
-__device__ __forceinline__ uint32_t fm_bg8(double bg) {
-    float f = fabsf(__double2float_rn(bg));        // double -> float32 first (A.7)
-    f = fminf(f, 255.0f);
-    // rne to integer through the 1.5*2^23 trick (f in [0, 255])
-    return __float_as_uint(__fadd_rn(f, 12582912.0f)) & 0x1FFu;
-}
-
 // One frame of one lane: 16 pixels (bytes of px[4]) -> 16 threshold bits (bit j = pixel j), background updated.
-// TAIL: the lane holds the N mod 16 remainder group (A.6: the product order of the AVX2 tail);
-// SAFE: alpha in [0, 1] and threshold >= 0, so bg stays in [0, 255] (no fabs / saturation) and
-//       rn(blur * alpha) = fma(2^52 + blur, alpha, -(2^52 * alpha)) exactly (no int -> double conversion);
-// INIT: first frame of the stream (ref_frame = blur.astype(float)).
+// TAIL: the lane holds the N mod 16 remainder group (A.6: the product order of the AVX2 tail, any alpha and threshold);
+// SAFE, INIT: as in fm_temporal_px.
 template <bool TAIL, bool SAFE, bool INIT>
 __device__ __forceinline__ uint32_t fm_temporal16(const uint32_t (&px)[4], double (&b)[16], int threshold, double alpha,
                                                   double beta) {
@@ -37,21 +23,15 @@ __device__ __forceinline__ uint32_t fm_temporal16(const uint32_t (&px)[4], doubl
 #pragma unroll
     for (int j = 0; j < 16; j++) {
         const uint32_t src = __byte_perm(px[j >> 2], 0, 0x4440 + (j & 3));
-        if (SAFE && !TAIL) {
-            const double X = __hiloint2double(0x43300000, (int)src);
-            if (INIT) b[j] = X - 4503599627370496.0;
-            const int q = __float_as_int(__fadd_rn(__double2float_rn(b[j]), 12582912.0f));     // 0x4B400000 + bg8
-            // bits = 2 * bits + (|bg8 - blur| > threshold): q - qoff - src in [0, 2 thr] unless above the threshold
-            asm("{\n .reg .u32 t;\n add.cc.u32 t, %1, %2;\n addc.u32 %0, %0, %0;\n}"
-                : "+r"(bits) : "r"((uint32_t)(q - qoff - (int)src)), "r"(nthr2));
-            b[j] = __fma_rn(b[j], beta, __fma_rn(X, alpha, nC));
-        } else {
+        if (TAIL) {
             const double sd = fm_u8_to_f64(src);
             if (INIT) b[j] = sd;
             int d = (int)src - (int)fm_bg8(b[j]);
             d = d < 0 ? -d : d;
             bits = 2u * bits + (d > threshold ? 1u : 0u);
-            b[j] = TAIL ? __fma_rn(sd, alpha, __dmul_rn(b[j], beta)) : __fma_rn(b[j], beta, __dmul_rn(sd, alpha));
+            b[j] = __fma_rn(sd, alpha, __dmul_rn(b[j], beta));
+        } else {
+            fm_temporal_px<SAFE, INIT>(src, b[j], bits, threshold, qoff, nthr2, alpha, beta, nC);
         }
     }
     return __brev(bits) >> 16;          // pixel 0 was pushed first

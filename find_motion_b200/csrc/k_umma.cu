@@ -40,30 +40,6 @@
 #define UB_BOFF 224
 #define UB_SMEM (2 * UB_GSTAGE + 2 * UB_PLANE + UB_BROWS * 32 + 1024 /* alignment */ + 64)
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                    const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-PFN_encodeTiled fm_tma_encoder();     // k_fused.cu
-int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);   // k_frontend.cu
-
-__device__ __forceinline__ uint32_t usmem(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void ub_mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(usmem(bar)), "r"(count));
-}
-__device__ __forceinline__ void ub_mbar_expect(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(usmem(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void ub_mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n.reg .pred p;\nUB_WAIT:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n@p bra UB_DONE;\nbra UB_WAIT;\nUB_DONE:\n}\n"
-        ::"r"(usmem(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void ub_tma_4d(void *dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, int c2, int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-        ::"r"(usmem(dst)), "l"(map), "r"(usmem(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
 // shared-memory matrix descriptors (sm_100 version bit set): K-major, no swizzle (LBO = stride of the two 16-byte K
 // chunks, SBO = stride of 8-row groups) and K-major SWIZZLE_128B (rows of 128 bytes, SBO = 1024)
 __device__ __forceinline__ uint64_t ub_desc_plain(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
@@ -80,7 +56,7 @@ __device__ __forceinline__ void ub_mma(uint32_t d_tmem, uint64_t adesc, uint64_t
         ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(0u) : "memory");
 }
 __device__ __forceinline__ void ub_commit(uint64_t *bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(usmem(bar)) : "memory");
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(fm_smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void ub_ld16(uint32_t taddr, uint32_t (&r)[16]) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
@@ -171,7 +147,7 @@ __device__ __forceinline__ uint32_t ub_epilogue(uint32_t tLo16, uint32_t tHi16, 
 #pragma unroll
         for (int wd = 0; wd < 4; wd++) {
             const uint32_t m4 = (M >> (4 * wd)) & 0xFu;
-            ow[wd] &= ~(((m4 * 0x00204081u) & 0x01010101u) * 0xFFu);              // masked pixels -> 0
+            ow[wd] = fm_clear_masked4(ow[wd], m4);
         }
         *reinterpret_cast<uint4 *>(blur_px) = o;
     }
@@ -184,22 +160,8 @@ __device__ __forceinline__ uint32_t ub_epilogue(uint32_t tLo16, uint32_t tHi16, 
             const int i = 2 * k + hlf;
             uint32_t sv = __byte_perm(Uu[k], 0, hlf ? 0x4443 : 0x4441);
             if (MASKED && (M & (1u << i))) sv = 0;                               // mask_off_areas paints BLACK into blur
-            if (SAFE) {
-                const double X = __hiloint2double(0x43300000, (int)sv);          // 2^52 + blur
-                if (init) bg[i] = X - 4503599627370496.0;                        // ref_frame = blur.astype(float)
-                const int q = __float_as_int(__fadd_rn(__double2float_rn(bg[i]), 12582912.0f));
-                // bits = 2 bits + (|bg8 - blur| > threshold): q - qoff - blur in [0, 2 thr] unless above the threshold
-                asm("{\n .reg .u32 t;\n add.cc.u32 t, %1, %2;\n addc.u32 %0, %0, %0;\n}" : "+r"(bits) : "r"((uint32_t)(q - p.qoff - (int)sv)), "r"(nthr2));
-                bg[i] = __fma_rn(bg[i], p.beta, __fma_rn(X, p.alpha, p.nC));     // fma(bg, 1 - a, rn(blur * a))
-            } else {
-                const double sd = __hiloint2double(0x43300000, (int)sv) - 4503599627370496.0;
-                if (init) bg[i] = sd;
-                const float f = fminf(fabsf(__double2float_rn(bg[i])), 255.0f);
-                const int b8 = __float_as_int(__fadd_rn(f, 12582912.0f)) & 0x1FF;
-                const int d = (int)sv - b8;
-                bits = 2u * bits + ((d < 0 ? -d : d) > p.threshold ? 1u : 0u);
-                bg[i] = __fma_rn(bg[i], p.beta, __dmul_rn(sd, p.alpha));
-            }
+            if (init) bg[i] = fm_u8_to_f64(sv);           // ref_frame = blur.astype(float); init is a run-time flag here
+            fm_temporal_px<SAFE, false>(sv, bg[i], bits, p.threshold, p.qoff, nthr2, p.alpha, p.beta, p.nC);
         }
     }
     return __brev(bits) >> 16;          // pixel 0 was pushed first
@@ -240,15 +202,15 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_blur(const __grid_consta
     for (int i = tid; i < UB_BROWS * 32 / 16; i += UB_THREADS)
         reinterpret_cast<uint4 *>(sBand)[i] = __ldg(reinterpret_cast<const uint4 *>(p.band) + i);
     if (tid == 0) {
-        ub_mbar_init(&bars[0], 1);
-        ub_mbar_init(&bars[1], 1);
-        ub_mbar_init(&bars[2], 1);
-        ub_mbar_init(&bars[3], 1);
-        ub_mbar_init(&bars[4], 1);
+        fm_mbar_init(&bars[0], 1);
+        fm_mbar_init(&bars[1], 1);
+        fm_mbar_init(&bars[2], 1);
+        fm_mbar_init(&bars[3], 1);
+        fm_mbar_init(&bars[4], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(usmem(tmem_slot)), "r"(512u) : "memory");
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(fm_smem_u32(tmem_slot)), "r"(512u) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // the band (generic-proxy writes) is read by the MMAs
@@ -280,16 +242,16 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_blur(const __grid_consta
 
     const uint32_t idesc1 = (2u << 4) | ((uint32_t)(UB_IN >> 3) << 17) | ((128u >> 4) << 24);      // S32 += U8 x U8, M128, N224
     const uint32_t idesc2 = (2u << 4) | ((uint32_t)(256 >> 3) << 17) | ((128u >> 4) << 24);        // N256: both byte planes
-    const uint32_t aBand = usmem(sBand), aGray = usmem(sGray), aLo = usmem(sLo), aHi = usmem(sHi);
+    const uint32_t aBand = fm_smem_u32(sBand), aGray = fm_smem_u32(sGray), aLo = fm_smem_u32(sLo), aHi = fm_smem_u32(sHi);
     auto issue_tma = [&](int t) {                 // thread 0
         uint64_t *bar = &bars[t & 1];
         unsigned char *dst = sGray + (t & 1) * UB_GSTAGE;
-        ub_mbar_expect(bar, UB_GSTAGE);
-        ub_tma_4d(dst, &tmap, bar, X0, Y0, t, s);
-        ub_tma_4d(dst + UB_IN * 128, &tmap, bar, X0 + 128, Y0, t, s);
+        fm_mbar_expect_tx(bar, UB_GSTAGE);
+        fm_tma_load_4d(dst, &tmap, bar, X0, Y0, t, s);
+        fm_tma_load_4d(dst + UB_IN * 128, &tmap, bar, X0 + 128, Y0, t, s);
     };
     auto issue_mma1 = [&](int t) {                // thread 0: horizontal pass of frame t into D1
-        ub_mbar_wait(&bars[t & 1], (t >> 1) & 1);
+        fm_mbar_wait(&bars[t & 1], (t >> 1) & 1);
         UB_FENCE_AFTER();
         const uint32_t g = aGray + (t & 1) * UB_GSTAGE;
 #pragma unroll
@@ -312,7 +274,7 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_blur(const __grid_consta
     if (p.prof && tid < 32) prof_acc[tid] = 0;
     long long prof_t = clock64();
     for (int t = 0; t < Ts; t++) {
-        ub_mbar_wait(&bars[2], t & 1);            // D1 of frame t is complete (and gray stage t & 1 has been read)
+        fm_mbar_wait(&bars[2], t & 1);            // D1 of frame t is complete (and gray stage t & 1 has been read)
         UB_FENCE_AFTER();
         UB_PROF(0);
         if (tid == 0 && t + 1 < Ts) issue_tma(t + 1);
@@ -335,7 +297,7 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_blur(const __grid_consta
             if (t + 1 < Ts) issue_mma1(t + 1);    // runs on the tensor pipe under the epilogue below
         }
         UB_PROF(5);
-        ub_mbar_wait(&bars[3], t & 1);
+        fm_mbar_wait(&bars[3], t & 1);
         UB_FENCE_AFTER();
         UB_PROF(6);
         uint8_t *bo = (p.blur_out && ok) ? p.blur_out + (((size_t)s * p.T + t) * p.h + py) * p.w + px : nullptr;
@@ -354,17 +316,6 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_blur(const __grid_consta
     __syncthreads();
     if (p.prof && tid < 32 && blockIdx.x == p.tilesX + 1 && blockIdx.y == 0) p.prof[tid] += prof_acc[tid];
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512u) : "memory");
-}
-
-__device__ __forceinline__ uint32_t ub_gray1(const uint8_t *q) { return (3735u * q[0] + 19235u * q[1] + 9798u * q[2] + 16384u) >> 15; }
-__device__ __forceinline__ uint32_t ub_gray4(uint32_t w0, uint32_t w1, uint32_t w2) {
-    const uint32_t C_BG = 7470u | (38470u << 16), C_R = 19596u;
-    const uint32_t C_xB = 7470u << 16, C_GR = 38470u | (19596u << 16);
-    uint32_t t0 = __dp2a_hi(C_R, w0, __dp2a_lo(C_BG, w0, 32768u));
-    uint32_t t1 = __dp2a_hi(C_xB, w0, __dp2a_lo(C_GR, w1, 32768u));
-    uint32_t t2 = __dp2a_hi(C_BG, w1, __dp2a_lo(C_R, w2, 32768u));
-    uint32_t t3 = __dp2a_hi(C_GR, w2, __dp2a_lo(C_xB, w2, 32768u));
-    return __byte_perm(__byte_perm(t0, t1, 0x0062), __byte_perm(t2, t3, 0x0062), 0x5410);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -427,13 +378,13 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
     for (int i = tid; i < G::BROWS * 32 / 16; i += UB_THREADS)
         reinterpret_cast<uint4 *>(sBand)[i] = __ldg(reinterpret_cast<const uint4 *>(p.band) + i);
     if (tid == 0) {
-        ub_mbar_init(&bars[0], 1);
-        ub_mbar_init(&bars[1], 1);
-        for (int i = 0; i < G::NST; i++) ub_mbar_init(&rbar[i], 1);
+        fm_mbar_init(&bars[0], 1);
+        fm_mbar_init(&bars[1], 1);
+        for (int i = 0; i < G::NST; i++) fm_mbar_init(&rbar[i], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(usmem(tmem_slot)), "r"(512u) : "memory");
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(fm_smem_u32(tmem_slot)), "r"(512u) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -464,7 +415,7 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
 
     const uint32_t idesc1 = (2u << 4) | ((uint32_t)(G::IN >> 3) << 17) | ((128u >> 4) << 24);
     const uint32_t idesc2 = (2u << 4) | ((uint32_t)(256 >> 3) << 17) | ((128u >> 4) << 24);        // N256: both byte planes
-    const uint32_t aBand = usmem(sBand), aGray = usmem(sGray), aLo = usmem(sLo), aHi = usmem(sHi);
+    const uint32_t aBand = fm_smem_u32(sBand), aGray = fm_smem_u32(sGray), aLo = fm_smem_u32(sLo), aHi = fm_smem_u32(sHi);
 
     // rows / columns of the gray tile that meet non-zero taps: tile row p <-> image row Y0 - RA + p
     const int p_lo = RA - r, p_hi = RA + TH + r;                   // [p_lo, p_hi)
@@ -477,14 +428,14 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
     auto issue_raw = [&](int g) {                 // thread 0
         const int t = g / NCH, c = g - t * NCH;
         uint64_t *bar = &rbar[g % G::NST];
-        ub_mbar_expect(bar, G::RSTAGE);
-        ub_tma_4d(sRaw + (g % G::NST) * G::RSTAGE, &tmap, bar, cx, Y0 - r + G::RC * c, t, s);
+        fm_mbar_expect_tx(bar, G::RSTAGE);
+        fm_tma_load_4d(sRaw + (g % G::NST) * G::RSTAGE, &tmap, bar, cx, Y0 - r + G::RC * c, t, s);
     };
     // BGR -> gray of frame t into the swizzled tile (all threads), chunk by chunk; re-arms the ring as stages drain
     auto convert = [&](int t) {
         for (int c = 0; c < NCH; c++) {
             const int g = t * NCH + c;
-            ub_mbar_wait(&rbar[g % G::NST], (g / G::NST) & 1);
+            fm_mbar_wait(&rbar[g % G::NST], (g / G::NST) & 1);
             const unsigned char *raw = sRaw + (g % G::NST) * G::RSTAGE;
             const int nun = u_hi - u_lo;
             for (int u = tid; u < G::RC * nun; u += UB_THREADS) {
@@ -494,10 +445,10 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
                     const uint4 *src = reinterpret_cast<const uint4 *>(raw + rr * G::RB + 48 * uu);
                     const uint4 a = src[0], b = src[1], d = src[2];
                     uint4 o;
-                    o.x = ub_gray4(a.x, a.y, a.z);
-                    o.y = ub_gray4(a.w, b.x, b.y);
-                    o.z = ub_gray4(b.z, b.w, d.x);
-                    o.w = ub_gray4(d.y, d.z, d.w);
+                    o.x = fm_gray4(a.x, a.y, a.z);
+                    o.y = fm_gray4(a.w, b.x, b.y);
+                    o.z = fm_gray4(b.z, b.w, d.x);
+                    o.w = fm_gray4(d.y, d.z, d.w);
                     *reinterpret_cast<uint4 *>(sGray + (uu >> 3) * (G::IN * 128) + pr * 128 + (((uu & 7) ^ (pr & 7)) << 4)) = o;
                 }
             }
@@ -560,7 +511,7 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
     const int yq_lo = p_lo >> 4, yq_hi = (p_hi + 15) >> 4;        // 16-row chunks of the horizontal sums that meet non-zero taps
 
     for (int t = 0; t < Ts; t++) {
-        ub_mbar_wait(&bars[0], t & 1);            // D1 of frame t is complete, the gray tile is free
+        fm_mbar_wait(&bars[0], t & 1);            // D1 of frame t is complete, the gray tile is free
         UB_FENCE_AFTER();
         ub_split<G::NU>(tD1 + lanebase, sLo, sHi, xl, rg, yq_lo, yq_hi);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -578,7 +529,7 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
             convert(t + 1);
             if (tid == 0) issue_mma1();           // ... and its horizontal pass under the epilogue below
         }
-        ub_mbar_wait(&bars[1], t & 1);
+        fm_mbar_wait(&bars[1], t & 1);
         UB_FENCE_AFTER();
         uint8_t *bo = (p.blur_out && ok) ? p.blur_out + (((size_t)s * p.T + t) * p.h + py) * p.w + px : nullptr;
         ub_frame_out<SAFE>(tLo + lanebase + 16 * rg, tHi + lanebase + 16 * rg, bg, M, ok, t == 0 && !has_bg, masked, p, th16, bo,
@@ -616,7 +567,7 @@ __global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ sr
         if (x >= 0 && x + 3 < w && aligned4) {
             if (BGR) {
                 const uint32_t *q = reinterpret_cast<const uint32_t *>(row + 3 * x);
-                out = ub_gray4(__ldg(q), __ldg(q + 1), __ldg(q + 2));
+                out = fm_gray4(__ldg(q), __ldg(q + 1), __ldg(q + 2));
             } else {
                 out = __ldg(reinterpret_cast<const uint32_t *>(row + x));
             }
@@ -625,7 +576,7 @@ __global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ sr
             for (int b = 0; b < 4; b++) {
                 if (xp + b < w + 2 * UB_PAD) {
                     const int xx = fm_reflect101(x + b, w);
-                    out |= (BGR ? ub_gray1(row + 3 * xx) : (uint32_t)row[xx]) << (8 * b);
+                    out |= (BGR ? fm_gray(row[3 * xx], row[3 * xx + 1], row[3 * xx + 2]) : (uint32_t)row[xx]) << (8 * b);
                 }
             }
         }
@@ -750,10 +701,6 @@ extern "C" void fm_umma_prof_dump(void) {
 
 // full-resolution mode, BGR frames straight into the tcgen05 kernel
 static int launch_umma_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
-    if ((((uintptr_t)frames) & 15) || (sstride & 15) || (fstride & 15)) {
-        fm_set_error("the tcgen05 front end needs 16-byte aligned frames and strides (TMA)");
-        return FM_EINVAL;
-    }
     int tilesX, tilesY, Wp, Hp;
     umma_geom(c, &tilesX, &tilesY, &Wp, &Hp);
     if (c->cfg.flags & FM_FLAG_KEEP_PLANES) {              // parity tap of the gray conversion
@@ -762,14 +709,8 @@ static int launch_umma_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, s
     }
     const int RA = c->umma_ra;
     CUtensorMap tmap;
-    cuuint64_t dims[4] = {(cuuint64_t)c->W * 3 / 4, (cuuint64_t)c->H, (cuuint64_t)T, (cuuint64_t)c->S};
-    cuuint64_t strides[3] = {(cuuint64_t)c->W * 3, (cuuint64_t)fstride, (cuuint64_t)(c->S > 1 ? sstride : fstride * T)};
-    cuuint32_t box[4] = {(cuuint32_t)(3 * (UB_T + 2 * RA) / 4), (cuuint32_t)(RA == 16 ? UfGeom<16>::RC : UfGeom<48>::RC), 1, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = fm_tma_encoder()(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, (void *)frames, dims, strides, box, estr,
-                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { fm_set_error("cuTensorMapEncodeTiled (BGR frames) failed (%d)", (int)r); return FM_ECUDA; }
+    int rc = fm_frames_tmap(c, frames, sstride, fstride, T, 3 * (UB_T + 2 * RA) / 4, RA == 16 ? UfGeom<16>::RC : UfGeom<48>::RC, &tmap);
+    if (rc) return rc;
     UfParams q;
     umma_params(c, T, tilesX, tilesY, q.u);
     q.u.band = c->uband_f;

@@ -34,52 +34,9 @@
 #define WV_NT 4            // column tiles per pass-2 CTA (cp.async double buffer)
 #define WT_COLS 16         // columns of a k_wide_vt CTA
 
-__device__ __forceinline__ uint32_t wsmem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void wldsm_x4(uint32_t addr, uint32_t (&r)[4]) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void wimma(int (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0,
-                                      uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+r"(d[0]), "+r"(d[1]), "+r"(d[2]), "+r"(d[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-// first step of a chain: D = A * B + c (the same constant in all four lanes)
-__device__ __forceinline__ void wimma0(int (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0,
-                                       uint32_t b1, int c) {
-    asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.u8.u8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%10,%10,%10,%10};"
-                 : "=r"(d[0]), "=r"(d[1]), "=r"(d[2]), "=r"(d[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1), "r"(c));
-}
 __device__ __forceinline__ void wcp_async16(uint32_t dst, const void *src, bool valid) {
     const int n = valid ? 16 : 0;                 // src-size 0: the 16 bytes are zero-filled
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(n) : "memory");
-}
-
-// mbarrier + TMA primitives (sm_100a PTX) of the TMA-staged pass 1
-__device__ __forceinline__ void wmbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(wsmem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void wmbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(wsmem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void wmbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WH_WAIT_LOOP:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra WH_WAIT_DONE;\n"
-        "bra WH_WAIT_LOOP;\n"
-        "WH_WAIT_DONE:\n"
-        "}\n" ::"r"(wsmem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void wtma_load_4d(uint32_t dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, int c2, int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-        ::"r"(dst), "l"(map), "r"(wsmem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
 }
 
 struct WideGeom {
@@ -166,20 +123,6 @@ __device__ __forceinline__ int wrow(int i, int n) {
     return (j >= 0 && j < n) ? j : fm_reflect101(i, n);
 }
 
-__device__ __forceinline__ uint32_t wgray1(const uint8_t *p) {
-    return (3735u * p[0] + 19235u * p[1] + 9798u * p[2] + 16384u) >> 15;
-}
-__device__ __forceinline__ uint32_t wgray4(uint32_t w0, uint32_t w1, uint32_t w2) {
-    // 4 BGR pixels in 3 words -> 4 gray bytes (two IDP.2A per pixel on doubled coefficients; Y is byte 2 of the sum)
-    const uint32_t C_BG = 7470u | (38470u << 16), C_R = 19596u;
-    const uint32_t C_xB = 7470u << 16, C_GR = 38470u | (19596u << 16);
-    uint32_t t0 = __dp2a_hi(C_R, w0, __dp2a_lo(C_BG, w0, 32768u));
-    uint32_t t1 = __dp2a_hi(C_xB, w0, __dp2a_lo(C_GR, w1, 32768u));
-    uint32_t t2 = __dp2a_hi(C_BG, w1, __dp2a_lo(C_R, w2, 32768u));
-    uint32_t t3 = __dp2a_hi(C_GR, w2, __dp2a_lo(C_xB, w2, 32768u));
-    return __byte_perm(__byte_perm(t0, t1, 0x0062), __byte_perm(t2, t3, 0x0062), 0x5410);
-}
-
 // BORDER_REFLECT_101 columns of a staged window from their mirror images inside the window (one reflection)
 __device__ __forceinline__ void wide_h_mirror(unsigned char *tile, int X0, int w, int r, int R16, int pitch) {
     const int tid = threadIdx.x;
@@ -223,10 +166,10 @@ __device__ __forceinline__ void wide_h_stage(unsigned char *tile, const uint8_t 
 #pragma unroll
                 for (int i = 0; i < 4; i++) {
                     uint4 o;
-                    o.x = wgray4(raw[i][0].x, raw[i][0].y, raw[i][0].z);
-                    o.y = wgray4(raw[i][0].w, raw[i][1].x, raw[i][1].y);
-                    o.z = wgray4(raw[i][1].z, raw[i][1].w, raw[i][2].x);
-                    o.w = wgray4(raw[i][2].y, raw[i][2].z, raw[i][2].w);
+                    o.x = fm_gray4(raw[i][0].x, raw[i][0].y, raw[i][0].z);
+                    o.y = fm_gray4(raw[i][0].w, raw[i][1].x, raw[i][1].y);
+                    o.z = fm_gray4(raw[i][1].z, raw[i][1].w, raw[i][2].x);
+                    o.w = fm_gray4(raw[i][2].y, raw[i][2].z, raw[i][2].w);
                     *reinterpret_cast<uint4 *>(tile + (wq + 8 * i) * pitch + 16 * u) = o;
                 }
             } else if (!mirror) {
@@ -234,7 +177,7 @@ __device__ __forceinline__ void wide_h_stage(unsigned char *tile, const uint8_t 
                 for (int b = 0; b < 16; b++) {
                     const int xx = 3 * fm_reflect101(x + b, w);
 #pragma unroll
-                    for (int i = 0; i < 4; i++) tile[(wq + 8 * i) * pitch + 16 * u + b] = (unsigned char)wgray1(rp[i] + xx);
+                    for (int i = 0; i < 4; i++) tile[(wq + 8 * i) * pitch + 16 * u + b] = (unsigned char)fm_gray(rp[i][xx], rp[i][xx + 1], rp[i][xx + 2]);
                 }
             }
         }
@@ -271,20 +214,20 @@ __device__ __forceinline__ void wide_h_products(const unsigned char *tile, const
     const int lane = threadIdx.x & 31, wq = threadIdx.x >> 5;
     if (X0 + 32 * wq >= w) return;                            // this warp's 32 columns are outside the image
     int acc[2][4][4];
-    const uint32_t abase = wsmem_u32(tile) + ((lane & 7) + 8 * ((lane >> 3) & 1)) * pitch + 32 * wq + 16 * (lane >> 4);
+    const uint32_t abase = fm_smem_u32(tile) + ((lane & 7) + 8 * ((lane >> 3) & 1)) * pitch + 32 * wq + 16 * (lane >> 4);
     auto step = [&](int s, auto first) {
         uint32_t a0[4], a1[4];
-        wldsm_x4(abase + 32 * s, a0);
-        wldsm_x4(abase + 32 * s + 16 * pitch, a1);
+        fm_ldsm_x4(abase + 32 * s, a0);
+        fm_ldsm_x4(abase + 32 * s + 16 * pitch, a1);
 #pragma unroll
         for (int nb = 0; nb < 4; nb++) {
             const uint2 b = tab[(4 * s - nb + 3) * 32 + lane];
             if (decltype(first)::value) {
-                wimma0(acc[0][nb], a0[0], a0[1], a0[2], a0[3], b.x, b.y, 0);
-                wimma0(acc[1][nb], a1[0], a1[1], a1[2], a1[3], b.x, b.y, 0);
+                fm_imma0(acc[0][nb], a0[0], a0[1], a0[2], a0[3], b.x, b.y, 0);
+                fm_imma0(acc[1][nb], a1[0], a1[1], a1[2], a1[3], b.x, b.y, 0);
             } else {
-                wimma(acc[0][nb], a0[0], a0[1], a0[2], a0[3], b.x, b.y);
-                wimma(acc[1][nb], a1[0], a1[1], a1[2], a1[3], b.x, b.y);
+                fm_imma(acc[0][nb], a0[0], a0[1], a0[2], a0[3], b.x, b.y);
+                fm_imma(acc[1][nb], a1[0], a1[1], a1[2], a1[3], b.x, b.y);
             }
         }
     };
@@ -352,12 +295,12 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_const
     const int Gbeg = blockIdx.y * gp, Gend = min(Gbeg + gp, NGa);
     auto interior = [&](int G) { return 32 * G - r >= 0 && 32 * G - r + 32 <= h; };    // CTA-uniform
     auto issue = [&](int G) {                  // one thread
-        wmbar_expect_tx(bar, (uint32_t)(nbox * boxbytes));
+        fm_mbar_expect_tx(bar, (uint32_t)(nbox * boxbytes));
         const int c0 = (3 * (X0 - R16)) / 4;                                 // u32 column (negative / past the row: zero-filled)
-        for (int b = 0; b < nbox; b++) wtma_load_4d(wsmem_u32(raw) + b * boxbytes, &tmap, bar, c0 + b * ubox * 12, 32 * G - r, f % T, f / T);
+        for (int b = 0; b < nbox; b++) fm_tma_load_4d(fm_smem_u32(raw) + b * boxbytes, &tmap, bar, c0 + b * ubox * 12, 32 * G - r, f % T, f / T);
     };
     if (tid == 0) {
-        wmbar_init(bar, 1);
+        fm_mbar_init(bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         if (interior(Gbeg)) issue(Gbeg);
@@ -370,7 +313,7 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_const
     for (int G = Gbeg; G < Gend; G++) {
         const bool more = G + 1 < Gend && interior(G + 1);
         if (interior(G)) {
-            wmbar_wait(bar, phase);
+            fm_mbar_wait(bar, phase);
             phase ^= 1;
             for (int u = tid; u < 32 * nunits; u += WH_THREADS) {
                 const int rr = (int)(((uint32_t)u * inv) >> 16), j = u - rr * nunits;
@@ -380,10 +323,10 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_const
                 const uint4 *q = reinterpret_cast<const uint4 *>(raw + jb * boxbytes + rr * (ubox * 48) + (j - jb * ubox) * 48);
                 const uint4 r0 = q[0], r1 = q[1], r2 = q[2];
                 uint4 o;
-                o.x = wgray4(r0.x, r0.y, r0.z);
-                o.y = wgray4(r0.w, r1.x, r1.y);
-                o.z = wgray4(r1.z, r1.w, r2.x);
-                o.w = wgray4(r2.y, r2.z, r2.w);
+                o.x = fm_gray4(r0.x, r0.y, r0.z);
+                o.y = fm_gray4(r0.w, r1.x, r1.y);
+                o.z = fm_gray4(r1.z, r1.w, r2.x);
+                o.w = fm_gray4(r2.y, r2.z, r2.w);
                 *reinterpret_cast<uint4 *>(tile + rr * pitch + 16 * j) = o;
             }
             __syncthreads();                                                 // raw stage consumed, window written
@@ -425,7 +368,7 @@ __global__ void __launch_bounds__(128, 4) k_wide_v(const uint4 *__restrict__ plo
     // staging: lane = column of the tile, warp = chunk row gh (2 * group + half) modulo 4, both planes
     const uint4 *gsrc = plo + (((size_t)f * NGa + G0) * 2 + wq) * w + XS + lane;
     const size_t pdiff = phi - plo;
-    const uint32_t sdst = wsmem_u32(sB) + (wq * WV_COLS + wv_slot(lane)) * 16;
+    const uint32_t sdst = fm_smem_u32(sB) + (wq * WV_COLS + wv_slot(lane)) * 16;
     const int ghmax = min(2 * NGt, 2 * (NGa - G0));              // chunk rows that exist in the planes
     auto issue = [&](int ct) {
         const bool okx = XS + ct * WV_COLS + lane < w;
@@ -462,14 +405,14 @@ __global__ void __launch_bounds__(128, 4) k_wide_v(const uint4 *__restrict__ plo
         __syncthreads();
         const int X0 = XS + ct * WV_COLS;
         int acc[2][2][4][4];       // [plane][row tile][column block][4]; the low plane starts at the rounding constant
-        const uint32_t sbase = wsmem_u32(sB + (ct & 1) * 2 * per);
+        const uint32_t sbase = fm_smem_u32(sB + (ct & 1) * 2 * per);
         auto step = [&](int s, auto first) {
             uint32_t bq[2][2][4];        // [plane][block pair][4]
 #pragma unroll
             for (int pl = 0; pl < 2; pl++)
 #pragma unroll
                 for (int np = 0; np < 2; np++)
-                    wldsm_x4(sbase + (pl * per + (wq + s) * 2 * WV_COLS) * 16 + boff[np], bq[pl][np]);
+                    fm_ldsm_x4(sbase + (pl * per + (wq + s) * 2 * WV_COLS) * 16 + boff[np], bq[pl][np]);
 #pragma unroll
             for (int mt = 0; mt < 2; mt++) {
                 const uint4 a = tab[(2 * s - mt + 1) * 32 + lane];
@@ -478,8 +421,8 @@ __global__ void __launch_bounds__(128, 4) k_wide_v(const uint4 *__restrict__ plo
 #pragma unroll
                     for (int nb = 0; nb < 4; nb++) {
                         const uint32_t b0 = bq[pl][nb >> 1][2 * (nb & 1)], b1 = bq[pl][nb >> 1][2 * (nb & 1) + 1];
-                        if (decltype(first)::value) wimma0(acc[pl][mt][nb], a.x, a.y, a.z, a.w, b0, b1, pl ? 0 : 32768);
-                        else wimma(acc[pl][mt][nb], a.x, a.y, a.z, a.w, b0, b1);
+                        if (decltype(first)::value) fm_imma0(acc[pl][mt][nb], a.x, a.y, a.z, a.w, b0, b1, pl ? 0 : 32768);
+                        else fm_imma(acc[pl][mt][nb], a.x, a.y, a.z, a.w, b0, b1);
                     }
             }
         };
@@ -511,8 +454,8 @@ __global__ void __launch_bounds__(128, 4) k_wide_v(const uint4 *__restrict__ plo
                     const uint32_t m = __ldg(mp + dy * wpr) >> (8 * t);
                     uint8_t *dst = dp0 + dy * w;
                     // masked pixels -> 0xFF bytes -> cleared
-                    const uint32_t o0 = wd[0] & ~((((m & 0xFu) * 0x00204081u) & 0x01010101u) * 0xFFu);
-                    const uint32_t o1 = wd[1] & ~(((((m >> 4) & 0xFu) * 0x00204081u) & 0x01010101u) * 0xFFu);
+                    const uint32_t o0 = fm_clear_masked4(wd[0], m & 0xFu);
+                    const uint32_t o1 = fm_clear_masked4(wd[1], (m >> 4) & 0xFu);
                     if ((w & 3) == 0) {
                         if (ok0) *reinterpret_cast<uint32_t *>(dst) = o0;
                         if (ok1) *reinterpret_cast<uint32_t *>(dst + 4) = o1;
@@ -555,23 +498,19 @@ struct WideVtParams {
 // 16 consecutive pixels of one row (blur bytes q, unmasked): polygon mask, threshold bits (bit j = pixel j), background update.
 // MASKED: the warp has masked pixels (M bit j = pixel j) or the parity tap is on; INIT: first frame of the stream.
 template <bool INIT, bool MASKED>
-__device__ __forceinline__ uint32_t wt_temporal16(uint4 q, uint32_t M, double (&bg)[16], int qoff, uint32_t nthr2, double alpha,
-                                                  double beta, double nC, uint8_t *blur_px) {
+__device__ __forceinline__ uint32_t wt_temporal16(uint4 q, uint32_t M, double (&bg)[16], int threshold, int qoff, uint32_t nthr2,
+                                                  double alpha, double beta, double nC, uint8_t *blur_px) {
     uint32_t w4[4] = {q.x, q.y, q.z, q.w};
     if (MASKED) {
 #pragma unroll
-        for (int k = 0; k < 4; k++) w4[k] &= ~(((((M >> (4 * k)) & 0xFu) * 0x00204081u) & 0x01010101u) * 0xFFu);   // BLACK into blur
+        for (int k = 0; k < 4; k++) w4[k] = fm_clear_masked4(w4[k], (M >> (4 * k)) & 0xFu);
         if (blur_px) *reinterpret_cast<uint4 *>(blur_px) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
     }
     uint32_t bits = 0;
 #pragma unroll
     for (int i = 0; i < 16; i++) {
         const uint32_t sv = __byte_perm(w4[i >> 2], 0, 0x4440 + (i & 3));
-        const double X = __hiloint2double(0x43300000, (int)sv);                     // 2^52 + blur
-        if (INIT) bg[i] = X - 4503599627370496.0;
-        const int qq = __float_as_int(__fadd_rn(__double2float_rn(bg[i]), 12582912.0f));
-        asm("{\n .reg .u32 t;\n add.cc.u32 t, %1, %2;\n addc.u32 %0, %0, %0;\n}" : "+r"(bits) : "r"((uint32_t)(qq - qoff - (int)sv)), "r"(nthr2));
-        bg[i] = __fma_rn(bg[i], beta, __fma_rn(X, alpha, nC));
+        fm_temporal_px<true, INIT>(sv, bg[i], bits, threshold, qoff, nthr2, alpha, beta, nC);
     }
     return __brev(bits) >> 16;       // bit j = pixel j
 }
@@ -600,7 +539,7 @@ __global__ void __launch_bounds__(128, 5) k_wide_vt(WideVtParams p) {
     const size_t fstride = (size_t)NGa * 2 * w;                               // uint4 per frame and plane
     const uint4 *gsrc = p.plo + ((size_t)s * T * NGa + G0) * 2 * w + (size_t)sgh * w + X0 + scol;
     const size_t pdiff = p.phi - p.plo;
-    const uint32_t sdst = wsmem_u32(sB) + (sgh * WT_COLS + wt_slot(scol)) * 16;
+    const uint32_t sdst = fm_smem_u32(sB) + (sgh * WT_COLS + wt_slot(scol)) * 16;
     const int ghmax = min(2 * NGt, 2 * (NGa - G0));
     auto issue = [&](int t) {
         const uint4 *sp = gsrc + (size_t)t * fstride;
@@ -656,11 +595,11 @@ __global__ void __launch_bounds__(128, 5) k_wide_vt(WideVtParams p) {
         }
         __syncthreads();
         int acc[2][2][2][4];       // [plane][row tile][column block][4]; the low plane starts at the rounding constant
-        const uint32_t sbase = wsmem_u32(sB + (t & 1) * 2 * per);
+        const uint32_t sbase = fm_smem_u32(sB + (t & 1) * 2 * per);
         auto step = [&](int sg, auto first) {
             uint32_t bq[2][4];
 #pragma unroll
-            for (int pl = 0; pl < 2; pl++) wldsm_x4(sbase + (pl * per + (wq + sg) * 2 * WT_COLS) * 16 + boff, bq[pl]);
+            for (int pl = 0; pl < 2; pl++) fm_ldsm_x4(sbase + (pl * per + (wq + sg) * 2 * WT_COLS) * 16 + boff, bq[pl]);
 #pragma unroll
             for (int mt = 0; mt < 2; mt++) {
                 const uint4 a = tab[(2 * sg - mt + 1) * 32 + lane];
@@ -668,8 +607,8 @@ __global__ void __launch_bounds__(128, 5) k_wide_vt(WideVtParams p) {
                 for (int pl = 0; pl < 2; pl++)
 #pragma unroll
                     for (int nb = 0; nb < 2; nb++) {
-                        if (decltype(first)::value) wimma0(acc[pl][mt][nb], a.x, a.y, a.z, a.w, bq[pl][2 * nb], bq[pl][2 * nb + 1], pl ? 0 : 32768);
-                        else wimma(acc[pl][mt][nb], a.x, a.y, a.z, a.w, bq[pl][2 * nb], bq[pl][2 * nb + 1]);
+                        if (decltype(first)::value) fm_imma0(acc[pl][mt][nb], a.x, a.y, a.z, a.w, bq[pl][2 * nb], bq[pl][2 * nb + 1], pl ? 0 : 32768);
+                        else fm_imma(acc[pl][mt][nb], a.x, a.y, a.z, a.w, bq[pl][2 * nb], bq[pl][2 * nb + 1]);
                     }
             }
         };
@@ -691,9 +630,9 @@ __global__ void __launch_bounds__(128, 5) k_wide_vt(WideVtParams p) {
         uint8_t *bo = (p.blur_out && y < h) ? p.blur_out + (((size_t)s * T + t) * h + y) * w + X0 : nullptr;
         asm volatile("" : "+r"(M));        // opaque per frame: keeps the single-bit tests of M from being hoisted
         uint32_t bits;
-        if (t == 0 && !has_bg) bits = wt_temporal16<true, true>(q, M, bg, qoff, nthr2, p.alpha, p.beta, nC, bo);
-        else if (masked) bits = wt_temporal16<false, true>(q, M, bg, qoff, nthr2, p.alpha, p.beta, nC, bo);
-        else bits = wt_temporal16<false, false>(q, M, bg, qoff, nthr2, p.alpha, p.beta, nC, nullptr);
+        if (t == 0 && !has_bg) bits = wt_temporal16<true, true>(q, M, bg, p.threshold, qoff, nthr2, p.alpha, p.beta, nC, bo);
+        else if (masked) bits = wt_temporal16<false, true>(q, M, bg, p.threshold, qoff, nthr2, p.alpha, p.beta, nC, bo);
+        else bits = wt_temporal16<false, false>(q, M, bg, p.threshold, qoff, nthr2, p.alpha, p.beta, nC, nullptr);
         if (y >= h) bits = 0;
         if (y < h) *tw = (uint16_t)bits;
         if (__any_sync(0xffffffffu, bits != 0) && lane == 0) {       // this warp's 32 rows hold something
@@ -736,14 +675,6 @@ int fm_launch_bg_export_wide(fm_ctx *c, int stream, double *dst_dev, cudaStream_
     FM_LAUNCH_CHECK();
     return FM_OK;
 }
-
-typedef CUresult (*PFN_encodeTiledW)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                     const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-PFN_encodeTiledW fm_tma_encoder();      // k_fused.cu
-
-// identity-resize gray plane (parity tap of the fused conversion), defined in k_frontend.cu
-int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
 
 // k = 1: GaussianBlur is the identity, only the polygon masks are painted (find_motion.py:494, 619-635)
 __global__ void __launch_bounds__(256) k_blur_identity(const uint8_t *__restrict__ gray, uint8_t *__restrict__ blur,
@@ -795,18 +726,8 @@ int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t
         const size_t smt = (size_t)nbox * 32 * ubox * 48 + smh + 16;
         static const long tma_kb = getenv("FM_WIDE_TMA_KB") ? atol(getenv("FM_WIDE_TMA_KB")) : 100;
         if (mirror && ubox <= 21 && smt <= (size_t)tma_kb * 1024) {
-            PFN_encodeTiledW enc = fm_tma_encoder();
-            if (!enc) { fm_set_error("cuTensorMapEncodeTiled not available"); return FM_ECUDA; }
-            CUtensorMap tmap;      // the call's frames as a 4-D u32 tensor: (W*3/4 words, H rows, T frames, S streams)
-            cuuint64_t dims[4] = {(cuuint64_t)c->W * 3 / 4, (cuuint64_t)c->H, (cuuint64_t)T, (cuuint64_t)c->S};
-            cuuint64_t strides[3] = {(cuuint64_t)c->W * 3, (cuuint64_t)(T > 1 ? fstride : (size_t)c->W * 3 * c->H),
-                                     (cuuint64_t)(c->S > 1 ? sstride : (T > 1 ? fstride * T : (size_t)c->W * 3 * c->H))};
-            cuuint32_t box[4] = {(cuuint32_t)(ubox * 12), 32, 1, 1};
-            cuuint32_t estr[4] = {1, 1, 1, 1};
-            CUresult cr = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, (void *)frames, dims, strides, box, estr,
-                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (cr != CUDA_SUCCESS) { fm_set_error("cuTensorMapEncodeTiled failed (%d)", (int)cr); return FM_ECUDA; }
+            CUtensorMap tmap;
+            if ((rc = fm_frames_tmap(c, frames, sstride, fstride, T, ubox * 12, 32, &tmap))) return rc;
             if ((rc = fm_ensure_smem((const void *)k_wide_h_tma, smt, c->cfg.device))) return rc;
             static const int gp = getenv("FM_WIDE_GP") ? std::max(1, atoi(getenv("FM_WIDE_GP"))) : 4;     // row groups per CTA (A/B: profiles/r2_wide_ab.txt)
             dim3 tgrid(hgrid.x, (g.NGa + gp - 1) / gp, F);

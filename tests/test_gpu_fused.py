@@ -6,7 +6,7 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 
-def _compare_with_oracle(W, H, n, T, kw, seed, n_streams=1):
+def _compare_with_oracle(W, H, n, T, kw, seed, n_streams=1, no_fused=False):
     import torch
     from find_motion_b200 import synth
     from find_motion_b200.engine import MotionEngine
@@ -14,8 +14,8 @@ def _compare_with_oracle(W, H, n, T, kw, seed, n_streams=1):
     clips = np.stack([synth.make_clip(W, H, n, seed=seed + s, fps=kw.get("fps", 30)) for s in range(n_streams)])
     orcs = [R.StreamOracle(W, H, **kw) for _ in range(n_streams)]
     dev = torch.from_numpy(clips).cuda()
-    with MotionEngine(W, H, n_streams=n_streams, max_frames=T, keep_planes=True, **kw) as eng:
-        assert eng.info["front_end"] == 0, "fused front end expected"
+    with MotionEngine(W, H, n_streams=n_streams, max_frames=T, keep_planes=True, no_fused=no_fused, **kw) as eng:
+        assert eng.info["front_end"] == (1 if no_fused else 0), "fused front end expected unless switched off"
         for t0 in range(0, n, T):
             t1 = min(n, t0 + T)
             stats = eng.process(dev[:, t0:t1])
@@ -51,9 +51,13 @@ def test_fused_kernel_sizes(k, blur_scale):
 
 
 def test_fused_avg_out_of_unit_range_still_exact():
-    """avg > 1 makes the background leave [0, 255]: the saturating/abs path of convertScaleAbs."""
-    kw = dict(fps=6, box_size=128, blur_scale=32, threshold=6, avg=1.7, min_time=0.3, cache_time=0.5)
-    _compare_with_oracle(128, 96, 10, 5, kw, seed=77)
+    """avg > 1 makes the background leave [0, 255]: the saturating/abs path of convertScaleAbs.  A negative threshold sets
+    every threshold bit.  Both take the variant of K1 without the carry form of the threshold test; the negative threshold
+    also runs through the generic front end at k = 5 (mma.sync Gaussian, then the separate temporal kernel)."""
+    for avg, threshold in ((1.7, 6), (0.3, -1)):
+        kw = dict(fps=6, box_size=128, blur_scale=32, threshold=threshold, avg=avg, min_time=0.3, cache_time=0.5)
+        _compare_with_oracle(128, 96, 10, 5, kw, seed=77)
+    _compare_with_oracle(128, 96, 10, 5, kw, seed=78, no_fused=True)
 
 
 def test_fused_multi_stream_1080p():

@@ -101,8 +101,9 @@ def test_umma_direct_full_frames(W, H, bs):
 
 @pytest.mark.parametrize("umma_apron", [False, True])
 def test_umma_blur_avg_outside_unit_range_and_k1(umma_apron):
-    kw = dict(fps=6, box_size=128, blur_scale=9, threshold=6, avg=1.7, min_time=0.3, cache_time=0.5)     # k = 15
-    _run(128, 96, 8, 4, kw, seed=930, no_fused=True, umma=True, umma_apron=umma_apron)
+    for avg, threshold in ((1.7, 6), (0.3, -1)):
+        kw = dict(fps=6, box_size=128, blur_scale=9, threshold=threshold, avg=avg, min_time=0.3, cache_time=0.5)     # k = 15
+        _run(128, 96, 8, 4, kw, seed=930, no_fused=True, umma=True, umma_apron=umma_apron)
     kw = dict(fps=6, box_size=128, blur_scale=128, threshold=6, avg=0.3, min_time=0.3, cache_time=0.5)   # k = 1: identity blur
     _run(128, 96, 8, 4, kw, seed=931, no_fused=True, umma=True, umma_apron=umma_apron)
 
