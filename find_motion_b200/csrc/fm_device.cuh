@@ -16,7 +16,8 @@ __device__ __forceinline__ void fm_mbar_init(uint64_t *bar, uint32_t count) {
 __device__ __forceinline__ void fm_mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(fm_smem_u32(bar)), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void fm_mbar_wait(uint64_t *bar, uint32_t parity) {
+// bar: shared-window address of the barrier (fm_smem_u32), for loops that keep it in a register
+__device__ __forceinline__ void fm_mbar_wait(uint32_t bar, uint32_t parity) {
     asm volatile(
         "{\n"
         ".reg .pred p;\n"
@@ -25,8 +26,9 @@ __device__ __forceinline__ void fm_mbar_wait(uint64_t *bar, uint32_t parity) {
         "@p bra WAIT_DONE;\n"
         "bra WAIT_LOOP;\n"
         "WAIT_DONE:\n"
-        "}\n" ::"r"(fm_smem_u32(bar)), "r"(parity) : "memory");
+        "}\n" ::"r"(bar), "r"(parity) : "memory");
 }
+__device__ __forceinline__ void fm_mbar_wait(uint64_t *bar, uint32_t parity) { fm_mbar_wait(fm_smem_u32(bar), parity); }
 // box (c0, c1, c2, c3) of a 4-D tensor map -> shared memory at `dst`; completes a transaction on `bar`
 __device__ __forceinline__ void fm_tma_load_4d(uint32_t dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, int c2,
                                                int c3) {

@@ -56,10 +56,30 @@ struct FusedParams {
     int b0, b1, b2, shift, rnd; // taps / g, and the rounding of the final shift (packed in both lanes)
     int threshold;
     double alpha, beta;
+    int qoff; uint32_t nthr2; double nC;    // fm_temporal_px's constants: read from the constant bank, not rebuilt per frame
     uint8_t *gray_out, *blur_out;   // [S][T][h][w], only with KEEP
     int *rawrange;                  // [S][T][2] (max y, max h-1-y) of rows with pixels above threshold
     uint4 bfr[32];                  // per lane: B fragments of the horizontal pass (fused_bfr)
+#ifdef FM_K1_PROF
+    long long *prof;                // development aid: [K1_NPROF] cycles per phase summed over CTAs (thread 0), [K1_NPROF] frames
+#endif
 };
+
+// Development aid (build with -DFM_K1_PROF, tools/k1_prof.py): clock64 of thread 0 of every CTA per phase of the frame
+// loop.  A phase that ends in a barrier includes the wait at it.  Off by default: the shipped code has no trace of it.
+enum { K1_WAIT, K1_GRAY, K1_BORDER, K1_HORIZ, K1_VERT, K1_TAIL, K1_NPROF };
+#ifdef FM_K1_PROF
+#define K1_PROF(slot)                                \
+    do {                                             \
+        if (tid == 0) {                              \
+            const long long now_ = clock64();        \
+            k1_prof[slot] += now_ - k1_prof_t;       \
+            k1_prof_t = now_;                        \
+        }                                            \
+    } while (0)
+#else
+#define K1_PROF(slot) do {} while (0)
+#endif
 
 // B fragments of the horizontal pass (constant per call): the banded tap matrix for the two 8-column output blocks of a
 // 32-byte window.  Output column n of block nb is gray byte 4 + 16 j + 8 nb + n of its row, window byte k is gray byte
@@ -95,6 +115,13 @@ __device__ __forceinline__ uint32_t nibble_transpose8(uint32_t x, int lane) {
     return x;
 }
 
+// a + b + c as one IADD3: written as C, the compiler adds c after the products of the vertical pass, one add more per word
+__device__ __forceinline__ uint32_t add3(uint32_t a, uint32_t b, uint32_t c) {
+    uint32_t d;
+    asm("add.u32 %0, %1, %2;\n\tadd.u32 %0, %0, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
+    return d;
+}
+
 // One thread: 5 rows of packed horizontal sums in -> ONE output row x 16 pixels (two segments of 8 consecutive pixels, 64
 // pixels apart, so that the 128-bit shared loads of a quarter-warp are contiguous): vertical pass, mask, threshold bits,
 // background update.  The 16 threshold bits of a thread are two bytes of the bit plane: no transposition across lanes.
@@ -104,9 +131,6 @@ template <bool KEEP, bool SAFE, bool INIT, bool MASKED, bool SH8>
 __device__ __forceinline__ uint32_t fused_rows(const uint32_t *shw, double (&bg)[FT_PX], uint32_t M, const FusedParams &p,
                                                uint8_t *blur_out, uint32_t vmask) {
     const uint32_t b0 = p.b0, b1 = p.b1, b2 = p.b2;
-    const int qoff = 0x4B400000 - p.threshold;
-    const unsigned nthr2 = ~(2u * (unsigned)p.threshold);
-    const double nC = -(4503599627370496.0 * p.alpha);
     uint32_t bits = 0;
 #pragma unroll
     for (int seg = 0; seg < 2; seg++) {
@@ -117,7 +141,7 @@ __device__ __forceinline__ uint32_t fused_rows(const uint32_t *shw, double (&bg)
         {
             const uint4 r0 = *reinterpret_cast<const uint4 *>(sp), r4 = *reinterpret_cast<const uint4 *>(sp + 4 * FH_WORDS);
             const uint32_t rn = SH8 ? 0x00800080u : (uint32_t)p.rnd;
-            if (SH8) { v[0] = r0.x + r4.x + rn; v[1] = r0.y + r4.y + rn; v[2] = r0.z + r4.z + rn; v[3] = r0.w + r4.w + rn; }
+            if (SH8) { v[0] = add3(r0.x, r4.x, rn); v[1] = add3(r0.y, r4.y, rn); v[2] = add3(r0.z, r4.z, rn); v[3] = add3(r0.w, r4.w, rn); }
             else { v[0] = b0 * (r0.x + r4.x) + rn; v[1] = b0 * (r0.y + r4.y) + rn; v[2] = b0 * (r0.z + r4.z) + rn; v[3] = b0 * (r0.w + r4.w) + rn; }
         }
         {
@@ -149,10 +173,17 @@ __device__ __forceinline__ uint32_t fused_rows(const uint32_t *shw, double (&bg)
             uint32_t sv = SH8 ? __byte_perm(v[c >> 1], 0, (c & 1) ? 0x4443 : 0x4441)
                               : ((c & 1) ? (v[c >> 1] >> 16) : (v[c >> 1] & 0xFFFFu));
             if (MASKED && (M & (1u << idx))) sv = 0;          // mask_off_areas paints BLACK into blur
-            fm_temporal_px<SAFE, INIT>(sv, bg[idx], bits, p.threshold, qoff, nthr2, p.alpha, p.beta, nC);
+            fm_temporal_px<SAFE, INIT>(sv, bg[idx], bits, p.threshold, p.qoff, p.nthr2, p.alpha, p.beta, p.nC);
         }
     }
     return __brev(bits) >> (32 - FT_PX);      // the first pixel was pushed first: bit idx = pixel idx
+}
+
+// Frame t of stream s has pixels above threshold in the 4 rows y .. y+3 of a warp: widen that frame's rawrange.
+__device__ __forceinline__ void rawrange_hit(const FusedParams &p, int s, int t, int y) {
+    int *rr = p.rawrange + 2 * ((size_t)s * p.T + t);
+    atomicMax(rr, min(y + 3, p.h - 1));
+    atomicMax(rr + 1, p.h - 1 - y);
 }
 
 // End of every CTA of K1.  K1 of call i+1 is launched as a programmatic dependent of k_decide of call i (fm_host.cu), so
@@ -246,6 +277,14 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
     const int hwin = warp & 7;                                  // the warp's 16-column window of the horizontal pass
     const uint32_t sg_lane = fm_smem_u32(sg) + ((lane & 7) + 8 * ((lane >> 3) & 1)) * (FG_WORDS * 4) + 16 * hwin + 16 * (lane >> 4);
     uint32_t *sh_lane = sh + (lane >> 2) * FH_WORDS + 8 * hwin + (lane & 3);
+    // the thread's first unit of the BGR -> gray conversion: stage bytes 4 + 24 tid .. (see below), gray words 2 tid, 2 tid + 1
+    const int rs_tid = 4 + 24 * tid;
+    uint2 *const sgt = reinterpret_cast<uint2 *>(sg) + tid;
+    const uint32_t bars_s = fm_smem_u32(bars);
+    uint32_t hits = 0;                  // bit t: frame t has a pixel above threshold in this warp's rows (Ts <= 32)
+#ifdef FM_K1_PROF
+    long long k1_prof[K1_NPROF] = {}, k1_prof_t = clock64();
+#endif
 
     for (int t = 0; t < Ts; t++) {
         // No barrier here: every thread that gets this far has passed the second barrier of frame t-1, i.e. all
@@ -254,28 +293,32 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
             fm_mbar_expect_tx(&bars[(t + 1) & 1], RAW_BYTES);
             fm_tma_load_4d(raw + ((t + 1) & 1) * RAW_STAGE, &tmap, &bars[(t + 1) & 1], cx, cy, t + 1, s);
         }
-        fm_mbar_wait(&bars[t & 1], (t >> 1) & 1);
+        fm_mbar_wait(bars_s + 8 * (t & 1), (t >> 1) & 1);
+        K1_PROF(K1_WAIT);
         // ---- staged BGR -> gray bytes in shared memory (tile + halo) ----
         {
             // the staged rows are dense (pitch 432 B = 36 groups of 4 pixels = 12 B, the first at byte 4 because the
             // TMA box must start 16 B aligned in global memory -- a box at x0 * 3 - 12 raises "illegal instruction") and
             // so are the gray rows (36 words): group u is raw + 4 + 12 u -> sg[u].
-            const unsigned char *rs = raw + (t & 1) * RAW_STAGE + 4;
-            // two units (8 pixels, 24 bytes -> 2 gray words) per step: half the address arithmetic and loop control
+            // two units (8 pixels, 24 bytes -> 2 gray words) per step: half the address arithmetic and loop control.  Unit
+            // u = tid + i * FUSED_THREADS: the offsets of all steps are immediates from the thread's own (rs, sgt), and
+            // only the last step, which not every thread has, is predicated.
+            constexpr int NU = FG_ROWS * FG_WORDS / 2, NFULL = NU / FUSED_THREADS;
+            const unsigned char *rs = raw + (t & 1) * RAW_STAGE + rs_tid;
 #pragma unroll
-            for (int i = 0; i < (FG_ROWS * FG_WORDS / 2 + FUSED_THREADS - 1) / FUSED_THREADS; i++) {
-                int u = tid + i * FUSED_THREADS;
-                if (u < FG_ROWS * FG_WORDS / 2) {
+            for (int i = 0; i <= NFULL; i++) {
+                if (i < NFULL || tid < NU - NFULL * FUSED_THREADS) {
                     // 24 bytes at byte 4 (mod 8) of the stage: 4 + 8 + 8 + 4
-                    const unsigned char *q = rs + u * 24;
+                    const unsigned char *q = rs + i * (24 * FUSED_THREADS);
                     const uint32_t a0 = *reinterpret_cast<const uint32_t *>(q), a5 = *reinterpret_cast<const uint32_t *>(q + 20);
                     const uint2 a12 = *reinterpret_cast<const uint2 *>(q + 4), a34 = *reinterpret_cast<const uint2 *>(q + 12);
                     const uint32_t g0 = fm_gray4(a0, a12.x, a12.y), g1 = fm_gray4(a34.x, a34.y, a5);
-                    *reinterpret_cast<uint2 *>(sg + 2 * u) = make_uint2(g0, g1);
+                    sgt[i * FUSED_THREADS] = make_uint2(g0, g1);
                 }
             }
         }
         __syncthreads();
+        K1_PROF(K1_GRAY);
         if (border) {               // BORDER_REFLECT_101 for the 2-pixel ring outside the image
             unsigned char *sb = reinterpret_cast<unsigned char *>(sg);
             for (int ry = tid; ry < FG_ROWS; ry += FUSED_THREADS) {
@@ -294,6 +337,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
             }
             __syncthreads();
         }
+        K1_PROF(K1_BORDER);
         if (KEEP) {
             for (int u = tid; u < FT_H * (FT_W / 4); u += FUSED_THREADS) {
                 int ry = u / (FT_W / 4), ux = u - ry * (FT_W / 4);
@@ -327,6 +371,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
             }
         }
         __syncthreads();
+        K1_PROF(K1_HORIZ);
         // ---- vertical pass on packed pairs (5 rows x 16 pixels per thread), then the temporal update ----
         const uint32_t *sgw = sh + trow * FH_WORDS + 4 * xg;
         asm volatile("" : "+r"(M));        // opaque per frame: keeps the 16 single-bit tests of M from being hoisted (and spilled)
@@ -337,18 +382,27 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
                                               : fused_rows<KEEP, SAFE, false, true, false>(sgw, bg, M, p, bo, vmask);
         else if (p.shift == 8) bits = fused_rows<KEEP, SAFE, false, false, true>(sgw, bg, M, p, bo, vmask);
         else bits = fused_rows<KEEP, SAFE, false, false, false>(sgw, bg, M, p, bo, vmask);
+        K1_PROF(K1_VERT);
         // ---- two bytes of the bit plane per thread ----
         if (!okA) bits = 0;
         if (!okB) bits &= 0xFFu;
         if (okA) tb[0] = (uint8_t)bits;
         if (okB) tb[8] = (uint8_t)(bits >> 8);
-        if (__any_sync(0xffffffffu, bits != 0) && lane == 0) {       // this warp's 4 rows hold something
-            int *rr = p.rawrange + 2 * ((size_t)s * p.T + t);
-            atomicMax(rr, min(y0 + 4 * warp + 3, h - 1));
-            atomicMax(rr + 1, h - 1 - (y0 + 4 * warp));
-        }
+        // rawrange: whether this warp's 4 rows hold something in frame t.  Up to 32 frames that is bit t of the
+        // warp-uniform `hits`, and the atomics of all frames go out once after the loop, one lane per frame.
+        const bool any = __any_sync(0xffffffffu, bits != 0);
+        if (Ts <= 32) hits |= (any ? 1u : 0u) << t;
+        else if (any && lane == 0) rawrange_hit(p, s, t, y0 + 4 * warp);
         tb += 4 * p.flatwords;
+        K1_PROF(K1_TAIL);
     }
+#ifdef FM_K1_PROF
+    if (tid == 0) {
+        for (int i = 0; i < K1_NPROF; i++) atomicAdd((unsigned long long *)p.prof + i, (unsigned long long)k1_prof[i]);
+        atomicAdd((unsigned long long *)p.prof + K1_NPROF, (unsigned long long)Ts);
+    }
+#endif
+    if (Ts <= 32 && ((hits >> lane) & 1u)) rawrange_hit(p, s, lane, y0 + 4 * warp);
 #pragma unroll
     for (int i = 0; i < FT_PX / 2; i++) bgt[i * 32] = make_double2(bg[2 * i], bg[2 * i + 1]);
     fused_exit(p);
@@ -377,6 +431,30 @@ size_t fm_fused_bg_doubles(const fm_ctx *c) {
     size_t tilesX = (c->w + FT_W - 1) / FT_W, tilesY = (c->h + FT_H - 1) / FT_H;
     return (size_t)c->S * tilesX * tilesY * FT_W * FT_H;
 }
+
+#ifdef FM_K1_PROF
+#include <cstdio>
+#include <cstring>
+
+static long long *k1_prof_buffer() {               // [K1_NPROF] cycles, [K1_NPROF] CTA-frames: managed, read by the host
+    static long long *buf = nullptr;
+    if (!buf && cudaMallocManaged(&buf, (K1_NPROF + 1) * sizeof(long long)) == cudaSuccess)
+        memset(buf, 0, (K1_NPROF + 1) * sizeof(long long));
+    return buf;
+}
+
+// cycles per CTA-frame of each phase since the last call (thread 0 of every CTA), then reset
+extern "C" void fm_k1_prof_dump(void) {
+    long long *b = k1_prof_buffer();
+    if (!b) return;
+    cudaDeviceSynchronize();
+    const double n = b[K1_NPROF] ? (double)b[K1_NPROF] : 1.0;
+    fprintf(stderr, "k1 phases (cycles per CTA-frame, thread 0, %lld CTA-frames): wait %.1f gray %.1f border %.1f "
+            "horizontal %.1f vertical %.1f tail %.1f\n", b[K1_NPROF], b[K1_WAIT] / n, b[K1_GRAY] / n, b[K1_BORDER] / n,
+            b[K1_HORIZ] / n, b[K1_VERT] / n, b[K1_TAIL] / n);
+    memset(b, 0, (K1_NPROF + 1) * sizeof(long long));
+}
+#endif
 
 #define FUSED_SMEM (2 * RAW_STAGE + FH_ROWS * FG_WORDS * 4 + FH_ROWS * FH_WORDS * 4 + 16)
 
@@ -409,9 +487,14 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     p.rnd = r1 | (r1 << 16);
     p.threshold = c->cfg.threshold;
     p.alpha = c->cfg.avg; p.beta = 1.0 - p.alpha;
+    p.qoff = (int)(0x4B400000u - (unsigned)p.threshold); p.nthr2 = ~(2u * (unsigned)p.threshold); p.nC = -(4503599627370496.0 * p.alpha);
     p.gray_out = c->gray; p.blur_out = c->blur;
     p.rawrange = fm_rawrange(c);
     p.stamp = c->stamp;
+#ifdef FM_K1_PROF
+    p.prof = k1_prof_buffer();
+    if (!p.prof) return FM_ECUDA;
+#endif
     const bool keep = (c->cfg.flags & FM_FLAG_KEEP_PLANES) != 0;
     const bool safe = p.alpha >= 0.0 && p.alpha <= 1.0 && p.threshold >= 0;
     fused_bfr(p);
