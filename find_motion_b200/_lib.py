@@ -56,6 +56,7 @@ FLAG_UMMA = 32
 FLAG_NO_ROWS = 64
 FLAG_UPSCALE = 128
 FLAG_DEVICE_CLIPS = 256
+FLAG_NV12 = 512
 
 # every symbol include/fm_gpu.h declares: name -> (restype, argtypes)
 _P = C.c_void_p

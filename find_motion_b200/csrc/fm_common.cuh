@@ -56,6 +56,9 @@ struct fm_ctx {
     int N;                     // w*h
     int ntiles;                // ceil(N / FM_TILE_PX)
     int resize_mode;           // 0 identity, 1 general tables, 2 integer ratio, 3 upscale (FM_FLAG_UPSCALE, k_upscale.cu)
+    size_t frame_bytes;        // bytes of one input frame: H * W * 3 (BGR) or H * W * 3 / 2 (FM_FLAG_NV12)
+    uint8_t *nv12_bgr;         // FM_FLAG_NV12 on the staged path: [S][Tmax][H][W][3] the call's frames converted to BGR
+                               // (k_nv12.cu), read by the BGR front end; null when none is needed
     bool fused;                // K1 fused stencil+background kernel drives the front end
     bool wide_fused;           // wide Gaussian: the vertical pass runs the temporal stage too (k_wide_vt)
     bool umma;                 // blur + temporal stage on tcgen05 tensor cores (k_umma.cu), k <= 97
@@ -113,8 +116,8 @@ struct fm_ctx {
     cudaStream_t copy_stream;  // host -> device frame copies
     cudaEvent_t ev_copied[2], ev_done[2];
     // device look-back cache (FM_FLAG_DEVICE_CLIPS, k_clips.cu)
-    uint8_t *clip_ring;        // [S][cache_frames] raw BGR frames, slots of clip_slot_bytes; null when cache_frames == 0
-    size_t clip_slot_bytes;    // H * W * 3 rounded up to 256
+    uint8_t *clip_ring;        // [S][cache_frames] raw input frames, slots of clip_slot_bytes; null when cache_frames == 0
+    size_t clip_slot_bytes;    // frame_bytes rounded up to 256
     long long *clip_base;      // [S] absolute frame number of the next frame of each stream
     FmClipCopy *clip_list;     // gather list [S * (cache_frames + Tmax)], then store list [S * min(cache_frames, Tmax)]
     int *clip_count;           // [2] entries of the two lists in the current call
@@ -250,6 +253,7 @@ int fm_clips_alloc(fm_ctx *c);
 void fm_clips_free(fm_ctx *c);
 int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
                     size_t ostride, cudaStream_t st);
+int fm_launch_nv12_bgr(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
 int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
 int fm_ccl_alloc(CclScratch *s, int frames, int h, int cap);
 void fm_ccl_free(CclScratch *s);

@@ -78,6 +78,32 @@ __device__ __forceinline__ uint32_t fm_gray4(uint32_t w0, uint32_t w1, uint32_t 
     return __byte_perm(__byte_perm(t0, t1, 0x0062), __byte_perm(t2, t3, 0x0062), 0x5410);
 }
 
+// ---- NV12 -> BGR exactly as cv2.cvtColor(COLOR_YUV2BGR_NV12): ITU-R BT.601 in 20-bit fixed point ----
+//   y' = max(Y - 16, 0) * 1220542,  u = U - 128,  v = V - 128
+//   R = sat((y' + 1673527 v + 2^19) >> 20),  G = sat((y' - 852492 v - 409993 u + 2^19) >> 20),  B = sat((y' + 2116026 u + 2^19) >> 20)
+// Chroma is nearest-neighbour (pixel (x, y) takes the U, V pair of UV row y/2, column pair x/2), so the chroma terms,
+// with the rounding folded in, are computed once per 2x2 block (fm_nv12_chroma) and shared by its four pixels.
+// Every intermediate fits an int32: |y'| + |2116026 u| < 2^30.
+struct FmChroma {
+    int r, g, b;
+};
+__device__ __forceinline__ FmChroma fm_nv12_chroma(uint32_t u, uint32_t v) {
+    const int uu = (int)u - 128, vv = (int)v - 128;
+    return FmChroma{1673527 * vv + (1 << 19), -852492 * vv - 409993 * uu + (1 << 19), 2116026 * uu + (1 << 19)};
+}
+__device__ __forceinline__ uint32_t fm_sat_q20(int x) { return (uint32_t)min(max(x >> 20, 0), 255); }
+__device__ __forceinline__ void fm_nv12_bgr(uint32_t y, const FmChroma &c, uint32_t &b, uint32_t &g, uint32_t &r) {
+    const int yy = max((int)y - 16, 0) * 1220542;
+    b = fm_sat_q20(yy + c.b);
+    g = fm_sat_q20(yy + c.g);
+    r = fm_sat_q20(yy + c.r);
+}
+__device__ __forceinline__ uint32_t fm_nv12_gray(uint32_t y, const FmChroma &c) {
+    uint32_t b, g, r;
+    fm_nv12_bgr(y, c, b, g, r);
+    return fm_gray(b, g, r);
+}
+
 __device__ __forceinline__ int fm_reflect101(int i, int n) {
     // BORDER_REFLECT_101 for any offset
     if ((unsigned)i < (unsigned)n) return i;

@@ -199,7 +199,7 @@ extern "C" int fm_ctx_destroy(fm_ctx *c) {
     cudaDeviceSynchronize();
     cudaFree(c->coef); cudaFree(c->wtab); cudaFree(c->uband); cudaFree(c->uband_f); cudaFree(c->gpad);
     cudaFree(c->g4start); cudaFree(c->g4n); cudaFree(c->g4off); cudaFree(c->g4w);
-    cudaFree(c->uxt); cudaFree(c->uyt);
+    cudaFree(c->uxt); cudaFree(c->uyt); cudaFree(c->nv12_bgr);
     fm_rows_free(c);
     fm_clips_free(c);
     cudaFree(c->xtab.start); cudaFree(c->xtab.idx); cudaFree(c->xtab.wt);
@@ -243,6 +243,16 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
                      cfg->frame_width);
         return FM_ERANGE;
     }
+    if ((cfg->flags & FM_FLAG_NV12) && ((cfg->frame_width | cfg->frame_height) & 1)) {
+        // the chroma plane has one U, V pair per 2 x 2 block (cv2's COLOR_YUV2BGR_NV12 refuses odd sizes as well)
+        fm_set_error("NV12 frames need an even width and height (%d x %d)", cfg->frame_width, cfg->frame_height);
+        return FM_ERANGE;
+    }
+    if ((cfg->flags & FM_FLAG_NV12) && (cfg->n_streams > 65535 || cfg->max_frames > 65535)) {
+        // the staging kernel's grid: one z index per stream, one y index per frame
+        fm_set_error("NV12 contexts take at most 65535 streams and 65535 frames per call");
+        return FM_ERANGE;
+    }
     int ndev = 0;
     FM_CUDA(cudaGetDeviceCount(&ndev));
     if (cfg->device < 0 || cfg->device >= ndev) {
@@ -256,6 +266,7 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     c->cfg = *cfg;
     c->S = cfg->n_streams; c->Tmax = cfg->max_frames;
     c->W = cfg->frame_width; c->H = cfg->frame_height;
+    c->frame_bytes = (cfg->flags & FM_FLAG_NV12) ? (size_t)c->W * c->H * 3 / 2 : (size_t)c->W * c->H * 3;
     // derived parameters, mirroring the Python expressions (true division on floats, int() truncation)
     const double W = c->W, H = c->H, box = cfg->box_size;
     c->w = cfg->box_size;
@@ -422,6 +433,14 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     if ((rc = fm_ccl_alloc(&c->ccl, nb, c->h, cap))) return fail(rc);
     if ((rc = fm_ccl_configure(c))) return fail(rc);
     if ((cfg->flags & FM_FLAG_DEVICE_CLIPS) && (rc = fm_clips_alloc(c))) return fail(rc);
+    // NV12: the fused front end reads the frames directly; every other front end reads them converted into a BGR slot
+    // (k_nv12.cu).  FM_NV12_STAGED builds (A/B of the two paths, tools/bench_nv12.py --ab-staged) stage them always.
+#ifdef FM_NV12_STAGED
+    const bool nv12_staged = true;
+#else
+    const bool nv12_staged = !c->fused;
+#endif
+    if ((cfg->flags & FM_FLAG_NV12) && nv12_staged) ALLOC(c->nv12_bgr, F * c->W * c->H * 3);
     FM_TRY(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
     FM_TRY(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     for (int i = 0; i < 2; i++) {
@@ -557,11 +576,22 @@ static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_
         if (c->fused) c->stamp = c->stamps + 4 * c->ev_pending++;
         else { ev = c->evs + 4 * c->ev_pending++; FM_CUDA(cudaEventRecord(ev[0], st)); }
     }
+    // NV12 on the staged path: the BGR front end reads the call's frames converted into the context's slot, packed as a
+    // dense BGR batch of the call; the device ring keeps the caller's NV12 frames
+    const uint8_t *fe = frames;
+    size_t fe_sstride = stream_stride, fe_fstride = frame_stride;
+    if (c->nv12_bgr) {
+        rc = fm_launch_nv12_bgr(c, frames, stream_stride, frame_stride, n_frames, st);
+        if (rc) { if (c->stamp) c->ev_pending--; c->stamp = nullptr; return rc; }
+        fe = c->nv12_bgr;
+        fe_fstride = (size_t)c->W * c->H * 3;
+        fe_sstride = fe_fstride * n_frames;
+    }
     if (c->fused) {
-        rc = fm_launch_fused(c, frames, stream_stride, frame_stride, n_frames, st);
+        rc = fm_launch_fused(c, fe, fe_sstride, fe_fstride, n_frames, st);
         if (rc) { if (c->stamp) c->ev_pending--; c->stamp = nullptr; return rc; }
     } else {
-        if ((rc = fm_launch_frontend(c, frames, stream_stride, frame_stride, n_frames, st))) return rc;
+        if ((rc = fm_launch_frontend(c, fe, fe_sstride, fe_fstride, n_frames, st))) return rc;
         if (ev) FM_CUDA(cudaEventRecord(ev[1], st));
         if (!c->wide_fused && !c->umma && (rc = fm_launch_temporal(c, n_frames, st))) return rc;
         if (ev) FM_CUDA(cudaEventRecord(ev[2], st));
@@ -617,7 +647,7 @@ extern "C" int fm_submit_host(fm_ctx *c, int slot, const uint8_t *frames_host, s
     }
     if (c->slot_T[slot]) { fm_set_error("slot %d still holds a batch: call fm_wait first", slot); return FM_EINVAL; }
     FM_CUDA(cudaSetDevice(c->cfg.device));
-    const size_t fb = (size_t)c->W * c->H * 3;
+    const size_t fb = c->frame_bytes;
     const size_t need = (size_t)c->S * n_frames * fb;
     if (c->stage_bytes[slot] < need) {
         cudaFree(c->stage_dev[slot]);

@@ -33,7 +33,7 @@ struct ClipPlanArgs {
     size_t slot_bytes;
     uint8_t *out;                  // null: no gather (the plain entry points only keep the ring up to date)
     size_t ostride;
-    size_t fb;                     // H * W * 3
+    size_t fb;                     // bytes of one input frame (fm_ctx::frame_bytes)
     int S, T, C;
     FmClipCopy *gather, *store;
     int *count;                    // [2] entries of the gather and of the store list
@@ -151,7 +151,7 @@ __global__ void __launch_bounds__(CLIP_COPY_THREADS) k_clip_store(const FmClipCo
 
 int fm_clips_alloc(fm_ctx *c) {
     const int C = c->info.cache_frames;
-    const size_t fb = (size_t)c->W * c->H * 3;
+    const size_t fb = c->frame_bytes;
     c->clip_slot_bytes = (fb + 255) & ~(size_t)255;
     if (C > 0) {
         const size_t ring = (size_t)c->S * C * c->clip_slot_bytes;
@@ -188,7 +188,7 @@ int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     a.frames = frames; a.sstride = sstride; a.fstride = fstride;
     a.ring = c->clip_ring; a.slot_bytes = c->clip_slot_bytes;
     a.out = out; a.ostride = ostride;
-    a.fb = (size_t)c->W * c->H * 3;
+    a.fb = c->frame_bytes;
     a.S = c->S; a.T = T; a.C = C;
     const size_t ng = (size_t)c->S * (C + c->Tmax);
     a.gather = c->clip_list; a.store = c->clip_list + ng;

@@ -38,6 +38,11 @@
 #define RAW_PITCH 432      // bytes per staged BGR row: bytes x0*3-16 .. x0*3+415 (TMA box of 108 u32)
 #define RAW_BYTES (RAW_PITCH * FG_ROWS)                 // bytes one TMA box delivers
 #define RAW_STAGE ((RAW_BYTES + 127) / 128 * 128)        // stage stride (TMA destinations are 128 B aligned)
+// NV12 (FM_FLAG_NV12): a stage holds two boxes, the luma rows y0-2 .. y0+FT_H+1 and the UV rows (y0-2)/2 .. that cover
+// them, each of bytes x0-16 .. x0+143 (40 u32: the box start must be 16 B aligned in global memory)
+#define NV_PITCH 160
+#define NV_Y_BYTES (NV_PITCH * FG_ROWS)                  // 5760 = 45 * 128: the UV box lands 128 B aligned after it
+#define NV_BYTES (NV_Y_BYTES + NV_PITCH * FG_ROWS / 2)   // <= RAW_BYTES: both fit the BGR stage
 
 struct FusedParams {
     int T, w, h, wpr;           // T = frames per stream of the call
@@ -205,8 +210,16 @@ __device__ __forceinline__ void fused_exit(const FusedParams &p) {
     }
 }
 
-template <bool KEEP, bool SAFE>
-__global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const __grid_constant__ CUtensorMap tmap, FusedParams p) {
+// 4 luma bytes of one row and the chroma of their two 2x2 blocks -> 4 gray bytes (fm_nv12_gray: cv2's COLOR_YUV2BGR_NV12)
+__device__ __forceinline__ uint32_t nv12_gray4(uint32_t y4, const FmChroma &c0, const FmChroma &c1) {
+    return fm_nv12_gray(y4 & 0xFFu, c0) | (fm_nv12_gray((y4 >> 8) & 0xFFu, c0) << 8) |
+           (fm_nv12_gray((y4 >> 16) & 0xFFu, c1) << 16) | (fm_nv12_gray(y4 >> 24, c1) << 24);
+}
+
+// NV12: frames arrive as the two boxes above (tmap = luma plane, tmap_uv = chroma plane); otherwise tmap_uv is unused
+template <bool KEEP, bool SAFE, bool NV12>
+__global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const __grid_constant__ CUtensorMap tmap, FusedParams p,
+                                                                         const __grid_constant__ CUtensorMap tmap_uv) {
     extern __shared__ __align__(128) unsigned char fsm[];
     unsigned char *raw = fsm;                                                  // [2][RAW_STAGE] staged BGR rows (TMA)
     uint32_t *sg = reinterpret_cast<uint32_t *>(fsm + 2 * RAW_STAGE);        // [FH_ROWS][FG_WORDS] gray bytes (FG_ROWS used)
@@ -259,8 +272,14 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
     }
     __syncthreads();
     if (tid == 0) {
-        fm_mbar_expect_tx(&bars[0], RAW_BYTES);
-        fm_tma_load_4d(raw, &tmap, &bars[0], cx, cy, 0, s);
+        if (NV12) {
+            fm_mbar_expect_tx(&bars[0], NV_BYTES);
+            fm_tma_load_4d(raw, &tmap, &bars[0], x0 / 4 - 4, y0 - 2, 0, s);
+            fm_tma_load_4d(raw + NV_Y_BYTES, &tmap_uv, &bars[0], x0 / 4 - 4, y0 / 2 - 1, 0, s);
+        } else {
+            fm_mbar_expect_tx(&bars[0], RAW_BYTES);
+            fm_tma_load_4d(raw, &tmap, &bars[0], cx, cy, 0, s);
+        }
     }
     // the thread's two bytes of the bit plane (row py, pixels px .. px+7 and px+64 .. px+71)
     uint8_t *tb = reinterpret_cast<uint8_t *>(p.tbits + ((size_t)s * p.T) * p.flatwords + (size_t)py * p.wpr) + (px >> 3);
@@ -290,13 +309,41 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
         // No barrier here: every thread that gets this far has passed the second barrier of frame t-1, i.e. all
         // conversions out of raw stage (t+1)&1 (frame t-1) and all reads of the gray plane are complete.
         if (tid == 0 && t + 1 < Ts) {
-            fm_mbar_expect_tx(&bars[(t + 1) & 1], RAW_BYTES);
-            fm_tma_load_4d(raw + ((t + 1) & 1) * RAW_STAGE, &tmap, &bars[(t + 1) & 1], cx, cy, t + 1, s);
+            if (NV12) {
+                unsigned char *dst = raw + ((t + 1) & 1) * RAW_STAGE;
+                fm_mbar_expect_tx(&bars[(t + 1) & 1], NV_BYTES);
+                fm_tma_load_4d(dst, &tmap, &bars[(t + 1) & 1], x0 / 4 - 4, y0 - 2, t + 1, s);
+                fm_tma_load_4d(dst + NV_Y_BYTES, &tmap_uv, &bars[(t + 1) & 1], x0 / 4 - 4, y0 / 2 - 1, t + 1, s);
+            } else {
+                fm_mbar_expect_tx(&bars[(t + 1) & 1], RAW_BYTES);
+                fm_tma_load_4d(raw + ((t + 1) & 1) * RAW_STAGE, &tmap, &bars[(t + 1) & 1], cx, cy, t + 1, s);
+            }
         }
         fm_mbar_wait(bars_s + 8 * (t & 1), (t >> 1) & 1);
         K1_PROF(K1_WAIT);
-        // ---- staged BGR -> gray bytes in shared memory (tile + halo) ----
-        {
+        // ---- staged BGR (or NV12) -> gray bytes in shared memory (tile + halo) ----
+        if (NV12) {
+            // unit = gray word u of the row pair 2k, 2k+1 (image rows y0-2+2k, +1; y0 is even): two luma words and the UV
+            // word of chroma row k (= image UV row y0/2-1+k), all at byte 12 + 4u of their box rows (columns x0-4+4u ..
+            // +3); the chroma terms of the word's two 2x2 blocks serve both rows.  Zero-filled bytes outside the image
+            // convert to some colour: the border step below overwrites every halo pixel the passes read, as with BGR.
+            constexpr int NU = (FG_ROWS / 2) * FG_WORDS, NFULL = NU / FUSED_THREADS;
+            const unsigned char *st = raw + (t & 1) * RAW_STAGE;
+#pragma unroll
+            for (int i = 0; i <= NFULL; i++) {
+                if (i < NFULL || tid < NU - NFULL * FUSED_THREADS) {
+                    const int un = tid + i * FUSED_THREADS, k = un / FG_WORDS, u = un - k * FG_WORDS;
+                    const unsigned char *yq = st + 2 * k * NV_PITCH + 12 + 4 * u;
+                    const uint32_t l0 = *reinterpret_cast<const uint32_t *>(yq);
+                    const uint32_t l1 = *reinterpret_cast<const uint32_t *>(yq + NV_PITCH);
+                    const uint32_t cw = *reinterpret_cast<const uint32_t *>(st + NV_Y_BYTES + k * NV_PITCH + 12 + 4 * u);
+                    const FmChroma c0 = fm_nv12_chroma(cw & 0xFFu, (cw >> 8) & 0xFFu);
+                    const FmChroma c1 = fm_nv12_chroma((cw >> 16) & 0xFFu, cw >> 24);
+                    sg[2 * k * FG_WORDS + u] = nv12_gray4(l0, c0, c1);
+                    sg[(2 * k + 1) * FG_WORDS + u] = nv12_gray4(l1, c0, c1);
+                }
+            }
+        } else {
             // the staged rows are dense (pitch 432 B = 36 groups of 4 pixels = 12 B, the first at byte 4 because the
             // TMA box must start 16 B aligned in global memory -- a box at x0 * 3 - 12 raises "illegal instruction") and
             // so are the gray rows (36 words): group u is raw + 4 + 12 u -> sg[u].
@@ -422,9 +469,11 @@ __global__ void k_bg_export_fused(const double *__restrict__ bg, double *__restr
     dst[(size_t)y * w + x] = bg[(base + (size_t)(idx >> 1) * 32 + lane) * 2 + (idx & 1)];
 }
 
+// NV12 needs nothing more: W % 32 == 0 makes the luma and chroma rows 16 B aligned, and with an even H (fm_ctx_create)
+// the frame (W * H * 3 / 2 bytes) and the chroma plane's offset (W * H) too; the caller's pointer and strides are checked
+// at launch, as with BGR
 bool fm_fused_supported(const fm_ctx *c) {
-    return c->resize_mode == 0 && c->k <= 5 && (c->w % 32) == 0 && c->w >= 4 && c->h >= 4 &&
-           ((size_t)c->W * c->H * 3) % 16 == 0;
+    return c->resize_mode == 0 && c->k <= 5 && (c->w % 32) == 0 && c->w >= 4 && c->h >= 4 && c->frame_bytes % 16 == 0;
 }
 
 size_t fm_fused_bg_doubles(const fm_ctx *c) {
@@ -458,10 +507,38 @@ extern "C" void fm_k1_prof_dump(void) {
 
 #define FUSED_SMEM (2 * RAW_STAGE + FH_ROWS * FG_WORDS * 4 + FH_ROWS * FH_WORDS * 4 + 16)
 
+// one plane of the call's NV12 frames (rows of W bytes) as a 4-D u32 tensor map with boxes of NV_PITCH bytes x box_rows
+static int nv12_plane_tmap(const fm_ctx *c, const uint8_t *plane, int rows, size_t sstride, size_t fstride, int T,
+                           int box_rows, CUtensorMap *out) {
+    PFN_encodeTiled enc = fm_tma_encoder();
+    if (!enc) { fm_set_error("cuTensorMapEncodeTiled not available"); return FM_ECUDA; }
+    const size_t dense = c->frame_bytes;        // stands in for the stride of a dimension of extent 1 (never applied)
+    cuuint64_t dims[4] = {(cuuint64_t)c->W / 4, (cuuint64_t)rows, (cuuint64_t)T, (cuuint64_t)c->S};
+    cuuint64_t strides[3] = {(cuuint64_t)c->W, (cuuint64_t)(T > 1 ? fstride : dense),
+                             (cuuint64_t)(c->S > 1 ? sstride : (T > 1 ? fstride * T : dense))};
+    cuuint32_t box[4] = {NV_PITCH / 4, (cuuint32_t)box_rows, 1, 1};
+    cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, (void *)plane, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { fm_set_error("cuTensorMapEncodeTiled (NV12 plane) failed (%d)", (int)r); return FM_ECUDA; }
+    return FM_OK;
+}
+
 int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
-    CUtensorMap tmap;
-    int rc = fm_frames_tmap(c, frames, sstride, fstride, T, RAW_PITCH / 4, FG_ROWS, &tmap);
-    if (rc) return rc;
+    CUtensorMap tmap, tmap_uv;
+    const bool nv12 = c->nv12_bgr == nullptr && (c->cfg.flags & FM_FLAG_NV12);     // NV12 read directly (no staged slot)
+    int rc;
+    if (nv12) {
+        if ((((uintptr_t)frames) | sstride | fstride) & 15) {
+            fm_set_error("the fused NV12 front end needs 16-byte aligned frames and strides");
+            return FM_EINVAL;
+        }
+        if ((rc = nv12_plane_tmap(c, frames, c->H, sstride, fstride, T, FG_ROWS, &tmap))) return rc;
+        if ((rc = nv12_plane_tmap(c, frames + (size_t)c->W * c->H, c->H / 2, sstride, fstride, T, FG_ROWS / 2, &tmap_uv))) return rc;
+    } else {
+        if ((rc = fm_frames_tmap(c, frames, sstride, fstride, T, RAW_PITCH / 4, FG_ROWS, &tmap))) return rc;
+        tmap_uv = tmap;                          // not read
+    }
     FusedParams p;
     p.T = T; p.nvalid = c->nvalid;
     p.w = c->w; p.h = c->h; p.wpr = c->wpr;
@@ -499,14 +576,17 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     const bool safe = p.alpha >= 0.0 && p.alpha <= 1.0 && p.threshold >= 0;
     fused_bfr(p);
     dim3 grid(p.tilesX, p.tilesY, c->S);
-    if ((rc = fm_ensure_smem((const void *)k_fused<true, true>, FUSED_SMEM, c->cfg.device))) return rc;
-    if ((rc = fm_ensure_smem((const void *)k_fused<true, false>, FUSED_SMEM, c->cfg.device))) return rc;
-    if ((rc = fm_ensure_smem((const void *)k_fused<false, true>, FUSED_SMEM, c->cfg.device))) return rc;
-    if ((rc = fm_ensure_smem((const void *)k_fused<false, false>, FUSED_SMEM, c->cfg.device))) return rc;
-    // a programmatic dependent of the contour stage of the previous call: see fused_exit
-    void (*kern)(const CUtensorMap, FusedParams) = keep ? (safe ? k_fused<true, true> : k_fused<true, false>)
-                                                        : (safe ? k_fused<false, true> : k_fused<false, false>);
-    (void)fm_launch_chained(kern, grid, dim3(FUSED_THREADS), FUSED_SMEM, st, tmap, p);
+    typedef void (*FusedKernel)(const CUtensorMap, FusedParams, const CUtensorMap);
+    const FusedKernel kerns[2][2][2] = {{{k_fused<false, false, false>, k_fused<false, false, true>},
+                                         {k_fused<false, true, false>, k_fused<false, true, true>}},
+                                        {{k_fused<true, false, false>, k_fused<true, false, true>},
+                                         {k_fused<true, true, false>, k_fused<true, true, true>}}};
+    const FusedKernel kern = kerns[keep][safe][nv12];
+    if ((rc = fm_ensure_smem((const void *)kern, FUSED_SMEM, c->cfg.device))) return rc;
+    // a programmatic dependent of the contour stage of the previous call: see fused_exit.  Not after the NV12 staging
+    // kernel (k_nv12.cu, FM_NV12_STAGED builds): K1 reads the frames before its wait, and that kernel writes them
+    if (c->nv12_bgr) kern<<<grid, FUSED_THREADS, FUSED_SMEM, st>>>(tmap, p, tmap_uv);
+    else (void)fm_launch_chained(kern, grid, dim3(FUSED_THREADS), FUSED_SMEM, st, tmap, p, tmap_uv);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }

@@ -20,11 +20,15 @@ class MotionEngine:
     def __init__(self, frame_width, frame_height, n_streams=1, max_frames=8, device=0, fps=30, box_size=100,
                  min_box_scale=50, cache_time=2.0, min_time=0.5, threshold=7, avg=0.1, blur_scale=20,
                  mask_areas=None, max_components=256, keep_planes=False, no_fused=False, no_umma=False, umma_apron=False, umma=False, no_rows=False,
-                 upscale=False, device_clips=False):
+                 upscale=False, device_clips=False, nv12=False):
         """upscale: accept box_size > frame_width (cv2's INTER_AREA upscale, bit-exact, as imutils.resize does it);
         without it such a geometry raises, as in earlier releases.
         device_clips: keep the look-back cache of raw frames on the GPU (n_streams x cache_frames frames) so that
-        process_clip can hand out the frames the reference writes to its *_motion.avi."""
+        process_clip can hand out the frames the reference writes to its *_motion.avi.
+        nv12: the frames are NV12 as GPU video decoders emit them, each [H * 3 // 2, W] uint8 (the luma rows, then the
+        interleaved U, V rows; W and H even), with the results of a BGR engine on cv2.cvtColor(frame,
+        cv2.COLOR_YUV2BGR_NV12).  process, process_clip, submit_host and process_host then take [S, T, H * 3 // 2, W],
+        and the clips are NV12 frames too."""
         self._lib = _lib.load()
         self._ctx = C.c_void_p()
         cfg = _lib.fm_config(
@@ -35,11 +39,14 @@ class MotionEngine:
             flags=(_lib.FLAG_KEEP_PLANES if keep_planes else 0) | (_lib.FLAG_NO_FUSED if no_fused else 0) |
             (_lib.FLAG_NO_UMMA if no_umma else 0) | (_lib.FLAG_UMMA_APRON if umma_apron else 0) | (_lib.FLAG_UMMA if umma else 0) |
             (_lib.FLAG_NO_ROWS if no_rows else 0) | (_lib.FLAG_UPSCALE if upscale else 0) |
-            (_lib.FLAG_DEVICE_CLIPS if device_clips else 0))
+            (_lib.FLAG_DEVICE_CLIPS if device_clips else 0) | (_lib.FLAG_NV12 if nv12 else 0))
         _lib.check(self._lib.fm_ctx_create(C.byref(cfg), C.byref(self._ctx)))
         self.device = device
         self.n_streams, self.max_frames = n_streams, max_frames
         self.W, self.H = frame_width, frame_height
+        self.nv12 = bool(nv12)
+        # shape of one input frame
+        self.frame_shape = (frame_height * 3 // 2, frame_width) if nv12 else (frame_height, frame_width, 3)
         inf = _lib.fm_info()
         _lib.check(self._lib.fm_ctx_info(self._ctx, C.byref(inf)))
         self.info = {f: getattr(inf, f) for f, _ in _lib.fm_info._fields_}
@@ -95,15 +102,20 @@ class MotionEngine:
         assert len(nv) == S and all(0 <= v <= T for v in nv), "n_valid: one count in [0, T] per stream"
         return (C.c_int32 * S)(*nv)
 
+    def _check_batch(self, shape):
+        """-> (S, T) of a batch [n_streams, T, *frame_shape]"""
+        assert len(shape) == 2 + len(self.frame_shape) and shape[0] == self.n_streams and \
+            tuple(shape[2:]) == self.frame_shape, f"frame geometry mismatch: want [{self.n_streams}, T, {self.frame_shape}]"
+        return shape[0], shape[1]
+
     def process(self, frames, sync=True, n_valid=None):
-        """frames: CUDA uint8 tensor [n_streams, T, H, W, 3] (BGR).  Returns the per-frame stats
-        as a structured numpy array [n_streams, T] (or the device tensor if sync=False).
+        """frames: CUDA uint8 tensor [n_streams, T, H, W, 3] (BGR; nv12: [n_streams, T, H * 3 // 2, W]).  Returns the
+        per-frame stats as a structured numpy array [n_streams, T] (or the device tensor if sync=False).
         n_valid: optional per-stream count of real frames in this call (ragged batch)."""
         import torch
 
-        assert frames.is_cuda and frames.dtype == torch.uint8 and frames.dim() == 5, "uint8 CUDA [S,T,H,W,3]"
-        S, T, H, W, ch = frames.shape
-        assert (S, H, W, ch) == (self.n_streams, self.H, self.W, 3), "frame geometry mismatch"
+        assert frames.is_cuda and frames.dtype == torch.uint8, "uint8 CUDA frames"
+        S, T = self._check_batch(frames.shape)
         assert frames[0, 0].is_contiguous()
         need = S * T * STATS_DTYPE.itemsize
         if self._stats_dev is None or self._stats_dev.numel() < need:
@@ -120,25 +132,26 @@ class MotionEngine:
 
     def process_clip(self, frames, n_valid=None, out=None):
         """process() that also returns the frames the reference writes to its *_motion.avi in this call (needs
-        device_clips=True).  frames: CUDA uint8 tensor [n_streams, T, H, W, 3].  out: optional CUDA uint8 tensor
-        [n_streams, >= cache_frames + T, H, W, 3] (dense frames) for them; by default one of
-        [n_streams, cache_frames + max_frames, H, W, 3] is allocated once and reused, so the views returned by one call
-        are overwritten by the next.  Runs on the current torch stream and synchronises.
-        Returns (stats [n_streams, T], clips): clips[s] is a view [n_out, H, W, 3] of `out` holding, in order, the
+        device_clips=True).  frames: CUDA uint8 tensor [n_streams, T, *frame_shape] (frame_shape = (H, W, 3), or
+        (H * 3 // 2, W) with nv12).  out: optional CUDA uint8 tensor [n_streams, >= cache_frames + T, *frame_shape]
+        (dense frames) for them; by default one of [n_streams, cache_frames + max_frames, *frame_shape] is allocated once
+        and reused, so the views returned by one call are overwritten by the next.  Runs on the current torch stream and
+        synchronises.
+        Returns (stats [n_streams, T], clips): clips[s] is a view [n_out, *frame_shape] of `out` holding, in order, the
         cached frames each frame of stream s flushes and the frame itself where it is written."""
         import torch
 
-        assert frames.is_cuda and frames.dtype == torch.uint8 and frames.dim() == 5, "uint8 CUDA [S,T,H,W,3]"
-        S, T, H, W, ch = frames.shape
-        assert (S, H, W, ch) == (self.n_streams, self.H, self.W, 3), "frame geometry mismatch"
+        assert frames.is_cuda and frames.dtype == torch.uint8, "uint8 CUDA frames"
+        S, T = self._check_batch(frames.shape)
         assert frames[0, 0].is_contiguous()
         if out is None:
             if self._clips_out is None:
-                self._clips_out = torch.empty((S, self.info["cache_frames"] + self.max_frames, H, W, 3), dtype=torch.uint8,
-                                              device=frames.device)
+                self._clips_out = torch.empty((S, self.info["cache_frames"] + self.max_frames) + self.frame_shape,
+                                              dtype=torch.uint8, device=frames.device)
             out = self._clips_out
-        assert out.is_cuda and out.dtype == torch.uint8 and out.dim() == 5 and out.shape[0] == S and \
-            tuple(out.shape[2:]) == (H, W, 3) and out[0].is_contiguous(), "uint8 CUDA [S, capacity, H, W, 3]"
+        assert out.is_cuda and out.dtype == torch.uint8 and out.dim() == 2 + len(self.frame_shape) and \
+            out.shape[0] == S and tuple(out.shape[2:]) == self.frame_shape and out[0].is_contiguous(), \
+            "uint8 CUDA [S, capacity, *frame_shape]"
         need = S * T * STATS_DTYPE.itemsize
         if self._stats_dev is None or self._stats_dev.numel() < need:
             self._stats_dev = torch.empty(S * self.max_frames * STATS_DTYPE.itemsize, dtype=torch.uint8,
@@ -168,11 +181,10 @@ class MotionEngine:
         return frames, frames.ctypes.data, frames.shape, frames.strides[0], frames.strides[1]
 
     def submit_host(self, slot, frames, n_valid=None):
-        """Pipelined host entry: enqueue the batch [n_streams, T, H, W, 3] (host array / pinned tensor) on slot 0 or 1
-        and return; wait_host(slot) gives its stats.  The buffer must stay untouched until then."""
+        """Pipelined host entry: enqueue the batch [n_streams, T, *frame_shape] (host array / pinned tensor) on slot 0
+        or 1 and return; wait_host(slot) gives its stats.  The buffer must stay untouched until then."""
         frames, ptr, shape, s0, s1 = self._host_view(frames)
-        S, T, H, W, ch = shape
-        assert (S, H, W, ch) == (self.n_streams, self.H, self.W, 3), "frame geometry mismatch"
+        S, T = self._check_batch(shape)
         _lib.check(self._lib.fm_submit_host(self._ctx, slot, C.c_void_p(ptr), s0, s1, T, self._nvalid(n_valid, S, T)))
         self._inflight[slot] = (T, frames)          # keeps the buffer alive
 
@@ -188,11 +200,10 @@ class MotionEngine:
         return out
 
     def process_host(self, frames):
-        """frames: host uint8 array / pinned tensor [n_streams, T, H, W, 3].  Copies in, runs,
+        """frames: host uint8 array / pinned tensor [n_streams, T, *frame_shape].  Copies in, runs,
         copies the stats out (the end-to-end call of the drop-in adapter)."""
         frames, ptr, shape, s0, s1 = self._host_view(frames)
-        S, T, H, W, ch = shape
-        assert (S, H, W, ch) == (self.n_streams, self.H, self.W, 3), "frame geometry mismatch"
+        S, T = self._check_batch(shape)
         out = np.empty((S, T), STATS_DTYPE)
         _lib.check(self._lib.fm_process_host(self._ctx, C.c_void_p(ptr), s0, s1, T, C.c_void_p(out.ctypes.data)))
         return out

@@ -38,7 +38,7 @@ typedef struct fm_ctx fm_ctx;
 typedef struct fm_config {
     int32_t device;          /* CUDA device ordinal */
     int32_t n_streams;       /* streams batched in this context */
-    int32_t frame_width;     /* W of the raw BGR frames (CAP_PROP_FRAME_WIDTH) */
+    int32_t frame_width;     /* W of the raw BGR (or, with FM_FLAG_NV12, NV12) frames (CAP_PROP_FRAME_WIDTH) */
     int32_t frame_height;    /* H */
     int32_t max_frames;      /* most frames per stream a single fm_process call will carry (T_max) */
     int32_t fps;             /* --fps, default 30 (find_motion.py:1463) */
@@ -66,8 +66,19 @@ typedef struct fm_config {
                                    SURVEY.md A.1), bit-exact, as imutils.resize does it.  Without the flag such a
                                    configuration is refused with FM_ERANGE */
 #define FM_FLAG_DEVICE_CLIPS 256 /* keep the look-back cache of raw frames on the device (a ring of cache_frames frames per
-                                   stream, n_streams * cache_frames * H * W * 3 bytes) and accept fm_process_clip.  Every
+                                   stream, n_streams * cache_frames slots of the frame size rounded up to 256 bytes:
+                                   H * W * 3, or H * W * 3 / 2 with FM_FLAG_NV12) and accept fm_process_clip.  Every
                                    hot-path call then keeps that ring up to date, so they mix freely with fm_process_clip */
+#define FM_FLAG_NV12        512 /* the frames are NV12, as hardware video decoders emit them: (H + H/2) rows of W bytes, the H
+                                   luma rows, then H/2 rows of interleaved U, V bytes (U first); W and H even (FM_ERANGE
+                                   otherwise).  Every entry point that takes frames reads W*H*3/2 bytes per frame; strides keep
+                                   their meaning in bytes.  Results are those of a BGR context on cv2.cvtColor(frame,
+                                   COLOR_YUV2BGR_NV12): BT.601 fixed point, chroma of pixel (x, y) from UV row y/2, bytes
+                                   2(x/2) and 2(x/2)+1.  With FM_FLAG_DEVICE_CLIPS the ring and the clips hold the NV12 frames.
+                                   Memory: the fused full-resolution front end (fm_info.front_end == 0) reads NV12 itself; every
+                                   other front end reads the frames converted into a BGR slot the context allocates,
+                                   n_streams * max_frames * H * W * 3 bytes (796 MB for 8 x 16 frames of 1080p), so such a
+                                   context needs more device memory than a BGR one.  At most 65535 streams and max_frames */
 
 /* Derived parameters, exactly as the reference computes them (SURVEY.md A.0). */
 typedef struct fm_info {
@@ -122,7 +133,8 @@ int fm_version(void);
 /* Replaces VideoMotion.__init__ + _calc_min_area + _make_gaussian + _load_video
  * (find_motion.py:299-380, 402-424, 478-484) for n_streams streams.  box_size > frame_width (a processing plane larger
  * than the frame, which imutils.resize produces with cv2's INTER_AREA upscale) needs FM_FLAG_UPSCALE; without it
- * fm_ctx_create returns FM_ERANGE. */
+ * fm_ctx_create returns FM_ERANGE.  So does an odd frame width or height with FM_FLAG_NV12.  Both checks come before
+ * any device query. */
 int fm_ctx_create(const fm_config *cfg, fm_ctx **out);
 int fm_ctx_destroy(fm_ctx *ctx);
 int fm_ctx_info(const fm_ctx *ctx, fm_info *info);
@@ -139,7 +151,7 @@ int fm_ctx_reset(fm_ctx *ctx, int stream);
 
 /* The hot path: for every stream s < n_streams and t < n_frames (in order), run
  * blur_frame -> mask_off_areas -> find_diff -> find_movement -> decide_output on the BGR frame
- *   frames + s * stream_stride + t * frame_stride          (H*W*3 bytes, HWC, uint8)
+ *   frames + s * stream_stride + t * frame_stride          (H*W*3 bytes, HWC, uint8; FM_FLAG_NV12: H*W*3/2 bytes NV12)
  * `frames` is a DEVICE pointer; work is enqueued on `cuda_stream` (a cudaStream_t, 0 = default)
  * and the call returns without synchronising.  stats_dev, if not NULL, is a device buffer of
  * n_streams * n_frames fm_frame_stats ([stream][frame]) filled by the call. */
@@ -156,7 +168,7 @@ int fm_process_ragged(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, 
 /* fm_process_ragged that also hands out the frames the reference writes to its *_motion.avi in this call (needs
  * FM_FLAG_DEVICE_CLIPS).  For stream s, with n_out[s] = sum of wrote + n_flush over its valid frames, it writes
  * n_out[s] raw BGR frames densely to the DEVICE buffer
- *   out_dev + s * out_stream_stride + i * H*W*3          (i < n_out[s])
+ *   out_dev + s * out_stream_stride + i * H*W*3          (i < n_out[s]; FM_FLAG_NV12: NV12 frames, i * H*W*3/2)
  * in the reference's order: for each frame in order, the n_flush cached frames it flushes (oldest first, taken from the
  * device ring or from this call's input), then the frame itself if `wrote` (find_motion.py:561-570, 583).  n_out
  * follows from the stats.  out_capacity is the room per stream in frames and must be at least cache_frames + n_frames,
@@ -167,7 +179,8 @@ int fm_process_clip(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, si
                     uint8_t *out_dev, size_t out_stream_stride, int out_capacity);
 
 /* Same with HOST buffers: copies the frames host->device (pinned memory recommended), runs the
- * path, copies the stats back and synchronises.  This is the call a drop-in adapter makes. */
+ * path, copies the stats back and synchronises.  This is the call a drop-in adapter makes.  With FM_FLAG_NV12 a frame
+ * is H*W*3/2 bytes, half the host->device traffic of BGR. */
 int fm_process_host(fm_ctx *ctx, const uint8_t *frames_host, size_t stream_stride,
                     size_t frame_stride, int n_frames, fm_frame_stats *stats_host);
 
