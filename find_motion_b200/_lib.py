@@ -57,6 +57,8 @@ FLAG_NO_ROWS = 64
 FLAG_UPSCALE = 128
 FLAG_DEVICE_CLIPS = 256
 FLAG_NV12 = 512
+FLAG_OBJECT_PLANES = 1024
+OBJECT_WIDTH = 300
 
 # every symbol include/fm_gpu.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
@@ -71,6 +73,7 @@ SYMBOLS = {
     "fm_process": (C.c_int, [_P, _P, C.c_size_t, C.c_size_t, C.c_int, _P, _P]),
     "fm_process_ragged": (C.c_int, [_P, _P, C.c_size_t, C.c_size_t, C.c_int, _P, _P, _P]),
     "fm_process_clip": (C.c_int, [_P, _P, C.c_size_t, C.c_size_t, C.c_int, _P, _P, _P, _P, C.c_size_t, C.c_int]),
+    "fm_object_planes": (C.c_int, [_P, _P, _P, C.c_size_t, C.c_int]),
     "fm_process_host": (C.c_int, [_P, _P, C.c_size_t, C.c_size_t, C.c_int, _P]),
     "fm_submit_host": (C.c_int, [_P, C.c_int, _P, C.c_size_t, C.c_size_t, C.c_int, _P]),
     "fm_wait": (C.c_int, [_P, C.c_int, _P]),

@@ -122,6 +122,18 @@ struct fm_ctx {
     FmClipCopy *clip_list;     // gather list [S * (cache_frames + Tmax)], then store list [S * min(cache_frames, Tmax)]
     int *clip_count;           // [2] entries of the two lists in the current call
     int clip_sms;              // multiprocessors of the device (grid of the copy kernels)
+    // detector input planes (FM_FLAG_OBJECT_PLANES, k_objects.cu): W x H -> FM_OBJECT_WIDTH x obj_h
+    int obj_h;
+    int obj_mode;              // 1 tables, 2 integer ratio (identity: fx = fy = 1), 3 upscale
+    int obj_fx, obj_fy;
+    ResizeTab obj_xtab, obj_ytab;
+    int2 *obj_uxt, *obj_uyt;
+    struct RowsPlan *obj_rows;    // BGR-output plan of k_resize_rows; null: not applicable
+    int *obj_idx;              // [S][Tmax] plane index of each frame of the last call, -1 = no plane
+    uint8_t *obj_bgr;          // FM_FLAG_NV12 on the fused front end: [S][Tmax][H][W][3] the written frames converted
+    int obj_src;               // the last hot-path call: 0 none (or failed), 1 a device entry point, 2 a host entry point
+    const uint8_t *obj_frames; // ... and its frames, as the caller passed them
+    size_t obj_sstride, obj_fstride;
     // timing
     bool timing;               // time the kernel groups: events around them, or stamps with the fused front end (no sync inside fm_process)
     cudaEvent_t *evs;          // [FM_TIMING_RING][4]
@@ -231,18 +243,25 @@ int fm_launch_bg_export_wide(fm_ctx *c, int stream, double *dst_dev, cudaStream_
 int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
 size_t fm_fused_bg_doubles(const fm_ctx *c);
 int fm_launch_bg_export_fused(fm_ctx *c, int stream, double *dst_dev, cudaStream_t st);
-int fm_launch_resize_bgr(int device, const uint8_t *src_dev, int W, int H, int w, int h, int mode, int fx, int fy,
-                         const ResizeTab &xt, const ResizeTab &yt, uint8_t *dst_dev, cudaStream_t st);
+int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, int S, int T, int W, int H,
+                         int w, int h, int mode, int fx, int fy, const ResizeTab &xt, const ResizeTab &yt, const int *oidx,
+                         uint8_t *dst_dev, size_t ostride, cudaStream_t st);
 size_t fm_upscale_smem(int w);
 int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, int T, int F, int W, int H, int w,
                       int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
-                      cudaStream_t st);
+                      const int *oidx, size_t ostride, cudaStream_t st);
 int fm_rows_plan(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx);
 void fm_rows_free(fm_ctx *c);
 int fm_rows_plan_describe(int W, int w, int h, const int *xstart, const int *xidx, const float *xwt, const int *ystart,
                           const int *yidx, fm_rows_plan_info *out);
+int fm_rows_plan_objects(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx);
 bool fm_rows_usable(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride);
 int fm_launch_resize_rows(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
+int fm_launch_resize_rows_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
+                                  size_t ostride, cudaStream_t st);
+int fm_launch_resize_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
+                             size_t ostride, cudaStream_t st);
+int fm_launch_object_plan(fm_ctx *c, int T, cudaStream_t st);
 bool fm_umma_supported(const fm_ctx *c);
 bool fm_umma_preferred(const fm_ctx *c);
 int fm_umma_init(fm_ctx *c, const int *taps);
@@ -253,7 +272,8 @@ int fm_clips_alloc(fm_ctx *c);
 void fm_clips_free(fm_ctx *c);
 int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
                     size_t ostride, cudaStream_t st);
-int fm_launch_nv12_bgr(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
+int fm_launch_nv12_bgr(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, const int *oidx,
+                       uint8_t *bgr, cudaStream_t st);
 int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
 int fm_ccl_alloc(CclScratch *s, int frames, int h, int cap);
 void fm_ccl_free(CclScratch *s);

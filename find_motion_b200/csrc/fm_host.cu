@@ -200,6 +200,9 @@ extern "C" int fm_ctx_destroy(fm_ctx *c) {
     cudaFree(c->coef); cudaFree(c->wtab); cudaFree(c->uband); cudaFree(c->uband_f); cudaFree(c->gpad);
     cudaFree(c->g4start); cudaFree(c->g4n); cudaFree(c->g4off); cudaFree(c->g4w);
     cudaFree(c->uxt); cudaFree(c->uyt); cudaFree(c->nv12_bgr);
+    cudaFree(c->obj_xtab.start); cudaFree(c->obj_xtab.idx); cudaFree(c->obj_xtab.wt);
+    cudaFree(c->obj_ytab.start); cudaFree(c->obj_ytab.idx); cudaFree(c->obj_ytab.wt);
+    cudaFree(c->obj_uxt); cudaFree(c->obj_uyt); cudaFree(c->obj_idx); cudaFree(c->obj_bgr);
     fm_rows_free(c);
     fm_clips_free(c);
     cudaFree(c->xtab.start); cudaFree(c->xtab.idx); cudaFree(c->xtab.wt);
@@ -251,6 +254,12 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     if ((cfg->flags & FM_FLAG_NV12) && (cfg->n_streams > 65535 || cfg->max_frames > 65535)) {
         // the staging kernel's grid: one z index per stream, one y index per frame
         fm_set_error("NV12 contexts take at most 65535 streams and 65535 frames per call");
+        return FM_ERANGE;
+    }
+    // find_objects' input plane: imutils.resize(frame.raw, width=300) (find_motion.py:703-706)
+    const int obj_h = (int)((double)cfg->frame_height * (FM_OBJECT_WIDTH / (double)cfg->frame_width));
+    if ((cfg->flags & FM_FLAG_OBJECT_PLANES) && obj_h < 1) {
+        fm_set_error("detector input plane of %d x %d frames is %d x 0", cfg->frame_width, cfg->frame_height, FM_OBJECT_WIDTH);
         return FM_ERANGE;
     }
     int ndev = 0;
@@ -441,6 +450,32 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     const bool nv12_staged = !c->fused;
 #endif
     if ((cfg->flags & FM_FLAG_NV12) && nv12_staged) ALLOC(c->nv12_bgr, F * c->W * c->H * 3);
+    if (cfg->flags & FM_FLAG_OBJECT_PLANES) {
+        // W x H -> 300 x obj_h, dispatched as cv::resize(INTER_AREA) does it (and as fm_resize_area does)
+        const int ow = FM_OBJECT_WIDTH;
+        c->obj_h = obj_h;
+        if (ow < c->W) {
+            const double sx = 1.0 / ((double)ow / W), sy = 1.0 / ((double)obj_h / H);
+            const int isx = (int)nearbyint(sx), isy = (int)nearbyint(sy);
+            if (fabs(sx - isx) < 2.220446049250313e-16 && fabs(sy - isy) < 2.220446049250313e-16) {
+                c->obj_mode = 2; c->obj_fx = isx; c->obj_fy = isy;
+            } else {
+                c->obj_mode = 1;
+                const HostTab xt = area_tab(c->W, ow), yt = area_tab(c->H, obj_h);
+                if ((rc = upload_tab(&c->obj_xtab, xt)) || (rc = upload_tab(&c->obj_ytab, yt))) return fail(rc);
+                if ((rc = fm_rows_plan_objects(c, xt.start.data(), xt.idx.data(), xt.wt.data(), yt.start.data(), yt.idx.data())))
+                    return fail(rc);
+            }
+        } else if (ow == c->W) {                               // obj_h == H: the integer ratio 1 x 1 is a copy
+            c->obj_mode = 2; c->obj_fx = c->obj_fy = 1;
+        } else {
+            c->obj_mode = 3;
+            if ((rc = upload(&c->obj_uxt, upscale_tab(c->W, ow))) || (rc = upload(&c->obj_uyt, upscale_tab(c->H, obj_h))))
+                return fail(rc);
+        }
+        ALLOC(c->obj_idx, F * sizeof(int));
+        if ((cfg->flags & FM_FLAG_NV12) && !c->nv12_bgr) ALLOC(c->obj_bgr, F * c->W * c->H * 3);
+    }
     FM_TRY(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
     FM_TRY(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     for (int i = 0; i < 2; i++) {
@@ -553,6 +588,7 @@ static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_
     FM_CUDA(cudaSetDevice(c->cfg.device));
     cudaStream_t st = (cudaStream_t)cuda_stream;
     int rc;
+    c->obj_src = 0;
     {   // frames of each stream that are real in this call (uploaded only when the vector changes)
         bool changed = false;
         for (int s = 0; s < c->S; s++) {
@@ -581,7 +617,7 @@ static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_
     const uint8_t *fe = frames;
     size_t fe_sstride = stream_stride, fe_fstride = frame_stride;
     if (c->nv12_bgr) {
-        rc = fm_launch_nv12_bgr(c, frames, stream_stride, frame_stride, n_frames, st);
+        rc = fm_launch_nv12_bgr(c, frames, stream_stride, frame_stride, n_frames, nullptr, c->nv12_bgr, st);
         if (rc) { if (c->stamp) c->ev_pending--; c->stamp = nullptr; return rc; }
         fe = c->nv12_bgr;
         fe_fstride = (size_t)c->W * c->H * 3;
@@ -606,6 +642,8 @@ static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_
         return rc;
     c->last_T = n_frames;
     c->planes_valid = true;
+    c->obj_src = 1;
+    c->obj_frames = frames; c->obj_sstride = stream_stride; c->obj_fstride = frame_stride;
     return FM_OK;
 }
 
@@ -634,6 +672,42 @@ extern "C" int fm_process_clip(fm_ctx *c, const uint8_t *frames, size_t stream_s
 extern "C" int fm_process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
                           int n_frames, void *cuda_stream, fm_frame_stats *stats_dev) {
     return process(c, frames, stream_stride, frame_stride, n_frames, nullptr, cuda_stream, stats_dev, nullptr, 0);
+}
+
+extern "C" int fm_object_planes(fm_ctx *c, void *cuda_stream, uint8_t *out_dev, size_t out_stream_stride, int out_capacity) {
+    if (!c || !out_dev) { fm_set_error("null argument"); return FM_EINVAL; }
+    if (!(c->cfg.flags & FM_FLAG_OBJECT_PLANES)) {
+        fm_set_error("fm_object_planes needs a context created with FM_FLAG_OBJECT_PLANES");
+        return FM_EINVAL;
+    }
+    if (c->obj_src != 1) {
+        fm_set_error(c->obj_src == 2 ? "the last call came through fm_process_host / fm_submit_host: no device frames to resize"
+                                     : "no fm_process / fm_process_ragged / fm_process_clip call to take the planes from");
+        return FM_EINVAL;
+    }
+    const int T = c->last_T;
+    const size_t plane = (size_t)FM_OBJECT_WIDTH * c->obj_h * 3;
+    if (out_capacity < T) {
+        fm_set_error("out_capacity %d < n_frames %d of the last call (the most planes it can have)", out_capacity, T);
+        return FM_EINVAL;
+    }
+    if (c->S > 1 && out_stream_stride < (size_t)out_capacity * plane) {
+        fm_set_error("out_stream_stride %zu < out_capacity %d x %zu bytes per plane", out_stream_stride, out_capacity, plane);
+        return FM_EINVAL;
+    }
+    FM_CUDA(cudaSetDevice(c->cfg.device));
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    int rc;
+    if ((rc = fm_launch_object_plan(c, T, st))) return rc;
+    const uint8_t *src = c->obj_frames;
+    size_t sstride = c->obj_sstride, fstride = c->obj_fstride;
+    if (c->cfg.flags & FM_FLAG_NV12) {      // the call's frames as BGR, packed as a dense batch of the call (k_nv12.cu)
+        if (c->obj_bgr && (rc = fm_launch_nv12_bgr(c, src, sstride, fstride, T, c->obj_idx, c->obj_bgr, st))) return rc;
+        src = c->obj_bgr ? c->obj_bgr : c->nv12_bgr;
+        fstride = (size_t)c->W * c->H * 3;
+        sstride = fstride * T;
+    }
+    return fm_launch_resize_objects(c, src, sstride, fstride, T, out_dev, out_stream_stride, st);
 }
 
 // ---- host buffers: pipelined (submit / wait on two slots) and the blocking form built on it ----
@@ -682,6 +756,7 @@ extern "C" int fm_submit_host(fm_ctx *c, int slot, const uint8_t *frames_host, s
     FM_CUDA(cudaStreamWaitEvent(st, c->ev_copied[slot], 0));
     int rc = fm_process_ragged(c, dev, fb * (size_t)n_frames, fb, n_frames, n_valid, st, nullptr);
     if (rc) return rc;
+    c->obj_src = 2;                                       // fm_object_planes would read a staging buffer that gets reused
     const size_t sb = (size_t)c->S * n_frames * sizeof(fm_frame_stats);
     FM_CUDA(cudaMemcpyAsync(c->stats_pinned[slot], c->stats, sb, cudaMemcpyDeviceToHost, st));
     FM_CUDA(cudaMemcpyAsync(c->err_pinned + slot, c->errflag, sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -901,7 +976,7 @@ extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H,
         FM_CUDA(cudaMalloc(&dst.p, (size_t)width * h * 3));
         FM_CUDA(cudaMemcpy(src.p, bgr_host, (size_t)W * H * 3, cudaMemcpyHostToDevice));
         if ((rc = fm_launch_upscale(device, (const uint8_t *)src.p, 0, 0, 1, 1, W, H, width, h, ut.x, ut.y, nullptr, nullptr,
-                                    (uint8_t *)dst.p, 0)))
+                                    (uint8_t *)dst.p, nullptr, 0, 0)))
             return rc;
         FM_CUDA(cudaMemcpy(out_host, dst.p, (size_t)width * h * 3, cudaMemcpyDeviceToHost));
         return FM_OK;
@@ -922,8 +997,8 @@ extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H,
     FM_CUDA(cudaMalloc(&src.p, (size_t)W * H * 3));
     FM_CUDA(cudaMalloc(&dst.p, (size_t)width * h * 3));
     FM_CUDA(cudaMemcpy(src.p, bgr_host, (size_t)W * H * 3, cudaMemcpyHostToDevice));
-    if ((rc = fm_launch_resize_bgr(device, (const uint8_t *)src.p, W, H, width, h, fast ? 2 : 1, isx, isy, tb.x, tb.y,
-                                   (uint8_t *)dst.p, 0)))
+    if ((rc = fm_launch_resize_bgr(device, (const uint8_t *)src.p, 0, 0, 1, 1, W, H, width, h, fast ? 2 : 1, isx, isy, tb.x,
+                                   tb.y, nullptr, (uint8_t *)dst.p, 0, 0)))
         return rc;
     FM_CUDA(cudaMemcpy(out_host, dst.p, (size_t)width * h * 3, cudaMemcpyDeviceToHost));
     return FM_OK;

@@ -48,11 +48,15 @@ struct K0Params {
 #define K0_THREADS 512
 #define K0_GROUPS 4       // source rows in flight (K0_THREADS/K0_GROUPS threads each)
 
-__global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p) {
+// oidx (with bgr_out): null, or [F] plane index (-1: skip the frame); frame f's plane then goes to
+// bgr_out + s * ostride + oidx[f] * h*w*3 (fm_object_planes)
+__global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const int *__restrict__ oidx, size_t ostride) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int f = blockIdx.y;
     const int s = f / p.T, t = f - s * p.T;
     if (p.nvalid && t >= __ldg(p.nvalid + s)) return;
+    const int o = oidx ? __ldg(oidx + f) : 0;
+    if (o < 0) return;
     const int dy = blockIdx.x;
     const uint8_t *src = p.frames + (size_t)s * p.sstride + (size_t)t * p.fstride;
     const int rowbytes = p.W * 3;
@@ -157,8 +161,8 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p) {
     }
     __syncthreads();
     if (p.bgr_out) {
-        uint8_t *o = p.bgr_out + ((size_t)f * p.h + dy) * w3;
-        for (int i = tid; i < w3; i += K0_THREADS) o[i] = small[i];
+        uint8_t *out = p.bgr_out + (oidx ? (size_t)s * ostride + ((size_t)o * p.h + dy) * w3 : ((size_t)f * p.h + dy) * w3);
+        for (int i = tid; i < w3; i += K0_THREADS) out[i] = small[i];
         return;
     }
     uint8_t *g = p.gray + ((size_t)f * p.h + dy) * p.w;
@@ -166,12 +170,14 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p) {
         g[dx] = (uint8_t)fm_gray(small[dx * 3], small[dx * 3 + 1], small[dx * 3 + 2]);
 }
 
-// standalone INTER_AREA resize of one BGR frame (device buffers); mode / tables as fm_ctx_create derives them
-int fm_launch_resize_bgr(int device, const uint8_t *src_dev, int W, int H, int w, int h, int mode, int fx, int fy,
-                         const ResizeTab &xt, const ResizeTab &yt, uint8_t *dst_dev, cudaStream_t st) {
+// INTER_AREA resize to BGR (device buffers); mode / tables as fm_ctx_create derives them.  One frame (fm_resize_area:
+// S = T = 1, oidx null) or the frames of a call with an oidx table (fm_object_planes)
+int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, int S, int T, int W, int H,
+                         int w, int h, int mode, int fx, int fy, const ResizeTab &xt, const ResizeTab &yt, const int *oidx,
+                         uint8_t *dst_dev, size_t ostride, cudaStream_t st) {
     K0Params p;
-    p.frames = src_dev; p.sstride = 0; p.fstride = 0;
-    p.T = 1; p.W = W; p.H = H; p.w = w; p.h = h;
+    p.frames = src_dev; p.sstride = sstride; p.fstride = fstride;
+    p.T = T; p.W = W; p.H = H; p.w = w; p.h = h;
     p.mode = mode; p.fx = fx; p.fy = fy;
     p.xstart = xt.start; p.xidx = xt.idx; p.xwt = xt.wt;
     p.ystart = yt.start; p.yidx = yt.idx; p.ywt = yt.wt;
@@ -185,8 +191,8 @@ int fm_launch_resize_bgr(int device, const uint8_t *src_dev, int W, int H, int w
     }
     int rc;
     if ((rc = fm_ensure_smem((const void *)k_resize_gray, smem, device))) return rc;
-    dim3 grid(h, 1);
-    k_resize_gray<<<grid, K0_THREADS, smem, st>>>(p);
+    dim3 grid(h, S * T);
+    k_resize_gray<<<grid, K0_THREADS, smem, st>>>(p, oidx, ostride);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }
@@ -440,7 +446,7 @@ int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t 
     if (c->resize_mode == 3) {        // upscale + gray into the gray plane (k_upscale.cu)
         int rc;
         if ((rc = fm_launch_upscale(c->cfg.device, frames, sstride, fstride, T, F, c->W, c->H, c->w, c->h, c->uxt, c->uyt,
-                                    c->nvalid, c->gray, nullptr, st)))
+                                    c->nvalid, c->gray, nullptr, nullptr, 0, st)))
             return rc;
     } else {
         K0Params p;
@@ -500,7 +506,7 @@ int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t 
             int rc;
             if ((rc = fm_ensure_smem((const void *)k_resize_gray, smem, c->cfg.device))) return rc;
             dim3 grid(c->h, F);
-            k_resize_gray<<<grid, K0_THREADS, smem, st>>>(p);
+            k_resize_gray<<<grid, K0_THREADS, smem, st>>>(p, nullptr, 0);
             FM_LAUNCH_CHECK();
         }
     }

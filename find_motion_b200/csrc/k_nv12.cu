@@ -26,16 +26,18 @@ __device__ __forceinline__ void nv12_row8(uint2 yv, const FmChroma (&c)[4], uint
 }
 
 // One thread per (row pair, unit): VEC = 8 columns with 8-byte loads and stores (W % 8 == 0, 8-byte aligned frames and
-// strides), otherwise one 2 x 2 block with byte accesses.  blockIdx.y = frame t, blockIdx.z = stream s.
+// strides), otherwise one 2 x 2 block with byte accesses.  blockIdx.y = frame t, blockIdx.z = stream s.  oidx (the
+// detector input planes of a fused context, k_objects.cu): null, or [S][T] and only the frames with oidx >= 0 are converted.
 template <bool VEC>
 __global__ void __launch_bounds__(NV12_THREADS) k_nv12_bgr(const uint8_t *__restrict__ frames, size_t sstride, size_t fstride,
                                                            int T, int W, int H, const int *__restrict__ nvalid,
-                                                           uint8_t *__restrict__ bgr, unsigned long long *stamp) {
+                                                           const int *__restrict__ oidx, uint8_t *__restrict__ bgr,
+                                                           unsigned long long *stamp) {
     fm_stamp_start(stamp);
     const int t = blockIdx.y, s = blockIdx.z, f = s * T + t;
     const int cols = VEC ? W / 8 : W / 2;
     const int u = blockIdx.x * NV12_THREADS + threadIdx.x;
-    if (t < __ldg(nvalid + s) && u < cols * (H / 2)) {
+    if ((oidx ? __ldg(oidx + f) >= 0 : t < __ldg(nvalid + s)) && u < cols * (H / 2)) {
         const int yb = u / cols, x = (u - yb * cols) * (VEC ? 8 : 2);
         const uint8_t *src = frames + (size_t)s * sstride + (size_t)t * fstride;
         const uint8_t *l0 = src + (size_t)(2 * yb) * W + x, *l1 = l0 + W;
@@ -65,12 +67,13 @@ __global__ void __launch_bounds__(NV12_THREADS) k_nv12_bgr(const uint8_t *__rest
     fm_stamp_end(stamp);
 }
 
-int fm_launch_nv12_bgr(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
+int fm_launch_nv12_bgr(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, const int *oidx,
+                       uint8_t *bgr, cudaStream_t st) {
     const bool vec = c->W % 8 == 0 && ((((uintptr_t)frames) | sstride | fstride) & 7) == 0;
     const int units = (vec ? c->W / 8 : c->W / 2) * (c->H / 2);
     const dim3 grid((units + NV12_THREADS - 1) / NV12_THREADS, T, c->S);     // S, T <= 65535: fm_ctx_create
-    if (vec) k_nv12_bgr<true><<<grid, NV12_THREADS, 0, st>>>(frames, sstride, fstride, T, c->W, c->H, c->nvalid, c->nv12_bgr, c->stamp);
-    else k_nv12_bgr<false><<<grid, NV12_THREADS, 0, st>>>(frames, sstride, fstride, T, c->W, c->H, c->nvalid, c->nv12_bgr, c->stamp);
+    if (vec) k_nv12_bgr<true><<<grid, NV12_THREADS, 0, st>>>(frames, sstride, fstride, T, c->W, c->H, c->nvalid, oidx, bgr, c->stamp);
+    else k_nv12_bgr<false><<<grid, NV12_THREADS, 0, st>>>(frames, sstride, fstride, T, c->W, c->H, c->nvalid, oidx, bgr, c->stamp);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }

@@ -14,7 +14,8 @@
 // different bank groups.
 //   phase 1: thread = source row: horizontal chains of the chunk's columns -> hs[column, channel][row]   (float32)
 //   phase 2: thread = (destination row, column, channel): vertical chain over the rows of its cell -> BGR byte
-// and at the end of the segment the BGR bytes become gray bytes of the processing plane.
+// and at the end of the segment the BGR bytes become gray bytes of the processing plane (or, in the BGR variant, are stored
+// as they are: the detector input plane of fm_object_planes, k_objects.cu).
 #include <cuda.h>
 
 #include <algorithm>
@@ -50,6 +51,10 @@ struct RowsParams {
     const float *ywt;
     uint8_t *gray;
     const int *nvalid;
+    // BGR variant (detector input planes, k_objects.cu): frame f's plane goes to out + s * ostride + oidx[f] * h*w*3
+    const int *oidx;
+    uint8_t *out;
+    size_t ostride;
 };
 
 __device__ __forceinline__ uint4 rr_lds128(uint32_t addr) {
@@ -117,11 +122,17 @@ __device__ __forceinline__ void rr_bar_arrive(int id, int count) {
 // producer + vertical chains (phase 2) + gray.  Named barriers 1 + (i & 1): "hs of chunk i complete and stage i & 1 read"
 // (row warps arrive, warp 5 waits); 3 + (i & 1): "hs buffer i & 1 consumed" (warp 5 arrives, row warps wait before chunk
 // i + 2), so the row warps run up to two chunks ahead of the vertical warp and never wait for each other.
+// BGR: warp 5 stores the band's BGR bytes as they are (the detector input plane) for the frames with oidx >= 0.
+template <bool BGR>
 __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(const __grid_constant__ CUtensorMap tmap, RowsParams p) {
     extern __shared__ __align__(128) unsigned char rsm[];
     const int tid = threadIdx.x;
     const int f = blockIdx.z, s = f / p.T, t = f - s * p.T;
-    if (t >= __ldg(p.nvalid + s)) return;                   // not a real frame of this (ragged) call
+    if constexpr (BGR) {
+        if (__ldg(p.oidx + f) < 0) return;                  // no plane for this frame
+    } else {
+        if (t >= __ldg(p.nvalid + s)) return;               // not a real frame of this (ragged) call
+    }
     const int CX = p.CX, BW = p.BW, NRp = p.NRp;
     const int DXU = CX * p.NCHU;
     const int dy0 = blockIdx.y * p.D, dy1 = min(dy0 + p.D, p.h), Dn = dy1 - dy0;
@@ -224,24 +235,37 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
         }
     }
     __syncwarp();
-    // ---- BGR -> gray (SURVEY.md A.2) ----
-    for (int i = lane; i < Dn * dxun; i += 32) {
-        const int dyl = i / dxun, dxo = i - dyl * dxun;
-        const unsigned char *q = bgr + (dyl * DXU + dxo) * 3;
-        p.gray[((size_t)f * p.h + dy0 + dyl) * p.w + dxa + dxo] =
-            (uint8_t)fm_gray(q[0], q[1], q[2]);
+    if constexpr (BGR) {
+        uint8_t *o = p.out + (size_t)s * p.ostride + ((size_t)__ldg(p.oidx + f) * p.h + dy0) * p.w * 3 + (size_t)dxa * 3;
+        const int rb = dxun * 3;
+        for (int i = lane; i < Dn * rb; i += 32) {
+            const int dyl = i / rb, b = i - dyl * rb;
+            o[(size_t)dyl * p.w * 3 + b] = bgr[dyl * DXU * 3 + b];
+        }
+    } else {
+        // ---- BGR -> gray (SURVEY.md A.2) ----
+        for (int i = lane; i < Dn * dxun; i += 32) {
+            const int dyl = i / dxun, dxo = i - dyl * dxun;
+            const unsigned char *q = bgr + (dyl * DXU + dxo) * 3;
+            p.gray[((size_t)f * p.h + dy0 + dyl) * p.w + dxa + dxo] =
+                (uint8_t)fm_gray(q[0], q[1], q[2]);
+        }
     }
 }
 
 // ---------------------------------------------------------------------------------------------
 // host: plan + launch
 // ---------------------------------------------------------------------------------------------
-void fm_rows_free(fm_ctx *c) {
-    RowsPlan *r = c->rows;
+static void rr_free(RowsPlan *&r) {
     if (!r) return;
     cudaFree(r->coltab); cudaFree(r->cstartw); cudaFree(r->rw);
     delete r;
-    c->rows = nullptr;
+    r = nullptr;
+}
+
+void fm_rows_free(fm_ctx *c) {
+    rr_free(c->rows);
+    rr_free(c->obj_rows);
 }
 
 template <typename T>
@@ -335,24 +359,34 @@ static bool rr_layout(int W, int w, int h, const int *xstart, const int *xidx, c
     return (w >= 2 && layout(2) && r->smem <= 56 * 1024) || layout(1);
 }
 
-// Builds the plan of the rows kernel for the context's decimation tables; leaves c->rows null when the geometry does not fit
-// (rr_layout) or FM_FLAG_NO_ROWS is set.
-int fm_rows_plan(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx) {
-    c->rows = nullptr;
+// Builds the plan of a W -> w x h decimation into *out; leaves it null when the geometry does not fit (rr_layout) or
+// FM_FLAG_NO_ROWS is set.
+static int rr_build(fm_ctx *c, const void *kern, int w, int h, const int *xstart, const int *xidx, const float *xwt,
+                    const int *ystart, const int *yidx, RowsPlan **out) {
+    *out = nullptr;
     if (c->cfg.flags & FM_FLAG_NO_ROWS) return FM_OK;
     RowsPlan *r = new RowsPlan();
     std::vector<int4> col;
     std::vector<float4> rw;
     std::vector<int> cstartw;
-    if (!rr_layout(c->W, c->w, c->h, xstart, xidx, xwt, ystart, yidx, r, col, rw, cstartw)) { delete r; return FM_OK; }
+    if (!rr_layout(c->W, w, h, xstart, xidx, xwt, ystart, yidx, r, col, rw, cstartw)) { delete r; return FM_OK; }
     if (!rr_upload(&r->coltab, col) || !rr_upload(&r->cstartw, cstartw) || !rr_upload(&r->rw, rw)) {
         cudaFree(r->coltab); cudaFree(r->cstartw); cudaFree(r->rw);
         delete r;
         fm_set_error("resize plan: out of device memory");
         return FM_ENOMEM;
     }
-    c->rows = r;
-    return fm_ensure_smem((const void *)k_resize_rows, r->smem, c->cfg.device);
+    *out = r;
+    return fm_ensure_smem(kern, r->smem, c->cfg.device);
+}
+
+// the processing plane (gray out) and the detector input plane (BGR out)
+int fm_rows_plan(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx) {
+    return rr_build(c, (const void *)k_resize_rows<false>, c->w, c->h, xstart, xidx, xwt, ystart, yidx, &c->rows);
+}
+int fm_rows_plan_objects(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx) {
+    return rr_build(c, (const void *)k_resize_rows<true>, FM_OBJECT_WIDTH, c->obj_h, xstart, xidx, xwt, ystart, yidx,
+                    &c->obj_rows);
 }
 
 // Plan of a geometry without a device (include/fm_gpu.h: fm_debug_rows_plan): the layout plus a re-check, tap by tap, that
@@ -396,20 +430,32 @@ bool fm_rows_usable(const fm_ctx *c, const uint8_t *frames, size_t sstride, size
     return c->rows && ((((uintptr_t)frames) | sstride | fstride) & 15) == 0;
 }
 
-int fm_launch_resize_rows(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
-    const RowsPlan *r = c->rows;
+template <bool BGR>
+static int rr_launch(const fm_ctx *c, const RowsPlan *r, int w, int h, const ResizeTab &yt, const uint8_t *frames,
+                     size_t sstride, size_t fstride, int T, uint8_t *out, size_t ostride, cudaStream_t st) {
     CUtensorMap tmap;
     int rc = fm_frames_tmap(c, frames, sstride, fstride, T, r->BW / 4, r->NR, &tmap);
     if (rc) return rc;
     RowsParams p;
-    p.T = T; p.w = c->w; p.h = c->h;
+    p.T = T; p.w = w; p.h = h;
     p.D = r->D; p.NR = r->NR; p.NRp = r->NRp; p.CX = r->CX; p.NCHU = r->NCHU; p.BW = r->BW;
     p.stage_stride = r->stage_stride;
     p.coltab = r->coltab; p.cstartw = r->cstartw; p.rw = r->rw;
-    p.ystart = c->ytab.start; p.yidx = c->ytab.idx; p.ywt = c->ytab.wt;
+    p.ystart = yt.start; p.yidx = yt.idx; p.ywt = yt.wt;
     p.gray = c->gray; p.nvalid = c->nvalid;
+    p.oidx = c->obj_idx; p.out = out; p.ostride = ostride;
     dim3 grid(r->segs, r->nbands, c->S * T);
-    k_resize_rows<<<grid, RR_THREADS + 32, r->smem, st>>>(tmap, p);
+    k_resize_rows<BGR><<<grid, RR_THREADS + 32, r->smem, st>>>(tmap, p);
     FM_LAUNCH_CHECK();
     return FM_OK;
+}
+
+int fm_launch_resize_rows(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
+    return rr_launch<false>(c, c->rows, c->w, c->h, c->ytab, frames, sstride, fstride, T, nullptr, 0, st);
+}
+
+int fm_launch_resize_rows_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
+                                  size_t ostride, cudaStream_t st) {
+    return rr_launch<true>(c, c->obj_rows, FM_OBJECT_WIDTH, c->obj_h, c->obj_ytab, frames, sstride, fstride, T, out,
+                           ostride, st);
 }

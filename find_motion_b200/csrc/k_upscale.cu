@@ -26,6 +26,8 @@ struct UpParams {
     const int *nvalid;          // [S] real frames of each stream in this call (null: every frame)
     uint8_t *gray;              // [F][h][w]
     uint8_t *bgr_out;           // [F][h][w][3] resized BGR instead of gray (fm_resize_area: the detector input plane)
+    const int *oidx;            // with bgr_out: null, or [F] plane index (-1: skip the frame); frame f's plane then goes to
+    size_t ostride;             //   bgr_out + s * ostride + oidx[f] * h*w*3 (fm_object_planes)
 };
 
 // horizontal pass of one source row into a staged row of u16 (hx >> 4), 4 destination columns per thread
@@ -62,6 +64,9 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
     const int f = blockIdx.y;                    // s*T + t
     const int s = f / p.T, t = f - s * p.T;
     if (p.nvalid && t >= __ldg(p.nvalid + s)) return;
+    const int oi = p.oidx ? __ldg(p.oidx + f) : 0;
+    if (oi < 0) return;
+    const size_t obase = p.oidx ? (size_t)s * p.ostride + (size_t)oi * p.h * (size_t)(3 * p.w) : (size_t)f * p.h * (size_t)(3 * p.w);
     const uint8_t *src = p.frames + (size_t)s * p.sstride + (size_t)t * p.fstride;
     const size_t rowbytes = (size_t)p.W * 3;
     const int pitch = (3 * p.w + 3) & ~3;        // u16 per staged row (rows 8-byte aligned)
@@ -108,7 +113,7 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
 #pragma unroll
             for (int i = 0; i < 12; i++) v[i] = min((((b0 * h0[i]) >> 16) + ((b1 * h1[i]) >> 16) + 2u) >> 2, 255u);
             if (p.bgr_out) {
-                uint8_t *o = p.bgr_out + ((size_t)f * p.h + dy) * (size_t)(3 * p.w) + 12 * q;
+                uint8_t *o = p.bgr_out + obase + (size_t)dy * (size_t)(3 * p.w) + 12 * q;
                 if (n == 4 && (((uintptr_t)o) & 3) == 0) {
 #pragma unroll
                     for (int k = 0; k < 3; k++)
@@ -139,11 +144,12 @@ size_t fm_upscale_smem(int w) { return (size_t)2 * ((3 * (size_t)w + 3) & ~(size
 
 int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, int T, int F, int W, int H, int w,
                       int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
-                      cudaStream_t st) {
+                      const int *oidx, size_t ostride, cudaStream_t st) {
     UpParams p;
     p.frames = frames; p.sstride = sstride; p.fstride = fstride;
     p.T = T; p.W = W; p.H = H; p.w = w; p.h = h;
     p.xt = xt; p.yt = yt; p.nvalid = nvalid; p.gray = gray; p.bgr_out = bgr_out;
+    p.oidx = oidx; p.ostride = ostride;
     // taller bands re-read fewer source rows; shorter ones keep every SM busy when there are few frames
     int band = UP_BAND_MAX;
     while (band > 4 && (size_t)((h + band - 1) / band) * F < 4 * 148) band >>= 1;

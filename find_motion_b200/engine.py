@@ -20,7 +20,7 @@ class MotionEngine:
     def __init__(self, frame_width, frame_height, n_streams=1, max_frames=8, device=0, fps=30, box_size=100,
                  min_box_scale=50, cache_time=2.0, min_time=0.5, threshold=7, avg=0.1, blur_scale=20,
                  mask_areas=None, max_components=256, keep_planes=False, no_fused=False, no_umma=False, umma_apron=False, umma=False, no_rows=False,
-                 upscale=False, device_clips=False, nv12=False):
+                 upscale=False, device_clips=False, nv12=False, object_planes=False):
         """upscale: accept box_size > frame_width (cv2's INTER_AREA upscale, bit-exact, as imutils.resize does it);
         without it such a geometry raises, as in earlier releases.
         device_clips: keep the look-back cache of raw frames on the GPU (n_streams x cache_frames frames) so that
@@ -28,7 +28,9 @@ class MotionEngine:
         nv12: the frames are NV12 as GPU video decoders emit them, each [H * 3 // 2, W] uint8 (the luma rows, then the
         interleaved U, V rows; W and H even), with the results of a BGR engine on cv2.cvtColor(frame,
         cv2.COLOR_YUV2BGR_NV12).  process, process_clip, submit_host and process_host then take [S, T, H * 3 // 2, W],
-        and the clips are NV12 frames too."""
+        and the clips are NV12 frames too.
+        object_planes: accept object_planes(), the input planes of the reference's find_objects for the frames each
+        process / process_clip call writes (imutils.resize(frame.raw, width=300), made on the GPU)."""
         self._lib = _lib.load()
         self._ctx = C.c_void_p()
         cfg = _lib.fm_config(
@@ -39,7 +41,8 @@ class MotionEngine:
             flags=(_lib.FLAG_KEEP_PLANES if keep_planes else 0) | (_lib.FLAG_NO_FUSED if no_fused else 0) |
             (_lib.FLAG_NO_UMMA if no_umma else 0) | (_lib.FLAG_UMMA_APRON if umma_apron else 0) | (_lib.FLAG_UMMA if umma else 0) |
             (_lib.FLAG_NO_ROWS if no_rows else 0) | (_lib.FLAG_UPSCALE if upscale else 0) |
-            (_lib.FLAG_DEVICE_CLIPS if device_clips else 0) | (_lib.FLAG_NV12 if nv12 else 0))
+            (_lib.FLAG_DEVICE_CLIPS if device_clips else 0) | (_lib.FLAG_NV12 if nv12 else 0) |
+            (_lib.FLAG_OBJECT_PLANES if object_planes else 0))
         _lib.check(self._lib.fm_ctx_create(C.byref(cfg), C.byref(self._ctx)))
         self.device = device
         self.n_streams, self.max_frames = n_streams, max_frames
@@ -54,6 +57,10 @@ class MotionEngine:
         self.max_components = inf.max_components
         self._stats_dev = None
         self._clips_out = None
+        self._objects_out = None
+        self._last_T = None              # frames per stream of the last process / process_clip call
+        # shape of one detector input plane (find_objects: imutils.resize(frame.raw, width=300))
+        self.object_shape = (int(frame_height * (_lib.OBJECT_WIDTH / float(frame_width))), _lib.OBJECT_WIDTH, 3)
         self._inflight = {}
         if mask_areas:
             self.set_masks(mask_areas)
@@ -124,6 +131,7 @@ class MotionEngine:
         st = torch.cuda.current_stream(frames.device).cuda_stream
         _lib.check(self._lib.fm_process_ragged(self._ctx, frames.data_ptr(), frames.stride(0), frames.stride(1), T,
                                                self._nvalid(n_valid, S, T), C.c_void_p(st), self._stats_dev.data_ptr()))
+        self._last_T = T
         if not sync:
             return self._stats_dev[:need]
         host = self._stats_dev[:need].cpu().numpy()
@@ -160,10 +168,41 @@ class MotionEngine:
         _lib.check(self._lib.fm_process_clip(self._ctx, frames.data_ptr(), frames.stride(0), frames.stride(1), T,
                                              self._nvalid(n_valid, S, T), C.c_void_p(st), self._stats_dev.data_ptr(),
                                              out.data_ptr(), out.stride(0), out.shape[1]))
+        self._last_T = T
         stats = self._stats_dev[:need].cpu().numpy().view(STATS_DTYPE).reshape(S, T)
         self.check()
         n_out = (stats["wrote"].astype(np.int64) + stats["n_flush"]).sum(axis=1)
         return stats, [out[s, :int(n_out[s])] for s in range(S)]
+
+    def object_planes(self, out=None):
+        """The input planes of the reference's find_objects (find_motion.py:572, 703-706) for the frames the last
+        process / process_clip call wrote (needs object_planes=True): cv2.resize(raw, (300, oh), INTER_AREA) of each,
+        bit-exact, made on the GPU from that call's frames (which must still hold them).  NV12 engines resize
+        cv2.cvtColor(frame, COLOR_YUV2BGR_NV12).  out: optional CUDA uint8 tensor [n_streams, >= T, *object_shape]; by
+        default one of [n_streams, max_frames, *object_shape] is allocated once and reused, so the views returned by one
+        call are overwritten by the next.  Runs on the current torch stream and synchronises.
+        Returns, per stream, (frame_indices, planes): the indices t of the written frames in the call, in order, and a
+        view [len(frame_indices), *object_shape] of `out` holding their planes."""
+        import torch
+
+        dev = torch.device("cuda", self.device)
+        if out is None:
+            if self._objects_out is None:
+                self._objects_out = torch.empty((self.n_streams, self.max_frames) + self.object_shape, dtype=torch.uint8,
+                                                device=dev)
+            out = self._objects_out
+        assert out.is_cuda and out.dtype == torch.uint8 and out.dim() == 5 and out.shape[0] == self.n_streams and \
+            tuple(out.shape[2:]) == self.object_shape and out[0].is_contiguous(), "uint8 CUDA [S, capacity, oh, 300, 3]"
+        st = torch.cuda.current_stream(out.device).cuda_stream
+        _lib.check(self._lib.fm_object_planes(self._ctx, C.c_void_p(st), out.data_ptr(), out.stride(0), out.shape[1]))
+        T = self._last_T
+        stats = self._stats_dev[:self.n_streams * T * STATS_DTYPE.itemsize].cpu().numpy().view(STATS_DTYPE)
+        self.check()
+        res = []
+        for s, wrote in enumerate(stats.reshape(self.n_streams, T)["wrote"]):
+            idx = np.flatnonzero(wrote)
+            res.append((idx, out[s, :len(idx)]))
+        return res
 
     def check(self):
         """Synchronise and raise if a call since the last check hit a device-side capacity error."""

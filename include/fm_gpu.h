@@ -61,7 +61,8 @@ typedef struct fm_config {
 #define FM_FLAG_UMMA        32  /* take the tcgen05 one-pass Gaussian wherever it applies (3 <= k <= 97, w % 32 == 0); without
                                    either flag the library picks the faster path for the geometry (measured: DESIGN.md) */
 #define FM_FLAG_NO_ROWS     64  /* default (resize) mode: never take the row-per-lane INTER_AREA kernel (k_resize_rows.cu);
-                                   the warp-per-destination-row kernels instead (A/B testing) */
+                                   the warp-per-destination-row kernels instead (A/B testing); the same for the planes of
+                                   fm_object_planes */
 #define FM_FLAG_UPSCALE     128 /* accept box_size > frame_width: cv2's INTER_AREA upscale (a fixed-point linear interpolation,
                                    SURVEY.md A.1), bit-exact, as imutils.resize does it.  Without the flag such a
                                    configuration is refused with FM_ERANGE */
@@ -79,6 +80,14 @@ typedef struct fm_config {
                                    other front end reads the frames converted into a BGR slot the context allocates,
                                    n_streams * max_frames * H * W * 3 bytes (796 MB for 8 x 16 frames of 1080p), so such a
                                    context needs more device memory than a BGR one.  At most 65535 streams and max_frames */
+#define FM_FLAG_OBJECT_PLANES 1024 /* accept fm_object_planes: find_objects' detector input of every written frame, on the
+                                   device.  fm_ctx_create derives the plane height oh = int(H * (300 / float(W))) (imutils.resize,
+                                   FM_OBJECT_WIDTH wide) and builds the INTER_AREA tables of W x H -> 300 x oh once; oh < 1 is
+                                   refused with FM_ERANGE before any device query.  Memory: [S][max_frames] ints of plane
+                                   indices, and with FM_FLAG_NV12 on the fused front end (fm_info.front_end == 0) a BGR slot
+                                   of n_streams * max_frames * H * W * 3 bytes like the staged one.  The hot-path entry
+                                   points launch nothing more and return the same results with the flag */
+#define FM_OBJECT_WIDTH 300     /* width of the detector input plane (find_motion.py:703-706 hard-codes it) */
 
 /* Derived parameters, exactly as the reference computes them (SURVEY.md A.0). */
 typedef struct fm_info {
@@ -177,6 +186,19 @@ int fm_process_ragged(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, 
 int fm_process_clip(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
                     int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev,
                     uint8_t *out_dev, size_t out_stream_stride, int out_capacity);
+
+/* find_objects' input planes (find_motion.py:572, 703-706) of the last hot-path call made through fm_process,
+ * fm_process_ragged or fm_process_clip (needs FM_FLAG_OBJECT_PLANES).  The context remembers that call's frames, strides
+ * and n_frames.  For stream s, with n_obj[s] = the number of its valid frames with wrote == 1, it writes n_obj[s] dense
+ * BGR planes of oh x 300 x 3 bytes (oh as for FM_FLAG_OBJECT_PLANES), in frame order, to the DEVICE buffer
+ *   out_dev + s * out_stream_stride + i * oh*300*3          (i < n_obj[s])
+ * each byte-identical to cv2.resize(raw, (300, oh), interpolation=cv2.INTER_AREA) of the written frame (the upscale for
+ * W < 300, a copy for W == 300).  The masks do not apply (find_objects reads frame.raw).  NV12 contexts resize
+ * cv2.cvtColor(frame, COLOR_YUV2BGR_NV12).  out_capacity is the room per stream in planes and must be at least the last
+ * call's n_frames.  Asynchronous on `cuda_stream`: the last call's frames must stay untouched until the planes are
+ * written, as for the call itself.  FM_EINVAL without the flag, for a short out_capacity, before the first device-entry
+ * call, and after fm_process_host / fm_submit_host (their frames live in the context's staging buffers). */
+int fm_object_planes(fm_ctx *ctx, void *cuda_stream, uint8_t *out_dev, size_t out_stream_stride, int out_capacity);
 
 /* Same with HOST buffers: copies the frames host->device (pinned memory recommended), runs the
  * path, copies the stats back and synchronises.  This is the call a drop-in adapter makes.  With FM_FLAG_NV12 a frame
