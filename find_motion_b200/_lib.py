@@ -48,6 +48,11 @@ class fm_rows_plan_info(C.Structure):
                                          "smem_bytes", "bands", "segs", "max_groups")]
 
 
+class fm_frames(C.Structure):
+    _fields_ = [("data", C.c_void_p), ("stream_stride", C.c_size_t), ("frame_stride", C.c_size_t),
+                ("row_pitch", C.c_size_t), ("uv_offset", C.c_int64)]
+
+
 FLAG_KEEP_PLANES = 1
 FLAG_NO_FUSED = 2
 FLAG_NO_UMMA = 8
@@ -73,6 +78,7 @@ SYMBOLS = {
     "fm_process": (C.c_int, [_P, _P, C.c_size_t, C.c_size_t, C.c_int, _P, _P]),
     "fm_process_ragged": (C.c_int, [_P, _P, C.c_size_t, C.c_size_t, C.c_int, _P, _P, _P]),
     "fm_process_clip": (C.c_int, [_P, _P, C.c_size_t, C.c_size_t, C.c_int, _P, _P, _P, _P, C.c_size_t, C.c_int]),
+    "fm_process_frames": (C.c_int, [_P, C.POINTER(fm_frames), C.c_int, _P, _P, _P, _P, C.c_size_t, C.c_int]),
     "fm_object_planes": (C.c_int, [_P, _P, _P, C.c_size_t, C.c_int]),
     "fm_process_host": (C.c_int, [_P, _P, C.c_size_t, C.c_size_t, C.c_int, _P]),
     "fm_submit_host": (C.c_int, [_P, C.c_int, _P, C.c_size_t, C.c_size_t, C.c_int, _P]),

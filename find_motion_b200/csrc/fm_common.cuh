@@ -133,7 +133,8 @@ struct fm_ctx {
     uint8_t *obj_bgr;          // FM_FLAG_NV12 on the fused front end: [S][Tmax][H][W][3] the written frames converted
     int obj_src;               // the last hot-path call: 0 none (or failed), 1 a device entry point, 2 a host entry point
     const uint8_t *obj_frames; // ... and its frames, as the caller passed them
-    size_t obj_sstride, obj_fstride;
+    size_t obj_sstride, obj_fstride, obj_pitch;
+    int64_t obj_uv;
     // timing
     bool timing;               // time the kernel groups: events around them, or stamps with the fused front end (no sync inside fm_process)
     cudaEvent_t *evs;          // [FM_TIMING_RING][4]
@@ -217,16 +218,19 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32
                                     const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 PFN_encodeTiled fm_tma_encoder();
-// The call's frames as a 4-D u32 tensor map (W*3/4 words, H rows, T frames, S streams) with boxes of box_words x box_rows
-// (out-of-range elements are zero-filled).  FM_EINVAL unless the frames, their strides and rows are 16-byte aligned.
-int fm_frames_tmap(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, int box_words, int box_rows,
-                   CUtensorMap *out);
+// The call's frames as a 4-D u32 tensor map (W*3/4 words, H rows `pitch` bytes apart, T frames, S streams) with boxes of
+// box_words x box_rows (out-of-range elements, the row padding included, are zero-filled).  FM_EINVAL unless the frames,
+// their strides, the pitch and the rows are 16-byte aligned.
+int fm_frames_tmap(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int box_words,
+                   int box_rows, CUtensorMap *out);
 
-// stage launchers (each enqueues on `st`, returns FM_OK / error)
-int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T,
+// stage launchers (each enqueues on `st`, returns FM_OK / error).  Frame (s, t) of the frames a launcher reads starts at
+// frames + s * sstride + t * fstride, its rows are `pitch` bytes apart (W * 3 when packed) and, for NV12, its chroma plane
+// starts `uv` bytes from the frame start (pitch * H when packed).
+int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T,
                        cudaStream_t st);
 int fm_launch_temporal(fm_ctx *c, int T, cudaStream_t st);
-int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
+int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int64_t uv, int T, cudaStream_t st);
 int fm_ccl_configure(fm_ctx *c);
 int fm_launch_morph_ccl(fm_ctx *c, int T, cudaStream_t st, fm_frame_stats *stats_out);
 int fm_launch_masks(fm_ctx *c, int stream, int n_polys, const int *offs, const int *pts_scaled,
@@ -240,14 +244,14 @@ int fm_wide_init(fm_ctx *c, const int *taps);
 bool fm_wide_fused_supported(const fm_ctx *c);
 size_t fm_wide_bg_doubles(const fm_ctx *c);
 int fm_launch_bg_export_wide(fm_ctx *c, int stream, double *dst_dev, cudaStream_t st);
-int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
+int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st);
 size_t fm_fused_bg_doubles(const fm_ctx *c);
 int fm_launch_bg_export_fused(fm_ctx *c, int stream, double *dst_dev, cudaStream_t st);
-int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, int S, int T, int W, int H,
+int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, size_t pitch, int S, int T, int W, int H,
                          int w, int h, int mode, int fx, int fy, const ResizeTab &xt, const ResizeTab &yt, const int *oidx,
                          uint8_t *dst_dev, size_t ostride, cudaStream_t st);
 size_t fm_upscale_smem(int w);
-int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, int T, int F, int W, int H, int w,
+int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int F, int W, int H, int w,
                       int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
                       const int *oidx, size_t ostride, cudaStream_t st);
 int fm_rows_plan(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx);
@@ -255,26 +259,26 @@ void fm_rows_free(fm_ctx *c);
 int fm_rows_plan_describe(int W, int w, int h, const int *xstart, const int *xidx, const float *xwt, const int *ystart,
                           const int *yidx, fm_rows_plan_info *out);
 int fm_rows_plan_objects(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx);
-bool fm_rows_usable(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride);
-int fm_launch_resize_rows(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
-int fm_launch_resize_rows_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
+bool fm_rows_usable(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch);
+int fm_launch_resize_rows(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st);
+int fm_launch_resize_rows_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, uint8_t *out,
                                   size_t ostride, cudaStream_t st);
-int fm_launch_resize_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
+int fm_launch_resize_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, uint8_t *out,
                              size_t ostride, cudaStream_t st);
 int fm_launch_object_plan(fm_ctx *c, int T, cudaStream_t st);
 bool fm_umma_supported(const fm_ctx *c);
 bool fm_umma_preferred(const fm_ctx *c);
 int fm_umma_init(fm_ctx *c, const int *taps);
 size_t fm_umma_bg_doubles(const fm_ctx *c);
-int fm_launch_umma_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
+int fm_launch_umma_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st);
 int fm_launch_bg_export_umma(fm_ctx *c, int stream, double *dst_dev, cudaStream_t st);
 int fm_clips_alloc(fm_ctx *c);
 void fm_clips_free(fm_ctx *c);
-int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
+int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int64_t uv, int T, uint8_t *out,
                     size_t ostride, cudaStream_t st);
-int fm_launch_nv12_bgr(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, const int *oidx,
+int fm_launch_nv12_bgr(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int64_t uv, int T, const int *oidx,
                        uint8_t *bgr, cudaStream_t st);
-int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st);
+int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st);
 int fm_ccl_alloc(CclScratch *s, int frames, int h, int cap);
 void fm_ccl_free(CclScratch *s);
 int fm_ccl_plane(int device, const uint8_t *plane_host, int w, int h, int max_n, fm_component *out,

@@ -53,18 +53,18 @@ PFN_encodeTiled fm_tma_encoder() {
     return fn;
 }
 
-int fm_frames_tmap(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, int box_words, int box_rows,
-                   CUtensorMap *out) {
-    const size_t row = (size_t)c->W * 3, dense = row * c->H;
-    if ((((uintptr_t)frames) | sstride | fstride | row) & 15) {
-        fm_set_error("the TMA front ends need 16-byte aligned frames, strides and rows");
+int fm_frames_tmap(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int box_words,
+                   int box_rows, CUtensorMap *out) {
+    const size_t row = (size_t)c->W * 3, dense = pitch * c->H;
+    if ((((uintptr_t)frames) | sstride | fstride | pitch | row) & 15) {
+        fm_set_error("the TMA front ends need 16-byte aligned frames, strides and rows (row pitch %zu)", pitch);
         return FM_EINVAL;
     }
     PFN_encodeTiled enc = fm_tma_encoder();
     if (!enc) { fm_set_error("cuTensorMapEncodeTiled not available"); return FM_ECUDA; }
     // the stride of a dimension of extent 1 is never applied: the dense size stands in for it (the caller's may be 0)
     cuuint64_t dims[4] = {(cuuint64_t)row / 4, (cuuint64_t)c->H, (cuuint64_t)T, (cuuint64_t)c->S};
-    cuuint64_t strides[3] = {(cuuint64_t)row, (cuuint64_t)(T > 1 ? fstride : dense),
+    cuuint64_t strides[3] = {(cuuint64_t)pitch, (cuuint64_t)(T > 1 ? fstride : dense),
                              (cuuint64_t)(c->S > 1 ? sstride : (T > 1 ? fstride * T : dense))};
     cuuint32_t box[4] = {(cuuint32_t)box_words, (cuuint32_t)box_rows, 1, 1};
     cuuint32_t estr[4] = {1, 1, 1, 1};
@@ -577,9 +577,11 @@ static int timing_drain(fm_ctx *c) {
 }
 
 // out: the motion-clip frames of fm_process_clip (null from the other entry points, which with FM_FLAG_DEVICE_CLIPS
-// still keep the device ring up to date)
-static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride, int n_frames,
-                   const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev, uint8_t *out, size_t out_stride) {
+// still keep the device ring up to date).  pitch / uv: the row pitch and the chroma offset, resolved (packed: W*3, or W
+// and W*H with FM_FLAG_NV12)
+static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride, size_t pitch, int64_t uv,
+                   int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev, uint8_t *out,
+                   size_t out_stride) {
     if (!c || !frames) { fm_set_error("null argument"); return FM_EINVAL; }
     if (n_frames < 1 || n_frames > c->Tmax) {
         fm_set_error("n_frames %d outside [1, max_frames=%d]", n_frames, c->Tmax);
@@ -615,19 +617,20 @@ static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_
     // NV12 on the staged path: the BGR front end reads the call's frames converted into the context's slot, packed as a
     // dense BGR batch of the call; the device ring keeps the caller's NV12 frames
     const uint8_t *fe = frames;
-    size_t fe_sstride = stream_stride, fe_fstride = frame_stride;
+    size_t fe_sstride = stream_stride, fe_fstride = frame_stride, fe_pitch = pitch;
     if (c->nv12_bgr) {
-        rc = fm_launch_nv12_bgr(c, frames, stream_stride, frame_stride, n_frames, nullptr, c->nv12_bgr, st);
+        rc = fm_launch_nv12_bgr(c, frames, stream_stride, frame_stride, pitch, uv, n_frames, nullptr, c->nv12_bgr, st);
         if (rc) { if (c->stamp) c->ev_pending--; c->stamp = nullptr; return rc; }
         fe = c->nv12_bgr;
-        fe_fstride = (size_t)c->W * c->H * 3;
+        fe_pitch = (size_t)c->W * 3;
+        fe_fstride = fe_pitch * c->H;
         fe_sstride = fe_fstride * n_frames;
     }
     if (c->fused) {
-        rc = fm_launch_fused(c, fe, fe_sstride, fe_fstride, n_frames, st);
+        rc = fm_launch_fused(c, fe, fe_sstride, fe_fstride, fe_pitch, uv, n_frames, st);
         if (rc) { if (c->stamp) c->ev_pending--; c->stamp = nullptr; return rc; }
     } else {
-        if ((rc = fm_launch_frontend(c, fe, fe_sstride, fe_fstride, n_frames, st))) return rc;
+        if ((rc = fm_launch_frontend(c, fe, fe_sstride, fe_fstride, fe_pitch, n_frames, st))) return rc;
         if (ev) FM_CUDA(cudaEventRecord(ev[1], st));
         if (!c->wide_fused && !c->umma && (rc = fm_launch_temporal(c, n_frames, st))) return rc;
         if (ev) FM_CUDA(cudaEventRecord(ev[2], st));
@@ -638,40 +641,81 @@ static int process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_
     if (c->fused) c->slot ^= 1;
     if (ev) FM_CUDA(cudaEventRecord(ev[3], st));
     if ((c->cfg.flags & FM_FLAG_DEVICE_CLIPS) &&
-        (rc = fm_launch_clips(c, frames, stream_stride, frame_stride, n_frames, out, out_stride, st)))
+        (rc = fm_launch_clips(c, frames, stream_stride, frame_stride, pitch, uv, n_frames, out, out_stride, st)))
         return rc;
     c->last_T = n_frames;
     c->planes_valid = true;
     c->obj_src = 1;
     c->obj_frames = frames; c->obj_sstride = stream_stride; c->obj_fstride = frame_stride;
+    c->obj_pitch = pitch; c->obj_uv = uv;
     return FM_OK;
+}
+
+// Every device entry point: the layout checks of fm_process_frames, then the clip rules of fm_process_clip (clip_out
+// non-null), all before anything is enqueued
+extern "C" int fm_process_frames(fm_ctx *c, const fm_frames *fr, int n_frames, const int32_t *n_valid, void *cuda_stream,
+                                 fm_frame_stats *stats_dev, uint8_t *clip_out, size_t clip_stream_stride, int clip_capacity) {
+    if (!c || !fr || !fr->data) { fm_set_error("null argument"); return FM_EINVAL; }
+    const bool nv12 = (c->cfg.flags & FM_FLAG_NV12) != 0;
+    const size_t row = nv12 ? (size_t)c->W : (size_t)c->W * 3;
+    const size_t pitch = fr->row_pitch ? fr->row_pitch : row;
+    if (pitch < row) {
+        fm_set_error("row_pitch %zu < %zu bytes of a row", pitch, row);
+        return FM_EINVAL;
+    }
+    const int64_t luma = (int64_t)(pitch * (c->H - 1) + row);           // bytes the luma rows of a frame span
+    const int64_t uv = nv12 ? (fr->uv_offset ? fr->uv_offset : (int64_t)(pitch * c->H)) : 0;
+    if (nv12 && uv < luma && uv + (int64_t)(pitch * (c->H / 2 - 1) + row) > 0) {
+        fm_set_error("uv_offset %lld: the chroma plane overlaps the luma plane (rows %zu bytes apart, luma spans %lld bytes)",
+                     (long long)uv, pitch, (long long)luma);
+        return FM_EINVAL;
+    }
+    const bool packed = pitch == row && (!nv12 || uv == (int64_t)(row * c->H));
+    if (!packed && c->fused) {      // k_fused reads by TMA only: refused here, before the call changes anything
+        const uintptr_t a = (uintptr_t)fr->data | fr->stream_stride | fr->frame_stride | pitch;
+        if (a & 15) {
+            fm_set_error("the fused front end reads by TMA: data %p, stream_stride %zu, frame_stride %zu and row_pitch %zu "
+                         "must be multiples of 16", (const void *)fr->data, fr->stream_stride, fr->frame_stride, pitch);
+            return FM_EINVAL;
+        }
+        if (nv12 && ((uintptr_t)(fr->data + uv) & 15)) {
+            fm_set_error("the fused front end reads by TMA: data + uv_offset (%lld) must be 16-byte aligned", (long long)uv);
+            return FM_EINVAL;
+        }
+    }
+    if (clip_out) {
+        if (!(c->cfg.flags & FM_FLAG_DEVICE_CLIPS)) {
+            fm_set_error("fm_process_clip needs a context created with FM_FLAG_DEVICE_CLIPS");
+            return FM_EINVAL;
+        }
+        if ((long long)clip_capacity < (long long)c->info.cache_frames + n_frames) {
+            fm_set_error("out_capacity %d < cache_frames %d + n_frames %d (the most frames one call can write)", clip_capacity,
+                         c->info.cache_frames, n_frames);
+            return FM_EINVAL;
+        }
+    }
+    return process(c, fr->data, fr->stream_stride, fr->frame_stride, pitch, uv, n_frames, n_valid, cuda_stream, stats_dev,
+                   clip_out, clip_stream_stride);
 }
 
 extern "C" int fm_process_ragged(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
                                  int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev) {
-    return process(c, frames, stream_stride, frame_stride, n_frames, n_valid, cuda_stream, stats_dev, nullptr, 0);
+    const fm_frames fr = {frames, stream_stride, frame_stride, 0, 0};
+    return fm_process_frames(c, &fr, n_frames, n_valid, cuda_stream, stats_dev, nullptr, 0, 0);
 }
 
 extern "C" int fm_process_clip(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
                                int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev,
                                uint8_t *out_dev, size_t out_stream_stride, int out_capacity) {
     if (!c || !frames || !out_dev) { fm_set_error("null argument"); return FM_EINVAL; }
-    if (!(c->cfg.flags & FM_FLAG_DEVICE_CLIPS)) {
-        fm_set_error("fm_process_clip needs a context created with FM_FLAG_DEVICE_CLIPS");
-        return FM_EINVAL;
-    }
-    if ((long long)out_capacity < (long long)c->info.cache_frames + n_frames) {
-        fm_set_error("out_capacity %d < cache_frames %d + n_frames %d (the most frames one call can write)", out_capacity,
-                     c->info.cache_frames, n_frames);
-        return FM_EINVAL;
-    }
-    return process(c, frames, stream_stride, frame_stride, n_frames, n_valid, cuda_stream, stats_dev, out_dev,
-                   out_stream_stride);
+    const fm_frames fr = {frames, stream_stride, frame_stride, 0, 0};
+    return fm_process_frames(c, &fr, n_frames, n_valid, cuda_stream, stats_dev, out_dev, out_stream_stride, out_capacity);
 }
 
 extern "C" int fm_process(fm_ctx *c, const uint8_t *frames, size_t stream_stride, size_t frame_stride,
                           int n_frames, void *cuda_stream, fm_frame_stats *stats_dev) {
-    return process(c, frames, stream_stride, frame_stride, n_frames, nullptr, cuda_stream, stats_dev, nullptr, 0);
+    const fm_frames fr = {frames, stream_stride, frame_stride, 0, 0};
+    return fm_process_frames(c, &fr, n_frames, nullptr, cuda_stream, stats_dev, nullptr, 0, 0);
 }
 
 extern "C" int fm_object_planes(fm_ctx *c, void *cuda_stream, uint8_t *out_dev, size_t out_stream_stride, int out_capacity) {
@@ -700,14 +744,16 @@ extern "C" int fm_object_planes(fm_ctx *c, void *cuda_stream, uint8_t *out_dev, 
     int rc;
     if ((rc = fm_launch_object_plan(c, T, st))) return rc;
     const uint8_t *src = c->obj_frames;
-    size_t sstride = c->obj_sstride, fstride = c->obj_fstride;
+    size_t sstride = c->obj_sstride, fstride = c->obj_fstride, pitch = c->obj_pitch;
     if (c->cfg.flags & FM_FLAG_NV12) {      // the call's frames as BGR, packed as a dense batch of the call (k_nv12.cu)
-        if (c->obj_bgr && (rc = fm_launch_nv12_bgr(c, src, sstride, fstride, T, c->obj_idx, c->obj_bgr, st))) return rc;
+        if (c->obj_bgr && (rc = fm_launch_nv12_bgr(c, src, sstride, fstride, pitch, c->obj_uv, T, c->obj_idx, c->obj_bgr, st)))
+            return rc;
         src = c->obj_bgr ? c->obj_bgr : c->nv12_bgr;
-        fstride = (size_t)c->W * c->H * 3;
+        pitch = (size_t)c->W * 3;
+        fstride = pitch * c->H;
         sstride = fstride * T;
     }
-    return fm_launch_resize_objects(c, src, sstride, fstride, T, out_dev, out_stream_stride, st);
+    return fm_launch_resize_objects(c, src, sstride, fstride, pitch, T, out_dev, out_stream_stride, st);
 }
 
 // ---- host buffers: pipelined (submit / wait on two slots) and the blocking form built on it ----
@@ -975,7 +1021,7 @@ extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H,
         FM_CUDA(cudaMalloc(&src.p, (size_t)W * H * 3));
         FM_CUDA(cudaMalloc(&dst.p, (size_t)width * h * 3));
         FM_CUDA(cudaMemcpy(src.p, bgr_host, (size_t)W * H * 3, cudaMemcpyHostToDevice));
-        if ((rc = fm_launch_upscale(device, (const uint8_t *)src.p, 0, 0, 1, 1, W, H, width, h, ut.x, ut.y, nullptr, nullptr,
+        if ((rc = fm_launch_upscale(device, (const uint8_t *)src.p, 0, 0, (size_t)W * 3, 1, 1, W, H, width, h, ut.x, ut.y, nullptr, nullptr,
                                     (uint8_t *)dst.p, nullptr, 0, 0)))
             return rc;
         FM_CUDA(cudaMemcpy(out_host, dst.p, (size_t)width * h * 3, cudaMemcpyDeviceToHost));
@@ -997,7 +1043,7 @@ extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H,
     FM_CUDA(cudaMalloc(&src.p, (size_t)W * H * 3));
     FM_CUDA(cudaMalloc(&dst.p, (size_t)width * h * 3));
     FM_CUDA(cudaMemcpy(src.p, bgr_host, (size_t)W * H * 3, cudaMemcpyHostToDevice));
-    if ((rc = fm_launch_resize_bgr(device, (const uint8_t *)src.p, 0, 0, 1, 1, W, H, width, h, fast ? 2 : 1, isx, isy, tb.x,
+    if ((rc = fm_launch_resize_bgr(device, (const uint8_t *)src.p, 0, 0, (size_t)W * 3, 1, 1, W, H, width, h, fast ? 2 : 1, isx, isy, tb.x,
                                    tb.y, nullptr, (uint8_t *)dst.p, 0, 0)))
         return rc;
     FM_CUDA(cudaMemcpy(out_host, dst.p, (size_t)width * h * 3, cudaMemcpyDeviceToHost));

@@ -13,7 +13,9 @@
 // in one launch and the stores in the next.
 //
 // Launches: k_clip_plan (one CTA, one warp per stream) writes both copy lists, k_clip_gather runs the gather list, then
-// k_clip_store the store list.  Without the flag none of this runs.
+// k_clip_store the store list.  Without the flag none of this runs.  Calls whose frames have a row pitch or a chroma
+// offset of their own (fm_process_frames) run k_clip_gather_pitched / k_clip_store_pitched instead: entries that read an
+// input frame copy its rows into the packed ring slot or output frame, ring slots are copied whole as above.
 #include <algorithm>
 
 #include "fm_common.cuh"
@@ -149,6 +151,64 @@ __global__ void __launch_bounds__(CLIP_COPY_THREADS) k_clip_store(const FmClipCo
     clip_copy(list, count, fb);
 }
 
+// The row layout of a pitched call's input frames: rows of rowbytes, `pitch` apart; rows >= luma_rows (the NV12 chroma
+// rows) start at uv + (row - luma_rows) * pitch.  Sources inside [ring, ring_end) are ring slots, dense like the outputs.
+struct ClipRows {
+    size_t pitch, rowbytes;
+    int64_t uv;
+    int luma_rows, rows, rows_per_item;
+    const uint8_t *ring, *ring_end;
+};
+
+// n bytes by the whole CTA: 16-byte streaming accesses when source and destination agree mod 16, bytes otherwise
+__device__ __forceinline__ void clip_span(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, size_t n) {
+    if ((((uintptr_t)src ^ (uintptr_t)dst) & 15) == 0) {
+        const size_t head = min(n, (size_t)((16 - ((uintptr_t)dst & 15)) & 15));
+        const size_t nv = (n - head) / 16, tail0 = head + nv * 16;
+        if (threadIdx.x < head) dst[threadIdx.x] = src[threadIdx.x];
+        if (threadIdx.x < n - tail0) dst[tail0 + threadIdx.x] = src[tail0 + threadIdx.x];
+        const int4 *s4 = reinterpret_cast<const int4 *>(src + head);
+        int4 *d4 = reinterpret_cast<int4 *>(dst + head);
+        for (size_t v = threadIdx.x; v < nv; v += CLIP_COPY_THREADS) __stcs(d4 + v, __ldcs(s4 + v));
+    } else {
+        for (size_t b = threadIdx.x; b < n; b += CLIP_COPY_THREADS) dst[b] = __ldcs(src + b);
+    }
+}
+
+// clip_copy for pitched calls: item (entry, ch) is chunk ch of a ring slot, or rows ch * rows_per_item .. of an input frame
+__device__ __forceinline__ void clip_copy_pitched(const FmClipCopy *__restrict__ list, const int *__restrict__ count, size_t fb,
+                                                  const ClipRows &g) {
+    const size_t nch = max((fb + CLIP_CHUNK_BYTES - 1) / CLIP_CHUNK_BYTES,
+                           (size_t)((g.rows + g.rows_per_item - 1) / g.rows_per_item));
+    const size_t items = (size_t)__ldg(count) * nch;
+    for (size_t it = blockIdx.x; it < items; it += gridDim.x) {
+        const size_t e = it / nch, ch = it % nch;
+        const FmClipCopy cp = list[e];
+        if (cp.src >= g.ring && cp.src < g.ring_end) {
+            const size_t b0 = ch * CLIP_CHUNK_BYTES;
+            if (b0 < fb) clip_span(cp.src + b0, cp.dst + b0, min((size_t)CLIP_CHUNK_BYTES, fb - b0));
+        } else {
+            const int r0 = (int)ch * g.rows_per_item, r1 = min(g.rows, r0 + g.rows_per_item);
+            for (int r = r0; r < r1; r++) {
+                const uint8_t *s = r < g.luma_rows ? cp.src + (size_t)r * g.pitch
+                                                   : cp.src + g.uv + (ptrdiff_t)((size_t)(r - g.luma_rows) * g.pitch);
+                clip_span(s, cp.dst + (size_t)r * g.rowbytes, g.rowbytes);
+            }
+        }
+    }
+}
+
+__global__ void __launch_bounds__(CLIP_COPY_THREADS) k_clip_gather_pitched(const FmClipCopy *__restrict__ list,
+                                                                           const int *__restrict__ count, size_t fb,
+                                                                           ClipRows g) {
+    clip_copy_pitched(list, count, fb, g);
+}
+__global__ void __launch_bounds__(CLIP_COPY_THREADS) k_clip_store_pitched(const FmClipCopy *__restrict__ list,
+                                                                          const int *__restrict__ count, size_t fb,
+                                                                          ClipRows g) {
+    clip_copy_pitched(list, count, fb, g);
+}
+
 int fm_clips_alloc(fm_ctx *c) {
     const int C = c->info.cache_frames;
     const size_t fb = c->frame_bytes;
@@ -179,8 +239,8 @@ void fm_clips_free(fm_ctx *c) {
     cudaFree(c->clip_ring); cudaFree(c->clip_base); cudaFree(c->clip_list); cudaFree(c->clip_count);
 }
 
-int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
-                    size_t ostride, cudaStream_t st) {
+int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int64_t uv, int T,
+                    uint8_t *out, size_t ostride, cudaStream_t st) {
     const int C = c->info.cache_frames;
     if (!out && C == 0) return FM_OK;                    // nothing to gather and no ring to keep
     ClipPlanArgs a;
@@ -195,6 +255,27 @@ int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     a.count = c->clip_count;
     k_clip_plan<<<1, CLIP_PLAN_THREADS, 0, st>>>(a);
     FM_LAUNCH_CHECK();
+    const bool nv12 = (c->cfg.flags & FM_FLAG_NV12) != 0;
+    ClipRows g;
+    g.rowbytes = nv12 ? (size_t)c->W : (size_t)c->W * 3;
+    g.pitch = pitch; g.uv = uv;
+    g.luma_rows = c->H; g.rows = nv12 ? c->H + c->H / 2 : c->H;
+    g.rows_per_item = (int)std::max<size_t>(1, CLIP_CHUNK_BYTES / g.rowbytes);
+    g.ring = c->clip_ring; g.ring_end = c->clip_ring ? c->clip_ring + (size_t)c->S * C * c->clip_slot_bytes : nullptr;
+    if (pitch != g.rowbytes || (nv12 && uv != (int64_t)(g.rowbytes * c->H))) {
+        const size_t nch = std::max((a.fb + CLIP_CHUNK_BYTES - 1) / CLIP_CHUNK_BYTES,
+                                    (size_t)((g.rows + g.rows_per_item - 1) / g.rows_per_item));
+        auto grid = [&](size_t entries) { return (int)std::max<size_t>(1, std::min<size_t>(entries * nch, (size_t)c->clip_sms * 8)); };
+        if (out) {
+            k_clip_gather_pitched<<<grid((size_t)c->S * (C + T)), CLIP_COPY_THREADS, 0, st>>>(a.gather, a.count, a.fb, g);
+            FM_LAUNCH_CHECK();
+        }
+        if (C > 0) {
+            k_clip_store_pitched<<<grid((size_t)c->S * std::min(C, T)), CLIP_COPY_THREADS, 0, st>>>(a.store, a.count + 1, a.fb, g);
+            FM_LAUNCH_CHECK();
+        }
+        return FM_OK;
+    }
     // grid: enough CTAs to keep every SM streaming, never more than the largest list could use
     const size_t nch = (a.fb + CLIP_CHUNK_BYTES - 1) / CLIP_CHUNK_BYTES;
     auto grid = [&](size_t entries) { return (int)std::max<size_t>(1, std::min<size_t>(entries * nch, (size_t)c->clip_sms * 8)); };

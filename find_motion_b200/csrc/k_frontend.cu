@@ -3,9 +3,10 @@
 // Replaces VideoMotion.blur_frame + mask_off_areas (find_motion/find_motion.py:487-494, 619-635).
 #include "fm_common.cuh"
 
-// identity-resize mode: one thread per 4 pixels of a frame (12 bytes in, 4 bytes out)
+// identity-resize mode: one thread per 4 pixels of a frame (12 bytes in, 4 bytes out).  Pixel i = y * w + x of a frame
+// is at y * pitch + 3 x; packed rows (pitch == 3 w) are one flat run, so 4 pixels may then straddle a row end
 __global__ void __launch_bounds__(256) k_gray(const uint8_t *__restrict__ frames, size_t sstride,
-                                              size_t fstride, int T, int N, uint8_t *__restrict__ gray,
+                                              size_t fstride, size_t pitch, int T, int w, int N, uint8_t *__restrict__ gray,
                                               const int *__restrict__ nvalid) {
     int f = blockIdx.y;   // s*T + t
     int s = f / T, t = f - s * T;
@@ -14,12 +15,16 @@ __global__ void __launch_bounds__(256) k_gray(const uint8_t *__restrict__ frames
     uint8_t *dst = gray + (size_t)f * N;
     int i4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (i4 >= N) return;
-    if (i4 + 4 <= N && ((((uintptr_t)src) & 3) == 0) && ((((uintptr_t)dst) & 3) == 0)) {
-        const uint32_t *p = reinterpret_cast<const uint32_t *>(src + (size_t)i4 * 3);
+    const bool flat = pitch == (size_t)w * 3;
+    const int y4 = flat ? 0 : i4 / w, x4 = i4 - y4 * w;
+    const uint8_t *q4 = flat ? src + (size_t)i4 * 3 : src + (size_t)y4 * pitch + (size_t)x4 * 3;
+    if (i4 + 4 <= N && (flat || x4 + 4 <= w) && ((((uintptr_t)q4) & 3) == 0) && ((((uintptr_t)dst) & 3) == 0)) {
+        const uint32_t *p = reinterpret_cast<const uint32_t *>(q4);
         *reinterpret_cast<uint32_t *>(dst + i4) = fm_gray4(__ldg(p), __ldg(p + 1), __ldg(p + 2));
     } else {
         for (int i = i4; i < min(i4 + 4, N); i++) {
-            const uint8_t *p = src + (size_t)i * 3;
+            const int y = i / w;
+            const uint8_t *p = src + (size_t)y * pitch + (size_t)(i - y * w) * 3;
             dst[i] = (uint8_t)fm_gray(p[0], p[1], p[2]);
         }
     }
@@ -33,6 +38,7 @@ __global__ void __launch_bounds__(256) k_gray(const uint8_t *__restrict__ frames
 struct K0Params {
     const uint8_t *frames;
     size_t sstride, fstride;
+    size_t pitch;                // bytes from one source row to the next (>= W * 3)
     int T, W, H, w, h;
     int mode, fx, fy;            // 1 = tables, 2 = integer ratio
     const int *xstart, *xidx;
@@ -82,7 +88,7 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const in
         int mis = 0;
         if (j < ny) {
             int sy = (p.mode == 1) ? p.yidx[y0 + j] : dy * p.fy + j;
-            const uint8_t *row = src + (size_t)sy * rowbytes;
+            const uint8_t *row = src + (size_t)sy * p.pitch;
             mis = (int)((uintptr_t)row & 15);
             const uint4 *row16 = reinterpret_cast<const uint4 *>(row - mis);
             int n16 = (mis + rowbytes + 15) >> 4;
@@ -172,11 +178,11 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const in
 
 // INTER_AREA resize to BGR (device buffers); mode / tables as fm_ctx_create derives them.  One frame (fm_resize_area:
 // S = T = 1, oidx null) or the frames of a call with an oidx table (fm_object_planes)
-int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, int S, int T, int W, int H,
-                         int w, int h, int mode, int fx, int fy, const ResizeTab &xt, const ResizeTab &yt, const int *oidx,
+int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, size_t pitch, int S, int T, int W,
+                         int H, int w, int h, int mode, int fx, int fy, const ResizeTab &xt, const ResizeTab &yt, const int *oidx,
                          uint8_t *dst_dev, size_t ostride, cudaStream_t st) {
     K0Params p;
-    p.frames = src_dev; p.sstride = sstride; p.fstride = fstride;
+    p.frames = src_dev; p.sstride = sstride; p.fstride = fstride; p.pitch = pitch;
     p.T = T; p.W = W; p.H = H; p.w = w; p.h = h;
     p.mode = mode; p.fx = fx; p.fy = fy;
     p.xstart = xt.start; p.xidx = xt.idx; p.xwt = xt.wt;
@@ -232,7 +238,7 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_warp(K0Params p,
     for (int j = 0; j < ny; j++) {
         const int sy = p.yidx[y0 + j];
         const float beta = p.ywt[y0 + j];
-        const uint8_t *seg = src + (size_t)sy * rowbytes + b_lo;          // first needed byte
+        const uint8_t *seg = src + (size_t)sy * p.pitch + b_lo;           // first needed byte
         const int nbytes = b_hi - b_lo;
         const int mis = (int)((uintptr_t)seg & 15);
         const uint4 *seg16 = reinterpret_cast<const uint4 *>(seg - mis);
@@ -332,7 +338,7 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
     uint4 *dst16 = reinterpret_cast<uint4 *>(rowbuf);
     // software pipeline: the 16-byte blocks of row j+1 are loaded into registers while row j is reduced
     uint4 pre[PF];
-    auto seg_of = [&](int j) { return src + (size_t)p.yidx[y0 + j] * rowbytes + b_lo; };
+    auto seg_of = [&](int j) { return src + (size_t)p.yidx[y0 + j] * p.pitch + b_lo; };
     auto issue = [&](int j) {
         const uint8_t *seg = seg_of(j);
         const int mis = (int)((uintptr_t)seg & 15);
@@ -430,27 +436,28 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
     }
 }
 
-int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
+int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
     dim3 grid(((c->N + 3) / 4 + 255) / 256, c->S * T);
-    k_gray<<<grid, 256, 0, st>>>(frames, sstride, fstride, T, c->N, c->gray, c->nvalid);
+    k_gray<<<grid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->w, c->N, c->gray, c->nvalid);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }
 
-int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T,
+int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T,
                        cudaStream_t st) {
     const int F = c->S * T;
     // every Gaussian the fused stencil does not take goes to the tensor-core blur (k_wide.cu)
     if (c->resize_mode == 0)          // gray fused into the first kernel of the blur
-        return c->umma ? fm_launch_umma_blur(c, frames, sstride, fstride, T, st) : fm_launch_wide_blur(c, frames, sstride, fstride, T, st);
+        return c->umma ? fm_launch_umma_blur(c, frames, sstride, fstride, pitch, T, st)
+                       : fm_launch_wide_blur(c, frames, sstride, fstride, pitch, T, st);
     if (c->resize_mode == 3) {        // upscale + gray into the gray plane (k_upscale.cu)
         int rc;
-        if ((rc = fm_launch_upscale(c->cfg.device, frames, sstride, fstride, T, F, c->W, c->H, c->w, c->h, c->uxt, c->uyt,
+        if ((rc = fm_launch_upscale(c->cfg.device, frames, sstride, fstride, pitch, T, F, c->W, c->H, c->w, c->h, c->uxt, c->uyt,
                                     c->nvalid, c->gray, nullptr, nullptr, 0, st)))
             return rc;
     } else {
         K0Params p;
-        p.frames = frames; p.sstride = sstride; p.fstride = fstride;
+        p.frames = frames; p.sstride = sstride; p.fstride = fstride; p.pitch = pitch;
         p.T = T; p.W = c->W; p.H = c->H; p.w = c->w; p.h = c->h;
         p.mode = c->resize_mode; p.fx = c->fx; p.fy = c->fy;
         p.xstart = c->xtab.start; p.xidx = c->xtab.idx; p.xwt = c->xtab.wt;
@@ -458,10 +465,10 @@ int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t 
         p.max_ytaps = c->resize_mode == 1 ? c->ytab.max_taps : c->fy;
         p.gray = c->gray; p.nvalid = c->nvalid; p.bgr_out = nullptr;
         int rowpitch = (c->W * 3 + 16 + 15) & ~15;
-        if (c->resize_mode == 1 && fm_rows_usable(c, frames, sstride, fstride)) {
+        if (c->resize_mode == 1 && fm_rows_usable(c, frames, sstride, fstride, pitch)) {
             // one source row per lane, TMA-staged (k_resize_rows.cu)
             int rc;
-            if ((rc = fm_launch_resize_rows(c, frames, sstride, fstride, T, st))) return rc;
+            if ((rc = fm_launch_resize_rows(c, frames, sstride, fstride, pitch, T, st))) return rc;
         } else if (c->resize_mode == 1) {
             // one warp per (frame, destination row, group of <= 32 destination columns)
             int nq = (c->w + 31) / 32, dxw = (c->w + nq - 1) / nq;
@@ -470,7 +477,7 @@ int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t 
             int rc;
             if ((rc = fm_ensure_smem((const void *)k_resize_gray_warp, smemw, c->cfg.device))) return rc;
             int tasks = c->h * F * nq;
-            const bool aligned4 = ((((uintptr_t)frames) | sstride | fstride | ((size_t)c->W * 3)) & 3) == 0;
+            const bool aligned4 = ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->W * 3)) & 3) == 0;
             if (aligned4 && c->g4w) {
                 if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, true>, smemw, c->cfg.device))) return rc;
                 if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, false>, smemw, c->cfg.device))) return rc;
@@ -510,5 +517,5 @@ int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t 
             FM_LAUNCH_CHECK();
         }
     }
-    return c->umma ? fm_launch_umma_blur(c, nullptr, 0, 0, T, st) : fm_launch_wide_blur(c, nullptr, 0, 0, T, st);
+    return c->umma ? fm_launch_umma_blur(c, nullptr, 0, 0, 0, T, st) : fm_launch_wide_blur(c, nullptr, 0, 0, 0, T, st);
 }

@@ -507,14 +507,15 @@ extern "C" void fm_k1_prof_dump(void) {
 
 #define FUSED_SMEM (2 * RAW_STAGE + FH_ROWS * FG_WORDS * 4 + FH_ROWS * FH_WORDS * 4 + 16)
 
-// one plane of the call's NV12 frames (rows of W bytes) as a 4-D u32 tensor map with boxes of NV_PITCH bytes x box_rows
-static int nv12_plane_tmap(const fm_ctx *c, const uint8_t *plane, int rows, size_t sstride, size_t fstride, int T,
+// one plane of the call's NV12 frames (rows of W bytes, `pitch` bytes apart) as a 4-D u32 tensor map with boxes of
+// NV_PITCH bytes x box_rows
+static int nv12_plane_tmap(const fm_ctx *c, const uint8_t *plane, int rows, size_t sstride, size_t fstride, size_t pitch, int T,
                            int box_rows, CUtensorMap *out) {
     PFN_encodeTiled enc = fm_tma_encoder();
     if (!enc) { fm_set_error("cuTensorMapEncodeTiled not available"); return FM_ECUDA; }
     const size_t dense = c->frame_bytes;        // stands in for the stride of a dimension of extent 1 (never applied)
     cuuint64_t dims[4] = {(cuuint64_t)c->W / 4, (cuuint64_t)rows, (cuuint64_t)T, (cuuint64_t)c->S};
-    cuuint64_t strides[3] = {(cuuint64_t)c->W, (cuuint64_t)(T > 1 ? fstride : dense),
+    cuuint64_t strides[3] = {(cuuint64_t)pitch, (cuuint64_t)(T > 1 ? fstride : dense),
                              (cuuint64_t)(c->S > 1 ? sstride : (T > 1 ? fstride * T : dense))};
     cuuint32_t box[4] = {NV_PITCH / 4, (cuuint32_t)box_rows, 1, 1};
     cuuint32_t estr[4] = {1, 1, 1, 1};
@@ -524,19 +525,20 @@ static int nv12_plane_tmap(const fm_ctx *c, const uint8_t *plane, int rows, size
     return FM_OK;
 }
 
-int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
+int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int64_t uv, int T,
+                    cudaStream_t st) {
     CUtensorMap tmap, tmap_uv;
     const bool nv12 = c->nv12_bgr == nullptr && (c->cfg.flags & FM_FLAG_NV12);     // NV12 read directly (no staged slot)
     int rc;
     if (nv12) {
-        if ((((uintptr_t)frames) | sstride | fstride) & 15) {
-            fm_set_error("the fused NV12 front end needs 16-byte aligned frames and strides");
+        if ((((uintptr_t)frames) | sstride | fstride | pitch | (size_t)uv) & 15) {
+            fm_set_error("the fused NV12 front end needs 16-byte aligned frames, strides, row pitch and chroma offset");
             return FM_EINVAL;
         }
-        if ((rc = nv12_plane_tmap(c, frames, c->H, sstride, fstride, T, FG_ROWS, &tmap))) return rc;
-        if ((rc = nv12_plane_tmap(c, frames + (size_t)c->W * c->H, c->H / 2, sstride, fstride, T, FG_ROWS / 2, &tmap_uv))) return rc;
+        if ((rc = nv12_plane_tmap(c, frames, c->H, sstride, fstride, pitch, T, FG_ROWS, &tmap))) return rc;
+        if ((rc = nv12_plane_tmap(c, frames + uv, c->H / 2, sstride, fstride, pitch, T, FG_ROWS / 2, &tmap_uv))) return rc;
     } else {
-        if ((rc = fm_frames_tmap(c, frames, sstride, fstride, T, RAW_PITCH / 4, FG_ROWS, &tmap))) return rc;
+        if ((rc = fm_frames_tmap(c, frames, sstride, fstride, pitch, T, RAW_PITCH / 4, FG_ROWS, &tmap))) return rc;
         tmap_uv = tmap;                          // not read
     }
     FusedParams p;

@@ -25,12 +25,13 @@ __device__ __forceinline__ void nv12_row8(uint2 yv, const FmChroma (&c)[4], uint
     dst[2] = make_uint2(o[4], o[5]);
 }
 
-// One thread per (row pair, unit): VEC = 8 columns with 8-byte loads and stores (W % 8 == 0, 8-byte aligned frames and
-// strides), otherwise one 2 x 2 block with byte accesses.  blockIdx.y = frame t, blockIdx.z = stream s.  oidx (the
+// One thread per (row pair, unit): VEC = 8 columns with 8-byte loads and stores (W % 8 == 0, 8-byte aligned frames,
+// strides, pitch and chroma offset), otherwise one 2 x 2 block with byte accesses.  Luma row y of a frame is at y * pitch,
+// chroma row y at uv + y * pitch.  blockIdx.y = frame t, blockIdx.z = stream s.  oidx (the
 // detector input planes of a fused context, k_objects.cu): null, or [S][T] and only the frames with oidx >= 0 are converted.
 template <bool VEC>
 __global__ void __launch_bounds__(NV12_THREADS) k_nv12_bgr(const uint8_t *__restrict__ frames, size_t sstride, size_t fstride,
-                                                           int T, int W, int H, const int *__restrict__ nvalid,
+                                                           size_t pitch, int64_t uv_off, int T, int W, int H, const int *__restrict__ nvalid,
                                                            const int *__restrict__ oidx, uint8_t *__restrict__ bgr,
                                                            unsigned long long *stamp) {
     fm_stamp_start(stamp);
@@ -40,8 +41,8 @@ __global__ void __launch_bounds__(NV12_THREADS) k_nv12_bgr(const uint8_t *__rest
     if ((oidx ? __ldg(oidx + f) >= 0 : t < __ldg(nvalid + s)) && u < cols * (H / 2)) {
         const int yb = u / cols, x = (u - yb * cols) * (VEC ? 8 : 2);
         const uint8_t *src = frames + (size_t)s * sstride + (size_t)t * fstride;
-        const uint8_t *l0 = src + (size_t)(2 * yb) * W + x, *l1 = l0 + W;
-        const uint8_t *uv = src + (size_t)(H + yb) * W + x;
+        const uint8_t *l0 = src + (size_t)(2 * yb) * pitch + x, *l1 = l0 + pitch;
+        const uint8_t *uv = src + uv_off + (ptrdiff_t)((size_t)yb * pitch + x);
         uint8_t *d0 = bgr + (((size_t)f * H + 2 * yb) * W + x) * 3, *d1 = d0 + (size_t)W * 3;
         if (VEC) {
             const uint2 cv = __ldg(reinterpret_cast<const uint2 *>(uv));
@@ -67,13 +68,13 @@ __global__ void __launch_bounds__(NV12_THREADS) k_nv12_bgr(const uint8_t *__rest
     fm_stamp_end(stamp);
 }
 
-int fm_launch_nv12_bgr(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, const int *oidx,
-                       uint8_t *bgr, cudaStream_t st) {
-    const bool vec = c->W % 8 == 0 && ((((uintptr_t)frames) | sstride | fstride) & 7) == 0;
+int fm_launch_nv12_bgr(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int64_t uv, int T,
+                       const int *oidx, uint8_t *bgr, cudaStream_t st) {
+    const bool vec = c->W % 8 == 0 && ((((uintptr_t)frames) | sstride | fstride | pitch | (size_t)uv) & 7) == 0;
     const int units = (vec ? c->W / 8 : c->W / 2) * (c->H / 2);
     const dim3 grid((units + NV12_THREADS - 1) / NV12_THREADS, T, c->S);     // S, T <= 65535: fm_ctx_create
-    if (vec) k_nv12_bgr<true><<<grid, NV12_THREADS, 0, st>>>(frames, sstride, fstride, T, c->W, c->H, c->nvalid, oidx, bgr, c->stamp);
-    else k_nv12_bgr<false><<<grid, NV12_THREADS, 0, st>>>(frames, sstride, fstride, T, c->W, c->H, c->nvalid, oidx, bgr, c->stamp);
+    if (vec) k_nv12_bgr<true><<<grid, NV12_THREADS, 0, st>>>(frames, sstride, fstride, pitch, uv, T, c->W, c->H, c->nvalid, oidx, bgr, c->stamp);
+    else k_nv12_bgr<false><<<grid, NV12_THREADS, 0, st>>>(frames, sstride, fstride, pitch, uv, T, c->W, c->H, c->nvalid, oidx, bgr, c->stamp);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }

@@ -38,14 +38,14 @@ int fm_launch_object_plan(fm_ctx *c, int T, cudaStream_t st) {
     return FM_OK;
 }
 
-int fm_launch_resize_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
-                             size_t ostride, cudaStream_t st) {
+int fm_launch_resize_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T,
+                             uint8_t *out, size_t ostride, cudaStream_t st) {
     const int w = FM_OBJECT_WIDTH, h = c->obj_h;
     if (c->obj_mode == 3)
-        return fm_launch_upscale(c->cfg.device, frames, sstride, fstride, T, c->S * T, c->W, c->H, w, h, c->obj_uxt,
+        return fm_launch_upscale(c->cfg.device, frames, sstride, fstride, pitch, T, c->S * T, c->W, c->H, w, h, c->obj_uxt,
                                  c->obj_uyt, nullptr, nullptr, out, c->obj_idx, ostride, st);
-    if (c->obj_rows && ((((uintptr_t)frames) | sstride | fstride) & 15) == 0)
-        return fm_launch_resize_rows_objects(c, frames, sstride, fstride, T, out, ostride, st);
-    return fm_launch_resize_bgr(c->cfg.device, frames, sstride, fstride, c->S, T, c->W, c->H, w, h, c->obj_mode, c->obj_fx,
+    if (c->obj_rows && ((((uintptr_t)frames) | sstride | fstride | pitch) & 15) == 0)
+        return fm_launch_resize_rows_objects(c, frames, sstride, fstride, pitch, T, out, ostride, st);
+    return fm_launch_resize_bgr(c->cfg.device, frames, sstride, fstride, pitch, c->S, T, c->W, c->H, w, h, c->obj_mode, c->obj_fx,
                                 c->obj_fy, c->obj_xtab, c->obj_ytab, c->obj_idx, out, ostride, st);
 }

@@ -426,15 +426,15 @@ int fm_rows_plan_describe(int W, int w, int h, const int *xstart, const int *xid
     return FM_OK;
 }
 
-bool fm_rows_usable(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride) {
-    return c->rows && ((((uintptr_t)frames) | sstride | fstride) & 15) == 0;
+bool fm_rows_usable(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch) {
+    return c->rows && ((((uintptr_t)frames) | sstride | fstride | pitch) & 15) == 0;
 }
 
 template <bool BGR>
 static int rr_launch(const fm_ctx *c, const RowsPlan *r, int w, int h, const ResizeTab &yt, const uint8_t *frames,
-                     size_t sstride, size_t fstride, int T, uint8_t *out, size_t ostride, cudaStream_t st) {
+                     size_t sstride, size_t fstride, size_t pitch, int T, uint8_t *out, size_t ostride, cudaStream_t st) {
     CUtensorMap tmap;
-    int rc = fm_frames_tmap(c, frames, sstride, fstride, T, r->BW / 4, r->NR, &tmap);
+    int rc = fm_frames_tmap(c, frames, sstride, fstride, pitch, T, r->BW / 4, r->NR, &tmap);
     if (rc) return rc;
     RowsParams p;
     p.T = T; p.w = w; p.h = h;
@@ -450,12 +450,13 @@ static int rr_launch(const fm_ctx *c, const RowsPlan *r, int w, int h, const Res
     return FM_OK;
 }
 
-int fm_launch_resize_rows(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
-    return rr_launch<false>(c, c->rows, c->w, c->h, c->ytab, frames, sstride, fstride, T, nullptr, 0, st);
+int fm_launch_resize_rows(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T,
+                          cudaStream_t st) {
+    return rr_launch<false>(c, c->rows, c->w, c->h, c->ytab, frames, sstride, fstride, pitch, T, nullptr, 0, st);
 }
 
-int fm_launch_resize_rows_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, uint8_t *out,
-                                  size_t ostride, cudaStream_t st) {
-    return rr_launch<true>(c, c->obj_rows, FM_OBJECT_WIDTH, c->obj_h, c->obj_ytab, frames, sstride, fstride, T, out,
+int fm_launch_resize_rows_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T,
+                                  uint8_t *out, size_t ostride, cudaStream_t st) {
+    return rr_launch<true>(c, c->obj_rows, FM_OBJECT_WIDTH, c->obj_h, c->obj_ytab, frames, sstride, fstride, pitch, T, out,
                            ostride, st);
 }

@@ -551,7 +551,7 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
 // (find_motion.py:493, SURVEY.md A.2).  One thread = 4 padded pixels.
 // ---------------------------------------------------------------------------------------------
 template <bool BGR>
-__global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ src, size_t sstride, size_t fstride, int T,
+__global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ src, size_t sstride, size_t fstride, size_t rpitch, int T,
                                                   uint8_t *__restrict__ gpad, int w, int h, int Wp, int Hp,
                                                   const int *__restrict__ nvalid, int aligned4) {
     const int f = blockIdx.z, s = f / T, t = f - s * T;
@@ -561,7 +561,7 @@ __global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ sr
     uint32_t out = 0;
     if (yp < h + 2 * UB_PAD && xp < w + 2 * UB_PAD) {
         const int y = fm_reflect101(yp - UB_PAD, h);
-        const uint8_t *row = BGR ? src + (size_t)s * sstride + (size_t)t * fstride + (size_t)y * w * 3
+        const uint8_t *row = BGR ? src + (size_t)s * sstride + (size_t)t * fstride + (size_t)y * rpitch
                                  : src + ((size_t)f * h + y) * w;
         const int x = xp - UB_PAD;
         if (x >= 0 && x + 3 < w && aligned4) {
@@ -700,16 +700,16 @@ extern "C" void fm_umma_prof_dump(void) {
 }
 
 // full-resolution mode, BGR frames straight into the tcgen05 kernel
-static int launch_umma_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
+static int launch_umma_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
     int tilesX, tilesY, Wp, Hp;
     umma_geom(c, &tilesX, &tilesY, &Wp, &Hp);
     if (c->cfg.flags & FM_FLAG_KEEP_PLANES) {              // parity tap of the gray conversion
-        int rc = fm_launch_gray_plane(c, frames, sstride, fstride, T, st);
+        int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
         if (rc) return rc;
     }
     const int RA = c->umma_ra;
     CUtensorMap tmap;
-    int rc = fm_frames_tmap(c, frames, sstride, fstride, T, 3 * (UB_T + 2 * RA) / 4, RA == 16 ? UfGeom<16>::RC : UfGeom<48>::RC, &tmap);
+    int rc = fm_frames_tmap(c, frames, sstride, fstride, pitch, T, 3 * (UB_T + 2 * RA) / 4, RA == 16 ? UfGeom<16>::RC : UfGeom<48>::RC, &tmap);
     if (rc) return rc;
     UfParams q;
     umma_params(c, T, tilesX, tilesY, q.u);
@@ -728,9 +728,12 @@ static int launch_umma_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, s
     return FM_OK;
 }
 
-// frames != nullptr: full-resolution mode (BGR -> padded gray in one kernel); else the resized gray plane c->gray
-int fm_launch_umma_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
-    if (frames && c->umma_direct && !(c->cfg.flags & FM_FLAG_UMMA_APRON)) return launch_umma_fused(c, frames, sstride, fstride, T, st);
+// frames != nullptr: full-resolution mode (BGR -> padded gray in one kernel); else the resized gray plane c->gray.  Pitched
+// rows that TMA cannot read (not 16-byte aligned) take the apron plane; packed ones keep the direct kernel's refusal.
+int fm_launch_umma_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
+    const bool tma_ok = pitch == (size_t)c->W * 3 || ((((uintptr_t)frames) | sstride | fstride | pitch) & 15) == 0;
+    if (frames && c->umma_direct && !(c->cfg.flags & FM_FLAG_UMMA_APRON) && tma_ok)
+        return launch_umma_fused(c, frames, sstride, fstride, pitch, T, st);
     if (!c->gpad) {                     // first call that needs the apron plane (A/B flag on a direct-capable context)
         FM_CUDA(cudaStreamSynchronize(st));
         FM_CUDA(cudaMalloc((void **)&c->gpad, fm_umma_pad_bytes(c)));
@@ -741,14 +744,14 @@ int fm_launch_umma_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t
     dim3 pgrid((Wp / 4 + 255) / 256, Hp, F);
     if (frames) {
         if (c->cfg.flags & FM_FLAG_KEEP_PLANES) {          // parity tap of the gray conversion
-            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, T, st);
+            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
             if (rc) return rc;
         }
-        const int al = ((((uintptr_t)frames) | sstride | fstride | ((size_t)c->w * 3)) & 3) == 0;
-        k_pad_gray<true><<<pgrid, 256, 0, st>>>(frames, sstride, fstride, T, c->gpad, c->w, c->h, Wp, Hp, c->nvalid, al);
+        const int al = ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->w * 3)) & 3) == 0;
+        k_pad_gray<true><<<pgrid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->gpad, c->w, c->h, Wp, Hp, c->nvalid, al);
     } else {
         const int al = (c->w & 3) == 0;
-        k_pad_gray<false><<<pgrid, 256, 0, st>>>(c->gray, 0, 0, T, c->gpad, c->w, c->h, Wp, Hp, c->nvalid, al);
+        k_pad_gray<false><<<pgrid, 256, 0, st>>>(c->gray, 0, 0, 0, T, c->gpad, c->w, c->h, Wp, Hp, c->nvalid, al);
     }
     FM_LAUNCH_CHECK();
     CUtensorMap tmap;

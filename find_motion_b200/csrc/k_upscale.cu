@@ -19,6 +19,7 @@
 struct UpParams {
     const uint8_t *frames;
     size_t sstride, fstride;
+    size_t pitch;               // bytes from one source row to the next (>= W * 3)
     int T, W, H, w, h;
     int band;                   // destination rows per CTA
     const int2 *xt;             // [w] (source x, a0 | a1 << 16)
@@ -68,7 +69,7 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
     if (oi < 0) return;
     const size_t obase = p.oidx ? (size_t)s * p.ostride + (size_t)oi * p.h * (size_t)(3 * p.w) : (size_t)f * p.h * (size_t)(3 * p.w);
     const uint8_t *src = p.frames + (size_t)s * p.sstride + (size_t)t * p.fstride;
-    const size_t rowbytes = (size_t)p.W * 3;
+    const size_t rowbytes = p.pitch;
     const int pitch = (3 * p.w + 3) & ~3;        // u16 per staged row (rows 8-byte aligned)
     uint16_t *rows = reinterpret_cast<uint16_t *>(smem);    // [2][pitch]: source row y lives in slot y & 1
     const int dy0 = blockIdx.x * p.band, dy1 = min(dy0 + p.band, p.h);
@@ -142,11 +143,11 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
 
 size_t fm_upscale_smem(int w) { return (size_t)2 * ((3 * (size_t)w + 3) & ~(size_t)3) * sizeof(uint16_t); }
 
-int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, int T, int F, int W, int H, int w,
-                      int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
+int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int F, int W, int H,
+                      int w, int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
                       const int *oidx, size_t ostride, cudaStream_t st) {
     UpParams p;
-    p.frames = frames; p.sstride = sstride; p.fstride = fstride;
+    p.frames = frames; p.sstride = sstride; p.fstride = fstride; p.pitch = pitch;
     p.T = T; p.W = W; p.H = H; p.w = w; p.h = h;
     p.xt = xt; p.yt = yt; p.nvalid = nvalid; p.gray = gray; p.bgr_out = bgr_out;
     p.oidx = oidx; p.ostride = ostride;

@@ -141,7 +141,7 @@ __device__ __forceinline__ void wide_h_mirror(unsigned char *tile, int X0, int w
 // padded row 32 G + rr) with register-staged global loads.  BGR: the BGR -> gray conversion is fused in. ----
 template <bool BGR>
 __device__ __forceinline__ void wide_h_stage(unsigned char *tile, const uint8_t *__restrict__ src, size_t sstride, size_t fstride,
-                                             int T, int f, int G, int X0, int w, int h, int r, int R16, int pitch) {
+                                             size_t rpitch, int T, int f, int G, int X0, int w, int h, int r, int R16, int pitch) {
     const int tid = threadIdx.x, lane = tid & 31, wq = tid >> 5;
     if (BGR) {
         // warp wq: rows wq, wq+8, wq+16, wq+24; lane: a unit of 16 pixels = 48 BGR bytes (three 128-bit loads); the
@@ -149,7 +149,7 @@ __device__ __forceinline__ void wide_h_stage(unsigned char *tile, const uint8_t 
         const uint8_t *fr = src + (size_t)(f / T) * sstride + (size_t)(f % T) * fstride;
         const uint8_t *rp[4];
 #pragma unroll
-        for (int i = 0; i < 4; i++) rp[i] = fr + (size_t)wrow(32 * G + wq + 8 * i - r, h) * (w * 3);
+        for (int i = 0; i < 4; i++) rp[i] = fr + (size_t)wrow(32 * G + wq + 8 * i - r, h) * rpitch;
         const int upr = pitch >> 4;
         const int xneed = min(X0 + WH_COLS, w) + r;           // first column no output of this CTA reads
         const bool mirror = R16 < w && R16 + r < WH_COLS;      // border columns are copies of staged columns (one reflection)
@@ -253,9 +253,11 @@ __device__ __forceinline__ void wide_h_products(const unsigned char *tile, const
 }
 
 // grid: (ceil(w / 256), NGa, F), 256 threads.  dynamic smem: 32 * pitch + (4 Sh + 3) * 256
-// BGR: src = the caller's frames (identity resize, 16-byte aligned rows); otherwise src = the gray plane [F][h][w].
+// BGR: src = the caller's frames (identity resize, 16-byte aligned rows rpitch bytes apart); otherwise src = the gray plane
+// [F][h][w].
 template <bool BGR>
-__global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h(const uint8_t *__restrict__ src, size_t sstride, size_t fstride, int T,
+__global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h(const uint8_t *__restrict__ src, size_t sstride, size_t fstride,
+                                                       size_t rpitch, int T,
                                                        uint32_t *__restrict__ plo, uint32_t *__restrict__ phi,
                                                        const uint2 *__restrict__ tabg, int w, int h, int r, int R16, int Sh,
                                                        int pitch, int NGa, const int *__restrict__ nvalid) {
@@ -266,7 +268,7 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h(const uint8_t *__restr
     const int f = blockIdx.z, G = blockIdx.y, X0 = blockIdx.x * WH_COLS;
     if (f % T >= __ldg(nvalid + f / T)) return;                             // not a real frame of this (ragged) call
     for (int i = tid; i < (4 * Sh + 3) * 32; i += WH_THREADS) tab[i] = __ldg(tabg + i);
-    wide_h_stage<BGR>(tile, src, sstride, fstride, T, f, G, X0, w, h, r, R16, pitch);
+    wide_h_stage<BGR>(tile, src, sstride, fstride, rpitch, T, f, G, X0, w, h, r, R16, pitch);
     __syncthreads();
     wide_h_products(tile, tab, f, G, X0, w, Sh, pitch, NGa, plo, phi);
 }
@@ -277,7 +279,8 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h(const uint8_t *__restr
 // that touch the top or bottom border need reflected rows and take the register-staged path.
 // dynamic smem: nbox * 32 * ubox * 48 (raw BGR)  +  32 * pitch  +  (4 Sh + 3) * 256  +  16
 __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_constant__ CUtensorMap tmap, const uint8_t *__restrict__ src,
-                                                           size_t sstride, size_t fstride, int T, uint32_t *__restrict__ plo,
+                                                           size_t sstride, size_t fstride, size_t rpitch, int T,
+                                                           uint32_t *__restrict__ plo,
                                                            uint32_t *__restrict__ phi, const uint2 *__restrict__ tabg, int w, int h,
                                                            int r, int R16, int Sh, int pitch, int NGa,
                                                            const int *__restrict__ nvalid, int nunits, int ubox, int nbox, int gp) {
@@ -336,7 +339,7 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_const
                 __syncthreads();
             }
         } else {
-            wide_h_stage<true>(tile, src, sstride, fstride, T, f, G, X0, w, h, r, R16, pitch);
+            wide_h_stage<true>(tile, src, sstride, fstride, rpitch, T, f, G, X0, w, h, r, R16, pitch);
             __syncthreads();
             if (more && tid == 0) issue(G + 1);                              // the raw stage is not in use
         }
@@ -688,10 +691,10 @@ __global__ void __launch_bounds__(256) k_blur_identity(const uint8_t *__restrict
 }
 
 // frames != nullptr: full-resolution mode, convert BGR -> gray while staging (no gray plane); else read c->gray
-int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, int T, cudaStream_t st) {
+int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
     if (c->k == 1) {
         if (frames) {
-            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, T, st);
+            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
             if (rc) return rc;
         }
         dim3 grid((c->w + 255) / 256, c->h, c->S * T);
@@ -712,10 +715,10 @@ int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t
     if ((rc = fm_ensure_smem((const void *)k_wide_h<false>, smh, c->cfg.device))) return rc;
     if ((rc = fm_ensure_smem((const void *)k_wide_v, smv, c->cfg.device))) return rc;
     dim3 hgrid((c->w + WH_COLS - 1) / WH_COLS, g.NGa, F);
-    const bool aligned16 = frames && ((((uintptr_t)frames) | sstride | fstride | ((size_t)c->w * 3)) & 15) == 0;
+    const bool aligned16 = frames && ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->w * 3)) & 15) == 0;
     if (aligned16) {
         if (c->cfg.flags & FM_FLAG_KEEP_PLANES) {
-            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, T, st);
+            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
             if (rc) return rc;
         }
         // TMA-staged pass 1 when the window of a CTA is one or two boxes and the CTA needs <= 100 KB (k <= ~200 at 1080p / 4K: k = 97 runs four CTAs
@@ -727,22 +730,22 @@ int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t
         static const long tma_kb = getenv("FM_WIDE_TMA_KB") ? atol(getenv("FM_WIDE_TMA_KB")) : 100;
         if (mirror && ubox <= 21 && smt <= (size_t)tma_kb * 1024) {
             CUtensorMap tmap;
-            if ((rc = fm_frames_tmap(c, frames, sstride, fstride, T, ubox * 12, 32, &tmap))) return rc;
+            if ((rc = fm_frames_tmap(c, frames, sstride, fstride, pitch, T, ubox * 12, 32, &tmap))) return rc;
             if ((rc = fm_ensure_smem((const void *)k_wide_h_tma, smt, c->cfg.device))) return rc;
             static const int gp = getenv("FM_WIDE_GP") ? std::max(1, atoi(getenv("FM_WIDE_GP"))) : 4;     // row groups per CTA (A/B: profiles/r2_wide_ab.txt)
             dim3 tgrid(hgrid.x, (g.NGa + gp - 1) / gp, F);
-            k_wide_h_tma<<<tgrid, WH_THREADS, smt, st>>>(tmap, frames, sstride, fstride, T, plo, phi, tabh, c->w, c->h, g.r, g.R16,
+            k_wide_h_tma<<<tgrid, WH_THREADS, smt, st>>>(tmap, frames, sstride, fstride, pitch, T, plo, phi, tabh, c->w, c->h, g.r, g.R16,
                                                          g.Sh, g.pitch, g.NGa, c->nvalid, nunits, ubox, nbox, gp);
         } else {
-            k_wide_h<true><<<hgrid, WH_THREADS, smh, st>>>(frames, sstride, fstride, T, plo, phi, tabh, c->w, c->h, g.r, g.R16,
+            k_wide_h<true><<<hgrid, WH_THREADS, smh, st>>>(frames, sstride, fstride, pitch, T, plo, phi, tabh, c->w, c->h, g.r, g.R16,
                                                            g.Sh, g.pitch, g.NGa, c->nvalid);
         }
     } else {
         if (frames) {
-            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, T, st);
+            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
             if (rc) return rc;
         }
-        k_wide_h<false><<<hgrid, WH_THREADS, smh, st>>>(c->gray, 0, 0, T, plo, phi, tabh, c->w, c->h, g.r, g.R16, g.Sh,
+        k_wide_h<false><<<hgrid, WH_THREADS, smh, st>>>(c->gray, 0, 0, 0, T, plo, phi, tabh, c->w, c->h, g.r, g.R16, g.Sh,
                                                         g.pitch, g.NGa, c->nvalid);
     }
     FM_LAUNCH_CHECK();

@@ -115,22 +115,54 @@ class MotionEngine:
             tuple(shape[2:]) == self.frame_shape, f"frame geometry mismatch: want [{self.n_streams}, T, {self.frame_shape}]"
         return shape[0], shape[1]
 
-    def process(self, frames, sync=True, n_valid=None):
-        """frames: CUDA uint8 tensor [n_streams, T, H, W, 3] (BGR; nv12: [n_streams, T, H * 3 // 2, W]).  Returns the
-        per-frame stats as a structured numpy array [n_streams, T] (or the device tensor if sync=False).
-        n_valid: optional per-stream count of real frames in this call (ragged batch)."""
+    def _device_batch(self, frames, chroma):
+        """-> (S, T, fm_frames or None) of a device batch.  None: every frame is packed (the plain entry points take the
+        batch).  Otherwise the rows are pitched (crop views, padded rows) or, with chroma, the NV12 planes are two views
+        of the same batch (luma [S, T, H, W] in frames, UV [S, T, H / 2, W] in chroma, e.g. slices of decoder surfaces)."""
         import torch
 
         assert frames.is_cuda and frames.dtype == torch.uint8, "uint8 CUDA frames"
+        if chroma is not None:
+            assert self.nv12, "chroma= is for nv12 engines"
+            assert chroma.is_cuda and chroma.dtype == torch.uint8 and chroma.device == frames.device, "uint8 CUDA chroma"
+            S, T = frames.shape[:2]
+            assert tuple(frames.shape) == (self.n_streams, T, self.H, self.W) and \
+                tuple(chroma.shape) == (self.n_streams, T, self.H // 2, self.W), \
+                f"want luma [{self.n_streams}, T, {self.H}, {self.W}] and chroma [{self.n_streams}, T, {self.H // 2}, {self.W}]"
+            assert frames.stride(-1) == 1 and chroma.stride() == frames.stride() and frames.stride(-2) >= self.W, \
+                "luma and chroma views need unit column strides and the same stream, frame and row strides"
+            assert chroma.data_ptr() != frames.data_ptr(), "the chroma plane starts at the luma plane"
+            return S, T, _lib.fm_frames(frames.data_ptr(), frames.stride(0), frames.stride(1), frames.stride(-2),
+                                        chroma.data_ptr() - frames.data_ptr())
         S, T = self._check_batch(frames.shape)
-        assert frames[0, 0].is_contiguous()
+        if frames[0, 0].is_contiguous():
+            return S, T, None
+        row = self.W if self.nv12 else 3 * self.W
+        assert frames.stride(-1) == 1 and (self.nv12 or frames.stride(-2) == 3) and \
+            frames.stride(2) >= row, "frames: unit byte stride, packed pixels and rows of at least the row bytes"
+        return S, T, _lib.fm_frames(frames.data_ptr(), frames.stride(0), frames.stride(1), frames.stride(2), 0)
+
+    def process(self, frames, sync=True, n_valid=None, chroma=None):
+        """frames: CUDA uint8 tensor [n_streams, T, H, W, 3] (BGR; nv12: [n_streams, T, H * 3 // 2, W]).  Returns the
+        per-frame stats as a structured numpy array [n_streams, T] (or the device tensor if sync=False).
+        n_valid: optional per-stream count of real frames in this call (ragged batch).
+        The rows of a frame may be pitched (a crop view such as frames[:, :, y0:y0 + H, x0:x0 + W], or padded rows):
+        pixels packed, rows at least W * 3 bytes apart.  nv12 engines also take the planes as two views with the same
+        strides: frames = luma [n_streams, T, H, W], chroma = UV [n_streams, T, H // 2, W] (slices of decoder surfaces)."""
+        import torch
+
+        S, T, layout = self._device_batch(frames, chroma)
         need = S * T * STATS_DTYPE.itemsize
         if self._stats_dev is None or self._stats_dev.numel() < need:
             self._stats_dev = torch.empty(S * self.max_frames * STATS_DTYPE.itemsize, dtype=torch.uint8,
                                           device=frames.device)
         st = torch.cuda.current_stream(frames.device).cuda_stream
-        _lib.check(self._lib.fm_process_ragged(self._ctx, frames.data_ptr(), frames.stride(0), frames.stride(1), T,
-                                               self._nvalid(n_valid, S, T), C.c_void_p(st), self._stats_dev.data_ptr()))
+        if layout is None:
+            _lib.check(self._lib.fm_process_ragged(self._ctx, frames.data_ptr(), frames.stride(0), frames.stride(1), T,
+                                                   self._nvalid(n_valid, S, T), C.c_void_p(st), self._stats_dev.data_ptr()))
+        else:
+            _lib.check(self._lib.fm_process_frames(self._ctx, C.byref(layout), T, self._nvalid(n_valid, S, T), C.c_void_p(st),
+                                                   self._stats_dev.data_ptr(), None, 0, 0))
         self._last_T = T
         if not sync:
             return self._stats_dev[:need]
@@ -138,7 +170,7 @@ class MotionEngine:
         self.check()
         return host.view(STATS_DTYPE).reshape(S, T)
 
-    def process_clip(self, frames, n_valid=None, out=None):
+    def process_clip(self, frames, n_valid=None, out=None, chroma=None):
         """process() that also returns the frames the reference writes to its *_motion.avi in this call (needs
         device_clips=True).  frames: CUDA uint8 tensor [n_streams, T, *frame_shape] (frame_shape = (H, W, 3), or
         (H * 3 // 2, W) with nv12).  out: optional CUDA uint8 tensor [n_streams, >= cache_frames + T, *frame_shape]
@@ -146,12 +178,11 @@ class MotionEngine:
         and reused, so the views returned by one call are overwritten by the next.  Runs on the current torch stream and
         synchronises.
         Returns (stats [n_streams, T], clips): clips[s] is a view [n_out, *frame_shape] of `out` holding, in order, the
-        cached frames each frame of stream s flushes and the frame itself where it is written."""
+        cached frames each frame of stream s flushes and the frame itself where it is written.  frames (and chroma) may
+        be laid out as process() takes them; the clips are packed frames."""
         import torch
 
-        assert frames.is_cuda and frames.dtype == torch.uint8, "uint8 CUDA frames"
-        S, T = self._check_batch(frames.shape)
-        assert frames[0, 0].is_contiguous()
+        S, T, layout = self._device_batch(frames, chroma)
         if out is None:
             if self._clips_out is None:
                 self._clips_out = torch.empty((S, self.info["cache_frames"] + self.max_frames) + self.frame_shape,
@@ -165,9 +196,13 @@ class MotionEngine:
             self._stats_dev = torch.empty(S * self.max_frames * STATS_DTYPE.itemsize, dtype=torch.uint8,
                                           device=frames.device)
         st = torch.cuda.current_stream(frames.device).cuda_stream
-        _lib.check(self._lib.fm_process_clip(self._ctx, frames.data_ptr(), frames.stride(0), frames.stride(1), T,
-                                             self._nvalid(n_valid, S, T), C.c_void_p(st), self._stats_dev.data_ptr(),
-                                             out.data_ptr(), out.stride(0), out.shape[1]))
+        if layout is None:
+            _lib.check(self._lib.fm_process_clip(self._ctx, frames.data_ptr(), frames.stride(0), frames.stride(1), T,
+                                                 self._nvalid(n_valid, S, T), C.c_void_p(st), self._stats_dev.data_ptr(),
+                                                 out.data_ptr(), out.stride(0), out.shape[1]))
+        else:
+            _lib.check(self._lib.fm_process_frames(self._ctx, C.byref(layout), T, self._nvalid(n_valid, S, T), C.c_void_p(st),
+                                                   self._stats_dev.data_ptr(), out.data_ptr(), out.stride(0), out.shape[1]))
         self._last_T = T
         stats = self._stats_dev[:need].cpu().numpy().view(STATS_DTYPE).reshape(S, T)
         self.check()

@@ -187,9 +187,30 @@ int fm_process_clip(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, si
                     int n_frames, const int32_t *n_valid, void *cuda_stream, fm_frame_stats *stats_dev,
                     uint8_t *out_dev, size_t out_stream_stride, int out_capacity);
 
+/* Where frame (s, t) of a call lives and how its rows are laid out: pitched rows (pitched allocations, crops of larger
+ * images) and hardware-decoder surfaces (luma pitch above W, chroma plane after the coded height) without a packing copy. */
+typedef struct fm_frames {
+    const uint8_t *data;        /* DEVICE pointer: frame (s, t) starts at data + s * stream_stride + t * frame_stride */
+    size_t stream_stride;
+    size_t frame_stride;
+    size_t row_pitch;           /* bytes from one row to the next, in both NV12 planes; 0 = packed (W*3, or W for NV12) */
+    int64_t uv_offset;          /* FM_FLAG_NV12: start of the chroma plane relative to the frame start (may be negative);
+                                   0 = row_pitch * H (chroma right after the luma rows) */
+} fm_frames;
+
+/* fm_process_ragged (clip_out == NULL) or fm_process_clip (clip_out != NULL, same flag and capacity rules) on frames laid
+ * out as `frames` describes.  Results, clip frames and detector input planes are those of the same frames packed; the
+ * outputs stay packed (clip frames of H*W*3 or H*W*3/2 bytes).  row_pitch must be at least the row bytes, and the two
+ * NV12 planes of a frame must not overlap.  Fused contexts (fm_info.front_end == 0) read the frames by TMA only and need
+ * data, the strides, row_pitch and data + uv_offset 16-byte aligned; every other front end takes any layout.  A refused
+ * call (FM_EINVAL) enqueues nothing and changes no state.  fm_process, fm_process_ragged and fm_process_clip are this
+ * call with row_pitch = 0. */
+int fm_process_frames(fm_ctx *ctx, const fm_frames *frames, int n_frames, const int32_t *n_valid, void *cuda_stream,
+                      fm_frame_stats *stats_dev, uint8_t *clip_out, size_t clip_stream_stride, int clip_capacity);
+
 /* find_objects' input planes (find_motion.py:572, 703-706) of the last hot-path call made through fm_process,
- * fm_process_ragged or fm_process_clip (needs FM_FLAG_OBJECT_PLANES).  The context remembers that call's frames, strides
- * and n_frames.  For stream s, with n_obj[s] = the number of its valid frames with wrote == 1, it writes n_obj[s] dense
+ * fm_process_ragged, fm_process_clip or fm_process_frames (needs FM_FLAG_OBJECT_PLANES).  The context remembers that
+ * call's frames, strides, row layout and n_frames.  For stream s, with n_obj[s] = the number of its valid frames with wrote == 1, it writes n_obj[s] dense
  * BGR planes of oh x 300 x 3 bytes (oh as for FM_FLAG_OBJECT_PLANES), in frame order, to the DEVICE buffer
  *   out_dev + s * out_stream_stride + i * oh*300*3          (i < n_obj[s])
  * each byte-identical to cv2.resize(raw, (300, oh), interpolation=cv2.INTER_AREA) of the written frame (the upscale for
