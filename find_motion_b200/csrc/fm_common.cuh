@@ -56,7 +56,7 @@ struct fm_ctx {
     int N;                     // w*h
     int ntiles;                // ceil(N / FM_TILE_PX)
     int resize_mode;           // 0 identity, 1 general tables, 2 integer ratio, 3 upscale (FM_FLAG_UPSCALE, k_upscale.cu)
-    size_t frame_bytes;        // bytes of one input frame: H * W * 3 (BGR) or H * W * 3 / 2 (FM_FLAG_NV12)
+    size_t frame_bytes;        // bytes of one input frame: H * W * 3 (BGR), H * W * 3 / 2 (FM_FLAG_NV12) or H * W (FM_FLAG_GRAY)
     uint8_t *nv12_bgr;         // FM_FLAG_NV12 on the staged path: [S][Tmax][H][W][3] the call's frames converted to BGR
                                // (k_nv12.cu), read by the BGR front end; null when none is needed
     bool fused;                // K1 fused stencil+background kernel drives the front end
@@ -218,15 +218,15 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32
                                     const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 PFN_encodeTiled fm_tma_encoder();
-// The call's frames as a 4-D u32 tensor map (W*3/4 words, H rows `pitch` bytes apart, T frames, S streams) with boxes of
+// The call's frames as a 4-D u32 tensor map (W*3/4 words, W/4 for gray frames, H rows `pitch` bytes apart, T frames, S streams) with boxes of
 // box_words x box_rows (out-of-range elements, the row padding included, are zero-filled).  FM_EINVAL unless the frames,
 // their strides, the pitch and the rows are 16-byte aligned.
 int fm_frames_tmap(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int box_words,
                    int box_rows, CUtensorMap *out);
 
 // stage launchers (each enqueues on `st`, returns FM_OK / error).  Frame (s, t) of the frames a launcher reads starts at
-// frames + s * sstride + t * fstride, its rows are `pitch` bytes apart (W * 3 when packed) and, for NV12, its chroma plane
-// starts `uv` bytes from the frame start (pitch * H when packed).
+// frames + s * sstride + t * fstride, its rows are `pitch` bytes apart (W * 3 when packed, W for gray frames) and, for NV12,
+// its chroma plane starts `uv` bytes from the frame start (pitch * H when packed).
 int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T,
                        cudaStream_t st);
 int fm_launch_temporal(fm_ctx *c, int T, cudaStream_t st);
@@ -249,14 +249,14 @@ size_t fm_fused_bg_doubles(const fm_ctx *c);
 int fm_launch_bg_export_fused(fm_ctx *c, int stream, double *dst_dev, cudaStream_t st);
 int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, size_t pitch, int S, int T, int W, int H,
                          int w, int h, int mode, int fx, int fy, const ResizeTab &xt, const ResizeTab &yt, const int *oidx,
-                         uint8_t *dst_dev, size_t ostride, cudaStream_t st);
+                         uint8_t *dst_dev, size_t ostride, cudaStream_t st, int channels);
 size_t fm_upscale_smem(int w);
 int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int F, int W, int H, int w,
                       int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
-                      const int *oidx, size_t ostride, cudaStream_t st);
+                      const int *oidx, size_t ostride, cudaStream_t st, int channels);
 int fm_rows_plan(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx);
 void fm_rows_free(fm_ctx *c);
-int fm_rows_plan_describe(int W, int w, int h, const int *xstart, const int *xidx, const float *xwt, const int *ystart,
+int fm_rows_plan_describe(int W, int w, int h, int channels, const int *xstart, const int *xidx, const float *xwt, const int *ystart,
                           const int *yidx, fm_rows_plan_info *out);
 int fm_rows_plan_objects(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx);
 bool fm_rows_usable(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch);

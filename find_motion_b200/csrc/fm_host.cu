@@ -55,7 +55,7 @@ PFN_encodeTiled fm_tma_encoder() {
 
 int fm_frames_tmap(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int box_words,
                    int box_rows, CUtensorMap *out) {
-    const size_t row = (size_t)c->W * 3, dense = pitch * c->H;
+    const size_t row = (size_t)c->W * ((c->cfg.flags & FM_FLAG_GRAY) ? 1 : 3), dense = pitch * c->H;
     if ((((uintptr_t)frames) | sstride | fstride | pitch | row) & 15) {
         fm_set_error("the TMA front ends need 16-byte aligned frames, strides and rows (row pitch %zu)", pitch);
         return FM_EINVAL;
@@ -239,6 +239,10 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
         fm_set_error("invalid configuration (streams/geometry/max_frames/box_size/blur_scale/min_box_scale)");
         return FM_EINVAL;
     }
+    if ((cfg->flags & FM_FLAG_GRAY) && (cfg->flags & FM_FLAG_NV12)) {
+        fm_set_error("FM_FLAG_GRAY and FM_FLAG_NV12 are two frame formats: set one of them");
+        return FM_EINVAL;
+    }
     if (cfg->box_size > cfg->frame_width && !(cfg->flags & FM_FLAG_UPSCALE)) {
         // INTER_AREA with a destination wider than the source is cv2's fixed-point linear upscale (SURVEY.md A.1):
         // opt-in with FM_FLAG_UPSCALE, so that binders of the earlier ABI keep their range check
@@ -275,7 +279,9 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     c->cfg = *cfg;
     c->S = cfg->n_streams; c->Tmax = cfg->max_frames;
     c->W = cfg->frame_width; c->H = cfg->frame_height;
-    c->frame_bytes = (cfg->flags & FM_FLAG_NV12) ? (size_t)c->W * c->H * 3 / 2 : (size_t)c->W * c->H * 3;
+    c->frame_bytes = (cfg->flags & FM_FLAG_NV12)   ? (size_t)c->W * c->H * 3 / 2
+                     : (cfg->flags & FM_FLAG_GRAY) ? (size_t)c->W * c->H
+                                                   : (size_t)c->W * c->H * 3;
     // derived parameters, mirroring the Python expressions (true division on floats, int() truncation)
     const double W = c->W, H = c->H, box = cfg->box_size;
     c->w = cfg->box_size;
@@ -389,7 +395,8 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     } while (0)
     // the fused front ends never materialise gray / blur planes (except as parity taps)
     const bool keep = (cfg->flags & FM_FLAG_KEEP_PLANES) != 0;
-    const bool need_gray = keep || !c->fused;
+    // gray frames at full resolution are the gray plane themselves
+    const bool need_gray = keep || (!c->fused && !((cfg->flags & FM_FLAG_GRAY) && c->resize_mode == 0));
     const bool need_blur = keep || !c->fused;
     ALLOC(c->gray, need_gray ? F * c->N : 16);
     ALLOC(c->hor, (c->fused || c->umma) ? 16 : 2 * fm_wide_plane_bytes(c));
@@ -657,10 +664,14 @@ extern "C" int fm_process_frames(fm_ctx *c, const fm_frames *fr, int n_frames, c
                                  fm_frame_stats *stats_dev, uint8_t *clip_out, size_t clip_stream_stride, int clip_capacity) {
     if (!c || !fr || !fr->data) { fm_set_error("null argument"); return FM_EINVAL; }
     const bool nv12 = (c->cfg.flags & FM_FLAG_NV12) != 0;
-    const size_t row = nv12 ? (size_t)c->W : (size_t)c->W * 3;
+    const size_t row = (nv12 || (c->cfg.flags & FM_FLAG_GRAY)) ? (size_t)c->W : (size_t)c->W * 3;
     const size_t pitch = fr->row_pitch ? fr->row_pitch : row;
     if (pitch < row) {
         fm_set_error("row_pitch %zu < %zu bytes of a row", pitch, row);
+        return FM_EINVAL;
+    }
+    if ((c->cfg.flags & FM_FLAG_GRAY) && fr->uv_offset) {
+        fm_set_error("uv_offset %lld: gray frames have no chroma plane", (long long)fr->uv_offset);
         return FM_EINVAL;
     }
     const int64_t luma = (int64_t)(pitch * (c->H - 1) + row);           // bytes the luma rows of a frame span
@@ -988,15 +999,21 @@ extern "C" int fm_debug_mask(fm_ctx *c, int stream, uint8_t *mask) {
 }
 
 // find_objects' input plane (find_motion.py:703-706): imutils.resize(frame.raw, width=300) = INTER_AREA, BGR out
-extern "C" int fm_debug_rows_plan(int W, int H, int box_size, fm_rows_plan_info *info) {
+extern "C" int fm_debug_rows_plan_channels(int W, int H, int box_size, int channels, fm_rows_plan_info *info) {
     if (!info || W < 1 || H < 1 || box_size < 1 || box_size > W) { fm_set_error("bad geometry"); return FM_EINVAL; }
+    if (channels != 1 && channels != 3) { fm_set_error("channels %d: 3 (BGR) or 1 (gray)", channels); return FM_EINVAL; }
     const int w = box_size, h = (int)((double)H * ((double)box_size / (double)W));          // imutils.resize
     memset(info, 0, sizeof(*info));
     if (h < 1 || (w == W && h == H)) return FM_OK;
     const double sx = 1.0 / ((double)w / W), sy = 1.0 / ((double)h / H);
     if (fabs(sx - nearbyint(sx)) < 2.220446049250313e-16 && fabs(sy - nearbyint(sy)) < 2.220446049250313e-16) return FM_OK;   // integer ratio
     const HostTab xt = area_tab(W, w), yt = area_tab(H, h);
-    return fm_rows_plan_describe(W, w, h, xt.start.data(), xt.idx.data(), xt.wt.data(), yt.start.data(), yt.idx.data(), info);
+    return fm_rows_plan_describe(W, w, h, channels, xt.start.data(), xt.idx.data(), xt.wt.data(), yt.start.data(), yt.idx.data(),
+                                 info);
+}
+
+extern "C" int fm_debug_rows_plan(int W, int H, int box_size, fm_rows_plan_info *info) {
+    return fm_debug_rows_plan_channels(W, H, box_size, 3, info);
 }
 
 extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H, int width, uint8_t *out_host, int *out_height) {
@@ -1022,7 +1039,7 @@ extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H,
         FM_CUDA(cudaMalloc(&dst.p, (size_t)width * h * 3));
         FM_CUDA(cudaMemcpy(src.p, bgr_host, (size_t)W * H * 3, cudaMemcpyHostToDevice));
         if ((rc = fm_launch_upscale(device, (const uint8_t *)src.p, 0, 0, (size_t)W * 3, 1, 1, W, H, width, h, ut.x, ut.y, nullptr, nullptr,
-                                    (uint8_t *)dst.p, nullptr, 0, 0)))
+                                    (uint8_t *)dst.p, nullptr, 0, 0, 3)))
             return rc;
         FM_CUDA(cudaMemcpy(out_host, dst.p, (size_t)width * h * 3, cudaMemcpyDeviceToHost));
         return FM_OK;
@@ -1044,7 +1061,7 @@ extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H,
     FM_CUDA(cudaMalloc(&dst.p, (size_t)width * h * 3));
     FM_CUDA(cudaMemcpy(src.p, bgr_host, (size_t)W * H * 3, cudaMemcpyHostToDevice));
     if ((rc = fm_launch_resize_bgr(device, (const uint8_t *)src.p, 0, 0, (size_t)W * 3, 1, 1, W, H, width, h, fast ? 2 : 1, isx, isy, tb.x,
-                                   tb.y, nullptr, (uint8_t *)dst.p, 0, 0)))
+                                   tb.y, nullptr, (uint8_t *)dst.p, 0, 0, 3)))
         return rc;
     FM_CUDA(cudaMemcpy(out_host, dst.p, (size_t)width * h * 3, cudaMemcpyDeviceToHost));
     return FM_OK;

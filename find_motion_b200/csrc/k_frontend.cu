@@ -3,8 +3,10 @@
 // Replaces VideoMotion.blur_frame + mask_off_areas (find_motion/find_motion.py:487-494, 619-635).
 #include "fm_common.cuh"
 
-// identity-resize mode: one thread per 4 pixels of a frame (12 bytes in, 4 bytes out).  Pixel i = y * w + x of a frame
-// is at y * pitch + 3 x; packed rows (pitch == 3 w) are one flat run, so 4 pixels may then straddle a row end
+// identity-resize mode: one thread per 4 pixels of a frame (12 bytes in, 4 bytes out; C = 1, gray frames: a copy).  Pixel
+// i = y * w + x of a frame is at y * pitch + C x; packed rows (pitch == C w) are one flat run, so 4 pixels may then straddle
+// a row end
+template <int C>
 __global__ void __launch_bounds__(256) k_gray(const uint8_t *__restrict__ frames, size_t sstride,
                                               size_t fstride, size_t pitch, int T, int w, int N, uint8_t *__restrict__ gray,
                                               const int *__restrict__ nvalid) {
@@ -15,17 +17,17 @@ __global__ void __launch_bounds__(256) k_gray(const uint8_t *__restrict__ frames
     uint8_t *dst = gray + (size_t)f * N;
     int i4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (i4 >= N) return;
-    const bool flat = pitch == (size_t)w * 3;
+    const bool flat = pitch == (size_t)w * C;
     const int y4 = flat ? 0 : i4 / w, x4 = i4 - y4 * w;
-    const uint8_t *q4 = flat ? src + (size_t)i4 * 3 : src + (size_t)y4 * pitch + (size_t)x4 * 3;
+    const uint8_t *q4 = flat ? src + (size_t)i4 * C : src + (size_t)y4 * pitch + (size_t)x4 * C;
     if (i4 + 4 <= N && (flat || x4 + 4 <= w) && ((((uintptr_t)q4) & 3) == 0) && ((((uintptr_t)dst) & 3) == 0)) {
         const uint32_t *p = reinterpret_cast<const uint32_t *>(q4);
-        *reinterpret_cast<uint32_t *>(dst + i4) = fm_gray4(__ldg(p), __ldg(p + 1), __ldg(p + 2));
+        *reinterpret_cast<uint32_t *>(dst + i4) = C == 1 ? __ldg(p) : fm_gray4(__ldg(p), __ldg(p + 1), __ldg(p + 2));
     } else {
         for (int i = i4; i < min(i4 + 4, N); i++) {
             const int y = i / w;
-            const uint8_t *p = src + (size_t)y * pitch + (size_t)(i - y * w) * 3;
-            dst[i] = (uint8_t)fm_gray(p[0], p[1], p[2]);
+            const uint8_t *p = src + (size_t)y * pitch + (size_t)(i - y * w) * C;
+            dst[i] = C == 1 ? p[0] : (uint8_t)fm_gray(p[0], p[1], p[2]);
         }
     }
 }
@@ -55,7 +57,9 @@ struct K0Params {
 #define K0_GROUPS 4       // source rows in flight (K0_THREADS/K0_GROUPS threads each)
 
 // oidx (with bgr_out): null, or [F] plane index (-1: skip the frame); frame f's plane then goes to
-// bgr_out + s * ostride + oidx[f] * h*w*3 (fm_object_planes)
+// bgr_out + s * ostride + oidx[f] * h*w*3 (fm_object_planes).  C: channels of the source (3 BGR, 1 gray); per channel the
+// chains are the same, and a gray source's resized byte is stored in all three channels of bgr_out
+template <int C>
 __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const int *__restrict__ oidx, size_t ostride) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int f = blockIdx.y;
@@ -65,11 +69,11 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const in
     if (o < 0) return;
     const int dy = blockIdx.x;
     const uint8_t *src = p.frames + (size_t)s * p.sstride + (size_t)t * p.fstride;
-    const int rowbytes = p.W * 3;
+    const int rowbytes = p.W * C;
     const int rowpitch = (rowbytes + 16 + 15) & ~15;          // room for a misaligned start
     unsigned char *rowbuf = smem;                               // [K0_GROUPS][rowpitch]
-    float *bufs = reinterpret_cast<float *>(smem + (size_t)K0_GROUPS * rowpitch);   // [ny][3w]
-    const int w3 = p.w * 3;
+    float *bufs = reinterpret_cast<float *>(smem + (size_t)K0_GROUPS * rowpitch);   // [ny][C w]
+    const int w3 = p.w * C;
     const int tid = threadIdx.x;
     const int gsz = K0_THREADS / K0_GROUPS;
     const int grp = tid / gsz, gt = tid - grp * gsz;
@@ -114,38 +118,38 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const in
             if (p.mode == 1) {
                 for (int dx = gt; dx < p.w; dx += gsz) {
                     int a = p.xstart[dx], b = p.xstart[dx + 1];
-                    float b0 = 0.f, b1 = 0.f, b2 = 0.f;
+                    float bc[C];
+#pragma unroll
+                    for (int ch = 0; ch < C; ch++) bc[ch] = 0.f;
                     for (int q = a; q < b; q++) {
-                        const unsigned char *px = rb + p.xidx[q] * 3;
+                        const unsigned char *px = rb + p.xidx[q] * C;
                         float al = p.xwt[q];
-                        b0 = __fadd_rn(b0, __fmul_rn((float)px[0], al));
-                        b1 = __fadd_rn(b1, __fmul_rn((float)px[1], al));
-                        b2 = __fadd_rn(b2, __fmul_rn((float)px[2], al));
+#pragma unroll
+                        for (int ch = 0; ch < C; ch++) bc[ch] = __fadd_rn(bc[ch], __fmul_rn((float)px[ch], al));
                     }
-                    out[dx * 3 + 0] = b0;
-                    out[dx * 3 + 1] = b1;
-                    out[dx * 3 + 2] = b2;
+#pragma unroll
+                    for (int ch = 0; ch < C; ch++) out[dx * C + ch] = bc[ch];
                 }
             } else {   // integer ratio: exact integer row sums, kept as int bit patterns
                 int *outi = reinterpret_cast<int *>(out);
                 for (int dx = gt; dx < p.w; dx += gsz) {
-                    int s0 = 0, s1 = 0, s2 = 0;
-                    const unsigned char *px = rb + dx * p.fx * 3;
-                    for (int q = 0; q < p.fx; q++, px += 3) {
-                        s0 += px[0];
-                        s1 += px[1];
-                        s2 += px[2];
+                    int sc[C];
+#pragma unroll
+                    for (int ch = 0; ch < C; ch++) sc[ch] = 0;
+                    const unsigned char *px = rb + dx * p.fx * C;
+                    for (int q = 0; q < p.fx; q++, px += C) {
+#pragma unroll
+                        for (int ch = 0; ch < C; ch++) sc[ch] += px[ch];
                     }
-                    outi[dx * 3 + 0] = s0;
-                    outi[dx * 3 + 1] = s1;
-                    outi[dx * 3 + 2] = s2;
+#pragma unroll
+                    for (int ch = 0; ch < C; ch++) outi[dx * C + ch] = sc[ch];
                 }
             }
         }
         __syncthreads();
     }
     // vertical chains + rounding + gray
-    unsigned char *small = rowbuf;        // reuse: [3w] resized BGR bytes of this row
+    unsigned char *small = rowbuf;        // reuse: [C w] resized bytes of this row
     for (int i = tid; i < w3; i += K0_THREADS) {
         int v;
         if (p.mode == 1) {
@@ -167,20 +171,22 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const in
     }
     __syncthreads();
     if (p.bgr_out) {
-        uint8_t *out = p.bgr_out + (oidx ? (size_t)s * ostride + ((size_t)o * p.h + dy) * w3 : ((size_t)f * p.h + dy) * w3);
-        for (int i = tid; i < w3; i += K0_THREADS) out[i] = small[i];
+        const int wb = p.w * 3;
+        uint8_t *out = p.bgr_out + (oidx ? (size_t)s * ostride + ((size_t)o * p.h + dy) * wb : ((size_t)f * p.h + dy) * wb);
+        for (int i = tid; i < wb; i += K0_THREADS) out[i] = C == 1 ? small[i / 3] : small[i];
         return;
     }
     uint8_t *g = p.gray + ((size_t)f * p.h + dy) * p.w;
     for (int dx = tid; dx < p.w; dx += K0_THREADS)
-        g[dx] = (uint8_t)fm_gray(small[dx * 3], small[dx * 3 + 1], small[dx * 3 + 2]);
+        g[dx] = C == 1 ? small[dx] : (uint8_t)fm_gray(small[dx * 3], small[dx * 3 + 1], small[dx * 3 + 2]);
 }
 
 // INTER_AREA resize to BGR (device buffers); mode / tables as fm_ctx_create derives them.  One frame (fm_resize_area:
-// S = T = 1, oidx null) or the frames of a call with an oidx table (fm_object_planes)
+// S = T = 1, oidx null) or the frames of a call with an oidx table (fm_object_planes).  channels: 3 (BGR source) or 1 (gray
+// source, its resize stored in B, G and R)
 int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, size_t pitch, int S, int T, int W,
                          int H, int w, int h, int mode, int fx, int fy, const ResizeTab &xt, const ResizeTab &yt, const int *oidx,
-                         uint8_t *dst_dev, size_t ostride, cudaStream_t st) {
+                         uint8_t *dst_dev, size_t ostride, cudaStream_t st, int channels) {
     K0Params p;
     p.frames = src_dev; p.sstride = sstride; p.fstride = fstride; p.pitch = pitch;
     p.T = T; p.W = W; p.H = H; p.w = w; p.h = h;
@@ -189,16 +195,18 @@ int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, siz
     p.ystart = yt.start; p.yidx = yt.idx; p.ywt = yt.wt;
     p.max_ytaps = mode == 1 ? yt.max_taps : fy;
     p.gray = nullptr; p.nvalid = nullptr; p.bgr_out = dst_dev;
-    const int rowpitch = (W * 3 + 16 + 15) & ~15;
-    const size_t smem = (size_t)K0_GROUPS * rowpitch + (size_t)p.max_ytaps * w * 3 * sizeof(float);
+    const int rowpitch = (W * channels + 16 + 15) & ~15;
+    const size_t smem = (size_t)K0_GROUPS * rowpitch + (size_t)p.max_ytaps * w * channels * sizeof(float);
     if (smem > 220 * 1024) {
         fm_set_error("resize needs %zu bytes of shared memory (frame too wide / ratio too large)", smem);
         return FM_ERANGE;
     }
     int rc;
-    if ((rc = fm_ensure_smem((const void *)k_resize_gray, smem, device))) return rc;
+    const void *kern = channels == 1 ? (const void *)k_resize_gray<1> : (const void *)k_resize_gray<3>;
+    if ((rc = fm_ensure_smem(kern, smem, device))) return rc;
     dim3 grid(h, S * T);
-    k_resize_gray<<<grid, K0_THREADS, smem, st>>>(p, oidx, ostride);
+    if (channels == 1) k_resize_gray<1><<<grid, K0_THREADS, smem, st>>>(p, oidx, ostride);
+    else k_resize_gray<3><<<grid, K0_THREADS, smem, st>>>(p, oidx, ostride);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }
@@ -211,7 +219,9 @@ int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, siz
 // ---------------------------------------------------------------------------------------------
 #define K0W_WARPS 8
 
-// task = ((frame * h + dy) * nq + q): the warp produces destination columns q*dxw .. q*dxw+dxw-1 (one per lane)
+// task = ((frame * h + dy) * nq + q): the warp produces destination columns q*dxw .. q*dxw+dxw-1 (one per lane).
+// C: channels of the source (3 BGR, 1 gray)
+template <int C>
 __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_warp(K0Params p, int segpitch, int tasks, int nq,
                                                                      int dxw) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -224,17 +234,17 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_warp(K0Params p,
     if (t >= __ldg(p.nvalid + s)) return;
     const uint8_t *src = p.frames + (size_t)s * p.sstride + (size_t)t * p.fstride;
     unsigned char *rowbuf = smem + (size_t)warp * segpitch;
-    const int rowbytes = p.W * 3;
+    const int rowbytes = p.W * C;
     const int y0 = p.ystart[dy], ny = p.ystart[dy + 1] - y0;
     const int dxa = q * dxw, dxb = min(dxa + dxw, p.w);
     const int dx = dxa + lane;
     const bool live = lane < dxw && dx < p.w;
     // source byte range of this warp's columns
-    const int b_lo = p.xidx[p.xstart[dxa]] * 3, b_hi = (p.xidx[p.xstart[dxb] - 1] + 1) * 3;
+    const int b_lo = p.xidx[p.xstart[dxa]] * C, b_hi = (p.xidx[p.xstart[dxb] - 1] + 1) * C;
     int xa = 0, xn = 0;
     int xfirst = 0;
     if (live) { xa = p.xstart[dx]; xn = p.xstart[dx + 1] - xa; xfirst = p.xidx[xa]; }
-    float s0 = 0.f, s1 = 0.f, s2 = 0.f;
+    float sc[C];
     for (int j = 0; j < ny; j++) {
         const int sy = p.yidx[y0 + j];
         const float beta = p.ywt[y0 + j];
@@ -261,30 +271,26 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_warp(K0Params p,
             }
         }
         __syncwarp();
-        const unsigned char *rb = rowbuf + mis - b_lo;                    // rb[3*x + c] = source pixel x
-        float b0 = 0.f, b1 = 0.f, b2 = 0.f;
-        const unsigned char *px = rb + xfirst * 3;      // the taps of a column are consecutive source pixels
+        const unsigned char *rb = rowbuf + mis - b_lo;                    // rb[C*x + c] = source pixel x
+        float bc[C];
+#pragma unroll
+        for (int ch = 0; ch < C; ch++) bc[ch] = 0.f;
+        const unsigned char *px = rb + xfirst * C;      // the taps of a column are consecutive source pixels
         const float *wt = p.xwt + xa;
 #pragma unroll 4
-        for (int qq = 0; qq < xn; qq++, px += 3) {
+        for (int qq = 0; qq < xn; qq++, px += C) {
             const float al = __ldg(wt + qq);
-            b0 = __fadd_rn(b0, __fmul_rn((float)px[0], al));
-            b1 = __fadd_rn(b1, __fmul_rn((float)px[1], al));
-            b2 = __fadd_rn(b2, __fmul_rn((float)px[2], al));
+#pragma unroll
+            for (int ch = 0; ch < C; ch++) bc[ch] = __fadd_rn(bc[ch], __fmul_rn((float)px[ch], al));
         }
-        if (j == 0) {
-            s0 = __fmul_rn(beta, b0); s1 = __fmul_rn(beta, b1); s2 = __fmul_rn(beta, b2);
-        } else {
-            s0 = __fadd_rn(s0, __fmul_rn(beta, b0));
-            s1 = __fadd_rn(s1, __fmul_rn(beta, b1));
-            s2 = __fadd_rn(s2, __fmul_rn(beta, b2));
-        }
+#pragma unroll
+        for (int ch = 0; ch < C; ch++) sc[ch] = j == 0 ? __fmul_rn(beta, bc[ch]) : __fadd_rn(sc[ch], __fmul_rn(beta, bc[ch]));
     }
     if (live) {
-        int v0 = min(max(__float2int_rn(s0), 0), 255);
-        int v1 = min(max(__float2int_rn(s1), 0), 255);
-        int v2 = min(max(__float2int_rn(s2), 0), 255);
-        p.gray[((size_t)f * p.h + dy) * p.w + dx] = (uint8_t)fm_gray(v0, v1, v2);
+        int v[C];
+#pragma unroll
+        for (int ch = 0; ch < C; ch++) v[ch] = min(max(__float2int_rn(sc[ch]), 0), 255);
+        p.gray[((size_t)f * p.h + dy) * p.w + dx] = C == 1 ? (uint8_t)v[0] : (uint8_t)fm_gray(v[0], v[C > 1 ? 1 : 0], v[C - 1]);
     }
 }
 
@@ -309,8 +315,9 @@ __device__ __noinline__ void copy_partial_block(unsigned char *d, const uint8_t 
 }
 
 #define K0_RG 7         // tap groups per destination column held in registers
-// PF = 16-byte blocks per lane of one source segment (registers used to prefetch the next row)
-template <int PF, bool INREG>
+// PF = 16-byte blocks per lane of one source segment (registers used to prefetch the next row).  C: channels of the source
+// (3 BGR: a group is 12 bytes; 1 gray: a group is one word)
+template <int PF, bool INREG, int C>
 __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K0GParams gp, int segpitch, int tasks,
                                                                    int nq, int dxw) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -323,15 +330,15 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
     if (t >= __ldg(p.nvalid + s)) return;
     const uint8_t *src = p.frames + (size_t)s * p.sstride + (size_t)t * p.fstride;
     unsigned char *rowbuf = smem + (size_t)warp * segpitch;
-    const int rowbytes = p.W * 3;
+    const int rowbytes = p.W * C;
     const int y0 = p.ystart[dy], ny = p.ystart[dy + 1] - y0;
     const int dxa = q * dxw, dxb = min(dxa + dxw, p.w);
     const int dx = dxa + lane;
     const bool live = lane < dxw && dx < p.w;
-    const int b_lo = gp.g4start[dxa] * 3;
-    const int b_hi = min((gp.g4start[dxb - 1] + 4 * gp.g4n[dxb - 1]) * 3, rowbytes);
+    const int b_lo = gp.g4start[dxa] * C;
+    const int b_hi = min((gp.g4start[dxb - 1] + 4 * gp.g4n[dxb - 1]) * C, rowbytes);
     const int nbytes = b_hi - b_lo;
-    int gs = b_lo / 3, gn = 0;          // idle lanes walk the start of the segment with zero weights
+    int gs = b_lo / C, gn = 0;          // idle lanes walk the start of the segment with zero weights
     const float4 *gw = gp.g4w;
     if (live) { gs = gp.g4start[dx]; gn = gp.g4n[dx]; gw += gp.g4off[dx]; }
     float s0 = 0.f, s1 = 0.f, s2 = 0.f;
@@ -392,7 +399,7 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
         const int mis = commit(j);
         __syncwarp();
         if (j + 1 < ny) issue(j + 1);
-        const uint32_t *wp = reinterpret_cast<const uint32_t *>(rowbuf + mis - b_lo + 3 * gs);
+        const uint32_t *wp = reinterpret_cast<const uint32_t *>(rowbuf + mis - b_lo + C * gs);
         float b0 = 0.f, b1 = 0.f, b2 = 0.f;
 #define FM_G4(W0, W1, W2, a, n)                                                                               \
         b0 = __fadd_rn(b0, fm_byte_mul(W0, 0, a.x, n.x)); b1 = __fadd_rn(b1, fm_byte_mul(W0, 1, a.x, n.x));       \
@@ -401,7 +408,23 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
         b0 = __fadd_rn(b0, fm_byte_mul(W1, 2, a.z, n.z)); b1 = __fadd_rn(b1, fm_byte_mul(W1, 3, a.z, n.z));       \
         b2 = __fadd_rn(b2, fm_byte_mul(W2, 0, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(W2, 1, a.w, n.w));       \
         b1 = __fadd_rn(b1, fm_byte_mul(W2, 2, a.w, n.w)); b2 = __fadd_rn(b2, fm_byte_mul(W2, 3, a.w, n.w));
-        if (inreg) {            // the column's weights live in registers for all source rows
+#define FM_G1(W0, a, n)                                                                                       \
+        b0 = __fadd_rn(b0, fm_byte_mul(W0, 0, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(W0, 1, a.y, n.y));       \
+        b0 = __fadd_rn(b0, fm_byte_mul(W0, 2, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(W0, 3, a.w, n.w));
+        if (C == 1 && inreg) {
+#pragma unroll
+            for (int g = 0; g < K0_RG; g++) {
+                if (g < gmax) FM_G1(wp[g], wr[g], wn[g])
+            }
+        } else if (C == 1) {
+#pragma unroll 2
+            for (int g = 0; g < gn; g++) {
+                const float4 a = __ldg(gw + g);
+                const float4 n = make_float4(__fmul_rn(a.x, -8388608.0f), __fmul_rn(a.y, -8388608.0f),
+                                             __fmul_rn(a.z, -8388608.0f), __fmul_rn(a.w, -8388608.0f));
+                FM_G1(wp[g], a, n)
+            }
+        } else if (inreg) {            // the column's weights live in registers for all source rows
 #pragma unroll
             for (int g = 0; g < K0_RG; g++) {
                 if (g < gmax) {     // warp-uniform: lanes with fewer groups add exact zeros (zero weights, finite bytes)
@@ -420,6 +443,7 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
             }
         }
 #undef FM_G4
+#undef FM_G1
         if (j == 0) {
             s0 = __fmul_rn(beta, b0); s1 = __fmul_rn(beta, b1); s2 = __fmul_rn(beta, b2);
         } else {
@@ -432,13 +456,54 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
         int v0 = min(max(__float2int_rn(s0), 0), 255);
         int v1 = min(max(__float2int_rn(s1), 0), 255);
         int v2 = min(max(__float2int_rn(s2), 0), 255);
-        p.gray[((size_t)f * p.h + dy) * p.w + dx] = (uint8_t)fm_gray(v0, v1, v2);
+        p.gray[((size_t)f * p.h + dy) * p.w + dx] = C == 1 ? (uint8_t)v0 : (uint8_t)fm_gray(v0, v1, v2);
     }
 }
 
 int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
     dim3 grid(((c->N + 3) / 4 + 255) / 256, c->S * T);
-    k_gray<<<grid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->w, c->N, c->gray, c->nvalid);
+    if (c->cfg.flags & FM_FLAG_GRAY) k_gray<1><<<grid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->w, c->N, c->gray, c->nvalid);
+    else k_gray<3><<<grid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->w, c->N, c->gray, c->nvalid);
+    FM_LAUNCH_CHECK();
+    return FM_OK;
+}
+
+template <int C>
+static int launch_resize_warps(fm_ctx *c, const K0Params &p, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch,
+                               int F, cudaStream_t st) {
+    // one warp per (frame, destination row, group of <= 32 destination columns)
+    int nq = (c->w + 31) / 32, dxw = (c->w + nq - 1) / nq;
+    int segpitch = ((c->W * C + nq - 1) / nq + C * (c->xtab.max_taps + 10) + 32 + 15) & ~15;
+    size_t smemw = (size_t)K0W_WARPS * segpitch;
+    int rc;
+    if ((rc = fm_ensure_smem((const void *)k_resize_gray_warp<C>, smemw, c->cfg.device))) return rc;
+    int tasks = c->h * F * nq;
+    const bool aligned4 = ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->W * C)) & 3) == 0;
+    if (aligned4 && c->g4w) {
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, true, C>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, false, C>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<8, true, C>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<8, false, C>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<16, true, C>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<16, false, C>, smemw, c->cfg.device))) return rc;
+        K0GParams gp;
+        gp.g4start = c->g4start; gp.g4n = c->g4n; gp.g4off = c->g4off; gp.g4w = c->g4w;
+        const int blocks16 = segpitch / 16 + 1;         // upper bound of 16-byte blocks per segment
+        const int gridw = (tasks + K0W_WARPS - 1) / K0W_WARPS;
+        const bool inreg = c->g4max <= K0_RG;
+#define FM_K0(PF)                                                                                                   \
+        do {                                                                                                        \
+            if (inreg) k_resize_gray_g4<PF, true, C><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, gp, segpitch, tasks, nq, dxw); \
+            else k_resize_gray_g4<PF, false, C><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, gp, segpitch, tasks, nq, dxw);     \
+        } while (0)
+        if (blocks16 <= 4 * 32) FM_K0(4);
+        else if (blocks16 <= 8 * 32) FM_K0(8);
+        else if (blocks16 <= 16 * 32) FM_K0(16);
+        else k_resize_gray_warp<C><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, segpitch, tasks, nq, dxw);
+#undef FM_K0
+    } else {
+        k_resize_gray_warp<C><<<(tasks + K0W_WARPS - 1) / K0W_WARPS, 32 * K0W_WARPS, smemw, st>>>(p, segpitch, tasks, nq, dxw);
+    }
     FM_LAUNCH_CHECK();
     return FM_OK;
 }
@@ -446,14 +511,16 @@ int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_
 int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T,
                        cudaStream_t st) {
     const int F = c->S * T;
+    const bool gray_in = (c->cfg.flags & FM_FLAG_GRAY) != 0;
+    const int C = gray_in ? 1 : 3;
     // every Gaussian the fused stencil does not take goes to the tensor-core blur (k_wide.cu)
-    if (c->resize_mode == 0)          // gray fused into the first kernel of the blur
+    if (c->resize_mode == 0)          // gray fused into the first kernel of the blur (gray frames: they are the gray plane)
         return c->umma ? fm_launch_umma_blur(c, frames, sstride, fstride, pitch, T, st)
                        : fm_launch_wide_blur(c, frames, sstride, fstride, pitch, T, st);
     if (c->resize_mode == 3) {        // upscale + gray into the gray plane (k_upscale.cu)
         int rc;
         if ((rc = fm_launch_upscale(c->cfg.device, frames, sstride, fstride, pitch, T, F, c->W, c->H, c->w, c->h, c->uxt, c->uyt,
-                                    c->nvalid, c->gray, nullptr, nullptr, 0, st)))
+                                    c->nvalid, c->gray, nullptr, nullptr, 0, st, C)))
             return rc;
     } else {
         K0Params p;
@@ -464,56 +531,26 @@ int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t 
         p.ystart = c->ytab.start; p.yidx = c->ytab.idx; p.ywt = c->ytab.wt;
         p.max_ytaps = c->resize_mode == 1 ? c->ytab.max_taps : c->fy;
         p.gray = c->gray; p.nvalid = c->nvalid; p.bgr_out = nullptr;
-        int rowpitch = (c->W * 3 + 16 + 15) & ~15;
+        int rowpitch = (c->W * C + 16 + 15) & ~15;
+        int rc;
         if (c->resize_mode == 1 && fm_rows_usable(c, frames, sstride, fstride, pitch)) {
             // one source row per lane, TMA-staged (k_resize_rows.cu)
-            int rc;
             if ((rc = fm_launch_resize_rows(c, frames, sstride, fstride, pitch, T, st))) return rc;
         } else if (c->resize_mode == 1) {
-            // one warp per (frame, destination row, group of <= 32 destination columns)
-            int nq = (c->w + 31) / 32, dxw = (c->w + nq - 1) / nq;
-            int segpitch = ((c->W * 3 + nq - 1) / nq + 3 * (c->xtab.max_taps + 10) + 32 + 15) & ~15;
-            size_t smemw = (size_t)K0W_WARPS * segpitch;
-            int rc;
-            if ((rc = fm_ensure_smem((const void *)k_resize_gray_warp, smemw, c->cfg.device))) return rc;
-            int tasks = c->h * F * nq;
-            const bool aligned4 = ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->W * 3)) & 3) == 0;
-            if (aligned4 && c->g4w) {
-                if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, true>, smemw, c->cfg.device))) return rc;
-                if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, false>, smemw, c->cfg.device))) return rc;
-                if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<8, true>, smemw, c->cfg.device))) return rc;
-                if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<8, false>, smemw, c->cfg.device))) return rc;
-                if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<16, true>, smemw, c->cfg.device))) return rc;
-                if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<16, false>, smemw, c->cfg.device))) return rc;
-                K0GParams gp;
-                gp.g4start = c->g4start; gp.g4n = c->g4n; gp.g4off = c->g4off; gp.g4w = c->g4w;
-                const int blocks16 = segpitch / 16 + 1;         // upper bound of 16-byte blocks per segment
-                const int gridw = (tasks + K0W_WARPS - 1) / K0W_WARPS;
-                const bool inreg = c->g4max <= K0_RG;
-#define FM_K0(PF)                                                                                                   \
-                do {                                                                                                \
-                    if (inreg) k_resize_gray_g4<PF, true><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, gp, segpitch, tasks, nq, dxw); \
-                    else k_resize_gray_g4<PF, false><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, gp, segpitch, tasks, nq, dxw);     \
-                } while (0)
-                if (blocks16 <= 4 * 32) FM_K0(4);
-                else if (blocks16 <= 8 * 32) FM_K0(8);
-                else if (blocks16 <= 16 * 32) FM_K0(16);
-                else k_resize_gray_warp<<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, segpitch, tasks, nq, dxw);
-#undef FM_K0
-            } else {
-                k_resize_gray_warp<<<(tasks + K0W_WARPS - 1) / K0W_WARPS, 32 * K0W_WARPS, smemw, st>>>(p, segpitch, tasks, nq, dxw);
-            }
-            FM_LAUNCH_CHECK();
+            if ((rc = gray_in ? launch_resize_warps<1>(c, p, frames, sstride, fstride, pitch, F, st)
+                              : launch_resize_warps<3>(c, p, frames, sstride, fstride, pitch, F, st)))
+                return rc;
         } else {
-            size_t smem = (size_t)K0_GROUPS * rowpitch + (size_t)p.max_ytaps * c->w * 3 * sizeof(float);
+            size_t smem = (size_t)K0_GROUPS * rowpitch + (size_t)p.max_ytaps * c->w * C * sizeof(float);
             if (smem > 220 * 1024) {
                 fm_set_error("resize front end needs %zu bytes of shared memory (frame too wide / ratio too large)", smem);
                 return FM_ERANGE;
             }
-            int rc;
-            if ((rc = fm_ensure_smem((const void *)k_resize_gray, smem, c->cfg.device))) return rc;
+            const void *kern = gray_in ? (const void *)k_resize_gray<1> : (const void *)k_resize_gray<3>;
+            if ((rc = fm_ensure_smem(kern, smem, c->cfg.device))) return rc;
             dim3 grid(c->h, F);
-            k_resize_gray<<<grid, K0_THREADS, smem, st>>>(p, nullptr, 0);
+            if (gray_in) k_resize_gray<1><<<grid, K0_THREADS, smem, st>>>(p, nullptr, 0);
+            else k_resize_gray<3><<<grid, K0_THREADS, smem, st>>>(p, nullptr, 0);
             FM_LAUNCH_CHECK();
         }
     }

@@ -43,6 +43,8 @@
 #define NV_PITCH 160
 #define NV_Y_BYTES (NV_PITCH * FG_ROWS)                  // 5760 = 45 * 128: the UV box lands 128 B aligned after it
 #define NV_BYTES (NV_Y_BYTES + NV_PITCH * FG_ROWS / 2)   // <= RAW_BYTES: both fit the BGR stage
+// Gray (FM_FLAG_GRAY): a stage holds the luma box alone, rows y0-2 .. y0+FT_H+1 of the caller's frame; no conversion
+enum { FUSED_BGR = 0, FUSED_NV12 = 1, FUSED_GRAY = 2 };     // source format of k_fused
 
 struct FusedParams {
     int T, w, h, wpr;           // T = frames per stream of the call
@@ -216,8 +218,9 @@ __device__ __forceinline__ uint32_t nv12_gray4(uint32_t y4, const FmChroma &c0, 
            (fm_nv12_gray((y4 >> 16) & 0xFFu, c1) << 16) | (fm_nv12_gray(y4 >> 24, c1) << 24);
 }
 
-// NV12: frames arrive as the two boxes above (tmap = luma plane, tmap_uv = chroma plane); otherwise tmap_uv is unused
-template <bool KEEP, bool SAFE, bool NV12>
+// NV12: frames arrive as the two boxes above (tmap = luma plane, tmap_uv = chroma plane); otherwise tmap_uv is unused.
+// GRAY: tmap = the gray frames as one plane of W-byte rows (the NV12 luma box)
+template <bool KEEP, bool SAFE, int SRC>
 __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const __grid_constant__ CUtensorMap tmap, FusedParams p,
                                                                          const __grid_constant__ CUtensorMap tmap_uv) {
     extern __shared__ __align__(128) unsigned char fsm[];
@@ -225,6 +228,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
     uint32_t *sg = reinterpret_cast<uint32_t *>(fsm + 2 * RAW_STAGE);        // [FH_ROWS][FG_WORDS] gray bytes (FG_ROWS used)
     uint32_t *sh = sg + FH_ROWS * FG_WORDS;                                  // [FH_ROWS][FH_WORDS] packed horizontal sums
     uint64_t *bars = reinterpret_cast<uint64_t *>(sh + FH_ROWS * FH_WORDS);
+    constexpr bool NV12 = SRC == FUSED_NV12, GRAY = SRC == FUSED_GRAY;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int s = blockIdx.z;
     const int tx = blockIdx.x, ty = blockIdx.y, tile = ty * p.tilesX + tx;
@@ -276,6 +280,9 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
             fm_mbar_expect_tx(&bars[0], NV_BYTES);
             fm_tma_load_4d(raw, &tmap, &bars[0], x0 / 4 - 4, y0 - 2, 0, s);
             fm_tma_load_4d(raw + NV_Y_BYTES, &tmap_uv, &bars[0], x0 / 4 - 4, y0 / 2 - 1, 0, s);
+        } else if (GRAY) {
+            fm_mbar_expect_tx(&bars[0], NV_Y_BYTES);
+            fm_tma_load_4d(raw, &tmap, &bars[0], x0 / 4 - 4, y0 - 2, 0, s);
         } else {
             fm_mbar_expect_tx(&bars[0], RAW_BYTES);
             fm_tma_load_4d(raw, &tmap, &bars[0], cx, cy, 0, s);
@@ -299,6 +306,12 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
     // the thread's first unit of the BGR -> gray conversion: stage bytes 4 + 24 tid .. (see below), gray words 2 tid, 2 tid + 1
     const int rs_tid = 4 + 24 * tid;
     uint2 *const sgt = reinterpret_cast<uint2 *>(sg) + tid;
+    // gray: the thread copies word gu of rows gr, gr + GROWS, ... (GROWS rows of FG_WORDS words per step): the offsets of
+    // every step are immediates from these two
+    constexpr int GROWS = FUSED_THREADS / FG_WORDS;
+    const int gr = tid / FG_WORDS, gu = tid - gr * FG_WORDS;
+    const int gs_tid = gr * NV_PITCH + 12 + 4 * gu;
+    uint32_t *const sgg = sg + gr * FG_WORDS + gu;
     const uint32_t bars_s = fm_smem_u32(bars);
     uint32_t hits = 0;                  // bit t: frame t has a pixel above threshold in this warp's rows (Ts <= 32)
 #ifdef FM_K1_PROF
@@ -314,6 +327,9 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
                 fm_mbar_expect_tx(&bars[(t + 1) & 1], NV_BYTES);
                 fm_tma_load_4d(dst, &tmap, &bars[(t + 1) & 1], x0 / 4 - 4, y0 - 2, t + 1, s);
                 fm_tma_load_4d(dst + NV_Y_BYTES, &tmap_uv, &bars[(t + 1) & 1], x0 / 4 - 4, y0 / 2 - 1, t + 1, s);
+            } else if (GRAY) {
+                fm_mbar_expect_tx(&bars[(t + 1) & 1], NV_Y_BYTES);
+                fm_tma_load_4d(raw + ((t + 1) & 1) * RAW_STAGE, &tmap, &bars[(t + 1) & 1], x0 / 4 - 4, y0 - 2, t + 1, s);
             } else {
                 fm_mbar_expect_tx(&bars[(t + 1) & 1], RAW_BYTES);
                 fm_tma_load_4d(raw + ((t + 1) & 1) * RAW_STAGE, &tmap, &bars[(t + 1) & 1], cx, cy, t + 1, s);
@@ -342,6 +358,16 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
                     sg[2 * k * FG_WORDS + u] = nv12_gray4(l0, c0, c1);
                     sg[(2 * k + 1) * FG_WORDS + u] = nv12_gray4(l1, c0, c1);
                 }
+            }
+        } else if (GRAY) {
+            // the stage already holds gray bytes: word u of a row (columns x0-4+4u .. +3) is at byte 12 + 4u of its box row.
+            // Zero-filled bytes outside the image are overwritten by the border step below, as with BGR.
+            const unsigned char *st = raw + (t & 1) * RAW_STAGE + gs_tid;
+            if (gr < GROWS) {
+#pragma unroll 1                // unrolled, the six loads in flight push the kernel to 40 spilled bytes (rolled: 20)
+                for (int i = 0; i < (FG_ROWS + GROWS - 1) / GROWS; i++)
+                    if ((i + 1) * GROWS <= FG_ROWS || gr + i * GROWS < FG_ROWS)
+                        sgg[i * GROWS * FG_WORDS] = *reinterpret_cast<const uint32_t *>(st + i * GROWS * NV_PITCH);
             }
         } else {
             // the staged rows are dense (pitch 432 B = 36 groups of 4 pixels = 12 B, the first at byte 4 because the
@@ -471,7 +497,7 @@ __global__ void k_bg_export_fused(const double *__restrict__ bg, double *__restr
 
 // NV12 needs nothing more: W % 32 == 0 makes the luma and chroma rows 16 B aligned, and with an even H (fm_ctx_create)
 // the frame (W * H * 3 / 2 bytes) and the chroma plane's offset (W * H) too; the caller's pointer and strides are checked
-// at launch, as with BGR
+// at launch, as with BGR.  Nor does gray: its rows and frames (W * H bytes) are 16 B aligned with W % 32 == 0
 bool fm_fused_supported(const fm_ctx *c) {
     return c->resize_mode == 0 && c->k <= 5 && (c->w % 32) == 0 && c->w >= 4 && c->h >= 4 && c->frame_bytes % 16 == 0;
 }
@@ -507,8 +533,8 @@ extern "C" void fm_k1_prof_dump(void) {
 
 #define FUSED_SMEM (2 * RAW_STAGE + FH_ROWS * FG_WORDS * 4 + FH_ROWS * FH_WORDS * 4 + 16)
 
-// one plane of the call's NV12 frames (rows of W bytes, `pitch` bytes apart) as a 4-D u32 tensor map with boxes of
-// NV_PITCH bytes x box_rows
+// one plane of the call's NV12 frames, or the gray frames (rows of W bytes, `pitch` bytes apart), as a 4-D u32 tensor map
+// with boxes of NV_PITCH bytes x box_rows
 static int nv12_plane_tmap(const fm_ctx *c, const uint8_t *plane, int rows, size_t sstride, size_t fstride, size_t pitch, int T,
                            int box_rows, CUtensorMap *out) {
     PFN_encodeTiled enc = fm_tma_encoder();
@@ -529,6 +555,7 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
                     cudaStream_t st) {
     CUtensorMap tmap, tmap_uv;
     const bool nv12 = c->nv12_bgr == nullptr && (c->cfg.flags & FM_FLAG_NV12);     // NV12 read directly (no staged slot)
+    const bool gray = (c->cfg.flags & FM_FLAG_GRAY) != 0;
     int rc;
     if (nv12) {
         if ((((uintptr_t)frames) | sstride | fstride | pitch | (size_t)uv) & 15) {
@@ -537,6 +564,13 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
         }
         if ((rc = nv12_plane_tmap(c, frames, c->H, sstride, fstride, pitch, T, FG_ROWS, &tmap))) return rc;
         if ((rc = nv12_plane_tmap(c, frames + uv, c->H / 2, sstride, fstride, pitch, T, FG_ROWS / 2, &tmap_uv))) return rc;
+    } else if (gray) {
+        if ((((uintptr_t)frames) | sstride | fstride | pitch) & 15) {
+            fm_set_error("the fused gray front end needs 16-byte aligned frames, strides and row pitch");
+            return FM_EINVAL;
+        }
+        if ((rc = nv12_plane_tmap(c, frames, c->H, sstride, fstride, pitch, T, FG_ROWS, &tmap))) return rc;
+        tmap_uv = tmap;                          // not read
     } else {
         if ((rc = fm_frames_tmap(c, frames, sstride, fstride, pitch, T, RAW_PITCH / 4, FG_ROWS, &tmap))) return rc;
         tmap_uv = tmap;                          // not read
@@ -579,11 +613,11 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     fused_bfr(p);
     dim3 grid(p.tilesX, p.tilesY, c->S);
     typedef void (*FusedKernel)(const CUtensorMap, FusedParams, const CUtensorMap);
-    const FusedKernel kerns[2][2][2] = {{{k_fused<false, false, false>, k_fused<false, false, true>},
-                                         {k_fused<false, true, false>, k_fused<false, true, true>}},
-                                        {{k_fused<true, false, false>, k_fused<true, false, true>},
-                                         {k_fused<true, true, false>, k_fused<true, true, true>}}};
-    const FusedKernel kern = kerns[keep][safe][nv12];
+#define FM_K1_SRCS(K, S) {k_fused<K, S, FUSED_BGR>, k_fused<K, S, FUSED_NV12>, k_fused<K, S, FUSED_GRAY>}
+    const FusedKernel kerns[2][2][3] = {{FM_K1_SRCS(false, false), FM_K1_SRCS(false, true)},
+                                        {FM_K1_SRCS(true, false), FM_K1_SRCS(true, true)}};
+#undef FM_K1_SRCS
+    const FusedKernel kern = kerns[keep][safe][nv12 ? FUSED_NV12 : gray ? FUSED_GRAY : FUSED_BGR];
     if ((rc = fm_ensure_smem((const void *)kern, FUSED_SMEM, c->cfg.device))) return rc;
     // a programmatic dependent of the contour stage of the previous call: see fused_exit.  Not after the NV12 staging
     // kernel (k_nv12.cu, FM_NV12_STAGED builds): K1 reads the frames before its wait, and that kernel writes them

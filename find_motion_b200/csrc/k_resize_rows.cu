@@ -16,6 +16,9 @@
 //   phase 2: thread = (destination row, column, channel): vertical chain over the rows of its cell -> BGR byte
 // and at the end of the segment the BGR bytes become gray bytes of the processing plane (or, in the BGR variant, are stored
 // as they are: the detector input plane of fm_object_planes, k_objects.cu).
+// C = 1 (FM_FLAG_GRAY): one-byte source pixels, a tap group of 4 pixels is one word instead of three, and each column has
+// one chain per row instead of three; per chain the products and sums are those of one channel of the BGR kernel.  The
+// gray variant stores the resized bytes as they are, the BGR one stores each in B, G and R.
 #include <cuda.h>
 
 #include <algorithm>
@@ -67,10 +70,10 @@ __device__ __forceinline__ uint4 rr_lds128(uint32_t addr) {
 // address `blk`, bytes realigned by `sel` (PRMT selector 0x3210 + 0x1111 * (byte offset & 3)); weights are warp-uniform
 // (broadcast loads).  The last block may reach past the column's last tap (other columns, the next row, the next shared
 // buffer): finite bytes that only meet zero weights or nothing at all.
-template <int WO, int NPG>
+template <int WO, int NPG, int C>
 __device__ __forceinline__ void rr_col_pass(uint32_t blk, uint32_t sel, const float4 *__restrict__ wp, float &b0, float &b1,
                                             float &b2) {
-    constexpr int NL = (WO + 3 * NPG) / 4 + 1;           // 16-byte blocks that hold words WO .. WO + 3 NPG
+    constexpr int NL = (WO + C * NPG) / 4 + 1;           // 16-byte blocks that hold words WO .. WO + C NPG
     uint32_t W[4 * NL];
 #pragma unroll
     for (int k = 0; k < NL; k++) {
@@ -80,29 +83,35 @@ __device__ __forceinline__ void rr_col_pass(uint32_t blk, uint32_t sel, const fl
 #pragma unroll
     for (int g = 0; g < NPG; g++) {          // straight-line code: the compiler schedules the weight loads ahead of their use
         const float4 a = __ldg(wp + 2 * g), n = __ldg(wp + 2 * g + 1);
-        const uint32_t X0 = __byte_perm(W[WO + 3 * g], W[WO + 3 * g + 1], sel);
-        const uint32_t X1 = __byte_perm(W[WO + 3 * g + 1], W[WO + 3 * g + 2], sel);
-        const uint32_t X2 = __byte_perm(W[WO + 3 * g + 2], W[WO + 3 * g + 3], sel);
-        // pixels in source order, channels B G R of each: the strictly ordered chains of resizeArea_
-        b0 = __fadd_rn(b0, fm_byte_mul(X0, 0, a.x, n.x)); b1 = __fadd_rn(b1, fm_byte_mul(X0, 1, a.x, n.x));
-        b2 = __fadd_rn(b2, fm_byte_mul(X0, 2, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(X0, 3, a.y, n.y));
-        b1 = __fadd_rn(b1, fm_byte_mul(X1, 0, a.y, n.y)); b2 = __fadd_rn(b2, fm_byte_mul(X1, 1, a.y, n.y));
-        b0 = __fadd_rn(b0, fm_byte_mul(X1, 2, a.z, n.z)); b1 = __fadd_rn(b1, fm_byte_mul(X1, 3, a.z, n.z));
-        b2 = __fadd_rn(b2, fm_byte_mul(X2, 0, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(X2, 1, a.w, n.w));
-        b1 = __fadd_rn(b1, fm_byte_mul(X2, 2, a.w, n.w)); b2 = __fadd_rn(b2, fm_byte_mul(X2, 3, a.w, n.w));
+        if constexpr (C == 1) {              // 4 pixels of one channel: one chain
+            const uint32_t X = __byte_perm(W[WO + g], W[WO + g + 1], sel);
+            b0 = __fadd_rn(b0, fm_byte_mul(X, 0, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(X, 1, a.y, n.y));
+            b0 = __fadd_rn(b0, fm_byte_mul(X, 2, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(X, 3, a.w, n.w));
+        } else {
+            const uint32_t X0 = __byte_perm(W[WO + 3 * g], W[WO + 3 * g + 1], sel);
+            const uint32_t X1 = __byte_perm(W[WO + 3 * g + 1], W[WO + 3 * g + 2], sel);
+            const uint32_t X2 = __byte_perm(W[WO + 3 * g + 2], W[WO + 3 * g + 3], sel);
+            // pixels in source order, channels B G R of each: the strictly ordered chains of resizeArea_
+            b0 = __fadd_rn(b0, fm_byte_mul(X0, 0, a.x, n.x)); b1 = __fadd_rn(b1, fm_byte_mul(X0, 1, a.x, n.x));
+            b2 = __fadd_rn(b2, fm_byte_mul(X0, 2, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(X0, 3, a.y, n.y));
+            b1 = __fadd_rn(b1, fm_byte_mul(X1, 0, a.y, n.y)); b2 = __fadd_rn(b2, fm_byte_mul(X1, 1, a.y, n.y));
+            b0 = __fadd_rn(b0, fm_byte_mul(X1, 2, a.z, n.z)); b1 = __fadd_rn(b1, fm_byte_mul(X1, 3, a.z, n.z));
+            b2 = __fadd_rn(b2, fm_byte_mul(X2, 0, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(X2, 1, a.w, n.w));
+            b1 = __fadd_rn(b1, fm_byte_mul(X2, 2, a.w, n.w)); b2 = __fadd_rn(b2, fm_byte_mul(X2, 3, a.w, n.w));
+        }
     }
 }
 
-template <int WO>
+template <int WO, int C>
 __device__ __forceinline__ void rr_col_pass_n(uint32_t blk, uint32_t sel, int npg, const float4 *__restrict__ wp, float &b0,
                                               float &b1, float &b2) {
     switch (npg) {                            // warp-uniform
-    case 1: rr_col_pass<WO, 1>(blk, sel, wp, b0, b1, b2); break;
-    case 2: rr_col_pass<WO, 2>(blk, sel, wp, b0, b1, b2); break;
-    case 3: rr_col_pass<WO, 3>(blk, sel, wp, b0, b1, b2); break;
-    case 4: rr_col_pass<WO, 4>(blk, sel, wp, b0, b1, b2); break;
-    case 5: rr_col_pass<WO, 5>(blk, sel, wp, b0, b1, b2); break;
-    default: rr_col_pass<WO, RR_GMAX>(blk, sel, wp, b0, b1, b2); break;
+    case 1: rr_col_pass<WO, 1, C>(blk, sel, wp, b0, b1, b2); break;
+    case 2: rr_col_pass<WO, 2, C>(blk, sel, wp, b0, b1, b2); break;
+    case 3: rr_col_pass<WO, 3, C>(blk, sel, wp, b0, b1, b2); break;
+    case 4: rr_col_pass<WO, 4, C>(blk, sel, wp, b0, b1, b2); break;
+    case 5: rr_col_pass<WO, 5, C>(blk, sel, wp, b0, b1, b2); break;
+    default: rr_col_pass<WO, RR_GMAX, C>(blk, sel, wp, b0, b1, b2); break;
     }
 }
 
@@ -123,7 +132,8 @@ __device__ __forceinline__ void rr_bar_arrive(int id, int count) {
 // (row warps arrive, warp 5 waits); 3 + (i & 1): "hs buffer i & 1 consumed" (warp 5 arrives, row warps wait before chunk
 // i + 2), so the row warps run up to two chunks ahead of the vertical warp and never wait for each other.
 // BGR: warp 5 stores the band's BGR bytes as they are (the detector input plane) for the frames with oidx >= 0.
-template <bool BGR>
+// C: channels of the source (3 BGR, 1 gray)
+template <bool BGR, int C>
 __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(const __grid_constant__ CUtensorMap tmap, RowsParams p) {
     extern __shared__ __align__(128) unsigned char rsm[];
     const int tid = threadIdx.x;
@@ -143,11 +153,11 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
     const int nrows = __ldg(p.yidx + yb + ytn - 1) - R0 + 1;
 
     unsigned char *stage = rsm;                                                    // [2][stage_stride]
-    float *hs = reinterpret_cast<float *>(rsm + 2 * (size_t)p.stage_stride);       // [2][CX * 3][NRp]
-    const int hsbuf = CX * 3 * NRp;
+    float *hs = reinterpret_cast<float *>(rsm + 2 * (size_t)p.stage_stride);       // [2][CX * C][NRp]
+    const int hsbuf = CX * C * NRp;
     float *yw = hs + 2 * hsbuf;                                                    // [2 NR] y weights of the band
     uint64_t *bars = reinterpret_cast<uint64_t *>((reinterpret_cast<uintptr_t>(yw + 2 * p.NR) + 7) & ~(uintptr_t)7);
-    unsigned char *bgr = reinterpret_cast<unsigned char *>(bars + 2);              // [D][DXU][3]
+    unsigned char *bgr = reinterpret_cast<unsigned char *>(bars + 2);              // [D][DXU][C]
     constexpr int NT = RR_THREADS + 32;
 
     if (tid == 0) {
@@ -177,20 +187,22 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
                     float b0 = 0.f, b1 = 0.f, b2 = 0.f;
 #pragma unroll 1
                     for (int g0 = 0; g0 < ci.y; g0 += RR_GMAX) {
-                        const int off = ci.x + 12 * g0;
+                        const int off = ci.x + 4 * C * g0;
                         const int npg = min(RR_GMAX, ci.y - g0);
                         const uint32_t blk = myrow + (uint32_t)(off & ~15);
                         switch ((off >> 2) & 3) {
-                        case 0: rr_col_pass_n<0>(blk, sel, npg, wp + 2 * g0, b0, b1, b2); break;
-                        case 1: rr_col_pass_n<1>(blk, sel, npg, wp + 2 * g0, b0, b1, b2); break;
-                        case 2: rr_col_pass_n<2>(blk, sel, npg, wp + 2 * g0, b0, b1, b2); break;
-                        default: rr_col_pass_n<3>(blk, sel, npg, wp + 2 * g0, b0, b1, b2); break;
+                        case 0: rr_col_pass_n<0, C>(blk, sel, npg, wp + 2 * g0, b0, b1, b2); break;
+                        case 1: rr_col_pass_n<1, C>(blk, sel, npg, wp + 2 * g0, b0, b1, b2); break;
+                        case 2: rr_col_pass_n<2, C>(blk, sel, npg, wp + 2 * g0, b0, b1, b2); break;
+                        default: rr_col_pass_n<3, C>(blk, sel, npg, wp + 2 * g0, b0, b1, b2); break;
                         }
                     }
                     if (tid < nrows) {        // lanes past the band's last row ran on rows of the box that nobody reads
-                        hw[(3 * dxl) * NRp] = b0;
-                        hw[(3 * dxl + 1) * NRp] = b1;
-                        hw[(3 * dxl + 2) * NRp] = b2;
+                        hw[(C * dxl) * NRp] = b0;
+                        if (C == 3) {
+                            hw[(C * dxl + 1) * NRp] = b1;
+                            hw[(C * dxl + 2) * NRp] = b2;
+                        }
                     }
                 }
             }
@@ -218,7 +230,7 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
         if (lane == 0 && i + 2 < nch) issue(i + 2);
         // vertical chains of the chunk's cells: task = (destination row, column, channel)
         const float *hb = hs + (i & 1) * hsbuf;
-        const int nq = cxn * 3, ntask = Dn * nq;
+        const int nq = cxn * C, ntask = Dn * nq;
         for (int task = lane; task < ntask; task += 32) {
             const int dyl = task / nq, q = task - dyl * nq;
             const int y0 = __ldg(p.ystart + dy0 + dyl), ny = __ldg(p.ystart + dy0 + dyl + 1) - y0;
@@ -227,7 +239,7 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
             float sum = __fmul_rn(wy[0], hp[0]);
             for (int j = 1; j < ny; j++) sum = __fadd_rn(sum, __fmul_rn(wy[j], hp[j]));
             const int v = min(max(__float2int_rn(sum), 0), 255);
-            bgr[(dyl * DXU + (dx0 - dxa)) * 3 + q] = (unsigned char)v;
+            bgr[(dyl * DXU + (dx0 - dxa)) * C + q] = (unsigned char)v;
         }
         if (i + 2 < nch) {
             __threadfence_block();
@@ -240,15 +252,15 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
         const int rb = dxun * 3;
         for (int i = lane; i < Dn * rb; i += 32) {
             const int dyl = i / rb, b = i - dyl * rb;
-            o[(size_t)dyl * p.w * 3 + b] = bgr[dyl * DXU * 3 + b];
+            o[(size_t)dyl * p.w * 3 + b] = C == 1 ? bgr[dyl * DXU + b / 3] : bgr[dyl * DXU * 3 + b];
         }
     } else {
         // ---- BGR -> gray (SURVEY.md A.2) ----
         for (int i = lane; i < Dn * dxun; i += 32) {
             const int dyl = i / dxun, dxo = i - dyl * dxun;
-            const unsigned char *q = bgr + (dyl * DXU + dxo) * 3;
+            const unsigned char *q = bgr + (dyl * DXU + dxo) * C;
             p.gray[((size_t)f * p.h + dy0 + dyl) * p.w + dxa + dxo] =
-                (uint8_t)fm_gray(q[0], q[1], q[2]);
+                C == 1 ? q[0] : (uint8_t)fm_gray(q[0], q[1], q[C - 1]);
         }
     }
 }
@@ -280,13 +292,13 @@ static int rr_env(const char *name, int dflt) {
     return (e && *e) ? atoi(e) : dflt;
 }
 
-// Host arithmetic of the plan (no CUDA): fills r and the three tables for the decimation tables of a geometry.  false: the
-// geometry does not fit the kernel (source rows not TMA-compatible, bands taller than the CTA, tiny ratios) and the
-// warp-per-row kernels stay in charge.
-static bool rr_layout(int W, int w, int h, const int *xstart, const int *xidx, const float *xwt, const int *ystart,
+// Host arithmetic of the plan (no CUDA): fills r and the three tables for the decimation tables of a geometry with C-byte
+// pixels (3 BGR, 1 gray).  false: the geometry does not fit the kernel (source rows not TMA-compatible, bands taller than
+// the CTA, tiny ratios) and the warp-per-row kernels stay in charge.
+static bool rr_layout(int W, int w, int h, int C, const int *xstart, const int *xidx, const float *xwt, const int *ystart,
                       const int *yidx, RowsPlan *r, std::vector<int4> &col, std::vector<float4> &rw, std::vector<int> &cstartw) {
     memset(r, 0, sizeof(*r));
-    if (((size_t)W * 3) % 16 != 0) return false;
+    if (((size_t)W * C) % 16 != 0) return false;
     // band height: the most destination rows whose source rows fit the CTA
     auto band_rows = [&](int D) {
         int mx = 0;
@@ -322,14 +334,14 @@ static bool rr_layout(int W, int w, int h, const int *xstart, const int *xidx, c
         const int nchunks = (w + cx - 1) / cx;
         for (int ch = 0; ch < nchunks; ch++) {
             const int dxa = ch * cx, dxb = std::min(dxa + cx, w);
-            const int cstart = (3 * xidx[xstart[dxa]]) & ~15;
+            const int cstart = (C * xidx[xstart[dxa]]) & ~15;
             cstartw.push_back(cstart / 4);
             for (int dx = dxa; dx < dxb; dx++) {
                 const int a = xstart[dx], b = xstart[dx + 1], first = xidx[a], nt = b - a;
                 for (int q = a; q < b; q++)
                     if (xidx[q] != first + (q - a)) return false;              // taps are consecutive pixels (always, for INTER_AREA)
                 // groups of 4 consecutive source pixels from the first tap on, zero-weight padded at the end
-                const int ng = (nt + 3) / 4, off = 3 * first - cstart;
+                const int ng = (nt + 3) / 4, off = C * first - cstart;
                 col[dx] = make_int4(off, ng, (int)rw.size(), 0);
                 for (int g = 0; g < ng; g++) {
                     float wv[4];
@@ -339,8 +351,8 @@ static bool rr_layout(int W, int w, int h, const int *xstart, const int *xidx, c
                 }
                 // 16-byte blocks the passes of this column read: block (off >> 4) + ((WO + 3 npg) >> 2) of the last pass
                 for (int g0 = 0; g0 < ng; g0 += RR_GMAX) {
-                    const int o = off + 12 * g0, npg = std::min(RR_GMAX, ng - g0);
-                    const int last = (o >> 4) + ((((o >> 2) & 3) + 3 * npg) >> 2);
+                    const int o = off + 4 * C * g0, npg = std::min(RR_GMAX, ng - g0);
+                    const int last = (o >> 4) + ((((o >> 2) & 3) + C * npg) >> 2);
                     BW = std::max(BW, 16 * (last + 1));
                 }
             }
@@ -350,8 +362,8 @@ static bool rr_layout(int W, int w, int h, const int *xstart, const int *xidx, c
         if (BW / 4 > 256) return false;        // TMA box limit
         r->BW = BW;
         r->stage_stride = (uint32_t)(((size_t)r->NR * BW + 127) / 128 * 128);
-        r->smem = 2 * (size_t)r->stage_stride + ((size_t)2 * cx * 3 * r->NRp + 2 * r->NR) * sizeof(float) + 8 + 16 +
-                  (size_t)r->D * DXU * 3;
+        r->smem = 2 * (size_t)r->stage_stride + ((size_t)2 * cx * C * r->NRp + 2 * r->NR) * sizeof(float) + 8 + 16 +
+                  (size_t)r->D * DXU * C;
         return r->smem <= 200 * 1024;
     };
     const int forced = rr_env("FM_K0_CX", 0);
@@ -361,7 +373,7 @@ static bool rr_layout(int W, int w, int h, const int *xstart, const int *xidx, c
 
 // Builds the plan of a W -> w x h decimation into *out; leaves it null when the geometry does not fit (rr_layout) or
 // FM_FLAG_NO_ROWS is set.
-static int rr_build(fm_ctx *c, const void *kern, int w, int h, const int *xstart, const int *xidx, const float *xwt,
+static int rr_build(fm_ctx *c, const void *kern, int w, int h, int C, const int *xstart, const int *xidx, const float *xwt,
                     const int *ystart, const int *yidx, RowsPlan **out) {
     *out = nullptr;
     if (c->cfg.flags & FM_FLAG_NO_ROWS) return FM_OK;
@@ -369,7 +381,7 @@ static int rr_build(fm_ctx *c, const void *kern, int w, int h, const int *xstart
     std::vector<int4> col;
     std::vector<float4> rw;
     std::vector<int> cstartw;
-    if (!rr_layout(c->W, w, h, xstart, xidx, xwt, ystart, yidx, r, col, rw, cstartw)) { delete r; return FM_OK; }
+    if (!rr_layout(c->W, w, h, C, xstart, xidx, xwt, ystart, yidx, r, col, rw, cstartw)) { delete r; return FM_OK; }
     if (!rr_upload(&r->coltab, col) || !rr_upload(&r->cstartw, cstartw) || !rr_upload(&r->rw, rw)) {
         cudaFree(r->coltab); cudaFree(r->cstartw); cudaFree(r->rw);
         delete r;
@@ -380,25 +392,30 @@ static int rr_build(fm_ctx *c, const void *kern, int w, int h, const int *xstart
     return fm_ensure_smem(kern, r->smem, c->cfg.device);
 }
 
+static int rr_channels(const fm_ctx *c) { return (c->cfg.flags & FM_FLAG_GRAY) ? 1 : 3; }
+
 // the processing plane (gray out) and the detector input plane (BGR out)
 int fm_rows_plan(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx) {
-    return rr_build(c, (const void *)k_resize_rows<false>, c->w, c->h, xstart, xidx, xwt, ystart, yidx, &c->rows);
+    const int C = rr_channels(c);
+    return rr_build(c, C == 1 ? (const void *)k_resize_rows<false, 1> : (const void *)k_resize_rows<false, 3>, c->w, c->h, C,
+                    xstart, xidx, xwt, ystart, yidx, &c->rows);
 }
 int fm_rows_plan_objects(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx) {
-    return rr_build(c, (const void *)k_resize_rows<true>, FM_OBJECT_WIDTH, c->obj_h, xstart, xidx, xwt, ystart, yidx,
-                    &c->obj_rows);
+    const int C = rr_channels(c);
+    return rr_build(c, C == 1 ? (const void *)k_resize_rows<true, 1> : (const void *)k_resize_rows<true, 3>, FM_OBJECT_WIDTH,
+                    c->obj_h, C, xstart, xidx, xwt, ystart, yidx, &c->obj_rows);
 }
 
 // Plan of a geometry without a device (include/fm_gpu.h: fm_debug_rows_plan): the layout plus a re-check, tap by tap, that
 // every shared-memory read of every column pass stays inside the chunk's box and meets the weight the tables give it.
-int fm_rows_plan_describe(int W, int w, int h, const int *xstart, const int *xidx, const float *xwt, const int *ystart,
+int fm_rows_plan_describe(int W, int w, int h, int C, const int *xstart, const int *xidx, const float *xwt, const int *ystart,
                           const int *yidx, fm_rows_plan_info *out) {
     RowsPlan r;
     std::vector<int4> col;
     std::vector<float4> rw;
     std::vector<int> cstartw;
     memset(out, 0, sizeof(*out));
-    if (!rr_layout(W, w, h, xstart, xidx, xwt, ystart, yidx, &r, col, rw, cstartw)) return FM_OK;
+    if (!rr_layout(W, w, h, C, xstart, xidx, xwt, ystart, yidx, &r, col, rw, cstartw)) return FM_OK;
     out->usable = 1;
     out->band_rows = r.D; out->box_rows = r.NR; out->chunk_cols = r.CX; out->seg_cols = r.CX * r.NCHU;
     out->box_bytes = r.BW; out->smem_bytes = (int32_t)r.smem; out->bands = r.nbands; out->segs = r.segs;
@@ -406,17 +423,17 @@ int fm_rows_plan_describe(int W, int w, int h, const int *xstart, const int *xid
         const int ch = dx / r.CX, a = xstart[dx], nt = xstart[dx + 1] - a;
         const int4 ci = col[dx];
         out->max_groups = std::max(out->max_groups, ci.y);
-        if (4 * cstartw[ch] + ci.x != 3 * xidx[a] || (cstartw[ch] & 3) || ci.x < 0) { fm_set_error("rows plan: column %d misplaced", dx); return FM_ERANGE; }
+        if (4 * cstartw[ch] + ci.x != C * xidx[a] || (cstartw[ch] & 3) || ci.x < 0) { fm_set_error("rows plan: column %d misplaced", dx); return FM_ERANGE; }
         for (int g = 0; g < ci.y; g++)
             for (int i = 0; i < 4; i++) {
                 const float wv = (&rw[ci.z + 2 * g].x)[i], nv = (&rw[ci.z + 2 * g + 1].x)[i];
                 const float want = 4 * g + i < nt ? xwt[a + 4 * g + i] : 0.0f;
                 if (wv != want || nv != -8388608.0f * want) { fm_set_error("rows plan: weight of column %d tap %d", dx, 4 * g + i); return FM_ERANGE; }
-                if (ci.x + 3 * (4 * g + i) + 2 >= r.BW) { fm_set_error("rows plan: column %d reads past the box", dx); return FM_ERANGE; }
+                if (ci.x + C * (4 * g + i) + C - 1 >= r.BW) { fm_set_error("rows plan: column %d reads past the box", dx); return FM_ERANGE; }
             }
         for (int g0 = 0; g0 < ci.y; g0 += RR_GMAX) {           // the 128-bit loads of a pass
-            const int o = ci.x + 12 * g0, npg = std::min(RR_GMAX, ci.y - g0);
-            if (16 * ((o >> 4) + ((((o >> 2) & 3) + 3 * npg) >> 2) + 1) > r.BW) { fm_set_error("rows plan: pass of column %d reads past the box", dx); return FM_ERANGE; }
+            const int o = ci.x + 4 * C * g0, npg = std::min(RR_GMAX, ci.y - g0);
+            if (16 * ((o >> 4) + ((((o >> 2) & 3) + C * npg) >> 2) + 1) > r.BW) { fm_set_error("rows plan: pass of column %d reads past the box", dx); return FM_ERANGE; }
         }
     }
     for (int b = 0; b < r.nbands; b++) {
@@ -445,7 +462,8 @@ static int rr_launch(const fm_ctx *c, const RowsPlan *r, int w, int h, const Res
     p.gray = c->gray; p.nvalid = c->nvalid;
     p.oidx = c->obj_idx; p.out = out; p.ostride = ostride;
     dim3 grid(r->segs, r->nbands, c->S * T);
-    k_resize_rows<BGR><<<grid, RR_THREADS + 32, r->smem, st>>>(tmap, p);
+    if (rr_channels(c) == 1) k_resize_rows<BGR, 1><<<grid, RR_THREADS + 32, r->smem, st>>>(tmap, p);
+    else k_resize_rows<BGR, 3><<<grid, RR_THREADS + 32, r->smem, st>>>(tmap, p);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }

@@ -548,7 +548,8 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
 
 // ---------------------------------------------------------------------------------------------
 // padded gray plane: gpad[f][yp][xp] = gray(reflect101(yp - 48), reflect101(xp - 48)); BGR: convert on the way
-// (find_motion.py:493, SURVEY.md A.2).  One thread = 4 padded pixels.
+// (find_motion.py:493, SURVEY.md A.2); otherwise src is a gray plane (the context's, or gray frames).  Frame (s, t) starts at
+// src + s * sstride + t * fstride, rows rpitch bytes apart.  One thread = 4 padded pixels.
 // ---------------------------------------------------------------------------------------------
 template <bool BGR>
 __global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ src, size_t sstride, size_t fstride, size_t rpitch, int T,
@@ -561,8 +562,7 @@ __global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ sr
     uint32_t out = 0;
     if (yp < h + 2 * UB_PAD && xp < w + 2 * UB_PAD) {
         const int y = fm_reflect101(yp - UB_PAD, h);
-        const uint8_t *row = BGR ? src + (size_t)s * sstride + (size_t)t * fstride + (size_t)y * rpitch
-                                 : src + ((size_t)f * h + y) * w;
+        const uint8_t *row = src + (size_t)s * sstride + (size_t)t * fstride + (size_t)y * rpitch;
         const int x = xp - UB_PAD;
         if (x >= 0 && x + 3 < w && aligned4) {
             if (BGR) {
@@ -637,10 +637,11 @@ static std::vector<uint8_t> make_band(const fm_ctx *c, const int *taps, int RA, 
     return band;
 }
 
-// the BGR frames can feed the tcgen05 kernel directly (TMA over the caller's frames, mirroring inside the tile)
+// the BGR frames can feed the tcgen05 kernel directly (TMA over the caller's frames, mirroring inside the tile); gray frames
+// take the apron plane, which k_pad_gray fills from them in place
 static bool umma_fused_geometry(const fm_ctx *c) {
     const int r = c->k >> 1;
-    return c->resize_mode == 0 && (c->W % 16) == 0 && c->w >= r + 2 && c->h >= r + 2;
+    return c->resize_mode == 0 && (c->W % 16) == 0 && c->w >= r + 2 && c->h >= r + 2 && !(c->cfg.flags & FM_FLAG_GRAY);
 }
 
 int fm_umma_init(fm_ctx *c, const int *taps) {
@@ -742,16 +743,21 @@ int fm_launch_umma_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t
     umma_geom(c, &tilesX, &tilesY, &Wp, &Hp);
     const int F = c->S * T;
     dim3 pgrid((Wp / 4 + 255) / 256, Hp, F);
-    if (frames) {
-        if (c->cfg.flags & FM_FLAG_KEEP_PLANES) {          // parity tap of the gray conversion
-            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
-            if (rc) return rc;
-        }
+    const bool gray_in = frames && (c->cfg.flags & FM_FLAG_GRAY);
+    if (frames && (c->cfg.flags & FM_FLAG_KEEP_PLANES)) {      // parity tap of the gray conversion (gray frames: a copy)
+        int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
+        if (rc) return rc;
+    }
+    if (frames && !gray_in) {
         const int al = ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->w * 3)) & 3) == 0;
         k_pad_gray<true><<<pgrid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->gpad, c->w, c->h, Wp, Hp, c->nvalid, al);
+    } else if (gray_in) {
+        const int al = ((((uintptr_t)frames) | sstride | fstride | pitch | (size_t)c->w) & 3) == 0;
+        k_pad_gray<false><<<pgrid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->gpad, c->w, c->h, Wp, Hp, c->nvalid, al);
     } else {
         const int al = (c->w & 3) == 0;
-        k_pad_gray<false><<<pgrid, 256, 0, st>>>(c->gray, 0, 0, 0, T, c->gpad, c->w, c->h, Wp, Hp, c->nvalid, al);
+        k_pad_gray<false><<<pgrid, 256, 0, st>>>(c->gray, (size_t)T * c->N, (size_t)c->N, (size_t)c->w, T, c->gpad, c->w, c->h, Wp,
+                                                 Hp, c->nvalid, al);
     }
     FM_LAUNCH_CHECK();
     CUtensorMap tmap;

@@ -19,7 +19,7 @@
 struct UpParams {
     const uint8_t *frames;
     size_t sstride, fstride;
-    size_t pitch;               // bytes from one source row to the next (>= W * 3)
+    size_t pitch;               // bytes from one source row to the next (>= W * channels)
     int T, W, H, w, h;
     int band;                   // destination rows per CTA
     const int2 *xt;             // [w] (source x, a0 | a1 << 16)
@@ -31,35 +31,38 @@ struct UpParams {
     size_t ostride;             //   bgr_out + s * ostride + oidx[f] * h*w*3 (fm_object_planes)
 };
 
-// horizontal pass of one source row into a staged row of u16 (hx >> 4), 4 destination columns per thread
+// horizontal pass of one source row into a staged row of u16 (hx >> 4), 4 destination columns per thread.  C: channels of
+// the source (3 BGR, 1 gray; each channel is interpolated the same way)
+template <int C>
 __device__ __forceinline__ void up_hrow(const UpParams &p, const uint8_t *__restrict__ row, uint16_t *out) {
     const int nq = (p.w + 3) >> 2;
     for (int q = threadIdx.x; q < nq; q += UP_THREADS) {
         const int dx0 = q * 4;
-        uint32_t v[12];
+        uint32_t v[4 * C];
 #pragma unroll
         for (int j = 0; j < 4; j++) {
             const int dx = min(dx0 + j, p.w - 1);                       // columns past w: computed, not stored
             const int2 xv = __ldg(p.xt + dx);
-            const uint8_t *a = row + 3 * xv.x;
-            const uint8_t *b = row + 3 * min(xv.x + 1, p.W - 1);
+            const uint8_t *a = row + C * xv.x;
+            const uint8_t *b = row + C * min(xv.x + 1, p.W - 1);
             const uint32_t a0 = (uint32_t)xv.y & 0xffffu, a1 = (uint32_t)xv.y >> 16;
 #pragma unroll
-            for (int ch = 0; ch < 3; ch++) v[3 * j + ch] = ((uint32_t)__ldg(a + ch) * a0 + (uint32_t)__ldg(b + ch) * a1) >> 4;
+            for (int ch = 0; ch < C; ch++) v[C * j + ch] = ((uint32_t)__ldg(a + ch) * a0 + (uint32_t)__ldg(b + ch) * a1) >> 4;
         }
-        uint16_t *o = out + 12 * q;
-        if (dx0 + 4 <= p.w) {                                           // 24 bytes at a multiple of 24: three 8-byte stores
+        uint16_t *o = out + 4 * C * q;
+        if (dx0 + 4 <= p.w) {                                           // 8 C bytes at a multiple of 8 C: C 8-byte stores
 #pragma unroll
-            for (int k = 0; k < 3; k++)
+            for (int k = 0; k < C; k++)
                 reinterpret_cast<uint2 *>(o)[k] = make_uint2(v[4 * k] | (v[4 * k + 1] << 16), v[4 * k + 2] | (v[4 * k + 3] << 16));
         } else {
 #pragma unroll
-            for (int i = 0; i < 12; i++)
-                if (i < 3 * (p.w - dx0)) o[i] = (uint16_t)v[i];
+            for (int i = 0; i < 4 * C; i++)
+                if (i < C * (p.w - dx0)) o[i] = (uint16_t)v[i];
         }
     }
 }
 
+template <int C>
 __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int f = blockIdx.y;                    // s*T + t
@@ -70,7 +73,7 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
     const size_t obase = p.oidx ? (size_t)s * p.ostride + (size_t)oi * p.h * (size_t)(3 * p.w) : (size_t)f * p.h * (size_t)(3 * p.w);
     const uint8_t *src = p.frames + (size_t)s * p.sstride + (size_t)t * p.fstride;
     const size_t rowbytes = p.pitch;
-    const int pitch = (3 * p.w + 3) & ~3;        // u16 per staged row (rows 8-byte aligned)
+    const int pitch = (C * p.w + 3) & ~3;        // u16 per staged row (rows 8-byte aligned)
     uint16_t *rows = reinterpret_cast<uint16_t *>(smem);    // [2][pitch]: source row y lives in slot y & 1
     const int dy0 = blockIdx.x * p.band, dy1 = min(dy0 + p.band, p.h);
     const int nq = (p.w + 3) >> 2;
@@ -83,8 +86,8 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
         const bool need1 = sy1 != sy0 && ((sy1 & 1) ? held1 : held0) != sy1;
         if (need0 || need1) {
             __syncthreads();                     // readers of the slot about to be replaced are done
-            if (need0) up_hrow(p, src + (size_t)sy0 * rowbytes, rows + (sy0 & 1) * pitch);
-            if (need1) up_hrow(p, src + (size_t)sy1 * rowbytes, rows + (sy1 & 1) * pitch);
+            if (need0) up_hrow<C>(p, src + (size_t)sy0 * rowbytes, rows + (sy0 & 1) * pitch);
+            if (need1) up_hrow<C>(p, src + (size_t)sy1 * rowbytes, rows + (sy1 & 1) * pitch);
             if (need0) { if (sy0 & 1) held1 = sy0; else held0 = sy0; }
             if (need1) { if (sy1 & 1) held1 = sy1; else held0 = sy1; }
             __syncthreads();
@@ -93,26 +96,29 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
         const uint32_t b0 = (uint32_t)yv.y & 0xffffu, b1 = (uint32_t)yv.y >> 16;
         for (int q = threadIdx.x; q < nq; q += UP_THREADS) {
             const int dx0 = q * 4, n = min(4, p.w - dx0);
-            uint32_t h0[12], h1[12];
+            uint32_t h0[4 * C], h1[4 * C];
             if (n == 4) {
 #pragma unroll
-                for (int k = 0; k < 3; k++) {
-                    const uint2 u = reinterpret_cast<const uint2 *>(r0 + 12 * q)[k];
-                    const uint2 l = reinterpret_cast<const uint2 *>(r1 + 12 * q)[k];
+                for (int k = 0; k < C; k++) {
+                    const uint2 u = reinterpret_cast<const uint2 *>(r0 + 4 * C * q)[k];
+                    const uint2 l = reinterpret_cast<const uint2 *>(r1 + 4 * C * q)[k];
                     h0[4 * k] = u.x & 0xffffu; h0[4 * k + 1] = u.x >> 16; h0[4 * k + 2] = u.y & 0xffffu; h0[4 * k + 3] = u.y >> 16;
                     h1[4 * k] = l.x & 0xffffu; h1[4 * k + 1] = l.x >> 16; h1[4 * k + 2] = l.y & 0xffffu; h1[4 * k + 3] = l.y >> 16;
                 }
             } else {
 #pragma unroll
-                for (int i = 0; i < 12; i++) {
-                    const int ii = min(i, 3 * n - 1);
-                    h0[i] = r0[12 * q + ii];
-                    h1[i] = r1[12 * q + ii];
+                for (int i = 0; i < 4 * C; i++) {
+                    const int ii = min(i, C * n - 1);
+                    h0[i] = r0[4 * C * q + ii];
+                    h1[i] = r1[4 * C * q + ii];
                 }
             }
-            uint32_t v[12];
+            uint32_t v[12];                              // 4 pixels x 3 channels (a gray source: its byte in all three)
 #pragma unroll
-            for (int i = 0; i < 12; i++) v[i] = min((((b0 * h0[i]) >> 16) + ((b1 * h1[i]) >> 16) + 2u) >> 2, 255u);
+            for (int i = 0; i < 12; i++) {
+                const int k = C == 1 ? i / 3 : i;
+                v[i] = min((((b0 * h0[k]) >> 16) + ((b1 * h1[k]) >> 16) + 2u) >> 2, 255u);
+            }
             if (p.bgr_out) {
                 uint8_t *o = p.bgr_out + obase + (size_t)dy * (size_t)(3 * p.w) + 12 * q;
                 if (n == 4 && (((uintptr_t)o) & 3) == 0) {
@@ -127,7 +133,7 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
             } else {
                 uint32_t g[4];
 #pragma unroll
-                for (int j = 0; j < 4; j++) g[j] = fm_gray(v[3 * j], v[3 * j + 1], v[3 * j + 2]);
+                for (int j = 0; j < 4; j++) g[j] = C == 1 ? v[3 * j] : fm_gray(v[3 * j], v[3 * j + 1], v[3 * j + 2]);
                 uint8_t *o = p.gray + ((size_t)f * p.h + dy) * (size_t)p.w + dx0;
                 if (n == 4 && (((uintptr_t)o) & 3) == 0) {
                     *reinterpret_cast<uint32_t *>(o) = g[0] | (g[1] << 8) | (g[2] << 16) | (g[3] << 24);
@@ -145,7 +151,7 @@ size_t fm_upscale_smem(int w) { return (size_t)2 * ((3 * (size_t)w + 3) & ~(size
 
 int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int F, int W, int H,
                       int w, int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
-                      const int *oidx, size_t ostride, cudaStream_t st) {
+                      const int *oidx, size_t ostride, cudaStream_t st, int channels) {
     UpParams p;
     p.frames = frames; p.sstride = sstride; p.fstride = fstride; p.pitch = pitch;
     p.T = T; p.W = W; p.H = H; p.w = w; p.h = h;
@@ -161,9 +167,11 @@ int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t 
         return FM_ERANGE;
     }
     int rc;
-    if ((rc = fm_ensure_smem((const void *)k_upscale_gray, smem, device))) return rc;
+    if ((rc = fm_ensure_smem(channels == 1 ? (const void *)k_upscale_gray<1> : (const void *)k_upscale_gray<3>, smem, device)))
+        return rc;
     dim3 grid((h + band - 1) / band, F);
-    k_upscale_gray<<<grid, UP_THREADS, smem, st>>>(p);
+    if (channels == 1) k_upscale_gray<1><<<grid, UP_THREADS, smem, st>>>(p);
+    else k_upscale_gray<3><<<grid, UP_THREADS, smem, st>>>(p);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }

@@ -187,10 +187,10 @@ __device__ __forceinline__ void wide_h_stage(unsigned char *tile, const uint8_t 
         }
     } else {
         const int words = pitch >> 2;
-        const uint8_t *fr = src + (size_t)f * h * w;
+        const uint8_t *fr = src + (size_t)(f / T) * sstride + (size_t)(f % T) * fstride;
 #pragma unroll 1
         for (int rr = wq; rr < 32; rr += WH_THREADS / 32) {
-            const uint8_t *row = fr + (size_t)wrow(32 * G + rr - r, h) * w;
+            const uint8_t *row = fr + (size_t)wrow(32 * G + rr - r, h) * rpitch;
             uint32_t *trow = reinterpret_cast<uint32_t *>(tile + rr * pitch);
             for (int cw = lane; cw < words; cw += 32) {
                 const int x = X0 - R16 + 4 * cw;
@@ -253,8 +253,8 @@ __device__ __forceinline__ void wide_h_products(const unsigned char *tile, const
 }
 
 // grid: (ceil(w / 256), NGa, F), 256 threads.  dynamic smem: 32 * pitch + (4 Sh + 3) * 256
-// BGR: src = the caller's frames (identity resize, 16-byte aligned rows rpitch bytes apart); otherwise src = the gray plane
-// [F][h][w].
+// BGR: src = the caller's frames (identity resize, 16-byte aligned rows rpitch bytes apart); otherwise src = a gray plane, rows
+// rpitch bytes apart (the context's [F][h][w], or the caller's gray frames with FM_FLAG_GRAY).
 template <bool BGR>
 __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h(const uint8_t *__restrict__ src, size_t sstride, size_t fstride,
                                                        size_t rpitch, int T,
@@ -679,26 +679,40 @@ int fm_launch_bg_export_wide(fm_ctx *c, int stream, double *dst_dev, cudaStream_
     return FM_OK;
 }
 
-// k = 1: GaussianBlur is the identity, only the polygon masks are painted (find_motion.py:494, 619-635)
-__global__ void __launch_bounds__(256) k_blur_identity(const uint8_t *__restrict__ gray, uint8_t *__restrict__ blur,
+// k = 1: GaussianBlur is the identity, only the polygon masks are painted (find_motion.py:494, 619-635).  The gray plane
+// of frame (s, t) starts at gray + s * sstride + t * fstride, its rows rpitch bytes apart
+__global__ void __launch_bounds__(256) k_blur_identity(const uint8_t *__restrict__ gray, size_t sstride, size_t fstride,
+                                                       size_t rpitch, uint8_t *__restrict__ blur,
                                                        const uint32_t *__restrict__ maskbits, int w, int h, int wpr, int T,
                                                        const int *__restrict__ nvalid) {
     const int f = blockIdx.z, y = blockIdx.y, x = blockIdx.x * blockDim.x + threadIdx.x;
     if (x >= w || f % T >= __ldg(nvalid + f / T)) return;
     const uint32_t m = __ldg(maskbits + ((size_t)(f / T) * h + y) * wpr + (x >> 5));
-    const size_t i = ((size_t)f * h + y) * w + x;
-    blur[i] = ((m >> (x & 31)) & 1u) ? (uint8_t)0 : gray[i];
+    const uint8_t v = gray[(size_t)(f / T) * sstride + (size_t)(f % T) * fstride + (size_t)y * rpitch + x];
+    blur[((size_t)f * h + y) * w + x] = ((m >> (x & 31)) & 1u) ? (uint8_t)0 : v;
 }
 
-// frames != nullptr: full-resolution mode, convert BGR -> gray while staging (no gray plane); else read c->gray
+// frames != nullptr: full-resolution mode, convert BGR -> gray while staging (no gray plane); else read c->gray.  Gray
+// frames (FM_FLAG_GRAY) are the gray plane: read in place, copied to c->gray only as the FM_FLAG_KEEP_PLANES tap
 int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
+    const uint8_t *gsrc = c->gray;                                   // the gray plane the passes read, and its layout
+    size_t gsstride = (size_t)T * c->N, gfstride = c->N, gpitch = c->w;
+    if (frames && (c->cfg.flags & FM_FLAG_GRAY)) {
+        if (c->cfg.flags & FM_FLAG_KEEP_PLANES) {
+            int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
+            if (rc) return rc;
+        }
+        gsrc = frames; gsstride = sstride; gfstride = fstride; gpitch = pitch;
+        frames = nullptr;
+    }
     if (c->k == 1) {
         if (frames) {
             int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
             if (rc) return rc;
         }
         dim3 grid((c->w + 255) / 256, c->h, c->S * T);
-        k_blur_identity<<<grid, 256, 0, st>>>(c->gray, c->blur, c->maskbits, c->w, c->h, c->wpr, T, c->nvalid);
+        k_blur_identity<<<grid, 256, 0, st>>>(gsrc, gsstride, gfstride, gpitch, c->blur, c->maskbits, c->w, c->h, c->wpr, T,
+                                              c->nvalid);
         FM_LAUNCH_CHECK();
         return FM_OK;
     }
@@ -745,8 +759,8 @@ int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t
             int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
             if (rc) return rc;
         }
-        k_wide_h<false><<<hgrid, WH_THREADS, smh, st>>>(c->gray, 0, 0, 0, T, plo, phi, tabh, c->w, c->h, g.r, g.R16, g.Sh,
-                                                        g.pitch, g.NGa, c->nvalid);
+        k_wide_h<false><<<hgrid, WH_THREADS, smh, st>>>(gsrc, gsstride, gfstride, gpitch, T, plo, phi, tabh, c->w, c->h, g.r,
+                                                        g.R16, g.Sh, g.pitch, g.NGa, c->nvalid);
     }
     FM_LAUNCH_CHECK();
     if (c->wide_fused) {

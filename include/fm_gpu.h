@@ -38,7 +38,7 @@ typedef struct fm_ctx fm_ctx;
 typedef struct fm_config {
     int32_t device;          /* CUDA device ordinal */
     int32_t n_streams;       /* streams batched in this context */
-    int32_t frame_width;     /* W of the raw BGR (or, with FM_FLAG_NV12, NV12) frames (CAP_PROP_FRAME_WIDTH) */
+    int32_t frame_width;     /* W of the raw BGR (or, with FM_FLAG_NV12, NV12; with FM_FLAG_GRAY, gray) frames (CAP_PROP_FRAME_WIDTH) */
     int32_t frame_height;    /* H */
     int32_t max_frames;      /* most frames per stream a single fm_process call will carry (T_max) */
     int32_t fps;             /* --fps, default 30 (find_motion.py:1463) */
@@ -87,6 +87,14 @@ typedef struct fm_config {
                                    indices, and with FM_FLAG_NV12 on the fused front end (fm_info.front_end == 0) a BGR slot
                                    of n_streams * max_frames * H * W * 3 bytes like the staged one.  The hot-path entry
                                    points launch nothing more and return the same results with the flag */
+#define FM_FLAG_GRAY        2048 /* the frames are single-channel gray, as thermal, IR and monochrome cameras deliver them: H
+                                   rows of W bytes.  Every entry point that takes frames reads W*H bytes per frame; strides keep
+                                   their meaning in bytes.  Results are those of a BGR context on cv2.cvtColor(frame,
+                                   COLOR_GRAY2BGR): every stats field, component, tap and the background.  Every front end
+                                   reads the one-byte pixels in place (no BGR slot).  With FM_FLAG_DEVICE_CLIPS the ring and
+                                   the clips hold gray frames of W*H bytes; fm_object_planes keeps its oh x 300 x 3 planes
+                                   (the one-channel resize stored in B, G and R).  FM_FLAG_GRAY | FM_FLAG_NV12 is refused with
+                                   FM_EINVAL before any device query */
 #define FM_OBJECT_WIDTH 300     /* width of the detector input plane (find_motion.py:703-706 hard-codes it) */
 
 /* Derived parameters, exactly as the reference computes them (SURVEY.md A.0). */
@@ -142,8 +150,8 @@ int fm_version(void);
 /* Replaces VideoMotion.__init__ + _calc_min_area + _make_gaussian + _load_video
  * (find_motion.py:299-380, 402-424, 478-484) for n_streams streams.  box_size > frame_width (a processing plane larger
  * than the frame, which imutils.resize produces with cv2's INTER_AREA upscale) needs FM_FLAG_UPSCALE; without it
- * fm_ctx_create returns FM_ERANGE.  So does an odd frame width or height with FM_FLAG_NV12.  Both checks come before
- * any device query. */
+ * fm_ctx_create returns FM_ERANGE.  So does an odd frame width or height with FM_FLAG_NV12.  FM_FLAG_GRAY together with
+ * FM_FLAG_NV12 returns FM_EINVAL.  These checks come before any device query. */
 int fm_ctx_create(const fm_config *cfg, fm_ctx **out);
 int fm_ctx_destroy(fm_ctx *ctx);
 int fm_ctx_info(const fm_ctx *ctx, fm_info *info);
@@ -160,7 +168,8 @@ int fm_ctx_reset(fm_ctx *ctx, int stream);
 
 /* The hot path: for every stream s < n_streams and t < n_frames (in order), run
  * blur_frame -> mask_off_areas -> find_diff -> find_movement -> decide_output on the BGR frame
- *   frames + s * stream_stride + t * frame_stride          (H*W*3 bytes, HWC, uint8; FM_FLAG_NV12: H*W*3/2 bytes NV12)
+ *   frames + s * stream_stride + t * frame_stride          (H*W*3 bytes, HWC, uint8; FM_FLAG_NV12: H*W*3/2 bytes NV12;
+ *                                                           FM_FLAG_GRAY: H*W bytes gray)
  * `frames` is a DEVICE pointer; work is enqueued on `cuda_stream` (a cudaStream_t, 0 = default)
  * and the call returns without synchronising.  stats_dev, if not NULL, is a device buffer of
  * n_streams * n_frames fm_frame_stats ([stream][frame]) filled by the call. */
@@ -177,7 +186,8 @@ int fm_process_ragged(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, 
 /* fm_process_ragged that also hands out the frames the reference writes to its *_motion.avi in this call (needs
  * FM_FLAG_DEVICE_CLIPS).  For stream s, with n_out[s] = sum of wrote + n_flush over its valid frames, it writes
  * n_out[s] raw BGR frames densely to the DEVICE buffer
- *   out_dev + s * out_stream_stride + i * H*W*3          (i < n_out[s]; FM_FLAG_NV12: NV12 frames, i * H*W*3/2)
+ *   out_dev + s * out_stream_stride + i * H*W*3          (i < n_out[s]; FM_FLAG_NV12: NV12 frames, i * H*W*3/2;
+ *                                                         FM_FLAG_GRAY: gray frames, i * H*W)
  * in the reference's order: for each frame in order, the n_flush cached frames it flushes (oldest first, taken from the
  * device ring or from this call's input), then the frame itself if `wrote` (find_motion.py:561-570, 583).  n_out
  * follows from the stats.  out_capacity is the room per stream in frames and must be at least cache_frames + n_frames,
@@ -193,14 +203,16 @@ typedef struct fm_frames {
     const uint8_t *data;        /* DEVICE pointer: frame (s, t) starts at data + s * stream_stride + t * frame_stride */
     size_t stream_stride;
     size_t frame_stride;
-    size_t row_pitch;           /* bytes from one row to the next, in both NV12 planes; 0 = packed (W*3, or W for NV12) */
+    size_t row_pitch;           /* bytes from one row to the next, in both NV12 planes; 0 = packed (W*3, or W for NV12
+                                   and gray) */
     int64_t uv_offset;          /* FM_FLAG_NV12: start of the chroma plane relative to the frame start (may be negative);
-                                   0 = row_pitch * H (chroma right after the luma rows) */
+                                   0 = row_pitch * H (chroma right after the luma rows).  Must be 0 otherwise with
+                                   FM_FLAG_GRAY (FM_EINVAL) */
 } fm_frames;
 
 /* fm_process_ragged (clip_out == NULL) or fm_process_clip (clip_out != NULL, same flag and capacity rules) on frames laid
  * out as `frames` describes.  Results, clip frames and detector input planes are those of the same frames packed; the
- * outputs stay packed (clip frames of H*W*3 or H*W*3/2 bytes).  row_pitch must be at least the row bytes, and the two
+ * outputs stay packed (clip frames of H*W*3, H*W*3/2 or, gray, H*W bytes).  row_pitch must be at least the row bytes, and the two
  * NV12 planes of a frame must not overlap.  Fused contexts (fm_info.front_end == 0) read the frames by TMA only and need
  * data, the strides, row_pitch and data + uv_offset 16-byte aligned; every other front end takes any layout.  A refused
  * call (FM_EINVAL) enqueues nothing and changes no state.  fm_process, fm_process_ragged and fm_process_clip are this
@@ -215,7 +227,8 @@ int fm_process_frames(fm_ctx *ctx, const fm_frames *frames, int n_frames, const 
  *   out_dev + s * out_stream_stride + i * oh*300*3          (i < n_obj[s])
  * each byte-identical to cv2.resize(raw, (300, oh), interpolation=cv2.INTER_AREA) of the written frame (the upscale for
  * W < 300, a copy for W == 300).  The masks do not apply (find_objects reads frame.raw).  NV12 contexts resize
- * cv2.cvtColor(frame, COLOR_YUV2BGR_NV12).  out_capacity is the room per stream in planes and must be at least the last
+ * cv2.cvtColor(frame, COLOR_YUV2BGR_NV12), gray contexts cv2.cvtColor(frame, COLOR_GRAY2BGR) (the one-channel resize
+ * in all three channels).  out_capacity is the room per stream in planes and must be at least the last
  * call's n_frames.  Asynchronous on `cuda_stream`: the last call's frames must stay untouched until the planes are
  * written, as for the call itself.  FM_EINVAL without the flag, for a short out_capacity, before the first device-entry
  * call, and after fm_process_host / fm_submit_host (their frames live in the context's staging buffers). */
@@ -223,7 +236,7 @@ int fm_object_planes(fm_ctx *ctx, void *cuda_stream, uint8_t *out_dev, size_t ou
 
 /* Same with HOST buffers: copies the frames host->device (pinned memory recommended), runs the
  * path, copies the stats back and synchronises.  This is the call a drop-in adapter makes.  With FM_FLAG_NV12 a frame
- * is H*W*3/2 bytes, half the host->device traffic of BGR. */
+ * is H*W*3/2 bytes, half the host->device traffic of BGR; with FM_FLAG_GRAY it is H*W bytes, a third. */
 int fm_process_host(fm_ctx *ctx, const uint8_t *frames_host, size_t stream_stride,
                     size_t frame_stride, int n_frames, fm_frame_stats *stats_host);
 
@@ -282,6 +295,10 @@ int fm_resize_area(int device, const uint8_t *bgr_host, int frame_width, int fra
  * re-checks, tap by tap, that every read of every column stays inside its TMA box and meets the weight cv2's table gives
  * it.  FM_OK with info->usable = 0 when the geometry is left to the warp-per-row kernels; FM_ERANGE if a check fails. */
 int fm_debug_rows_plan(int frame_width, int frame_height, int box_size, fm_rows_plan_info *info);
+
+/* fm_debug_rows_plan for frames of `channels` bytes per pixel: 3 (BGR, what fm_debug_rows_plan checks) or 1 (FM_FLAG_GRAY,
+ * whose plan reads W-byte rows and 4-byte tap groups).  FM_EINVAL for any other count. */
+int fm_debug_rows_plan_channels(int frame_width, int frame_height, int box_size, int channels, fm_rows_plan_info *info);
 
 /* Number of kernels this library has launched since load (bench.py's gpu_launches). */
 uint64_t fm_launch_count(void);

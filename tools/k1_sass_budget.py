@@ -1,7 +1,7 @@
 """Static instruction budget of K1 (k_fused), per phase, from the sm_100a SASS.  Needs nvcc, no GPU.
 
 Compiles csrc/k_fused.cu with build.py's flags plus `-Xptxas -v` into a cubin, disassembles the benchmarked
-instantiation (KEEP off, SAFE on: `k_fused<false, true>`) with nvdisasm's inline line information, and attributes each
+instantiation (KEEP off, SAFE on, BGR source: `k_fused<false, true, FUSED_BGR>`) with nvdisasm's inline line information, and attributes each
 instruction to the line of the kernel body it comes from (for inlined code: the outermost call site).  The phases are
 the marked sections of the frame loop in the source, so the table follows the code when lines move:
 
@@ -31,10 +31,10 @@ sys.path.insert(0, ROOT)
 from find_motion_b200 import build as B  # noqa: E402
 
 SRC = os.path.join(B.CSRC, "k_fused.cu")
-KERNEL = "_Z7k_fusedILb0ELb1EEv14CUtensorMap_st11FusedParams"
+KERNEL = "_Z7k_fusedILb0ELb1ELi0EEv14CUtensorMap_st11FusedParamsS0_"
 MARKERS = [  # (phase that starts at the first line containing the text, text)
     ("loop top", "for (int t = 0; t < Ts; t++)"),
-    ("gray", "// ---- staged BGR -> gray"),
+    ("gray", "// ---- staged BGR"),
     ("border", "if (border)"),
     ("horizontal", "// ---- horizontal pass"),
     ("vertical", "// ---- vertical pass"),
@@ -114,7 +114,7 @@ def main():
         if ph in ("vertical", "tail"):
             sites[loc] = sites.get(loc, 0) + 1
 
-    print("k_fused<false, true> (KEEP off, SAFE on): %s; %s" % (regs, spill))
+    print("k_fused<false, true, FUSED_BGR> (KEEP off, SAFE on): %s; %s" % (regs, spill))
     order = ["before the loop"] + [n for n, _ in MARKERS] + ["after the loop"]
     print("%-16s %6s" % ("phase", "SASS"))
     for n in order:
