@@ -64,6 +64,8 @@ FLAG_DEVICE_CLIPS = 256
 FLAG_NV12 = 512
 FLAG_OBJECT_PLANES = 1024
 FLAG_GRAY = 2048
+FLAG_RGB = 4096
+FLAG_ALPHA = 8192
 OBJECT_WIDTH = 300
 
 # every symbol include/fm_gpu.h declares: name -> (restype, argtypes)
@@ -95,6 +97,7 @@ SYMBOLS = {
     "fm_resize_area": (C.c_int, [C.c_int, _P, C.c_int, C.c_int, C.c_int, _P, C.POINTER(C.c_int)]),
     "fm_debug_rows_plan": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(fm_rows_plan_info)]),
     "fm_debug_rows_plan_channels": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(fm_rows_plan_info)]),
+    "fm_debug_rows_plan_format": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int32, C.POINTER(fm_rows_plan_info)]),
     "fm_launch_count": (C.c_uint64, []),
     "fm_timing_enable": (C.c_int, [_P, C.c_int]),
     "fm_timing_reset": (C.c_int, [_P]),

@@ -8,6 +8,7 @@
 #include <stdint.h>
 
 #include <atomic>
+#include <type_traits>
 #include <utility>
 
 #include "../../include/fm_gpu.h"
@@ -49,6 +50,18 @@ struct CclScratch {            // run-based labelling scratch for `frames` frame
     int *bbox;                 // [frames][slots][4]  xmin, ymin, xmax, ymax
 };
 
+// f(std::integral_constant<int, C>, std::integral_constant<bool, RGB>) for the pixel format (C bytes a pixel: 1 gray, 3
+// BGR / RGB, 4 BGRA / RGBA; RGB: R first): one call per kernel family picks its instantiation
+template <typename F>
+void fm_px_dispatch(int px_bytes, bool rgb, F &&f) {
+    using I1 = std::integral_constant<int, 1>; using I3 = std::integral_constant<int, 3>; using I4 = std::integral_constant<int, 4>;
+    using B0 = std::integral_constant<bool, false>; using B1 = std::integral_constant<bool, true>;
+    if (px_bytes == 1) f(I1{}, B0{});
+    else if (px_bytes == 4) { if (rgb) f(I4{}, B1{}); else f(I4{}, B0{}); }
+    else if (rgb) f(I3{}, B1{});
+    else f(I3{}, B0{});
+}
+
 struct fm_ctx {
     fm_config cfg;
     fm_info info;
@@ -56,7 +69,14 @@ struct fm_ctx {
     int N;                     // w*h
     int ntiles;                // ceil(N / FM_TILE_PX)
     int resize_mode;           // 0 identity, 1 general tables, 2 integer ratio, 3 upscale (FM_FLAG_UPSCALE, k_upscale.cu)
-    size_t frame_bytes;        // bytes of one input frame: H * W * 3 (BGR), H * W * 3 / 2 (FM_FLAG_NV12) or H * W (FM_FLAG_GRAY)
+    size_t frame_bytes;        // bytes of one input frame: H * W * 3 (BGR, FM_FLAG_RGB), H * W * 3 / 2 (FM_FLAG_NV12) or H * W
+                               // (FM_FLAG_GRAY)
+    // the pixel format, resolved once from the flags by fm_ctx_create (fm_pixel_format); every launcher reads these
+    int px_bytes;              // bytes per pixel of the frames the BGR / gray front ends read: 3 (BGR, RGB, and NV12's BGR
+                               // slot), 4 (FM_FLAG_ALPHA: BGRA, RGBA) or 1 (FM_FLAG_GRAY)
+    bool rgb;                  // FM_FLAG_RGB: pixels are R, G, B in memory; only the gray weights and the byte order of the
+                               // detector input planes depend on it
+    size_t row_bytes;          // bytes of one packed row of the caller's frames: W * px_bytes, or W (NV12 luma)
     uint8_t *nv12_bgr;         // FM_FLAG_NV12 on the staged path: [S][Tmax][H][W][3] the call's frames converted to BGR
                                // (k_nv12.cu), read by the BGR front end; null when none is needed
     bool fused;                // K1 fused stencil+background kernel drives the front end
@@ -249,11 +269,11 @@ size_t fm_fused_bg_doubles(const fm_ctx *c);
 int fm_launch_bg_export_fused(fm_ctx *c, int stream, double *dst_dev, cudaStream_t st);
 int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, size_t pitch, int S, int T, int W, int H,
                          int w, int h, int mode, int fx, int fy, const ResizeTab &xt, const ResizeTab &yt, const int *oidx,
-                         uint8_t *dst_dev, size_t ostride, cudaStream_t st, int channels);
-size_t fm_upscale_smem(int w);
+                         uint8_t *dst_dev, size_t ostride, cudaStream_t st, int channels, bool rgb = false);
+size_t fm_upscale_smem(int w, int channels);
 int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int F, int W, int H, int w,
                       int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
-                      const int *oidx, size_t ostride, cudaStream_t st, int channels);
+                      const int *oidx, size_t ostride, cudaStream_t st, int channels, bool rgb = false);
 int fm_rows_plan(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx);
 void fm_rows_free(fm_ctx *c);
 int fm_rows_plan_describe(int W, int w, int h, int channels, const int *xstart, const int *xidx, const float *xwt, const int *ystart,

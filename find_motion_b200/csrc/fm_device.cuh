@@ -62,19 +62,34 @@ __device__ __forceinline__ void fm_imma0(int (&d)[4], uint32_t a0, uint32_t a1, 
 }
 
 // ---- gray (SURVEY.md A.2): Y = (3735 B + 19235 G + 9798 R + 16384) >> 15 ----
-__device__ __forceinline__ uint32_t fm_gray(uint32_t b, uint32_t g, uint32_t r) {
-    return (3735u * b + 19235u * g + 9798u * r + 16384u) >> 15;
+// RGB: the caller's pixels are R first (FM_FLAG_RGB), so the B and R weights trade places; p0, p1, p2 are the pixel's bytes
+// in memory order
+template <bool RGB = false>
+__device__ __forceinline__ uint32_t fm_gray(uint32_t p0, uint32_t g, uint32_t p2) {
+    return RGB ? (3735u * p2 + 19235u * g + 9798u * p0 + 16384u) >> 15 : (3735u * p0 + 19235u * g + 9798u * p2 + 16384u) >> 15;
 }
 // 4 BGR pixels in 3 words -> 4 gray bytes.  The same Y computed as (7470 B + 38470 G + 19596 R + 32768) >> 16 with two
 // 16-bit x 8-bit dot products per pixel (IDP.2A); the lo/hi byte-pair selection of IDP.2A picks each pixel's bytes straight
-// out of the three words.  The result is byte 2 of the accumulator.
+// out of the three words.  The result is byte 2 of the accumulator.  RGB: 4 RGB pixels, the B and R constants swapped.
+template <bool RGB = false>
 __device__ __forceinline__ uint32_t fm_gray4(uint32_t w0, uint32_t w1, uint32_t w2) {
-    const uint32_t C_BG = 7470u | (38470u << 16), C_R = 19596u;              // byte pairs [B,G], [R,x]
-    const uint32_t C_xB = 7470u << 16, C_GR = 38470u | (19596u << 16);       // byte pairs [x,B], [G,R]
+    constexpr uint32_t WB = RGB ? 19596u : 7470u, WR = RGB ? 7470u : 19596u;   // weights of bytes 0 and 2 of a pixel
+    const uint32_t C_BG = WB | (38470u << 16), C_R = WR;                     // byte pairs [B,G], [R,x]
+    const uint32_t C_xB = WB << 16, C_GR = 38470u | (WR << 16);              // byte pairs [x,B], [G,R]
     uint32_t t0 = __dp2a_hi(C_R, w0, __dp2a_lo(C_BG, w0, 32768u));           // w0 = [B0,G0,R0,B1]
     uint32_t t1 = __dp2a_hi(C_xB, w0, __dp2a_lo(C_GR, w1, 32768u));          // w1 = [G1,R1,B2,G2]
     uint32_t t2 = __dp2a_hi(C_BG, w1, __dp2a_lo(C_R, w2, 32768u));           // w2 = [R2,B3,G3,R3]
     uint32_t t3 = __dp2a_hi(C_GR, w2, __dp2a_lo(C_xB, w2, 32768u));
+    return __byte_perm(__byte_perm(t0, t1, 0x0062), __byte_perm(t2, t3, 0x0062), 0x5410);
+}
+// 4 four-byte pixels (BGRA, or RGBA with RGB), one word each -> 4 gray bytes: the same two IDP.2A per pixel, the fourth byte
+// weighted 0
+template <bool RGB = false>
+__device__ __forceinline__ uint32_t fm_gray4a(uint4 q) {
+    constexpr uint32_t WB = RGB ? 19596u : 7470u, WR = RGB ? 7470u : 19596u;
+    const uint32_t C_BG = WB | (38470u << 16), C_R = WR;                     // byte pairs [B,G], [R,A]
+    const uint32_t t0 = __dp2a_hi(C_R, q.x, __dp2a_lo(C_BG, q.x, 32768u)), t1 = __dp2a_hi(C_R, q.y, __dp2a_lo(C_BG, q.y, 32768u));
+    const uint32_t t2 = __dp2a_hi(C_R, q.z, __dp2a_lo(C_BG, q.z, 32768u)), t3 = __dp2a_hi(C_R, q.w, __dp2a_lo(C_BG, q.w, 32768u));
     return __byte_perm(__byte_perm(t0, t1, 0x0062), __byte_perm(t2, t3, 0x0062), 0x5410);
 }
 

@@ -55,7 +55,7 @@ PFN_encodeTiled fm_tma_encoder() {
 
 int fm_frames_tmap(const fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int box_words,
                    int box_rows, CUtensorMap *out) {
-    const size_t row = (size_t)c->W * ((c->cfg.flags & FM_FLAG_GRAY) ? 1 : 3), dense = pitch * c->H;
+    const size_t row = (size_t)c->W * c->px_bytes, dense = pitch * c->H;
     if ((((uintptr_t)frames) | sstride | fstride | pitch | row) & 15) {
         fm_set_error("the TMA front ends need 16-byte aligned frames, strides and rows (row pitch %zu)", pitch);
         return FM_EINVAL;
@@ -231,6 +231,26 @@ extern "C" int fm_ctx_destroy(fm_ctx *c) {
     return FM_OK;
 }
 
+// The pixel format the flags select, decided here once for fm_ctx_create and fm_debug_rows_plan_format: bytes per pixel
+// of the frames the BGR / gray front ends read (NV12's staged slot is BGR) and whether R comes first.  false (with the
+// error set) for two formats at once.
+static bool fm_pixel_format(int32_t flags, int *px_bytes, bool *rgb) {
+    if ((flags & FM_FLAG_GRAY) && (flags & FM_FLAG_NV12)) {
+        fm_set_error("FM_FLAG_GRAY and FM_FLAG_NV12 are two frame formats: set one of them");
+        return false;
+    }
+    for (int32_t f : {FM_FLAG_RGB, FM_FLAG_ALPHA}) {
+        if ((flags & f) && (flags & (FM_FLAG_NV12 | FM_FLAG_GRAY))) {
+            fm_set_error("%s and %s are two frame formats: set one of them", f == FM_FLAG_RGB ? "FM_FLAG_RGB" : "FM_FLAG_ALPHA",
+                         (flags & FM_FLAG_NV12) ? "FM_FLAG_NV12" : "FM_FLAG_GRAY");
+            return false;
+        }
+    }
+    *px_bytes = (flags & FM_FLAG_GRAY) ? 1 : (flags & FM_FLAG_ALPHA) ? 4 : 3;
+    *rgb = (flags & FM_FLAG_RGB) != 0;
+    return true;
+}
+
 extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     if (!cfg || !out) { fm_set_error("null argument"); return FM_EINVAL; }
     *out = nullptr;
@@ -239,10 +259,9 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
         fm_set_error("invalid configuration (streams/geometry/max_frames/box_size/blur_scale/min_box_scale)");
         return FM_EINVAL;
     }
-    if ((cfg->flags & FM_FLAG_GRAY) && (cfg->flags & FM_FLAG_NV12)) {
-        fm_set_error("FM_FLAG_GRAY and FM_FLAG_NV12 are two frame formats: set one of them");
-        return FM_EINVAL;
-    }
+    int px_bytes;
+    bool rgb;
+    if (!fm_pixel_format(cfg->flags, &px_bytes, &rgb)) return FM_EINVAL;
     if (cfg->box_size > cfg->frame_width && !(cfg->flags & FM_FLAG_UPSCALE)) {
         // INTER_AREA with a destination wider than the source is cv2's fixed-point linear upscale (SURVEY.md A.1):
         // opt-in with FM_FLAG_UPSCALE, so that binders of the earlier ABI keep their range check
@@ -279,9 +298,9 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     c->cfg = *cfg;
     c->S = cfg->n_streams; c->Tmax = cfg->max_frames;
     c->W = cfg->frame_width; c->H = cfg->frame_height;
-    c->frame_bytes = (cfg->flags & FM_FLAG_NV12)   ? (size_t)c->W * c->H * 3 / 2
-                     : (cfg->flags & FM_FLAG_GRAY) ? (size_t)c->W * c->H
-                                                   : (size_t)c->W * c->H * 3;
+    c->px_bytes = px_bytes; c->rgb = rgb;
+    c->row_bytes = (cfg->flags & FM_FLAG_NV12) ? (size_t)c->W : (size_t)c->W * px_bytes;
+    c->frame_bytes = (cfg->flags & FM_FLAG_NV12) ? (size_t)c->W * c->H * 3 / 2 : c->row_bytes * c->H;
     // derived parameters, mirroring the Python expressions (true division on floats, int() truncation)
     const double W = c->W, H = c->H, box = cfg->box_size;
     c->w = cfg->box_size;
@@ -326,7 +345,7 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
             return fail(FM_ERANGE);
         }
         c->resize_mode = 3;
-        if (fm_upscale_smem(c->w) > 200 * 1024) { fm_set_error("processing width %d too large to upscale", c->w); return fail(FM_ERANGE); }
+        if (fm_upscale_smem(c->w, c->px_bytes) > 200 * 1024) { fm_set_error("processing width %d too large to upscale", c->w); return fail(FM_ERANGE); }
         if ((rc = upload(&c->uxt, upscale_tab(c->W, c->w)))) return fail(rc);
         if ((rc = upload(&c->uyt, upscale_tab(c->H, c->h)))) return fail(rc);
     } else {
@@ -396,7 +415,7 @@ extern "C" int fm_ctx_create(const fm_config *cfg, fm_ctx **out) {
     // the fused front ends never materialise gray / blur planes (except as parity taps)
     const bool keep = (cfg->flags & FM_FLAG_KEEP_PLANES) != 0;
     // gray frames at full resolution are the gray plane themselves
-    const bool need_gray = keep || (!c->fused && !((cfg->flags & FM_FLAG_GRAY) && c->resize_mode == 0));
+    const bool need_gray = keep || (!c->fused && !(c->px_bytes == 1 && c->resize_mode == 0));
     const bool need_blur = keep || !c->fused;
     ALLOC(c->gray, need_gray ? F * c->N : 16);
     ALLOC(c->hor, (c->fused || c->umma) ? 16 : 2 * fm_wide_plane_bytes(c));
@@ -664,14 +683,15 @@ extern "C" int fm_process_frames(fm_ctx *c, const fm_frames *fr, int n_frames, c
                                  fm_frame_stats *stats_dev, uint8_t *clip_out, size_t clip_stream_stride, int clip_capacity) {
     if (!c || !fr || !fr->data) { fm_set_error("null argument"); return FM_EINVAL; }
     const bool nv12 = (c->cfg.flags & FM_FLAG_NV12) != 0;
-    const size_t row = (nv12 || (c->cfg.flags & FM_FLAG_GRAY)) ? (size_t)c->W : (size_t)c->W * 3;
+    const size_t row = c->row_bytes;
     const size_t pitch = fr->row_pitch ? fr->row_pitch : row;
     if (pitch < row) {
         fm_set_error("row_pitch %zu < %zu bytes of a row", pitch, row);
         return FM_EINVAL;
     }
-    if ((c->cfg.flags & FM_FLAG_GRAY) && fr->uv_offset) {
-        fm_set_error("uv_offset %lld: gray frames have no chroma plane", (long long)fr->uv_offset);
+    if ((c->px_bytes != 3 || c->rgb) && !nv12 && fr->uv_offset) {
+        fm_set_error("uv_offset %lld: %s frames have no chroma plane", (long long)fr->uv_offset,
+                     c->px_bytes == 1 ? "gray" : c->px_bytes == 4 ? (c->rgb ? "RGBA" : "BGRA") : "RGB");
         return FM_EINVAL;
     }
     const int64_t luma = (int64_t)(pitch * (c->H - 1) + row);           // bytes the luma rows of a frame span
@@ -999,9 +1019,9 @@ extern "C" int fm_debug_mask(fm_ctx *c, int stream, uint8_t *mask) {
 }
 
 // find_objects' input plane (find_motion.py:703-706): imutils.resize(frame.raw, width=300) = INTER_AREA, BGR out
-extern "C" int fm_debug_rows_plan_channels(int W, int H, int box_size, int channels, fm_rows_plan_info *info) {
+// the self-checked rows plan of a geometry for px_bytes-byte pixels (1, 3 or 4)
+static int rows_plan_px(int W, int H, int box_size, int channels, fm_rows_plan_info *info) {
     if (!info || W < 1 || H < 1 || box_size < 1 || box_size > W) { fm_set_error("bad geometry"); return FM_EINVAL; }
-    if (channels != 1 && channels != 3) { fm_set_error("channels %d: 3 (BGR) or 1 (gray)", channels); return FM_EINVAL; }
     const int w = box_size, h = (int)((double)H * ((double)box_size / (double)W));          // imutils.resize
     memset(info, 0, sizeof(*info));
     if (h < 1 || (w == W && h == H)) return FM_OK;
@@ -1012,8 +1032,24 @@ extern "C" int fm_debug_rows_plan_channels(int W, int H, int box_size, int chann
                                  info);
 }
 
+extern "C" int fm_debug_rows_plan_channels(int W, int H, int box_size, int channels, fm_rows_plan_info *info) {
+    if (channels != 1 && channels != 3) { fm_set_error("channels %d: 3 (BGR) or 1 (gray)", channels); return FM_EINVAL; }
+    return rows_plan_px(W, H, box_size, channels, info);
+}
+
 extern "C" int fm_debug_rows_plan(int W, int H, int box_size, fm_rows_plan_info *info) {
     return fm_debug_rows_plan_channels(W, H, box_size, 3, info);
+}
+
+extern "C" int fm_debug_rows_plan_format(int W, int H, int box_size, int32_t flags, fm_rows_plan_info *info) {
+    if (flags & ~(FM_FLAG_RGB | FM_FLAG_ALPHA | FM_FLAG_GRAY)) {
+        fm_set_error("flags %d: a combination of FM_FLAG_RGB and FM_FLAG_ALPHA, or FM_FLAG_GRAY", (int)flags);
+        return FM_EINVAL;
+    }
+    int px_bytes;
+    bool rgb;
+    if (!fm_pixel_format(flags, &px_bytes, &rgb)) return FM_EINVAL;
+    return rows_plan_px(W, H, box_size, px_bytes, info);
 }
 
 extern "C" int fm_resize_area(int device, const uint8_t *bgr_host, int W, int H, int width, uint8_t *out_host, int *out_height) {

@@ -257,7 +257,7 @@ int fm_launch_clips(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     FM_LAUNCH_CHECK();
     const bool nv12 = (c->cfg.flags & FM_FLAG_NV12) != 0;
     ClipRows g;
-    g.rowbytes = (nv12 || (c->cfg.flags & FM_FLAG_GRAY)) ? (size_t)c->W : (size_t)c->W * 3;
+    g.rowbytes = c->row_bytes;
     g.pitch = pitch; g.uv = uv;
     g.luma_rows = c->H; g.rows = nv12 ? c->H + c->H / 2 : c->H;
     g.rows_per_item = (int)std::max<size_t>(1, CLIP_CHUNK_BYTES / g.rowbytes);

@@ -5,8 +5,8 @@
 
 // identity-resize mode: one thread per 4 pixels of a frame (12 bytes in, 4 bytes out; C = 1, gray frames: a copy).  Pixel
 // i = y * w + x of a frame is at y * pitch + C x; packed rows (pitch == C w) are one flat run, so 4 pixels may then straddle
-// a row end
-template <int C>
+// a row end.  RGB: R-first pixels (FM_FLAG_RGB)
+template <int C, bool RGB = false>
 __global__ void __launch_bounds__(256) k_gray(const uint8_t *__restrict__ frames, size_t sstride,
                                               size_t fstride, size_t pitch, int T, int w, int N, uint8_t *__restrict__ gray,
                                               const int *__restrict__ nvalid) {
@@ -22,12 +22,14 @@ __global__ void __launch_bounds__(256) k_gray(const uint8_t *__restrict__ frames
     const uint8_t *q4 = flat ? src + (size_t)i4 * C : src + (size_t)y4 * pitch + (size_t)x4 * C;
     if (i4 + 4 <= N && (flat || x4 + 4 <= w) && ((((uintptr_t)q4) & 3) == 0) && ((((uintptr_t)dst) & 3) == 0)) {
         const uint32_t *p = reinterpret_cast<const uint32_t *>(q4);
-        *reinterpret_cast<uint32_t *>(dst + i4) = C == 1 ? __ldg(p) : fm_gray4(__ldg(p), __ldg(p + 1), __ldg(p + 2));
+        *reinterpret_cast<uint32_t *>(dst + i4) = C == 1   ? __ldg(p)
+            : C == 4 ? fm_gray4a<RGB>(make_uint4(__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3)))
+                     : fm_gray4<RGB>(__ldg(p), __ldg(p + 1), __ldg(p + 2));
     } else {
         for (int i = i4; i < min(i4 + 4, N); i++) {
             const int y = i / w;
             const uint8_t *p = src + (size_t)y * pitch + (size_t)(i - y * w) * C;
-            dst[i] = C == 1 ? p[0] : (uint8_t)fm_gray(p[0], p[1], p[2]);
+            dst[i] = C == 1 ? p[0] : (uint8_t)fm_gray<RGB>(p[0], p[1], p[2]);
         }
     }
 }
@@ -58,8 +60,9 @@ struct K0Params {
 
 // oidx (with bgr_out): null, or [F] plane index (-1: skip the frame); frame f's plane then goes to
 // bgr_out + s * ostride + oidx[f] * h*w*3 (fm_object_planes).  C: channels of the source (3 BGR, 1 gray); per channel the
-// chains are the same, and a gray source's resized byte is stored in all three channels of bgr_out
-template <int C>
+// chains are the same, and a gray source's resized byte is stored in all three channels of bgr_out.  RGB: R-first source
+// pixels, whose resized bytes go to bgr_out in BGR order
+template <int C, bool RGB = false>
 __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const int *__restrict__ oidx, size_t ostride) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int f = blockIdx.y;
@@ -73,7 +76,8 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const in
     const int rowpitch = (rowbytes + 16 + 15) & ~15;          // room for a misaligned start
     unsigned char *rowbuf = smem;                               // [K0_GROUPS][rowpitch]
     float *bufs = reinterpret_cast<float *>(smem + (size_t)K0_GROUPS * rowpitch);   // [ny][C w]
-    const int w3 = p.w * C;
+    constexpr int NC = C == 4 ? 3 : C;          // chains per column: the fourth byte of BGRA / RGBA is not resized
+    const int w3 = p.w * NC;
     const int tid = threadIdx.x;
     const int gsz = K0_THREADS / K0_GROUPS;
     const int grp = tid / gsz, gt = tid - grp * gsz;
@@ -118,31 +122,31 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const in
             if (p.mode == 1) {
                 for (int dx = gt; dx < p.w; dx += gsz) {
                     int a = p.xstart[dx], b = p.xstart[dx + 1];
-                    float bc[C];
+                    float bc[NC];
 #pragma unroll
-                    for (int ch = 0; ch < C; ch++) bc[ch] = 0.f;
+                    for (int ch = 0; ch < NC; ch++) bc[ch] = 0.f;
                     for (int q = a; q < b; q++) {
                         const unsigned char *px = rb + p.xidx[q] * C;
                         float al = p.xwt[q];
 #pragma unroll
-                        for (int ch = 0; ch < C; ch++) bc[ch] = __fadd_rn(bc[ch], __fmul_rn((float)px[ch], al));
+                        for (int ch = 0; ch < NC; ch++) bc[ch] = __fadd_rn(bc[ch], __fmul_rn((float)px[ch], al));
                     }
 #pragma unroll
-                    for (int ch = 0; ch < C; ch++) out[dx * C + ch] = bc[ch];
+                    for (int ch = 0; ch < NC; ch++) out[dx * NC + ch] = bc[ch];
                 }
             } else {   // integer ratio: exact integer row sums, kept as int bit patterns
                 int *outi = reinterpret_cast<int *>(out);
                 for (int dx = gt; dx < p.w; dx += gsz) {
-                    int sc[C];
+                    int sc[NC];
 #pragma unroll
-                    for (int ch = 0; ch < C; ch++) sc[ch] = 0;
+                    for (int ch = 0; ch < NC; ch++) sc[ch] = 0;
                     const unsigned char *px = rb + dx * p.fx * C;
                     for (int q = 0; q < p.fx; q++, px += C) {
 #pragma unroll
-                        for (int ch = 0; ch < C; ch++) sc[ch] += px[ch];
+                        for (int ch = 0; ch < NC; ch++) sc[ch] += px[ch];
                     }
 #pragma unroll
-                    for (int ch = 0; ch < C; ch++) outi[dx * C + ch] = sc[ch];
+                    for (int ch = 0; ch < NC; ch++) outi[dx * NC + ch] = sc[ch];
                 }
             }
         }
@@ -173,20 +177,20 @@ __global__ void __launch_bounds__(K0_THREADS) k_resize_gray(K0Params p, const in
     if (p.bgr_out) {
         const int wb = p.w * 3;
         uint8_t *out = p.bgr_out + (oidx ? (size_t)s * ostride + ((size_t)o * p.h + dy) * wb : ((size_t)f * p.h + dy) * wb);
-        for (int i = tid; i < wb; i += K0_THREADS) out[i] = C == 1 ? small[i / 3] : small[i];
+        for (int i = tid; i < wb; i += K0_THREADS) out[i] = C == 1 ? small[i / 3] : RGB ? small[i + 2 - 2 * (i % 3)] : small[i];
         return;
     }
     uint8_t *g = p.gray + ((size_t)f * p.h + dy) * p.w;
     for (int dx = tid; dx < p.w; dx += K0_THREADS)
-        g[dx] = C == 1 ? small[dx] : (uint8_t)fm_gray(small[dx * 3], small[dx * 3 + 1], small[dx * 3 + 2]);
+        g[dx] = C == 1 ? small[dx] : (uint8_t)fm_gray<RGB>(small[dx * 3], small[dx * 3 + 1], small[dx * 3 + 2]);
 }
 
 // INTER_AREA resize to BGR (device buffers); mode / tables as fm_ctx_create derives them.  One frame (fm_resize_area:
 // S = T = 1, oidx null) or the frames of a call with an oidx table (fm_object_planes).  channels: 3 (BGR source) or 1 (gray
-// source, its resize stored in B, G and R)
+// source, its resize stored in B, G and R); rgb: R-first three-byte source
 int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, size_t fstride, size_t pitch, int S, int T, int W,
                          int H, int w, int h, int mode, int fx, int fy, const ResizeTab &xt, const ResizeTab &yt, const int *oidx,
-                         uint8_t *dst_dev, size_t ostride, cudaStream_t st, int channels) {
+                         uint8_t *dst_dev, size_t ostride, cudaStream_t st, int channels, bool rgb) {
     K0Params p;
     p.frames = src_dev; p.sstride = sstride; p.fstride = fstride; p.pitch = pitch;
     p.T = T; p.W = W; p.H = H; p.w = w; p.h = h;
@@ -201,12 +205,14 @@ int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, siz
         fm_set_error("resize needs %zu bytes of shared memory (frame too wide / ratio too large)", smem);
         return FM_ERANGE;
     }
-    int rc;
-    const void *kern = channels == 1 ? (const void *)k_resize_gray<1> : (const void *)k_resize_gray<3>;
-    if ((rc = fm_ensure_smem(kern, smem, device))) return rc;
+    int rc = FM_OK;
     dim3 grid(h, S * T);
-    if (channels == 1) k_resize_gray<1><<<grid, K0_THREADS, smem, st>>>(p, oidx, ostride);
-    else k_resize_gray<3><<<grid, K0_THREADS, smem, st>>>(p, oidx, ostride);
+    fm_px_dispatch(channels, rgb, [&](auto C, auto RGB) {
+        const void *kern = (const void *)k_resize_gray<C.value, RGB.value>;
+        if ((rc = fm_ensure_smem(kern, smem, device))) return;
+        k_resize_gray<C.value, RGB.value><<<grid, K0_THREADS, smem, st>>>(p, oidx, ostride);
+    });
+    if (rc) return rc;
     FM_LAUNCH_CHECK();
     return FM_OK;
 }
@@ -220,8 +226,8 @@ int fm_launch_resize_bgr(int device, const uint8_t *src_dev, size_t sstride, siz
 #define K0W_WARPS 8
 
 // task = ((frame * h + dy) * nq + q): the warp produces destination columns q*dxw .. q*dxw+dxw-1 (one per lane).
-// C: channels of the source (3 BGR, 1 gray)
-template <int C>
+// C: channels of the source (3 BGR, 1 gray); RGB: R-first three-byte source
+template <int C, bool RGB = false>
 __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_warp(K0Params p, int segpitch, int tasks, int nq,
                                                                      int dxw) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -244,7 +250,8 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_warp(K0Params p,
     int xa = 0, xn = 0;
     int xfirst = 0;
     if (live) { xa = p.xstart[dx]; xn = p.xstart[dx + 1] - xa; xfirst = p.xidx[xa]; }
-    float sc[C];
+    constexpr int NC = C == 4 ? 3 : C;          // chains per column: the fourth byte of BGRA / RGBA is not resized
+    float sc[NC];
     for (int j = 0; j < ny; j++) {
         const int sy = p.yidx[y0 + j];
         const float beta = p.ywt[y0 + j];
@@ -272,25 +279,25 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_warp(K0Params p,
         }
         __syncwarp();
         const unsigned char *rb = rowbuf + mis - b_lo;                    // rb[C*x + c] = source pixel x
-        float bc[C];
+        float bc[NC];
 #pragma unroll
-        for (int ch = 0; ch < C; ch++) bc[ch] = 0.f;
+        for (int ch = 0; ch < NC; ch++) bc[ch] = 0.f;
         const unsigned char *px = rb + xfirst * C;      // the taps of a column are consecutive source pixels
         const float *wt = p.xwt + xa;
 #pragma unroll 4
         for (int qq = 0; qq < xn; qq++, px += C) {
             const float al = __ldg(wt + qq);
 #pragma unroll
-            for (int ch = 0; ch < C; ch++) bc[ch] = __fadd_rn(bc[ch], __fmul_rn((float)px[ch], al));
+            for (int ch = 0; ch < NC; ch++) bc[ch] = __fadd_rn(bc[ch], __fmul_rn((float)px[ch], al));
         }
 #pragma unroll
-        for (int ch = 0; ch < C; ch++) sc[ch] = j == 0 ? __fmul_rn(beta, bc[ch]) : __fadd_rn(sc[ch], __fmul_rn(beta, bc[ch]));
+        for (int ch = 0; ch < NC; ch++) sc[ch] = j == 0 ? __fmul_rn(beta, bc[ch]) : __fadd_rn(sc[ch], __fmul_rn(beta, bc[ch]));
     }
     if (live) {
-        int v[C];
+        int v[NC];
 #pragma unroll
-        for (int ch = 0; ch < C; ch++) v[ch] = min(max(__float2int_rn(sc[ch]), 0), 255);
-        p.gray[((size_t)f * p.h + dy) * p.w + dx] = C == 1 ? (uint8_t)v[0] : (uint8_t)fm_gray(v[0], v[C > 1 ? 1 : 0], v[C - 1]);
+        for (int ch = 0; ch < NC; ch++) v[ch] = min(max(__float2int_rn(sc[ch]), 0), 255);
+        p.gray[((size_t)f * p.h + dy) * p.w + dx] = C == 1 ? (uint8_t)v[0] : (uint8_t)fm_gray<RGB>(v[0], v[NC > 1 ? 1 : 0], v[NC - 1]);
     }
 }
 
@@ -316,8 +323,8 @@ __device__ __noinline__ void copy_partial_block(unsigned char *d, const uint8_t 
 
 #define K0_RG 7         // tap groups per destination column held in registers
 // PF = 16-byte blocks per lane of one source segment (registers used to prefetch the next row).  C: channels of the source
-// (3 BGR: a group is 12 bytes; 1 gray: a group is one word)
-template <int PF, bool INREG, int C>
+// (3 BGR: a group is 12 bytes; 1 gray: a group is one word); RGB: R-first three-byte source
+template <int PF, bool INREG, int C, bool RGB = false>
 __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K0GParams gp, int segpitch, int tasks,
                                                                    int nq, int dxw) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -408,10 +415,32 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
         b0 = __fadd_rn(b0, fm_byte_mul(W1, 2, a.z, n.z)); b1 = __fadd_rn(b1, fm_byte_mul(W1, 3, a.z, n.z));       \
         b2 = __fadd_rn(b2, fm_byte_mul(W2, 0, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(W2, 1, a.w, n.w));       \
         b1 = __fadd_rn(b1, fm_byte_mul(W2, 2, a.w, n.w)); b2 = __fadd_rn(b2, fm_byte_mul(W2, 3, a.w, n.w));
+#define FM_G4A(W0, W1, W2, W3, a, n)                                                                          \
+        b0 = __fadd_rn(b0, fm_byte_mul(W0, 0, a.x, n.x)); b1 = __fadd_rn(b1, fm_byte_mul(W0, 1, a.x, n.x));       \
+        b2 = __fadd_rn(b2, fm_byte_mul(W0, 2, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(W1, 0, a.y, n.y));       \
+        b1 = __fadd_rn(b1, fm_byte_mul(W1, 1, a.y, n.y)); b2 = __fadd_rn(b2, fm_byte_mul(W1, 2, a.y, n.y));       \
+        b0 = __fadd_rn(b0, fm_byte_mul(W2, 0, a.z, n.z)); b1 = __fadd_rn(b1, fm_byte_mul(W2, 1, a.z, n.z));       \
+        b2 = __fadd_rn(b2, fm_byte_mul(W2, 2, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(W3, 0, a.w, n.w));       \
+        b1 = __fadd_rn(b1, fm_byte_mul(W3, 1, a.w, n.w)); b2 = __fadd_rn(b2, fm_byte_mul(W3, 2, a.w, n.w));
 #define FM_G1(W0, a, n)                                                                                       \
         b0 = __fadd_rn(b0, fm_byte_mul(W0, 0, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(W0, 1, a.y, n.y));       \
         b0 = __fadd_rn(b0, fm_byte_mul(W0, 2, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(W0, 3, a.w, n.w));
-        if (C == 1 && inreg) {
+        if (C == 4 && inreg) {          // four-byte pixels: a group is 4 words, the fourth byte of each is skipped
+#pragma unroll
+            for (int g = 0; g < K0_RG; g++) {
+                if (g < gmax) {     // braces: the macro is several statements, all of them guarded
+                    FM_G4A(wp[4 * g], wp[4 * g + 1], wp[4 * g + 2], wp[4 * g + 3], wr[g], wn[g])
+                }
+            }
+        } else if (C == 4) {
+#pragma unroll 2
+            for (int g = 0; g < gn; g++) {
+                const float4 a = __ldg(gw + g);
+                const float4 n = make_float4(__fmul_rn(a.x, -8388608.0f), __fmul_rn(a.y, -8388608.0f),
+                                             __fmul_rn(a.z, -8388608.0f), __fmul_rn(a.w, -8388608.0f));
+                FM_G4A(wp[4 * g], wp[4 * g + 1], wp[4 * g + 2], wp[4 * g + 3], a, n)
+            }
+        } else if (C == 1 && inreg) {
 #pragma unroll
             for (int g = 0; g < K0_RG; g++) {
                 if (g < gmax) FM_G1(wp[g], wr[g], wn[g])
@@ -444,6 +473,7 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
         }
 #undef FM_G4
 #undef FM_G1
+#undef FM_G4A
         if (j == 0) {
             s0 = __fmul_rn(beta, b0); s1 = __fmul_rn(beta, b1); s2 = __fmul_rn(beta, b2);
         } else {
@@ -456,19 +486,20 @@ __global__ void __launch_bounds__(32 * K0W_WARPS) k_resize_gray_g4(K0Params p, K
         int v0 = min(max(__float2int_rn(s0), 0), 255);
         int v1 = min(max(__float2int_rn(s1), 0), 255);
         int v2 = min(max(__float2int_rn(s2), 0), 255);
-        p.gray[((size_t)f * p.h + dy) * p.w + dx] = C == 1 ? (uint8_t)v0 : (uint8_t)fm_gray(v0, v1, v2);
+        p.gray[((size_t)f * p.h + dy) * p.w + dx] = C == 1 ? (uint8_t)v0 : (uint8_t)fm_gray<RGB>(v0, v1, v2);
     }
 }
 
 int fm_launch_gray_plane(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
     dim3 grid(((c->N + 3) / 4 + 255) / 256, c->S * T);
-    if (c->cfg.flags & FM_FLAG_GRAY) k_gray<1><<<grid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->w, c->N, c->gray, c->nvalid);
-    else k_gray<3><<<grid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->w, c->N, c->gray, c->nvalid);
+    fm_px_dispatch(c->px_bytes, c->rgb, [&](auto C, auto RGB) {
+        k_gray<C.value, RGB.value><<<grid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->w, c->N, c->gray, c->nvalid);
+    });
     FM_LAUNCH_CHECK();
     return FM_OK;
 }
 
-template <int C>
+template <int C, bool RGB = false>
 static int launch_resize_warps(fm_ctx *c, const K0Params &p, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch,
                                int F, cudaStream_t st) {
     // one warp per (frame, destination row, group of <= 32 destination columns)
@@ -476,16 +507,16 @@ static int launch_resize_warps(fm_ctx *c, const K0Params &p, const uint8_t *fram
     int segpitch = ((c->W * C + nq - 1) / nq + C * (c->xtab.max_taps + 10) + 32 + 15) & ~15;
     size_t smemw = (size_t)K0W_WARPS * segpitch;
     int rc;
-    if ((rc = fm_ensure_smem((const void *)k_resize_gray_warp<C>, smemw, c->cfg.device))) return rc;
+    if ((rc = fm_ensure_smem((const void *)k_resize_gray_warp<C, RGB>, smemw, c->cfg.device))) return rc;
     int tasks = c->h * F * nq;
     const bool aligned4 = ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->W * C)) & 3) == 0;
     if (aligned4 && c->g4w) {
-        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, true, C>, smemw, c->cfg.device))) return rc;
-        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, false, C>, smemw, c->cfg.device))) return rc;
-        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<8, true, C>, smemw, c->cfg.device))) return rc;
-        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<8, false, C>, smemw, c->cfg.device))) return rc;
-        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<16, true, C>, smemw, c->cfg.device))) return rc;
-        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<16, false, C>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, true, C, RGB>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<4, false, C, RGB>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<8, true, C, RGB>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<8, false, C, RGB>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<16, true, C, RGB>, smemw, c->cfg.device))) return rc;
+        if ((rc = fm_ensure_smem((const void *)k_resize_gray_g4<16, false, C, RGB>, smemw, c->cfg.device))) return rc;
         K0GParams gp;
         gp.g4start = c->g4start; gp.g4n = c->g4n; gp.g4off = c->g4off; gp.g4w = c->g4w;
         const int blocks16 = segpitch / 16 + 1;         // upper bound of 16-byte blocks per segment
@@ -493,16 +524,16 @@ static int launch_resize_warps(fm_ctx *c, const K0Params &p, const uint8_t *fram
         const bool inreg = c->g4max <= K0_RG;
 #define FM_K0(PF)                                                                                                   \
         do {                                                                                                        \
-            if (inreg) k_resize_gray_g4<PF, true, C><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, gp, segpitch, tasks, nq, dxw); \
-            else k_resize_gray_g4<PF, false, C><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, gp, segpitch, tasks, nq, dxw);     \
+            if (inreg) k_resize_gray_g4<PF, true, C, RGB><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, gp, segpitch, tasks, nq, dxw); \
+            else k_resize_gray_g4<PF, false, C, RGB><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, gp, segpitch, tasks, nq, dxw);     \
         } while (0)
         if (blocks16 <= 4 * 32) FM_K0(4);
         else if (blocks16 <= 8 * 32) FM_K0(8);
         else if (blocks16 <= 16 * 32) FM_K0(16);
-        else k_resize_gray_warp<C><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, segpitch, tasks, nq, dxw);
+        else k_resize_gray_warp<C, RGB><<<gridw, 32 * K0W_WARPS, smemw, st>>>(p, segpitch, tasks, nq, dxw);
 #undef FM_K0
     } else {
-        k_resize_gray_warp<C><<<(tasks + K0W_WARPS - 1) / K0W_WARPS, 32 * K0W_WARPS, smemw, st>>>(p, segpitch, tasks, nq, dxw);
+        k_resize_gray_warp<C, RGB><<<(tasks + K0W_WARPS - 1) / K0W_WARPS, 32 * K0W_WARPS, smemw, st>>>(p, segpitch, tasks, nq, dxw);
     }
     FM_LAUNCH_CHECK();
     return FM_OK;
@@ -511,8 +542,7 @@ static int launch_resize_warps(fm_ctx *c, const K0Params &p, const uint8_t *fram
 int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T,
                        cudaStream_t st) {
     const int F = c->S * T;
-    const bool gray_in = (c->cfg.flags & FM_FLAG_GRAY) != 0;
-    const int C = gray_in ? 1 : 3;
+    const int C = c->px_bytes;
     // every Gaussian the fused stencil does not take goes to the tensor-core blur (k_wide.cu)
     if (c->resize_mode == 0)          // gray fused into the first kernel of the blur (gray frames: they are the gray plane)
         return c->umma ? fm_launch_umma_blur(c, frames, sstride, fstride, pitch, T, st)
@@ -520,7 +550,7 @@ int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t 
     if (c->resize_mode == 3) {        // upscale + gray into the gray plane (k_upscale.cu)
         int rc;
         if ((rc = fm_launch_upscale(c->cfg.device, frames, sstride, fstride, pitch, T, F, c->W, c->H, c->w, c->h, c->uxt, c->uyt,
-                                    c->nvalid, c->gray, nullptr, nullptr, 0, st, C)))
+                                    c->nvalid, c->gray, nullptr, nullptr, 0, st, C, c->rgb)))
             return rc;
     } else {
         K0Params p;
@@ -537,20 +567,22 @@ int fm_launch_frontend(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t 
             // one source row per lane, TMA-staged (k_resize_rows.cu)
             if ((rc = fm_launch_resize_rows(c, frames, sstride, fstride, pitch, T, st))) return rc;
         } else if (c->resize_mode == 1) {
-            if ((rc = gray_in ? launch_resize_warps<1>(c, p, frames, sstride, fstride, pitch, F, st)
-                              : launch_resize_warps<3>(c, p, frames, sstride, fstride, pitch, F, st)))
-                return rc;
+            fm_px_dispatch(c->px_bytes, c->rgb, [&](auto Cx, auto RGB) {
+                rc = launch_resize_warps<Cx.value, RGB.value>(c, p, frames, sstride, fstride, pitch, F, st);
+            });
+            if (rc) return rc;
         } else {
             size_t smem = (size_t)K0_GROUPS * rowpitch + (size_t)p.max_ytaps * c->w * C * sizeof(float);
             if (smem > 220 * 1024) {
                 fm_set_error("resize front end needs %zu bytes of shared memory (frame too wide / ratio too large)", smem);
                 return FM_ERANGE;
             }
-            const void *kern = gray_in ? (const void *)k_resize_gray<1> : (const void *)k_resize_gray<3>;
-            if ((rc = fm_ensure_smem(kern, smem, c->cfg.device))) return rc;
             dim3 grid(c->h, F);
-            if (gray_in) k_resize_gray<1><<<grid, K0_THREADS, smem, st>>>(p, nullptr, 0);
-            else k_resize_gray<3><<<grid, K0_THREADS, smem, st>>>(p, nullptr, 0);
+            fm_px_dispatch(c->px_bytes, c->rgb, [&](auto Cx, auto RGB) {
+                if ((rc = fm_ensure_smem((const void *)k_resize_gray<Cx.value, RGB.value>, smem, c->cfg.device))) return;
+                k_resize_gray<Cx.value, RGB.value><<<grid, K0_THREADS, smem, st>>>(p, nullptr, 0);
+            });
+            if (rc) return rc;
             FM_LAUNCH_CHECK();
         }
     }

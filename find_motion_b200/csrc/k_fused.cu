@@ -44,7 +44,14 @@
 #define NV_Y_BYTES (NV_PITCH * FG_ROWS)                  // 5760 = 45 * 128: the UV box lands 128 B aligned after it
 #define NV_BYTES (NV_Y_BYTES + NV_PITCH * FG_ROWS / 2)   // <= RAW_BYTES: both fit the BGR stage
 // Gray (FM_FLAG_GRAY): a stage holds the luma box alone, rows y0-2 .. y0+FT_H+1 of the caller's frame; no conversion
-enum { FUSED_BGR = 0, FUSED_NV12 = 1, FUSED_GRAY = 2 };     // source format of k_fused
+// Four-byte pixels (FM_FLAG_ALPHA): a stage holds one box of the tile's pixels x0-4 .. x0+139 as u32 words, 576-byte
+// rows; one 16-byte word of 4 pixels is one gray word, no realignment.  Two such stages make the CTA's shared memory
+// FUSED_SMEM_A4 = 61,456 B (BGR: 51,216 B), so three CTAs fit an SM instead of four (DESIGN §4.9)
+#define A4_PITCH 576
+#define A4_BYTES (A4_PITCH * FG_ROWS)
+#define A4_STAGE ((A4_BYTES + 127) / 128 * 128)
+enum { FUSED_BGR = 0, FUSED_NV12 = 1, FUSED_GRAY = 2, FUSED_RGB = 3, FUSED_BGRA = 4, FUSED_RGBA = 5 };
+// source format of k_fused (RGB, RGBA: the gray weights of bytes 0 and 2 swapped)
 
 struct FusedParams {
     int T, w, h, wpr;           // T = frames per stream of the call
@@ -224,8 +231,10 @@ template <bool KEEP, bool SAFE, int SRC>
 __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const __grid_constant__ CUtensorMap tmap, FusedParams p,
                                                                          const __grid_constant__ CUtensorMap tmap_uv) {
     extern __shared__ __align__(128) unsigned char fsm[];
-    unsigned char *raw = fsm;                                                  // [2][RAW_STAGE] staged BGR rows (TMA)
-    uint32_t *sg = reinterpret_cast<uint32_t *>(fsm + 2 * RAW_STAGE);        // [FH_ROWS][FG_WORDS] gray bytes (FG_ROWS used)
+    constexpr bool A4 = SRC == FUSED_BGRA || SRC == FUSED_RGBA, RGBO = SRC == FUSED_RGB || SRC == FUSED_RGBA;
+    constexpr int STG = A4 ? A4_STAGE : RAW_STAGE;
+    unsigned char *raw = fsm;                                                  // [2][STG] staged BGR rows (TMA)
+    uint32_t *sg = reinterpret_cast<uint32_t *>(fsm + 2 * STG);              // [FH_ROWS][FG_WORDS] gray bytes (FG_ROWS used)
     uint32_t *sh = sg + FH_ROWS * FG_WORDS;                                  // [FH_ROWS][FH_WORDS] packed horizontal sums
     uint64_t *bars = reinterpret_cast<uint64_t *>(sh + FH_ROWS * FH_WORDS);
     constexpr bool NV12 = SRC == FUSED_NV12, GRAY = SRC == FUSED_GRAY;
@@ -267,7 +276,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
     if (okB) M |= ((__ldg(p.maskbits + ((size_t)s * h + py) * p.wpr + ((px + 64) >> 5)) >> (px & 31)) & 0xFFu) << 8;
     const bool wmasked = __any_sync(0xffffffffu, M != 0);       // warp-uniform choice of the masked variant
     // TMA pipeline: frame t+1 lands in the other stage while frame t is being processed
-    const int cx = (x0 * 3) / 4 - 4, cy = y0 - 2;        // box origin in (u32 column, row); OOB is zero-filled
+    const int cx = A4 ? x0 - 4 : (x0 * 3) / 4 - 4, cy = y0 - 2;     // box origin in (u32 column, row); OOB is zero-filled
     if (tid == 0) {
         fm_mbar_init(&bars[0], 1);
         fm_mbar_init(&bars[1], 1);
@@ -284,7 +293,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
             fm_mbar_expect_tx(&bars[0], NV_Y_BYTES);
             fm_tma_load_4d(raw, &tmap, &bars[0], x0 / 4 - 4, y0 - 2, 0, s);
         } else {
-            fm_mbar_expect_tx(&bars[0], RAW_BYTES);
+            fm_mbar_expect_tx(&bars[0], A4 ? A4_BYTES : RAW_BYTES);
             fm_tma_load_4d(raw, &tmap, &bars[0], cx, cy, 0, s);
         }
     }
@@ -323,16 +332,16 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
         // conversions out of raw stage (t+1)&1 (frame t-1) and all reads of the gray plane are complete.
         if (tid == 0 && t + 1 < Ts) {
             if (NV12) {
-                unsigned char *dst = raw + ((t + 1) & 1) * RAW_STAGE;
+                unsigned char *dst = raw + ((t + 1) & 1) * STG;
                 fm_mbar_expect_tx(&bars[(t + 1) & 1], NV_BYTES);
                 fm_tma_load_4d(dst, &tmap, &bars[(t + 1) & 1], x0 / 4 - 4, y0 - 2, t + 1, s);
                 fm_tma_load_4d(dst + NV_Y_BYTES, &tmap_uv, &bars[(t + 1) & 1], x0 / 4 - 4, y0 / 2 - 1, t + 1, s);
             } else if (GRAY) {
                 fm_mbar_expect_tx(&bars[(t + 1) & 1], NV_Y_BYTES);
-                fm_tma_load_4d(raw + ((t + 1) & 1) * RAW_STAGE, &tmap, &bars[(t + 1) & 1], x0 / 4 - 4, y0 - 2, t + 1, s);
+                fm_tma_load_4d(raw + ((t + 1) & 1) * STG, &tmap, &bars[(t + 1) & 1], x0 / 4 - 4, y0 - 2, t + 1, s);
             } else {
-                fm_mbar_expect_tx(&bars[(t + 1) & 1], RAW_BYTES);
-                fm_tma_load_4d(raw + ((t + 1) & 1) * RAW_STAGE, &tmap, &bars[(t + 1) & 1], cx, cy, t + 1, s);
+                fm_mbar_expect_tx(&bars[(t + 1) & 1], A4 ? A4_BYTES : RAW_BYTES);
+                fm_tma_load_4d(raw + ((t + 1) & 1) * STG, &tmap, &bars[(t + 1) & 1], cx, cy, t + 1, s);
             }
         }
         fm_mbar_wait(bars_s + 8 * (t & 1), (t >> 1) & 1);
@@ -344,7 +353,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
             // +3); the chroma terms of the word's two 2x2 blocks serve both rows.  Zero-filled bytes outside the image
             // convert to some colour: the border step below overwrites every halo pixel the passes read, as with BGR.
             constexpr int NU = (FG_ROWS / 2) * FG_WORDS, NFULL = NU / FUSED_THREADS;
-            const unsigned char *st = raw + (t & 1) * RAW_STAGE;
+            const unsigned char *st = raw + (t & 1) * STG;
 #pragma unroll
             for (int i = 0; i <= NFULL; i++) {
                 if (i < NFULL || tid < NU - NFULL * FUSED_THREADS) {
@@ -362,12 +371,19 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
         } else if (GRAY) {
             // the stage already holds gray bytes: word u of a row (columns x0-4+4u .. +3) is at byte 12 + 4u of its box row.
             // Zero-filled bytes outside the image are overwritten by the border step below, as with BGR.
-            const unsigned char *st = raw + (t & 1) * RAW_STAGE + gs_tid;
+            const unsigned char *st = raw + (t & 1) * STG + gs_tid;
             if (gr < GROWS) {
 #pragma unroll 1                // unrolled, the six loads in flight push the kernel to 40 spilled bytes (rolled: 20)
                 for (int i = 0; i < (FG_ROWS + GROWS - 1) / GROWS; i++)
                     if ((i + 1) * GROWS <= FG_ROWS || gr + i * GROWS < FG_ROWS)
                         sgg[i * GROWS * FG_WORDS] = *reinterpret_cast<const uint32_t *>(st + i * GROWS * NV_PITCH);
+            }
+        } else if (A4) {
+            // word u of a gray row (columns x0-4+4u .. +3) is the 16-byte word u of its box row
+            const unsigned char *st = raw + (t & 1) * STG;
+            for (int un = tid; un < FG_ROWS * FG_WORDS; un += FUSED_THREADS) {
+                const int k = un / FG_WORDS, u = un - k * FG_WORDS;
+                sg[k * FG_WORDS + u] = fm_gray4a<RGBO>(*reinterpret_cast<const uint4 *>(st + k * A4_PITCH + 16 * u));
             }
         } else {
             // the staged rows are dense (pitch 432 B = 36 groups of 4 pixels = 12 B, the first at byte 4 because the
@@ -377,7 +393,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
             // u = tid + i * FUSED_THREADS: the offsets of all steps are immediates from the thread's own (rs, sgt), and
             // only the last step, which not every thread has, is predicated.
             constexpr int NU = FG_ROWS * FG_WORDS / 2, NFULL = NU / FUSED_THREADS;
-            const unsigned char *rs = raw + (t & 1) * RAW_STAGE + rs_tid;
+            const unsigned char *rs = raw + (t & 1) * STG + rs_tid;
 #pragma unroll
             for (int i = 0; i <= NFULL; i++) {
                 if (i < NFULL || tid < NU - NFULL * FUSED_THREADS) {
@@ -385,7 +401,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, FUSED_MIN_CTAS) k_fused(const _
                     const unsigned char *q = rs + i * (24 * FUSED_THREADS);
                     const uint32_t a0 = *reinterpret_cast<const uint32_t *>(q), a5 = *reinterpret_cast<const uint32_t *>(q + 20);
                     const uint2 a12 = *reinterpret_cast<const uint2 *>(q + 4), a34 = *reinterpret_cast<const uint2 *>(q + 12);
-                    const uint32_t g0 = fm_gray4(a0, a12.x, a12.y), g1 = fm_gray4(a34.x, a34.y, a5);
+                    const uint32_t g0 = fm_gray4<RGBO>(a0, a12.x, a12.y), g1 = fm_gray4<RGBO>(a34.x, a34.y, a5);
                     sgt[i * FUSED_THREADS] = make_uint2(g0, g1);
                 }
             }
@@ -532,6 +548,8 @@ extern "C" void fm_k1_prof_dump(void) {
 #endif
 
 #define FUSED_SMEM (2 * RAW_STAGE + FH_ROWS * FG_WORDS * 4 + FH_ROWS * FH_WORDS * 4 + 16)
+#define FUSED_SMEM_A4 (2 * A4_STAGE + FH_ROWS * FG_WORDS * 4 + FH_ROWS * FH_WORDS * 4 + 16)
+static_assert(FUSED_SMEM_A4 == 61456, "DESIGN §4.9 states this budget");
 
 // one plane of the call's NV12 frames, or the gray frames (rows of W bytes, `pitch` bytes apart), as a 4-D u32 tensor map
 // with boxes of NV_PITCH bytes x box_rows
@@ -555,7 +573,7 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
                     cudaStream_t st) {
     CUtensorMap tmap, tmap_uv;
     const bool nv12 = c->nv12_bgr == nullptr && (c->cfg.flags & FM_FLAG_NV12);     // NV12 read directly (no staged slot)
-    const bool gray = (c->cfg.flags & FM_FLAG_GRAY) != 0;
+    const bool gray = c->px_bytes == 1;
     int rc;
     if (nv12) {
         if ((((uintptr_t)frames) | sstride | fstride | pitch | (size_t)uv) & 15) {
@@ -572,7 +590,9 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
         if ((rc = nv12_plane_tmap(c, frames, c->H, sstride, fstride, pitch, T, FG_ROWS, &tmap))) return rc;
         tmap_uv = tmap;                          // not read
     } else {
-        if ((rc = fm_frames_tmap(c, frames, sstride, fstride, pitch, T, RAW_PITCH / 4, FG_ROWS, &tmap))) return rc;
+        if ((rc = fm_frames_tmap(c, frames, sstride, fstride, pitch, T, c->px_bytes == 4 ? A4_PITCH / 4 : RAW_PITCH / 4, FG_ROWS,
+                                 &tmap)))
+            return rc;
         tmap_uv = tmap;                          // not read
     }
     FusedParams p;
@@ -613,16 +633,20 @@ int fm_launch_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fst
     fused_bfr(p);
     dim3 grid(p.tilesX, p.tilesY, c->S);
     typedef void (*FusedKernel)(const CUtensorMap, FusedParams, const CUtensorMap);
-#define FM_K1_SRCS(K, S) {k_fused<K, S, FUSED_BGR>, k_fused<K, S, FUSED_NV12>, k_fused<K, S, FUSED_GRAY>}
-    const FusedKernel kerns[2][2][3] = {{FM_K1_SRCS(false, false), FM_K1_SRCS(false, true)},
+#define FM_K1_SRCS(K, S) {k_fused<K, S, FUSED_BGR>, k_fused<K, S, FUSED_NV12>, k_fused<K, S, FUSED_GRAY>, k_fused<K, S, FUSED_RGB>, \
+                          k_fused<K, S, FUSED_BGRA>, k_fused<K, S, FUSED_RGBA>}
+    const FusedKernel kerns[2][2][6] = {{FM_K1_SRCS(false, false), FM_K1_SRCS(false, true)},
                                         {FM_K1_SRCS(true, false), FM_K1_SRCS(true, true)}};
 #undef FM_K1_SRCS
-    const FusedKernel kern = kerns[keep][safe][nv12 ? FUSED_NV12 : gray ? FUSED_GRAY : FUSED_BGR];
-    if ((rc = fm_ensure_smem((const void *)kern, FUSED_SMEM, c->cfg.device))) return rc;
+    const int src = nv12 ? FUSED_NV12 : gray ? FUSED_GRAY : c->px_bytes == 4 ? (c->rgb ? FUSED_RGBA : FUSED_BGRA)
+                                                 : c->rgb ? FUSED_RGB : FUSED_BGR;
+    const FusedKernel kern = kerns[keep][safe][src];
+    const int smem = c->px_bytes == 4 ? FUSED_SMEM_A4 : FUSED_SMEM;
+    if ((rc = fm_ensure_smem((const void *)kern, smem, c->cfg.device))) return rc;
     // a programmatic dependent of the contour stage of the previous call: see fused_exit.  Not after the NV12 staging
     // kernel (k_nv12.cu, FM_NV12_STAGED builds): K1 reads the frames before its wait, and that kernel writes them
-    if (c->nv12_bgr) kern<<<grid, FUSED_THREADS, FUSED_SMEM, st>>>(tmap, p, tmap_uv);
-    else (void)fm_launch_chained(kern, grid, dim3(FUSED_THREADS), FUSED_SMEM, st, tmap, p, tmap_uv);
+    if (c->nv12_bgr) kern<<<grid, FUSED_THREADS, smem, st>>>(tmap, p, tmap_uv);
+    else (void)fm_launch_chained(kern, grid, dim3(FUSED_THREADS), smem, st, tmap, p, tmap_uv);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }

@@ -12,6 +12,7 @@
 // NV12 contexts resize the BGR slot: the staged front ends already hold the call's frames converted there; a fused
 // context first converts its written frames into its own slot with k_nv12_bgr.  Gray contexts (FM_FLAG_GRAY) resize their
 // one channel in place (k_resize_rows<true, 1>, k_resize_gray<1>, k_upscale_gray<1>) and store each byte in B, G and R.
+// RGB contexts (FM_FLAG_RGB) resize their frames in place and store each pixel's bytes in BGR order (the RGB instantiations).
 #include "fm_common.cuh"
 
 #define OBJ_PLAN_THREADS 1024
@@ -42,12 +43,12 @@ int fm_launch_object_plan(fm_ctx *c, int T, cudaStream_t st) {
 int fm_launch_resize_objects(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T,
                              uint8_t *out, size_t ostride, cudaStream_t st) {
     const int w = FM_OBJECT_WIDTH, h = c->obj_h;
-    const int C = (c->cfg.flags & FM_FLAG_GRAY) ? 1 : 3;
+    const int C = c->px_bytes;
     if (c->obj_mode == 3)
         return fm_launch_upscale(c->cfg.device, frames, sstride, fstride, pitch, T, c->S * T, c->W, c->H, w, h, c->obj_uxt,
-                                 c->obj_uyt, nullptr, nullptr, out, c->obj_idx, ostride, st, C);
+                                 c->obj_uyt, nullptr, nullptr, out, c->obj_idx, ostride, st, C, c->rgb);
     if (c->obj_rows && ((((uintptr_t)frames) | sstride | fstride | pitch) & 15) == 0)
         return fm_launch_resize_rows_objects(c, frames, sstride, fstride, pitch, T, out, ostride, st);
     return fm_launch_resize_bgr(c->cfg.device, frames, sstride, fstride, pitch, c->S, T, c->W, c->H, w, h, c->obj_mode, c->obj_fx,
-                                c->obj_fy, c->obj_xtab, c->obj_ytab, c->obj_idx, out, ostride, st, C);
+                                c->obj_fy, c->obj_xtab, c->obj_ytab, c->obj_idx, out, ostride, st, C, c->rgb);
 }

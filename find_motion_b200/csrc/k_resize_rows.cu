@@ -19,6 +19,10 @@
 // C = 1 (FM_FLAG_GRAY): one-byte source pixels, a tap group of 4 pixels is one word instead of three, and each column has
 // one chain per row instead of three; per chain the products and sums are those of one channel of the BGR kernel.  The
 // gray variant stores the resized bytes as they are, the BGR one stores each in B, G and R.
+// C = 4 (FM_FLAG_ALPHA): four-byte pixels, a tap group of 4 pixels is 4 aligned words (no realignment), three chains per
+// row and column as for BGR, and the fourth byte of each pixel is never read into a chain.
+// RGB (FM_FLAG_RGB): the three-byte (or four-byte) plan unchanged; only the gray step weighs byte 0 as R and byte 2 as B, and the BGR
+// variant stores each pixel's bytes in BGR order.
 #include <cuda.h>
 
 #include <algorithm>
@@ -83,7 +87,15 @@ __device__ __forceinline__ void rr_col_pass(uint32_t blk, uint32_t sel, const fl
 #pragma unroll
     for (int g = 0; g < NPG; g++) {          // straight-line code: the compiler schedules the weight loads ahead of their use
         const float4 a = __ldg(wp + 2 * g), n = __ldg(wp + 2 * g + 1);
-        if constexpr (C == 1) {              // 4 pixels of one channel: one chain
+        if constexpr (C == 4) {              // 4 four-byte pixels, one aligned word each: the fourth byte never enters a chain
+            const uint32_t X0 = W[WO + 4 * g], X1 = W[WO + 4 * g + 1], X2 = W[WO + 4 * g + 2], X3 = W[WO + 4 * g + 3];
+            b0 = __fadd_rn(b0, fm_byte_mul(X0, 0, a.x, n.x)); b1 = __fadd_rn(b1, fm_byte_mul(X0, 1, a.x, n.x));
+            b2 = __fadd_rn(b2, fm_byte_mul(X0, 2, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(X1, 0, a.y, n.y));
+            b1 = __fadd_rn(b1, fm_byte_mul(X1, 1, a.y, n.y)); b2 = __fadd_rn(b2, fm_byte_mul(X1, 2, a.y, n.y));
+            b0 = __fadd_rn(b0, fm_byte_mul(X2, 0, a.z, n.z)); b1 = __fadd_rn(b1, fm_byte_mul(X2, 1, a.z, n.z));
+            b2 = __fadd_rn(b2, fm_byte_mul(X2, 2, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(X3, 0, a.w, n.w));
+            b1 = __fadd_rn(b1, fm_byte_mul(X3, 1, a.w, n.w)); b2 = __fadd_rn(b2, fm_byte_mul(X3, 2, a.w, n.w));
+        } else if constexpr (C == 1) {       // 4 pixels of one channel: one chain
             const uint32_t X = __byte_perm(W[WO + g], W[WO + g + 1], sel);
             b0 = __fadd_rn(b0, fm_byte_mul(X, 0, a.x, n.x)); b0 = __fadd_rn(b0, fm_byte_mul(X, 1, a.y, n.y));
             b0 = __fadd_rn(b0, fm_byte_mul(X, 2, a.z, n.z)); b0 = __fadd_rn(b0, fm_byte_mul(X, 3, a.w, n.w));
@@ -132,8 +144,8 @@ __device__ __forceinline__ void rr_bar_arrive(int id, int count) {
 // (row warps arrive, warp 5 waits); 3 + (i & 1): "hs buffer i & 1 consumed" (warp 5 arrives, row warps wait before chunk
 // i + 2), so the row warps run up to two chunks ahead of the vertical warp and never wait for each other.
 // BGR: warp 5 stores the band's BGR bytes as they are (the detector input plane) for the frames with oidx >= 0.
-// C: channels of the source (3 BGR, 1 gray)
-template <bool BGR, int C>
+// C: channels of the source (3 BGR, 1 gray); RGB: R-first three-byte source
+template <bool BGR, int C, bool RGB = false>
 __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(const __grid_constant__ CUtensorMap tmap, RowsParams p) {
     extern __shared__ __align__(128) unsigned char rsm[];
     const int tid = threadIdx.x;
@@ -144,6 +156,7 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
         if (t >= __ldg(p.nvalid + s)) return;               // not a real frame of this (ragged) call
     }
     const int CX = p.CX, BW = p.BW, NRp = p.NRp;
+    constexpr int NC = C == 4 ? 3 : C;       // chains (and resized bytes) per column: BGRA / RGBA resize three channels
     const int DXU = CX * p.NCHU;
     const int dy0 = blockIdx.y * p.D, dy1 = min(dy0 + p.D, p.h), Dn = dy1 - dy0;
     const int dxa = blockIdx.x * DXU, dxb = min(dxa + DXU, p.w), dxun = dxb - dxa;
@@ -153,11 +166,11 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
     const int nrows = __ldg(p.yidx + yb + ytn - 1) - R0 + 1;
 
     unsigned char *stage = rsm;                                                    // [2][stage_stride]
-    float *hs = reinterpret_cast<float *>(rsm + 2 * (size_t)p.stage_stride);       // [2][CX * C][NRp]
-    const int hsbuf = CX * C * NRp;
+    float *hs = reinterpret_cast<float *>(rsm + 2 * (size_t)p.stage_stride);       // [2][CX * NC][NRp]
+    const int hsbuf = CX * NC * NRp;
     float *yw = hs + 2 * hsbuf;                                                    // [2 NR] y weights of the band
     uint64_t *bars = reinterpret_cast<uint64_t *>((reinterpret_cast<uintptr_t>(yw + 2 * p.NR) + 7) & ~(uintptr_t)7);
-    unsigned char *bgr = reinterpret_cast<unsigned char *>(bars + 2);              // [D][DXU][C]
+    unsigned char *bgr = reinterpret_cast<unsigned char *>(bars + 2);              // [D][DXU][NC]
     constexpr int NT = RR_THREADS + 32;
 
     if (tid == 0) {
@@ -198,10 +211,10 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
                         }
                     }
                     if (tid < nrows) {        // lanes past the band's last row ran on rows of the box that nobody reads
-                        hw[(C * dxl) * NRp] = b0;
-                        if (C == 3) {
-                            hw[(C * dxl + 1) * NRp] = b1;
-                            hw[(C * dxl + 2) * NRp] = b2;
+                        hw[(NC * dxl) * NRp] = b0;
+                        if (NC == 3) {
+                            hw[(NC * dxl + 1) * NRp] = b1;
+                            hw[(NC * dxl + 2) * NRp] = b2;
                         }
                     }
                 }
@@ -230,7 +243,7 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
         if (lane == 0 && i + 2 < nch) issue(i + 2);
         // vertical chains of the chunk's cells: task = (destination row, column, channel)
         const float *hb = hs + (i & 1) * hsbuf;
-        const int nq = cxn * C, ntask = Dn * nq;
+        const int nq = cxn * NC, ntask = Dn * nq;
         for (int task = lane; task < ntask; task += 32) {
             const int dyl = task / nq, q = task - dyl * nq;
             const int y0 = __ldg(p.ystart + dy0 + dyl), ny = __ldg(p.ystart + dy0 + dyl + 1) - y0;
@@ -239,7 +252,7 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
             float sum = __fmul_rn(wy[0], hp[0]);
             for (int j = 1; j < ny; j++) sum = __fadd_rn(sum, __fmul_rn(wy[j], hp[j]));
             const int v = min(max(__float2int_rn(sum), 0), 255);
-            bgr[(dyl * DXU + (dx0 - dxa)) * C + q] = (unsigned char)v;
+            bgr[(dyl * DXU + (dx0 - dxa)) * NC + q] = (unsigned char)v;
         }
         if (i + 2 < nch) {
             __threadfence_block();
@@ -252,15 +265,15 @@ __global__ void __launch_bounds__(RR_THREADS + 32, RR_MIN_CTAS) k_resize_rows(co
         const int rb = dxun * 3;
         for (int i = lane; i < Dn * rb; i += 32) {
             const int dyl = i / rb, b = i - dyl * rb;
-            o[(size_t)dyl * p.w * 3 + b] = C == 1 ? bgr[dyl * DXU + b / 3] : bgr[dyl * DXU * 3 + b];
+            o[(size_t)dyl * p.w * 3 + b] = C == 1 ? bgr[dyl * DXU + b / 3] : bgr[dyl * DXU * 3 + (RGB ? b + 2 - 2 * (b % 3) : b)];
         }
     } else {
         // ---- BGR -> gray (SURVEY.md A.2) ----
         for (int i = lane; i < Dn * dxun; i += 32) {
             const int dyl = i / dxun, dxo = i - dyl * dxun;
-            const unsigned char *q = bgr + (dyl * DXU + dxo) * C;
+            const unsigned char *q = bgr + (dyl * DXU + dxo) * NC;
             p.gray[((size_t)f * p.h + dy0 + dyl) * p.w + dxa + dxo] =
-                C == 1 ? q[0] : (uint8_t)fm_gray(q[0], q[1], q[C - 1]);
+                C == 1 ? q[0] : (uint8_t)fm_gray<RGB>(q[0], q[1], q[NC - 1]);
         }
     }
 }
@@ -362,8 +375,9 @@ static bool rr_layout(int W, int w, int h, int C, const int *xstart, const int *
         if (BW / 4 > 256) return false;        // TMA box limit
         r->BW = BW;
         r->stage_stride = (uint32_t)(((size_t)r->NR * BW + 127) / 128 * 128);
-        r->smem = 2 * (size_t)r->stage_stride + ((size_t)2 * cx * C * r->NRp + 2 * r->NR) * sizeof(float) + 8 + 16 +
-                  (size_t)r->D * DXU * C;
+        const int nc = C == 4 ? 3 : C;         // chains per column
+        r->smem = 2 * (size_t)r->stage_stride + ((size_t)2 * cx * nc * r->NRp + 2 * r->NR) * sizeof(float) + 8 + 16 +
+                  (size_t)r->D * DXU * nc;
         return r->smem <= 200 * 1024;
     };
     const int forced = rr_env("FM_K0_CX", 0);
@@ -392,18 +406,21 @@ static int rr_build(fm_ctx *c, const void *kern, int w, int h, int C, const int 
     return fm_ensure_smem(kern, r->smem, c->cfg.device);
 }
 
-static int rr_channels(const fm_ctx *c) { return (c->cfg.flags & FM_FLAG_GRAY) ? 1 : 3; }
+// the instantiation of k_resize_rows for the context's pixel format
+template <bool BGR>
+static const void *rr_kernel(const fm_ctx *c) {
+    const void *k = nullptr;
+    fm_px_dispatch(c->px_bytes, c->rgb, [&](auto C, auto RGB) { k = (const void *)k_resize_rows<BGR, C.value, RGB.value>; });
+    return k;
+}
 
 // the processing plane (gray out) and the detector input plane (BGR out)
 int fm_rows_plan(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx) {
-    const int C = rr_channels(c);
-    return rr_build(c, C == 1 ? (const void *)k_resize_rows<false, 1> : (const void *)k_resize_rows<false, 3>, c->w, c->h, C,
-                    xstart, xidx, xwt, ystart, yidx, &c->rows);
+    return rr_build(c, rr_kernel<false>(c), c->w, c->h, c->px_bytes, xstart, xidx, xwt, ystart, yidx, &c->rows);
 }
 int fm_rows_plan_objects(fm_ctx *c, const int *xstart, const int *xidx, const float *xwt, const int *ystart, const int *yidx) {
-    const int C = rr_channels(c);
-    return rr_build(c, C == 1 ? (const void *)k_resize_rows<true, 1> : (const void *)k_resize_rows<true, 3>, FM_OBJECT_WIDTH,
-                    c->obj_h, C, xstart, xidx, xwt, ystart, yidx, &c->obj_rows);
+    return rr_build(c, rr_kernel<true>(c), FM_OBJECT_WIDTH, c->obj_h, c->px_bytes, xstart, xidx, xwt, ystart, yidx,
+                    &c->obj_rows);
 }
 
 // Plan of a geometry without a device (include/fm_gpu.h: fm_debug_rows_plan): the layout plus a re-check, tap by tap, that
@@ -423,7 +440,7 @@ int fm_rows_plan_describe(int W, int w, int h, int C, const int *xstart, const i
         const int ch = dx / r.CX, a = xstart[dx], nt = xstart[dx + 1] - a;
         const int4 ci = col[dx];
         out->max_groups = std::max(out->max_groups, ci.y);
-        if (4 * cstartw[ch] + ci.x != C * xidx[a] || (cstartw[ch] & 3) || ci.x < 0) { fm_set_error("rows plan: column %d misplaced", dx); return FM_ERANGE; }
+        if (4 * cstartw[ch] + ci.x != C * xidx[a] || (cstartw[ch] & 3) || ci.x < 0 || (C == 4 && (ci.x & 3))) { fm_set_error("rows plan: column %d misplaced", dx); return FM_ERANGE; }
         for (int g = 0; g < ci.y; g++)
             for (int i = 0; i < 4; i++) {
                 const float wv = (&rw[ci.z + 2 * g].x)[i], nv = (&rw[ci.z + 2 * g + 1].x)[i];
@@ -462,8 +479,9 @@ static int rr_launch(const fm_ctx *c, const RowsPlan *r, int w, int h, const Res
     p.gray = c->gray; p.nvalid = c->nvalid;
     p.oidx = c->obj_idx; p.out = out; p.ostride = ostride;
     dim3 grid(r->segs, r->nbands, c->S * T);
-    if (rr_channels(c) == 1) k_resize_rows<BGR, 1><<<grid, RR_THREADS + 32, r->smem, st>>>(tmap, p);
-    else k_resize_rows<BGR, 3><<<grid, RR_THREADS + 32, r->smem, st>>>(tmap, p);
+    fm_px_dispatch(c->px_bytes, c->rgb, [&](auto C, auto RGB) {
+        k_resize_rows<BGR, C.value, RGB.value><<<grid, RR_THREADS + 32, r->smem, st>>>(tmap, p);
+    });
     FM_LAUNCH_CHECK();
     return FM_OK;
 }

@@ -351,7 +351,8 @@ struct UfParams {
     int r;                      // kernel radius (k >> 1) <= RA
 };
 
-template <int RA, bool SAFE>
+// RGB: R-first frames (FM_FLAG_RGB)
+template <int RA, bool SAFE, bool RGB = false>
 __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_constant__ CUtensorMap tmap, UfParams q) {
     using G = UfGeom<RA>;
     const UmmaParams &p = q.u;
@@ -445,10 +446,10 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
                     const uint4 *src = reinterpret_cast<const uint4 *>(raw + rr * G::RB + 48 * uu);
                     const uint4 a = src[0], b = src[1], d = src[2];
                     uint4 o;
-                    o.x = fm_gray4(a.x, a.y, a.z);
-                    o.y = fm_gray4(a.w, b.x, b.y);
-                    o.z = fm_gray4(b.z, b.w, d.x);
-                    o.w = fm_gray4(d.y, d.z, d.w);
+                    o.x = fm_gray4<RGB>(a.x, a.y, a.z);
+                    o.y = fm_gray4<RGB>(a.w, b.x, b.y);
+                    o.z = fm_gray4<RGB>(b.z, b.w, d.x);
+                    o.w = fm_gray4<RGB>(d.y, d.z, d.w);
                     *reinterpret_cast<uint4 *>(sGray + (uu >> 3) * (G::IN * 128) + pr * 128 + (((uu & 7) ^ (pr & 7)) << 4)) = o;
                 }
             }
@@ -549,9 +550,10 @@ __global__ void __launch_bounds__(UB_THREADS, 1) k_umma_fused(const __grid_const
 // ---------------------------------------------------------------------------------------------
 // padded gray plane: gpad[f][yp][xp] = gray(reflect101(yp - 48), reflect101(xp - 48)); BGR: convert on the way
 // (find_motion.py:493, SURVEY.md A.2); otherwise src is a gray plane (the context's, or gray frames).  Frame (s, t) starts at
-// src + s * sstride + t * fstride, rows rpitch bytes apart.  One thread = 4 padded pixels.
+// src + s * sstride + t * fstride, rows rpitch bytes apart.  One thread = 4 padded pixels.  RGB: R-first frames; PX: bytes
+// per pixel of the frames (3, or 4 with FM_FLAG_ALPHA)
 // ---------------------------------------------------------------------------------------------
-template <bool BGR>
+template <bool BGR, bool RGB = false, int PX = 3>
 __global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ src, size_t sstride, size_t fstride, size_t rpitch, int T,
                                                   uint8_t *__restrict__ gpad, int w, int h, int Wp, int Hp,
                                                   const int *__restrict__ nvalid, int aligned4) {
@@ -566,8 +568,9 @@ __global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ sr
         const int x = xp - UB_PAD;
         if (x >= 0 && x + 3 < w && aligned4) {
             if (BGR) {
-                const uint32_t *q = reinterpret_cast<const uint32_t *>(row + 3 * x);
-                out = fm_gray4(__ldg(q), __ldg(q + 1), __ldg(q + 2));
+                const uint32_t *q = reinterpret_cast<const uint32_t *>(row + PX * x);
+                if constexpr (PX == 4) out = fm_gray4a<RGB>(make_uint4(__ldg(q), __ldg(q + 1), __ldg(q + 2), __ldg(q + 3)));
+                else out = fm_gray4<RGB>(__ldg(q), __ldg(q + 1), __ldg(q + 2));
             } else {
                 out = __ldg(reinterpret_cast<const uint32_t *>(row + x));
             }
@@ -576,7 +579,7 @@ __global__ void __launch_bounds__(256) k_pad_gray(const uint8_t *__restrict__ sr
             for (int b = 0; b < 4; b++) {
                 if (xp + b < w + 2 * UB_PAD) {
                     const int xx = fm_reflect101(x + b, w);
-                    out |= (BGR ? fm_gray(row[3 * xx], row[3 * xx + 1], row[3 * xx + 2]) : (uint32_t)row[xx]) << (8 * b);
+                    out |= (BGR ? fm_gray<RGB>(row[PX * xx], row[PX * xx + 1], row[PX * xx + 2]) : (uint32_t)row[xx]) << (8 * b);
                 }
             }
         }
@@ -637,11 +640,20 @@ static std::vector<uint8_t> make_band(const fm_ctx *c, const int *taps, int RA, 
     return band;
 }
 
-// the BGR frames can feed the tcgen05 kernel directly (TMA over the caller's frames, mirroring inside the tile); gray frames
-// take the apron plane, which k_pad_gray fills from them in place
+// the BGR (and RGB) frames can feed the tcgen05 kernel directly (TMA over the caller's frames, mirroring inside the tile);
+// gray and four-byte frames take the apron plane, which k_pad_gray fills from them in place
 static bool umma_fused_geometry(const fm_ctx *c) {
     const int r = c->k >> 1;
-    return c->resize_mode == 0 && (c->W % 16) == 0 && c->w >= r + 2 && c->h >= r + 2 && !(c->cfg.flags & FM_FLAG_GRAY);
+    return c->resize_mode == 0 && (c->W % 16) == 0 && c->w >= r + 2 && c->h >= r + 2 && c->px_bytes == 3;
+}
+
+template <bool RGB>
+static int umma_fused_smem(const fm_ctx *c) {
+    int rc;
+    if ((rc = fm_ensure_smem((const void *)k_umma_fused<16, true, RGB>, UfGeom<16>::SMEM, c->cfg.device))) return rc;
+    if ((rc = fm_ensure_smem((const void *)k_umma_fused<16, false, RGB>, UfGeom<16>::SMEM, c->cfg.device))) return rc;
+    if ((rc = fm_ensure_smem((const void *)k_umma_fused<48, true, RGB>, UfGeom<48>::SMEM, c->cfg.device))) return rc;
+    return fm_ensure_smem((const void *)k_umma_fused<48, false, RGB>, UfGeom<48>::SMEM, c->cfg.device);
 }
 
 int fm_umma_init(fm_ctx *c, const int *taps) {
@@ -657,10 +669,7 @@ int fm_umma_init(fm_ctx *c, const int *taps) {
                                 : make_band(c, taps, 48, UfGeom<48>::BROWS, UfGeom<48>::BOFF);
         FM_CUDA(cudaMalloc((void **)&c->uband_f, band.size()));
         FM_CUDA(cudaMemcpy(c->uband_f, band.data(), band.size(), cudaMemcpyHostToDevice));
-        if ((rc = fm_ensure_smem((const void *)k_umma_fused<16, true>, UfGeom<16>::SMEM, c->cfg.device))) return rc;
-        if ((rc = fm_ensure_smem((const void *)k_umma_fused<16, false>, UfGeom<16>::SMEM, c->cfg.device))) return rc;
-        if ((rc = fm_ensure_smem((const void *)k_umma_fused<48, true>, UfGeom<48>::SMEM, c->cfg.device))) return rc;
-        if ((rc = fm_ensure_smem((const void *)k_umma_fused<48, false>, UfGeom<48>::SMEM, c->cfg.device))) return rc;
+        if ((rc = c->rgb ? umma_fused_smem<true>(c) : umma_fused_smem<false>(c))) return rc;
     } else {
         FM_CUDA(cudaMalloc((void **)&c->gpad, fm_umma_pad_bytes(c)));      // apron plane of the resize modes
     }
@@ -700,7 +709,18 @@ extern "C" void fm_umma_prof_dump(void) {
     memset(b, 0, 32 * sizeof(long long));
 }
 
-// full-resolution mode, BGR frames straight into the tcgen05 kernel
+template <bool RGB>
+static void umma_fused_launch(int RA, bool safe, dim3 grid, cudaStream_t st, const CUtensorMap &tmap, const UfParams &q) {
+    if (RA == 16) {
+        if (safe) k_umma_fused<16, true, RGB><<<grid, UB_THREADS, UfGeom<16>::SMEM, st>>>(tmap, q);
+        else k_umma_fused<16, false, RGB><<<grid, UB_THREADS, UfGeom<16>::SMEM, st>>>(tmap, q);
+    } else {
+        if (safe) k_umma_fused<48, true, RGB><<<grid, UB_THREADS, UfGeom<48>::SMEM, st>>>(tmap, q);
+        else k_umma_fused<48, false, RGB><<<grid, UB_THREADS, UfGeom<48>::SMEM, st>>>(tmap, q);
+    }
+}
+
+// full-resolution mode, BGR (or RGB) frames straight into the tcgen05 kernel
 static int launch_umma_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
     int tilesX, tilesY, Wp, Hp;
     umma_geom(c, &tilesX, &tilesY, &Wp, &Hp);
@@ -718,13 +738,8 @@ static int launch_umma_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, s
     q.r = c->k >> 1;
     const bool safe = q.u.alpha >= 0.0 && q.u.alpha <= 1.0 && q.u.threshold >= 0;
     dim3 grid(tilesX * tilesY, c->S);
-    if (RA == 16) {
-        if (safe) k_umma_fused<16, true><<<grid, UB_THREADS, UfGeom<16>::SMEM, st>>>(tmap, q);
-        else k_umma_fused<16, false><<<grid, UB_THREADS, UfGeom<16>::SMEM, st>>>(tmap, q);
-    } else {
-        if (safe) k_umma_fused<48, true><<<grid, UB_THREADS, UfGeom<48>::SMEM, st>>>(tmap, q);
-        else k_umma_fused<48, false><<<grid, UB_THREADS, UfGeom<48>::SMEM, st>>>(tmap, q);
-    }
+    if (c->rgb) umma_fused_launch<true>(RA, safe, grid, st, tmap, q);
+    else umma_fused_launch<false>(RA, safe, grid, st, tmap, q);
     FM_LAUNCH_CHECK();
     return FM_OK;
 }
@@ -732,7 +747,7 @@ static int launch_umma_fused(fm_ctx *c, const uint8_t *frames, size_t sstride, s
 // frames != nullptr: full-resolution mode (BGR -> padded gray in one kernel); else the resized gray plane c->gray.  Pitched
 // rows that TMA cannot read (not 16-byte aligned) take the apron plane; packed ones keep the direct kernel's refusal.
 int fm_launch_umma_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
-    const bool tma_ok = pitch == (size_t)c->W * 3 || ((((uintptr_t)frames) | sstride | fstride | pitch) & 15) == 0;
+    const bool tma_ok = pitch == (size_t)c->W * c->px_bytes || ((((uintptr_t)frames) | sstride | fstride | pitch) & 15) == 0;
     if (frames && c->umma_direct && !(c->cfg.flags & FM_FLAG_UMMA_APRON) && tma_ok)
         return launch_umma_fused(c, frames, sstride, fstride, pitch, T, st);
     if (!c->gpad) {                     // first call that needs the apron plane (A/B flag on a direct-capable context)
@@ -743,16 +758,20 @@ int fm_launch_umma_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t
     umma_geom(c, &tilesX, &tilesY, &Wp, &Hp);
     const int F = c->S * T;
     dim3 pgrid((Wp / 4 + 255) / 256, Hp, F);
-    const bool gray_in = frames && (c->cfg.flags & FM_FLAG_GRAY);
+    const bool gray_in = frames && c->px_bytes == 1;
     if (frames && (c->cfg.flags & FM_FLAG_KEEP_PLANES)) {      // parity tap of the gray conversion (gray frames: a copy)
         int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
         if (rc) return rc;
     }
     if (frames && !gray_in) {
-        const int al = ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->w * 3)) & 3) == 0;
-        k_pad_gray<true><<<pgrid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->gpad, c->w, c->h, Wp, Hp, c->nvalid, al);
+        const int al = ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->W * c->px_bytes)) & 3) == 0;
+        fm_px_dispatch(c->px_bytes, c->rgb, [&](auto Cx, auto RGB) {
+            constexpr int P = Cx.value == 4 ? 4 : 3;
+            k_pad_gray<true, RGB.value, P><<<pgrid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->gpad, c->w, c->h, Wp, Hp,
+                                                                  c->nvalid, al);
+        });
     } else if (gray_in) {
-        const int al = ((((uintptr_t)frames) | sstride | fstride | pitch | (size_t)c->w) & 3) == 0;
+        const int al = ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->W * c->px_bytes)) & 3) == 0;
         k_pad_gray<false><<<pgrid, 256, 0, st>>>(frames, sstride, fstride, pitch, T, c->gpad, c->w, c->h, Wp, Hp, c->nvalid, al);
     } else {
         const int al = (c->w & 3) == 0;

@@ -62,7 +62,8 @@ __device__ __forceinline__ void up_hrow(const UpParams &p, const uint8_t *__rest
     }
 }
 
-template <int C>
+// RGB: R-first three-byte source pixels; their channels are put in BGR order as they leave the vertical pass
+template <int C, bool RGB = false>
 __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int f = blockIdx.y;                    // s*T + t
@@ -113,10 +114,10 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
                     h1[i] = r1[4 * C * q + ii];
                 }
             }
-            uint32_t v[12];                              // 4 pixels x 3 channels (a gray source: its byte in all three)
+            uint32_t v[12];                              // 4 pixels x 3 channels, BGR (a gray source: its byte in all three)
 #pragma unroll
             for (int i = 0; i < 12; i++) {
-                const int k = C == 1 ? i / 3 : i;
+                const int k = C == 1 ? i / 3 : C == 4 ? 4 * (i / 3) + (RGB ? 2 - i % 3 : i % 3) : RGB ? i + 2 - 2 * (i % 3) : i;
                 v[i] = min((((b0 * h0[k]) >> 16) + ((b1 * h1[k]) >> 16) + 2u) >> 2, 255u);
             }
             if (p.bgr_out) {
@@ -147,11 +148,13 @@ __global__ void __launch_bounds__(UP_THREADS) k_upscale_gray(UpParams p) {
     }
 }
 
-size_t fm_upscale_smem(int w) { return (size_t)2 * ((3 * (size_t)w + 3) & ~(size_t)3) * sizeof(uint16_t); }
+size_t fm_upscale_smem(int w, int channels) {
+    return (size_t)2 * (((size_t)(channels > 3 ? channels : 3) * w + 3) & ~(size_t)3) * sizeof(uint16_t);
+}
 
 int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, int F, int W, int H,
                       int w, int h, const int2 *xt, const int2 *yt, const int *nvalid, uint8_t *gray, uint8_t *bgr_out,
-                      const int *oidx, size_t ostride, cudaStream_t st, int channels) {
+                      const int *oidx, size_t ostride, cudaStream_t st, int channels, bool rgb) {
     UpParams p;
     p.frames = frames; p.sstride = sstride; p.fstride = fstride; p.pitch = pitch;
     p.T = T; p.W = W; p.H = H; p.w = w; p.h = h;
@@ -161,17 +164,19 @@ int fm_launch_upscale(int device, const uint8_t *frames, size_t sstride, size_t 
     int band = UP_BAND_MAX;
     while (band > 4 && (size_t)((h + band - 1) / band) * F < 4 * 148) band >>= 1;
     p.band = band;
-    const size_t smem = fm_upscale_smem(w);
+    const size_t smem = fm_upscale_smem(w, channels);
     if (smem > 200 * 1024) {
         fm_set_error("upscale needs %zu bytes of shared memory (destination width %d too large)", smem, w);
         return FM_ERANGE;
     }
     int rc;
-    if ((rc = fm_ensure_smem(channels == 1 ? (const void *)k_upscale_gray<1> : (const void *)k_upscale_gray<3>, smem, device)))
-        return rc;
     dim3 grid((h + band - 1) / band, F);
-    if (channels == 1) k_upscale_gray<1><<<grid, UP_THREADS, smem, st>>>(p);
-    else k_upscale_gray<3><<<grid, UP_THREADS, smem, st>>>(p);
+    rc = FM_OK;
+    fm_px_dispatch(channels, rgb, [&](auto C, auto RGB) {
+        if ((rc = fm_ensure_smem((const void *)k_upscale_gray<C.value, RGB.value>, smem, device))) return;
+        k_upscale_gray<C.value, RGB.value><<<grid, UP_THREADS, smem, st>>>(p);
+    });
+    if (rc) return rc;
     FM_LAUNCH_CHECK();
     return FM_OK;
 }

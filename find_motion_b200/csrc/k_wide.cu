@@ -138,14 +138,15 @@ __device__ __forceinline__ void wide_h_mirror(unsigned char *tile, int X0, int w
 }
 
 // ---- pass 1, step A: stage the gray window of a CTA (shared column cc <-> image column X0 - R16 + cc, reflected; row rr <->
-// padded row 32 G + rr) with register-staged global loads.  BGR: the BGR -> gray conversion is fused in. ----
-template <bool BGR>
+// padded row 32 G + rr) with register-staged global loads.  BGR: the BGR -> gray conversion is fused in (RGB: R-first
+// pixels; PX = 4: four-byte BGRA / RGBA pixels). ----
+template <bool BGR, bool RGB = false, int PX = 3>
 __device__ __forceinline__ void wide_h_stage(unsigned char *tile, const uint8_t *__restrict__ src, size_t sstride, size_t fstride,
                                              size_t rpitch, int T, int f, int G, int X0, int w, int h, int r, int R16, int pitch) {
     const int tid = threadIdx.x, lane = tid & 31, wq = tid >> 5;
     if (BGR) {
-        // warp wq: rows wq, wq+8, wq+16, wq+24; lane: a unit of 16 pixels = 48 BGR bytes (three 128-bit loads); the
-        // loads of the four rows are issued before the first conversion
+        // warp wq: rows wq, wq+8, wq+16, wq+24; lane: a unit of 16 pixels = 48 BGR bytes (three 128-bit loads; PX = 4:
+        // 64 bytes, four); the loads of the four rows are issued before the first conversion
         const uint8_t *fr = src + (size_t)(f / T) * sstride + (size_t)(f % T) * fstride;
         const uint8_t *rp[4];
 #pragma unroll
@@ -157,27 +158,35 @@ __device__ __forceinline__ void wide_h_stage(unsigned char *tile, const uint8_t 
             const int x = X0 - R16 + 16 * u;
             if (x >= xneed) continue;
             if (x >= 0 && x + 15 < w) {
-                uint4 raw[4][3];
+                uint4 raw[4][PX];
 #pragma unroll
                 for (int i = 0; i < 4; i++) {
-                    const uint4 *q = reinterpret_cast<const uint4 *>(rp[i] + 3 * x);
-                    raw[i][0] = __ldg(q); raw[i][1] = __ldg(q + 1); raw[i][2] = __ldg(q + 2);
+                    const uint4 *q = reinterpret_cast<const uint4 *>(rp[i] + PX * x);
+#pragma unroll
+                    for (int k = 0; k < PX; k++) raw[i][k] = __ldg(q + k);
                 }
 #pragma unroll
                 for (int i = 0; i < 4; i++) {
                     uint4 o;
-                    o.x = fm_gray4(raw[i][0].x, raw[i][0].y, raw[i][0].z);
-                    o.y = fm_gray4(raw[i][0].w, raw[i][1].x, raw[i][1].y);
-                    o.z = fm_gray4(raw[i][1].z, raw[i][1].w, raw[i][2].x);
-                    o.w = fm_gray4(raw[i][2].y, raw[i][2].z, raw[i][2].w);
+                    if constexpr (PX == 4) {
+                        o = make_uint4(fm_gray4a<RGB>(raw[i][0]), fm_gray4a<RGB>(raw[i][1]), fm_gray4a<RGB>(raw[i][2]),
+                                       fm_gray4a<RGB>(raw[i][3]));
+                    } else {
+                        o.x = fm_gray4<RGB>(raw[i][0].x, raw[i][0].y, raw[i][0].z);
+                        o.y = fm_gray4<RGB>(raw[i][0].w, raw[i][1].x, raw[i][1].y);
+                        o.z = fm_gray4<RGB>(raw[i][1].z, raw[i][1].w, raw[i][2].x);
+                        o.w = fm_gray4<RGB>(raw[i][2].y, raw[i][2].z, raw[i][2].w);
+                    }
                     *reinterpret_cast<uint4 *>(tile + (wq + 8 * i) * pitch + 16 * u) = o;
                 }
-            } else if (!mirror) {
+            } else if (!mirror || (PX == 4 && x >= 0 && x < w)) {
+                // PX = 4: rows of 4 W bytes are 16-byte aligned for any W % 4 == 0, so the last unit may straddle the right
+                // edge (three-byte rows are aligned only for W % 16 == 0); its columns inside the image are staged here
 #pragma unroll 1
                 for (int b = 0; b < 16; b++) {
-                    const int xx = 3 * fm_reflect101(x + b, w);
+                    const int xx = PX * fm_reflect101(x + b, w);
 #pragma unroll
-                    for (int i = 0; i < 4; i++) tile[(wq + 8 * i) * pitch + 16 * u + b] = (unsigned char)fm_gray(rp[i][xx], rp[i][xx + 1], rp[i][xx + 2]);
+                    for (int i = 0; i < 4; i++) tile[(wq + 8 * i) * pitch + 16 * u + b] = (unsigned char)fm_gray<RGB>(rp[i][xx], rp[i][xx + 1], rp[i][xx + 2]);
                 }
             }
         }
@@ -254,8 +263,9 @@ __device__ __forceinline__ void wide_h_products(const unsigned char *tile, const
 
 // grid: (ceil(w / 256), NGa, F), 256 threads.  dynamic smem: 32 * pitch + (4 Sh + 3) * 256
 // BGR: src = the caller's frames (identity resize, 16-byte aligned rows rpitch bytes apart); otherwise src = a gray plane, rows
-// rpitch bytes apart (the context's [F][h][w], or the caller's gray frames with FM_FLAG_GRAY).
-template <bool BGR>
+// rpitch bytes apart (the context's [F][h][w], or the caller's gray frames with FM_FLAG_GRAY).  RGB: R-first frames; PX:
+// bytes per pixel of the frames (3, or 4 with FM_FLAG_ALPHA)
+template <bool BGR, bool RGB = false, int PX = 3>
 __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h(const uint8_t *__restrict__ src, size_t sstride, size_t fstride,
                                                        size_t rpitch, int T,
                                                        uint32_t *__restrict__ plo, uint32_t *__restrict__ phi,
@@ -268,7 +278,7 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h(const uint8_t *__restr
     const int f = blockIdx.z, G = blockIdx.y, X0 = blockIdx.x * WH_COLS;
     if (f % T >= __ldg(nvalid + f / T)) return;                             // not a real frame of this (ragged) call
     for (int i = tid; i < (4 * Sh + 3) * 32; i += WH_THREADS) tab[i] = __ldg(tabg + i);
-    wide_h_stage<BGR>(tile, src, sstride, fstride, rpitch, T, f, G, X0, w, h, r, R16, pitch);
+    wide_h_stage<BGR, RGB, PX>(tile, src, sstride, fstride, rpitch, T, f, G, X0, w, h, r, R16, pitch);
     __syncthreads();
     wide_h_products(tile, tab, f, G, X0, w, Sh, pitch, NGa, plo, phi);
 }
@@ -277,7 +287,9 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h(const uint8_t *__restr
 // boxes of 32 rows x (ubox units of 16 pixels = 48 bytes) for the whole CTA, every lane then converts units out of shared memory
 // (no per-thread global addresses, no idle lanes: 22 units per row at k = 97 left 10 of 32 lanes without work above).  Row groups
 // that touch the top or bottom border need reflected rows and take the register-staged path.
-// dynamic smem: nbox * 32 * ubox * 48 (raw BGR)  +  32 * pitch  +  (4 Sh + 3) * 256  +  16
+// dynamic smem: nbox * 32 * ubox * 16 PX (raw pixels)  +  32 * pitch  +  (4 Sh + 3) * 256  +  16.  RGB: R-first frames; PX:
+// bytes per pixel (3, or 4 with FM_FLAG_ALPHA: a unit of 16 pixels is four 16-byte words, each one gray word)
+template <bool RGB = false, int PX = 3>
 __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_constant__ CUtensorMap tmap, const uint8_t *__restrict__ src,
                                                            size_t sstride, size_t fstride, size_t rpitch, int T,
                                                            uint32_t *__restrict__ plo,
@@ -285,7 +297,8 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_const
                                                            int r, int R16, int Sh, int pitch, int NGa,
                                                            const int *__restrict__ nvalid, int nunits, int ubox, int nbox, int gp) {
     extern __shared__ __align__(128) unsigned char wsmt[];
-    const int boxbytes = 32 * ubox * 48;                                     // a multiple of 128
+    constexpr int UB = 16 * PX;                                              // bytes of a unit of 16 pixels
+    const int boxbytes = 32 * ubox * UB;                                     // a multiple of 128
     unsigned char *raw = wsmt;                                               // [nbox][32][ubox * 48] staged BGR rows
     unsigned char *tile = raw + nbox * boxbytes;                             // [32][pitch] gray bytes
     uint2 *tab = reinterpret_cast<uint2 *>(tile + 32 * pitch);              // [4 Sh + 3][32]
@@ -299,8 +312,8 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_const
     auto interior = [&](int G) { return 32 * G - r >= 0 && 32 * G - r + 32 <= h; };    // CTA-uniform
     auto issue = [&](int G) {                  // one thread
         fm_mbar_expect_tx(bar, (uint32_t)(nbox * boxbytes));
-        const int c0 = (3 * (X0 - R16)) / 4;                                 // u32 column (negative / past the row: zero-filled)
-        for (int b = 0; b < nbox; b++) fm_tma_load_4d(fm_smem_u32(raw) + b * boxbytes, &tmap, bar, c0 + b * ubox * 12, 32 * G - r, f % T, f / T);
+        const int c0 = (PX * (X0 - R16)) / 4;                                // u32 column (negative / past the row: zero-filled)
+        for (int b = 0; b < nbox; b++) fm_tma_load_4d(fm_smem_u32(raw) + b * boxbytes, &tmap, bar, c0 + b * ubox * (UB / 4), 32 * G - r, f % T, f / T);
     };
     if (tid == 0) {
         fm_mbar_init(bar, 1);
@@ -323,13 +336,17 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_const
                 const int x = X0 - R16 + 16 * j;
                 if (x < 0 || x >= w || x >= xneed) continue;                 // border columns come from their mirror images below
                 const int jb = j >= ubox ? 1 : 0;
-                const uint4 *q = reinterpret_cast<const uint4 *>(raw + jb * boxbytes + rr * (ubox * 48) + (j - jb * ubox) * 48);
-                const uint4 r0 = q[0], r1 = q[1], r2 = q[2];
+                const uint4 *q = reinterpret_cast<const uint4 *>(raw + jb * boxbytes + rr * (ubox * UB) + (j - jb * ubox) * UB);
                 uint4 o;
-                o.x = fm_gray4(r0.x, r0.y, r0.z);
-                o.y = fm_gray4(r0.w, r1.x, r1.y);
-                o.z = fm_gray4(r1.z, r1.w, r2.x);
-                o.w = fm_gray4(r2.y, r2.z, r2.w);
+                if constexpr (PX == 4) {
+                    o = make_uint4(fm_gray4a<RGB>(q[0]), fm_gray4a<RGB>(q[1]), fm_gray4a<RGB>(q[2]), fm_gray4a<RGB>(q[3]));
+                } else {
+                    const uint4 r0 = q[0], r1 = q[1], r2 = q[2];
+                    o.x = fm_gray4<RGB>(r0.x, r0.y, r0.z);
+                    o.y = fm_gray4<RGB>(r0.w, r1.x, r1.y);
+                    o.z = fm_gray4<RGB>(r1.z, r1.w, r2.x);
+                    o.w = fm_gray4<RGB>(r2.y, r2.z, r2.w);
+                }
                 *reinterpret_cast<uint4 *>(tile + rr * pitch + 16 * j) = o;
             }
             __syncthreads();                                                 // raw stage consumed, window written
@@ -339,7 +356,7 @@ __global__ void __launch_bounds__(WH_THREADS, 4) k_wide_h_tma(const __grid_const
                 __syncthreads();
             }
         } else {
-            wide_h_stage<true>(tile, src, sstride, fstride, rpitch, T, f, G, X0, w, h, r, R16, pitch);
+            wide_h_stage<true, RGB, PX>(tile, src, sstride, fstride, rpitch, T, f, G, X0, w, h, r, R16, pitch);
             __syncthreads();
             if (more && tid == 0) issue(G + 1);                              // the raw stage is not in use
         }
@@ -697,7 +714,7 @@ __global__ void __launch_bounds__(256) k_blur_identity(const uint8_t *__restrict
 int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t fstride, size_t pitch, int T, cudaStream_t st) {
     const uint8_t *gsrc = c->gray;                                   // the gray plane the passes read, and its layout
     size_t gsstride = (size_t)T * c->N, gfstride = c->N, gpitch = c->w;
-    if (frames && (c->cfg.flags & FM_FLAG_GRAY)) {
+    if (frames && c->px_bytes == 1) {
         if (c->cfg.flags & FM_FLAG_KEEP_PLANES) {
             int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
             if (rc) return rc;
@@ -725,35 +742,43 @@ int fm_launch_wide_blur(fm_ctx *c, const uint8_t *frames, size_t sstride, size_t
     const size_t smh = (size_t)32 * g.pitch + (size_t)(4 * g.Sh + 3) * 256;
     const size_t smv = (size_t)4 * (4 + g.Sv - 1) * 2 * WV_COLS * 16 + (size_t)2 * g.Sv * 512;
     int rc;
-    if ((rc = fm_ensure_smem((const void *)k_wide_h<true>, smh, c->cfg.device))) return rc;
     if ((rc = fm_ensure_smem((const void *)k_wide_h<false>, smh, c->cfg.device))) return rc;
     if ((rc = fm_ensure_smem((const void *)k_wide_v, smv, c->cfg.device))) return rc;
     dim3 hgrid((c->w + WH_COLS - 1) / WH_COLS, g.NGa, F);
-    const bool aligned16 = frames && ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->w * 3)) & 15) == 0;
+    const bool aligned16 = frames && ((((uintptr_t)frames) | sstride | fstride | pitch | ((size_t)c->W * c->px_bytes)) & 15) == 0;
     if (aligned16) {
         if (c->cfg.flags & FM_FLAG_KEEP_PLANES) {
             int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);
             if (rc) return rc;
         }
         // TMA-staged pass 1 when the window of a CTA is one or two boxes and the CTA needs <= 100 KB (k <= ~200 at 1080p / 4K: k = 97 runs four CTAs
-        // per SM, k = 193 three; measured against the register-staged path in profiles/r2_wide_ab.txt)
+        // per SM, k = 193 three; measured against the register-staged path in profiles/r2_wide_ab.txt).  A box row is at
+        // most 256 words: 21 units of 16 three-byte pixels, 16 of four-byte ones
+        const int PX = c->px_bytes, umax = PX == 4 ? 16 : 21;
         const bool mirror = g.R16 < c->w && g.R16 + g.r < WH_COLS;
         const int nunits = (g.R16 + WH_COLS + g.r + 15) / 16;
-        const int nbox = nunits > 21 ? 2 : 1, ubox = (nunits + nbox - 1) / nbox;
-        const size_t smt = (size_t)nbox * 32 * ubox * 48 + smh + 16;
+        const int nbox = nunits > umax ? 2 : 1, ubox = (nunits + nbox - 1) / nbox;
+        const size_t smt = (size_t)nbox * 32 * ubox * 16 * PX + smh + 16;
         static const long tma_kb = getenv("FM_WIDE_TMA_KB") ? atol(getenv("FM_WIDE_TMA_KB")) : 100;
-        if (mirror && ubox <= 21 && smt <= (size_t)tma_kb * 1024) {
-            CUtensorMap tmap;
-            if ((rc = fm_frames_tmap(c, frames, sstride, fstride, pitch, T, ubox * 12, 32, &tmap))) return rc;
-            if ((rc = fm_ensure_smem((const void *)k_wide_h_tma, smt, c->cfg.device))) return rc;
-            static const int gp = getenv("FM_WIDE_GP") ? std::max(1, atoi(getenv("FM_WIDE_GP"))) : 4;     // row groups per CTA (A/B: profiles/r2_wide_ab.txt)
-            dim3 tgrid(hgrid.x, (g.NGa + gp - 1) / gp, F);
-            k_wide_h_tma<<<tgrid, WH_THREADS, smt, st>>>(tmap, frames, sstride, fstride, pitch, T, plo, phi, tabh, c->w, c->h, g.r, g.R16,
-                                                         g.Sh, g.pitch, g.NGa, c->nvalid, nunits, ubox, nbox, gp);
-        } else {
-            k_wide_h<true><<<hgrid, WH_THREADS, smh, st>>>(frames, sstride, fstride, pitch, T, plo, phi, tabh, c->w, c->h, g.r, g.R16,
-                                                           g.Sh, g.pitch, g.NGa, c->nvalid);
-        }
+        const bool tma = mirror && ubox <= umax && smt <= (size_t)tma_kb * 1024;
+        CUtensorMap tmap;
+        if (tma && (rc = fm_frames_tmap(c, frames, sstride, fstride, pitch, T, ubox * 4 * PX, 32, &tmap))) return rc;
+        static const int gp = getenv("FM_WIDE_GP") ? std::max(1, atoi(getenv("FM_WIDE_GP"))) : 4;     // row groups per CTA (A/B: profiles/r2_wide_ab.txt)
+        fm_px_dispatch(c->px_bytes, c->rgb, [&](auto Cx, auto RGB) {
+            constexpr int P = Cx.value == 4 ? 4 : 3;
+            if (tma) {
+                if ((rc = fm_ensure_smem((const void *)k_wide_h_tma<RGB.value, P>, smt, c->cfg.device))) return;
+                dim3 tgrid(hgrid.x, (g.NGa + gp - 1) / gp, F);
+                k_wide_h_tma<RGB.value, P><<<tgrid, WH_THREADS, smt, st>>>(tmap, frames, sstride, fstride, pitch, T, plo, phi, tabh,
+                                                                           c->w, c->h, g.r, g.R16, g.Sh, g.pitch, g.NGa, c->nvalid,
+                                                                           nunits, ubox, nbox, gp);
+            } else {
+                if ((rc = fm_ensure_smem((const void *)k_wide_h<true, RGB.value, P>, smh, c->cfg.device))) return;
+                k_wide_h<true, RGB.value, P><<<hgrid, WH_THREADS, smh, st>>>(frames, sstride, fstride, pitch, T, plo, phi, tabh, c->w,
+                                                                             c->h, g.r, g.R16, g.Sh, g.pitch, g.NGa, c->nvalid);
+            }
+        });
+        if (rc) return rc;
     } else {
         if (frames) {
             int rc = fm_launch_gray_plane(c, frames, sstride, fstride, pitch, T, st);

@@ -20,7 +20,7 @@ class MotionEngine:
     def __init__(self, frame_width, frame_height, n_streams=1, max_frames=8, device=0, fps=30, box_size=100,
                  min_box_scale=50, cache_time=2.0, min_time=0.5, threshold=7, avg=0.1, blur_scale=20,
                  mask_areas=None, max_components=256, keep_planes=False, no_fused=False, no_umma=False, umma_apron=False, umma=False, no_rows=False,
-                 upscale=False, device_clips=False, nv12=False, object_planes=False, gray=False):
+                 upscale=False, device_clips=False, nv12=False, object_planes=False, gray=False, rgb=False, alpha=False):
         """upscale: accept box_size > frame_width (cv2's INTER_AREA upscale, bit-exact, as imutils.resize does it);
         without it such a geometry raises, as in earlier releases.
         device_clips: keep the look-back cache of raw frames on the GPU (n_streams x cache_frames frames) so that
@@ -35,7 +35,14 @@ class MotionEngine:
         a BGR engine on cv2.cvtColor(frame, cv2.COLOR_GRAY2BGR) and a third of the bytes per frame (at full resolution
         with a Gaussian wider than 5 taps the device path is slower than BGR input: INTEGRATION.md).  process,
         process_clip, submit_host and process_host then take [S, T, H, W], and the clips are gray frames too; the
-        object planes stay [oh, 300, 3].  Not together with nv12."""
+        object planes stay [oh, 300, 3].  Not together with nv12.
+        rgb: the frames are RGB, [H, W, 3] uint8 with R first (DALI, PIL, PyAV rgb24, torchvision.io.read_video), read in
+        place with the results of a BGR engine on cv2.cvtColor(frame, cv2.COLOR_RGB2BGR).  The clips are the caller's
+        RGB frames; the object planes stay BGR.  Not together with nv12 or gray.
+        alpha: four bytes a pixel, [H, W, 4] uint8: B, G, R, A (with rgb: R, G, B, A), as DeepStream, graphics interop and
+        desktop capture deliver them, read in place with the results of a BGR engine on cv2.cvtColor(frame,
+        COLOR_BGRA2BGR) (COLOR_RGBA2BGR); the fourth byte never affects a result.  The clips are the caller's four-byte
+        frames; the object planes stay BGR.  Not together with nv12 or gray."""
         self._lib = _lib.load()
         self._ctx = C.c_void_p()
         cfg = _lib.fm_config(
@@ -47,15 +54,16 @@ class MotionEngine:
             (_lib.FLAG_NO_UMMA if no_umma else 0) | (_lib.FLAG_UMMA_APRON if umma_apron else 0) | (_lib.FLAG_UMMA if umma else 0) |
             (_lib.FLAG_NO_ROWS if no_rows else 0) | (_lib.FLAG_UPSCALE if upscale else 0) |
             (_lib.FLAG_DEVICE_CLIPS if device_clips else 0) | (_lib.FLAG_NV12 if nv12 else 0) |
-            (_lib.FLAG_OBJECT_PLANES if object_planes else 0) | (_lib.FLAG_GRAY if gray else 0))
+            (_lib.FLAG_OBJECT_PLANES if object_planes else 0) | (_lib.FLAG_GRAY if gray else 0) |
+            (_lib.FLAG_RGB if rgb else 0) | (_lib.FLAG_ALPHA if alpha else 0))
         _lib.check(self._lib.fm_ctx_create(C.byref(cfg), C.byref(self._ctx)))
         self.device = device
         self.n_streams, self.max_frames = n_streams, max_frames
         self.W, self.H = frame_width, frame_height
-        self.nv12, self.gray = bool(nv12), bool(gray)
+        self.nv12, self.gray, self.rgb, self.alpha = bool(nv12), bool(gray), bool(rgb), bool(alpha)
         # shape of one input frame
         self.frame_shape = (frame_height * 3 // 2, frame_width) if nv12 else \
-            (frame_height, frame_width) if gray else (frame_height, frame_width, 3)
+            (frame_height, frame_width) if gray else (frame_height, frame_width, 4 if alpha else 3)
         inf = _lib.fm_info()
         _lib.check(self._lib.fm_ctx_info(self._ctx, C.byref(inf)))
         self.info = {f: getattr(inf, f) for f, _ in _lib.fm_info._fields_}
@@ -143,13 +151,14 @@ class MotionEngine:
         S, T = self._check_batch(frames.shape)
         if frames[0, 0].is_contiguous():
             return S, T, None
-        row = self.W if self.nv12 or self.gray else 3 * self.W
-        assert frames.stride(-1) == 1 and (self.nv12 or self.gray or frames.stride(-2) == 3) and \
+        px = 1 if self.nv12 or self.gray else self.frame_shape[-1]
+        row = px * self.W
+        assert frames.stride(-1) == 1 and (px == 1 or frames.stride(-2) == px) and \
             frames.stride(2) >= row, "frames: unit byte stride, packed pixels and rows of at least the row bytes"
         return S, T, _lib.fm_frames(frames.data_ptr(), frames.stride(0), frames.stride(1), frames.stride(2), 0)
 
     def process(self, frames, sync=True, n_valid=None, chroma=None):
-        """frames: CUDA uint8 tensor [n_streams, T, H, W, 3] (BGR; nv12: [n_streams, T, H * 3 // 2, W]; gray:
+        """frames: CUDA uint8 tensor [n_streams, T, H, W, 3] (BGR, or RGB with rgb; [..., 4] with alpha; nv12: [n_streams, T, H * 3 // 2, W]; gray:
         [n_streams, T, H, W]).  Returns the
         per-frame stats as a structured numpy array [n_streams, T] (or the device tensor if sync=False).
         n_valid: optional per-stream count of real frames in this call (ragged batch).
@@ -221,7 +230,7 @@ class MotionEngine:
         """The input planes of the reference's find_objects (find_motion.py:572, 703-706) for the frames the last
         process / process_clip call wrote (needs object_planes=True): cv2.resize(raw, (300, oh), INTER_AREA) of each,
         bit-exact, made on the GPU from that call's frames (which must still hold them).  NV12 engines resize
-        cv2.cvtColor(frame, COLOR_YUV2BGR_NV12), gray engines cv2.cvtColor(frame, COLOR_GRAY2BGR).  out: optional CUDA uint8 tensor [n_streams, >= T, *object_shape]; by
+        cv2.cvtColor(frame, COLOR_YUV2BGR_NV12), gray engines cv2.cvtColor(frame, COLOR_GRAY2BGR), RGB engines cv2.cvtColor(frame, COLOR_RGB2BGR).  out: optional CUDA uint8 tensor [n_streams, >= T, *object_shape]; by
         default one of [n_streams, max_frames, *object_shape] is allocated once and reused, so the views returned by one
         call are overwritten by the next.  Runs on the current torch stream and synchronises.
         Returns, per stream, (frame_indices, planes): the indices t of the written frames in the call, in order, and a

@@ -95,6 +95,22 @@ typedef struct fm_config {
                                    the clips hold gray frames of W*H bytes; fm_object_planes keeps its oh x 300 x 3 planes
                                    (the one-channel resize stored in B, G and R).  FM_FLAG_GRAY | FM_FLAG_NV12 is refused with
                                    FM_EINVAL before any device query */
+#define FM_FLAG_RGB         4096 /* the frames are packed RGB, 3 bytes a pixel in the order R, G, B, as PyTorch-side decoders
+                                   (DALI, PIL, PyAV rgb24, torchvision.io.read_video) hand them out.  Results are exactly those
+                                   of a BGR context on cv2.cvtColor(frame, COLOR_RGB2BGR): every stats field, component, tap
+                                   and the background.  Every front end reads the pixels in place (no channel flip).  With
+                                   FM_FLAG_DEVICE_CLIPS the ring and the clips hold the caller's RGB frames byte for byte;
+                                   fm_object_planes keeps its oh x 300 x 3 BGR planes.  Strides and row_pitch keep their
+                                   meaning in bytes (row_pitch >= W*3); fm_frames.uv_offset must be 0.  FM_FLAG_RGB together
+                                   with FM_FLAG_NV12 or FM_FLAG_GRAY is refused with FM_EINVAL before any device query */
+#define FM_FLAG_ALPHA       8192 /* four bytes a pixel: B, G, R, A (with FM_FLAG_RGB: R, G, B, A), as DeepStream's NvBufSurface,
+                                   CUDA-OpenGL/Vulkan interop textures and desktop capture deliver them.  Results are exactly
+                                   those of a BGR context on cv2.cvtColor(frame, COLOR_BGRA2BGR) (COLOR_RGBA2BGR); the fourth
+                                   byte never affects a result.  Every entry point that takes frames reads W*H*4 bytes per
+                                   frame; row_pitch >= W*4; fm_frames.uv_offset must be 0.  With FM_FLAG_DEVICE_CLIPS the ring
+                                   and the clips hold the caller's four-byte frames byte for byte, alpha included;
+                                   fm_object_planes keeps its oh x 300 x 3 BGR planes.  Together with FM_FLAG_NV12 or
+                                   FM_FLAG_GRAY it is refused with FM_EINVAL before any device query */
 #define FM_OBJECT_WIDTH 300     /* width of the detector input plane (find_motion.py:703-706 hard-codes it) */
 
 /* Derived parameters, exactly as the reference computes them (SURVEY.md A.0). */
@@ -151,7 +167,7 @@ int fm_version(void);
  * (find_motion.py:299-380, 402-424, 478-484) for n_streams streams.  box_size > frame_width (a processing plane larger
  * than the frame, which imutils.resize produces with cv2's INTER_AREA upscale) needs FM_FLAG_UPSCALE; without it
  * fm_ctx_create returns FM_ERANGE.  So does an odd frame width or height with FM_FLAG_NV12.  FM_FLAG_GRAY together with
- * FM_FLAG_NV12 returns FM_EINVAL.  These checks come before any device query. */
+ * FM_FLAG_NV12, and FM_FLAG_RGB or FM_FLAG_ALPHA together with either, return FM_EINVAL.  These checks come before any device query. */
 int fm_ctx_create(const fm_config *cfg, fm_ctx **out);
 int fm_ctx_destroy(fm_ctx *ctx);
 int fm_ctx_info(const fm_ctx *ctx, fm_info *info);
@@ -169,7 +185,8 @@ int fm_ctx_reset(fm_ctx *ctx, int stream);
 /* The hot path: for every stream s < n_streams and t < n_frames (in order), run
  * blur_frame -> mask_off_areas -> find_diff -> find_movement -> decide_output on the BGR frame
  *   frames + s * stream_stride + t * frame_stride          (H*W*3 bytes, HWC, uint8; FM_FLAG_NV12: H*W*3/2 bytes NV12;
- *                                                           FM_FLAG_GRAY: H*W bytes gray)
+ *                                                           FM_FLAG_GRAY: H*W bytes gray; FM_FLAG_RGB: H*W*3 bytes RGB;
+ *                                                           FM_FLAG_ALPHA: H*W*4 bytes BGRA, or RGBA with FM_FLAG_RGB)
  * `frames` is a DEVICE pointer; work is enqueued on `cuda_stream` (a cudaStream_t, 0 = default)
  * and the call returns without synchronising.  stats_dev, if not NULL, is a device buffer of
  * n_streams * n_frames fm_frame_stats ([stream][frame]) filled by the call. */
@@ -187,7 +204,9 @@ int fm_process_ragged(fm_ctx *ctx, const uint8_t *frames, size_t stream_stride, 
  * FM_FLAG_DEVICE_CLIPS).  For stream s, with n_out[s] = sum of wrote + n_flush over its valid frames, it writes
  * n_out[s] raw BGR frames densely to the DEVICE buffer
  *   out_dev + s * out_stream_stride + i * H*W*3          (i < n_out[s]; FM_FLAG_NV12: NV12 frames, i * H*W*3/2;
- *                                                         FM_FLAG_GRAY: gray frames, i * H*W)
+ *                                                         FM_FLAG_GRAY: gray frames, i * H*W;
+ *                                                         FM_FLAG_RGB: the caller's RGB frames, i * H*W*3;
+ *                                                         FM_FLAG_ALPHA: the caller's four-byte frames, i * H*W*4)
  * in the reference's order: for each frame in order, the n_flush cached frames it flushes (oldest first, taken from the
  * device ring or from this call's input), then the frame itself if `wrote` (find_motion.py:561-570, 583).  n_out
  * follows from the stats.  out_capacity is the room per stream in frames and must be at least cache_frames + n_frames,
@@ -203,11 +222,11 @@ typedef struct fm_frames {
     const uint8_t *data;        /* DEVICE pointer: frame (s, t) starts at data + s * stream_stride + t * frame_stride */
     size_t stream_stride;
     size_t frame_stride;
-    size_t row_pitch;           /* bytes from one row to the next, in both NV12 planes; 0 = packed (W*3, or W for NV12
-                                   and gray) */
+    size_t row_pitch;           /* bytes from one row to the next, in both NV12 planes; 0 = packed (W*3 for BGR and RGB,
+                                   W*4 with FM_FLAG_ALPHA, W for NV12 and gray) */
     int64_t uv_offset;          /* FM_FLAG_NV12: start of the chroma plane relative to the frame start (may be negative);
                                    0 = row_pitch * H (chroma right after the luma rows).  Must be 0 otherwise with
-                                   FM_FLAG_GRAY (FM_EINVAL) */
+                                   FM_FLAG_GRAY, FM_FLAG_RGB or FM_FLAG_ALPHA (FM_EINVAL) */
 } fm_frames;
 
 /* fm_process_ragged (clip_out == NULL) or fm_process_clip (clip_out != NULL, same flag and capacity rules) on frames laid
@@ -228,7 +247,8 @@ int fm_process_frames(fm_ctx *ctx, const fm_frames *frames, int n_frames, const 
  * each byte-identical to cv2.resize(raw, (300, oh), interpolation=cv2.INTER_AREA) of the written frame (the upscale for
  * W < 300, a copy for W == 300).  The masks do not apply (find_objects reads frame.raw).  NV12 contexts resize
  * cv2.cvtColor(frame, COLOR_YUV2BGR_NV12), gray contexts cv2.cvtColor(frame, COLOR_GRAY2BGR) (the one-channel resize
- * in all three channels).  out_capacity is the room per stream in planes and must be at least the last
+ * in all three channels); RGB, BGRA and RGBA contexts give BGR planes, those of
+ * cv2.cvtColor(frame, COLOR_RGB2BGR / COLOR_BGRA2BGR / COLOR_RGBA2BGR).  out_capacity is the room per stream in planes and must be at least the last
  * call's n_frames.  Asynchronous on `cuda_stream`: the last call's frames must stay untouched until the planes are
  * written, as for the call itself.  FM_EINVAL without the flag, for a short out_capacity, before the first device-entry
  * call, and after fm_process_host / fm_submit_host (their frames live in the context's staging buffers). */
@@ -236,7 +256,8 @@ int fm_object_planes(fm_ctx *ctx, void *cuda_stream, uint8_t *out_dev, size_t ou
 
 /* Same with HOST buffers: copies the frames host->device (pinned memory recommended), runs the
  * path, copies the stats back and synchronises.  This is the call a drop-in adapter makes.  With FM_FLAG_NV12 a frame
- * is H*W*3/2 bytes, half the host->device traffic of BGR; with FM_FLAG_GRAY it is H*W bytes, a third. */
+ * is H*W*3/2 bytes, half the host->device traffic of BGR; with FM_FLAG_GRAY it is H*W bytes, a third; with FM_FLAG_RGB
+ * the H*W*3 bytes, with FM_FLAG_ALPHA the H*W*4 bytes, are copied as given. */
 int fm_process_host(fm_ctx *ctx, const uint8_t *frames_host, size_t stream_stride,
                     size_t frame_stride, int n_frames, fm_frame_stats *stats_host);
 
@@ -299,6 +320,13 @@ int fm_debug_rows_plan(int frame_width, int frame_height, int box_size, fm_rows_
 /* fm_debug_rows_plan for frames of `channels` bytes per pixel: 3 (BGR, what fm_debug_rows_plan checks) or 1 (FM_FLAG_GRAY,
  * whose plan reads W-byte rows and 4-byte tap groups).  FM_EINVAL for any other count. */
 int fm_debug_rows_plan_channels(int frame_width, int frame_height, int box_size, int channels, fm_rows_plan_info *info);
+
+/* fm_debug_rows_plan for the pixel format `flags` selects, as fm_ctx_create resolves it: 0 (BGR) and FM_FLAG_RGB (the same
+ * three-byte plan; the order only moves the gray weights), FM_FLAG_ALPHA and FM_FLAG_RGB | FM_FLAG_ALPHA (the four-byte
+ * plan: a tap group of 4 pixels is 4 aligned words, the fourth byte of each never enters a chain) or FM_FLAG_GRAY
+ * (fm_debug_rows_plan_channels(..., 1, ...)).  FM_EINVAL for two formats at once, and for any other flag, NV12 included
+ * (its rows plan reads the BGR slot). */
+int fm_debug_rows_plan_format(int frame_width, int frame_height, int box_size, int32_t flags, fm_rows_plan_info *info);
 
 /* Number of kernels this library has launched since load (bench.py's gpu_launches). */
 uint64_t fm_launch_count(void);
